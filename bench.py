@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W          # the CUDA path (this repo)
     python bench.py --impl reference --gpus N ...          # the reference algorithm on host CPUs
     python bench.py --envs-total E --gpus N ...            # strong scaling: E envs sharded over N GPUs
+    python bench.py ... --dump-outputs DIR                 # also write the last timed step's outputs to DIR/*.npy
 
 Workload (N=1): BASELINE.json configs[3], the configuration the headline target is quoted
 on: MultiOptLRs, 2-layer MLP 784->64->10 on synthetic MNIST-shaped data (60000 rows),
@@ -27,6 +28,10 @@ Reported on one JSON line:
   cpu_baseline  the oracle on the host cores, on a bounded sample of the same workload:
             "port" = vectorised numpy (SURVEY 8d path ii), "faithful" = per-env Python
             objects, thread per env over pipes (path i)
+
+--dump-outputs DIR writes what the last timed step returned on rank 0 (see dump_outputs). Data,
+permutations, initial weights and actions are all seeded, so two builds run with the same
+arguments get the same inputs and their files can be compared array for array.
 """
 import argparse
 import contextlib
@@ -232,6 +237,34 @@ def reference_arm(args):
 
 
 # -------------------------------------------------------------------------- GPU arm
+DUMP_OBS_ROWS = 1 << 18           # observation rows written by --dump-outputs: 262144 x 15 float32 = 15.7 MB
+
+
+def dump_outputs(out_dir, obs, reward, done, info):
+    """Write the outputs of one env.step() to out_dir/<name>.npy, every value finite: obs [rows, obs_dim]
+    float32, reward [E] float32, done [E] float32 (0 / 1), info [E, 16] float64 and info_nonfinite
+    [E, 16] float32.  info holds non-finite values by design, as the reference does: the loss column is
+    NaN (the reference's None) unless the episode ended, and sums of ratios that nan_to_num set to the
+    float maximum overflow to +inf.  Such entries are written as 0 in info.npy and marked in
+    info_nonfinite.npy (0 finite, 1 NaN, 2 +inf, 3 -inf).  At the bench shape the observation matrix
+    is 12.5 GB, so only a fixed sample of DUMP_OBS_ROWS of its rows is written:
+    np.random.default_rng(0).choice(rows, DUMP_OBS_ROWS, replace=False), sorted (every row when
+    there are no more than that)."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rows = obs.shape[0]
+    if rows > DUMP_OBS_ROWS:
+        pick = np.sort(np.random.default_rng(0).choice(rows, DUMP_OBS_ROWS, replace=False))
+        obs = obs.index_select(0, torch.as_tensor(pick, device=obs.device))
+    info = info.double().cpu().numpy()
+    nonfinite = np.select([np.isnan(info), np.isposinf(info), np.isneginf(info)], [1, 2, 3], 0).astype(np.float32)
+    arrays = {'obs': obs.float().cpu().numpy(), 'reward': reward.float().cpu().numpy(),
+              'done': done.float().cpu().numpy(), 'info': np.where(nonfinite == 0, info, 0.0),
+              'info_nonfinite': nonfinite}
+    for name, array in arrays.items():
+        np.save(os.path.join(out_dir, name + '.npy'), array)
+
+
 def sampled_parity(env, feats, labels, actions, max_batches=MAX_BATCHES, depth=HIST, spec=None):
     """One env step checked against the oracle for the sampled envs {0, 1, E/3, 2E/3, E-2, E-1}:
     the oracle (the checker, oracle/step_check.py) is seeded with the device's own state of those
@@ -361,6 +394,9 @@ def gpu_arm(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
     value = envs_all * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        # env.step() returns these buffers themselves: they hold the last timed step's outputs until the next step
+        dump_outputs(args.dump_outputs, env.obs, env.reward, env.done, env.info)
 
     # ---- parity: one more step, replayed by the oracle for six sampled envs from the device's own state
     parity = sampled_parity(env, feats, labels, actions[0]) if rank == 0 else None
@@ -543,7 +579,13 @@ def main():
     parser.add_argument('--skip-policy-loop', action='store_true', help='skip the device policy-in-the-loop figure')
     parser.add_argument('--skip-faithful', action='store_true', help='skip the ~25 s per-env-object CPU baseline')
     parser.add_argument('--cpu-steps', type=int, default=30, help='steps of the vectorised CPU baseline sample (~12 s at 30)')
+    parser.add_argument('--dump-outputs', metavar='DIR', default=None,
+                        help='write the outputs of the last timed step (rank 0) to DIR/<name>.npy')
     args = parser.parse_args()
+    if args.steps < 1:
+        parser.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'b200':
+        parser.error('--dump-outputs writes the outputs of the CUDA path (--impl b200)')
     if args.impl == 'reference':
         reference_arm(args)
         return
