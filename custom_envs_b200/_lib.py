@@ -28,7 +28,8 @@ EXPORTS = (
     'b2d_last_error', 'b2d_resize_nearest', 'b2d_minmax_workspace', 'b2d_column_minmax',
     'b2d_normalize', 'b2d_rank_workspace', 'b2d_label_ranks', 'b2d_onehot', 'b2d_shuffle_permutations',
     # shared per-agent policy (include/b200policy.h)
-    'b2p_create', 'b2p_destroy', 'b2p_last_error', 'b2p_set_weights', 'b2p_act', 'b2p_act_env', 'b2p_set_seed_counter')
+    'b2p_create', 'b2p_destroy', 'b2p_last_error', 'b2p_set_weights', 'b2p_act', 'b2p_act_env', 'b2p_set_seed_counter',
+    'b2p_set_value_weights', 'b2p_step', 'b2p_step_env', 'b2p_gae')
 DTYPE_U8, DTYPE_I32, DTYPE_F32, DTYPE_F64 = range(4)
 
 
@@ -39,6 +40,11 @@ class Config(ctypes.Structure):
         'history_version', 'observation_version', 'action_version', 'reward_version',
         'row_order', 'index_mode', 'auto_reset', 'reserved')] + [
         ('hidden_more', ctypes.c_int32 * MAX_LAYERS), ('init_seed', ctypes.c_uint64)]
+
+
+class StepOut(ctypes.Structure):
+    """b2p_step_out: device pointers of the outputs of one b2p_step / b2p_step_env launch (NULL = not computed)."""
+    _fields_ = [(name, ctypes.c_void_p) for name in ('actions', 'actions_raw', 'values', 'neglogp', 'obs_bf16')]
 
 
 class B200EnvError(RuntimeError):
@@ -104,6 +110,10 @@ def load():
     lib.b2p_set_seed_counter.argtypes = [vp, vp]
     lib.b2p_act.argtypes = [vp, vp, i64, vp, f32, u64, f32, f32, vp]
     lib.b2p_act_env.argtypes = [vp, vp, vp, f32, u64, f32, f32, vp]
+    lib.b2p_set_value_weights.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.b2p_step.argtypes = [vp, vp, i64, ctypes.POINTER(StepOut), f32, f32, u64, f32, f32, vp]
+    lib.b2p_step_env.argtypes = [vp, vp, ctypes.POINTER(StepOut), f32, f32, u64, f32, f32, vp]
+    lib.b2p_gae.argtypes = [vp, vp, vp, i32, i64, i64, ctypes.c_double, ctypes.c_double, vp, vp, vp]
     if lib.b2e_abi_version() != 2:
         raise B200EnvError('libb200env.so ABI version mismatch')
     _lib = lib

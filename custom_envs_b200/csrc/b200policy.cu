@@ -52,8 +52,13 @@ constexpr int OFF_B2 = OFF_B1 + B1_BYTES, B2_BYTES = (HID / 8) * SBO2;
 constexpr int OFF_W3 = OFF_B2 + B2_BYTES;
 constexpr int SMEM_BYTES = OFF_W3 + (HID + 4) * 4 + 128;   // + slack to align the base to 128 bytes
 constexpr int TMEM_COLS = GROUPS <= 4 ? 256 : 512;    // 64 columns per group: D2 overwrites D1, which is fully read before the second layer's MMAs are issued
-static_assert(G_BYTES % 128 == 0 && OFF_B1 % 128 == 0 && OFF_B2 % 128 == 0, "operand blocks are 128-byte aligned");
-static_assert(SMEM_BYTES <= 227 * 1024, "shared memory");
+// the step kernel (b2p_step*) adds the value tower's operands behind the action tower's; it runs the two towers
+// one after the other in the same TMEM columns and A2 buffer
+constexpr int OFF_VB1 = (OFF_W3 + (HID + 4) * 4 + 127) / 128 * 128, OFF_VB2 = OFF_VB1 + B1_BYTES, OFF_VW3 = OFF_VB2 + B2_BYTES;
+constexpr int SMEM_STEP_BYTES = OFF_VW3 + (HID + 4) * 4 + 128;
+static_assert(G_BYTES % 128 == 0 && OFF_B1 % 128 == 0 && OFF_B2 % 128 == 0 && OFF_VB1 % 128 == 0 && OFF_VB2 % 128 == 0,
+              "operand blocks are 128-byte aligned");
+static_assert(SMEM_BYTES <= 227 * 1024 && SMEM_STEP_BYTES <= 227 * 1024, "shared memory");
 
 struct Args {
     const float *w1, *b1, *w2, *b2, *w3, *b3;
@@ -65,6 +70,15 @@ struct Args {
     const unsigned long long *seed_counter;   // added to seed when set (b2p_set_seed_counter)
     float noise_std, low, high;
     int obs_dim, bulk_ok;
+};
+
+// the rest of stable-baselines' model.step / model.value (b2p_step*): a NULL output is not computed
+struct StepArgs {
+    const float *w1, *b1, *w2, *b2, *w3, *b3;      // value tower (vf), NULL without values
+    float *raw, *values, *neglogp;                  // [rows]; Args::out holds the clipped actions
+    uint4 *obs16;                                   // [rows][16] bf16 = 2 x uint4 per row
+    float nlp_const;                                // 0.5 log(2 pi) + log_std
+    int want_pi;                                    // any action output requested
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -143,8 +157,11 @@ __device__ __forceinline__ float row_noise(unsigned long long seed, long long ro
 
 // FRONT: 0 = dense observation rows, 1 = rings with max_history 5 (every index a compile-time constant),
 // 2 = rings with any max_history <= 5
-template <int FRONT, int TANH>
-__global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constant__ Args a, const __grid_constant__ Dev d) {
+// STEP: the b2p_step* variant (value tower, raw actions, neglogp, observation store; StepArgs); the b2p_act* instantiations
+// ignore `s`
+template <int FRONT, int TANH, bool STEP = false>
+__global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constant__ Args a, const __grid_constant__ Dev d,
+                                                            const __grid_constant__ StepArgs s) {
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t obs_full[GROUPS][2];
     __shared__ __align__(8) uint64_t mma_bar[GROUPS];
@@ -180,6 +197,23 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
     }
     if (tid < HID) w3s[tid] = a.w3[tid];
     if (tid == HID) w3s[HID] = a.b3[0];
+    if constexpr (STEP) {
+        if (s.values) {
+            for (int i = tid; i < HID * K1; i += THREADS) {
+                const int n = i / K1, k = i - n * K1;
+                const float v = k < od ? s.w1[n * od + k] : (k == K1 - 1 ? s.b1[n] : 0.f);
+                *reinterpret_cast<unsigned short *>(sm + OFF_VB1 + (n >> 3) * SBO1 + (k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2) = bf16_bits(v);
+            }
+            for (int i = tid; i < HID * K2; i += THREADS) {
+                const int n = i / K2, k = i - n * K2;
+                const float v = k < HID ? s.w2[n * HID + k] : (k == HID ? s.b2[n] : 0.f);
+                *reinterpret_cast<unsigned short *>(sm + OFF_VB2 + (n >> 3) * SBO2 + (k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2) = bf16_bits(v);
+            }
+            float *const vw3s = reinterpret_cast<float *>(sm + OFF_VW3);
+            if (tid < HID) vw3s[tid] = s.w3[tid];
+            if (tid == HID) vw3s[HID] = s.b3[0];
+        }
+    }
     {   // constant columns of this thread's A2 row: k = 64 is the bias 1, k = 65..79 are zero
         unsigned char *row = A2 + (gt >> 3) * SBO2 + (gt & 7) * 16;
         *reinterpret_cast<uint4 *>(row + 8 * 128) = make_uint4(0x00003F80u, 0u, 0u, 0u);
@@ -194,6 +228,12 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
     const uint64_t a1d = make_desc(sbase + g * G_BYTES + NSTG * STAGE_BYTES, 128, SBO1);
     const uint64_t a2d = make_desc(sbase + g * G_BYTES + NSTG * STAGE_BYTES + A1_BYTES, 128, SBO2);
     const uint64_t b1d = make_desc(sbase + OFF_B1, 128, SBO1), b2d = make_desc(sbase + OFF_B2, 128, SBO2);
+    // the value tower's B descriptors: the action tower's moved by the offset of its operands (start address field,
+    // 16-byte units; formed where used, so that they hold no registers across the tile loop)
+    constexpr uint64_t VDESC_SHIFT = (uint64_t)((OFF_VB1 - OFF_B1) >> 4);
+    static_assert(OFF_VB2 - OFF_B2 == OFF_VB1 - OFF_B1, "both value-tower operands sit at the same offset");
+    auto want_pi = [&]() -> bool { return !STEP || s.want_pi; };     // read from the parameter space, never held in a register
+    auto want_v = [&]() -> bool { return STEP && s.values; };
     const uint32_t tm1 = tmem + 64 * g, tm2 = tm1;
     const uint32_t tlane = (uint32_t)(wq * 32) << 16;
     const float b3 = w3s[HID];
@@ -323,20 +363,39 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
 #pragma unroll
             for (int k = 0; k < XMAX; ++k) x[k] = (live && k < od) ? st[k] : 0.f;
         }
+        // ---- row of the output vectors (the next b2e_step gathers the action through the same row table)
+        auto out_row = [&](bool &live) -> long long {
+            if (RING) {
+                const int p = cur_tp * TILE + gt;
+                live = p < d.P;
+                return (long long)cur_e * d.P + (live ? (d.row_lex ? d.row_of_param[p] : p) : 0);
+            }
+            live = tile * TILE + gt < a.rows;
+            return tile * TILE + gt;
+        };
         // ---- A1 = [x | 0 | 1] as bf16, this thread's row
         {
             unsigned char *row = A1 + (gt >> 3) * SBO1 + (gt & 7) * 16;
-            *reinterpret_cast<uint4 *>(row) = make_uint4(pack_bf16x2(x[0], x[1]), pack_bf16x2(x[2], x[3]),
-                                                         pack_bf16x2(x[4], x[5]), pack_bf16x2(x[6], x[7]));
+            const uint4 lo = make_uint4(pack_bf16x2(x[0], x[1]), pack_bf16x2(x[2], x[3]), pack_bf16x2(x[4], x[5]), pack_bf16x2(x[6], x[7]));
+            *reinterpret_cast<uint4 *>(row) = lo;
             *reinterpret_cast<uint4 *>(row + 128) = make_uint4(pack_bf16x2(x[8], x[9]), pack_bf16x2(x[10], x[11]),
                                                                pack_bf16x2(x[12], x[13]), pack_bf16x2(x[14], 1.0f));
+            if constexpr (STEP) {           // the observation store: the row as the MMA reads it, bias column -> 0
+                bool live;
+                const long long orow = s.obs16 ? out_row(live) : 0;
+                if (s.obs16 && live) {
+                    s.obs16[2 * orow] = lo;
+                    s.obs16[2 * orow + 1] = make_uint4(pack_bf16x2(x[8], x[9]), pack_bf16x2(x[10], x[11]),
+                                                       pack_bf16x2(x[12], x[13]), pack_bf16x2(x[14], 0.f));
+                }
+            }
         }
         fence_async();
         tc_fence_before();
         group_bar(g);
-        if (gt == 0) {
+        if (gt == 0 && (want_pi() || want_v())) {
             tc_fence_after();
-            mma_bf16(tm1, a1d, b1d, idesc, 0u);
+            mma_bf16(tm1, a1d, want_pi() ? b1d : b1d + VDESC_SHIFT, idesc, 0u);
             mma_commit(&mma_bar[g]);
         }
         if (!RING && NSTG == 1 && c.valid) fetch_dense(c.tile, 0);      // the single staging buffer is free again (barrier above)
@@ -345,84 +404,156 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
         const int next_e = c.e, next_tp = c.tp;
         if (RING && have_next) load_ring(c, nxt);             // in flight under this tile's work
         if (have_next) advance(c);
-        mbar_wait(&mma_bar[g], mph);
-        mph ^= 1u;
-        tc_fence_after();
-        // ---- A2 = tanh(D1) as bf16, 16 accumulator columns at a time (register budget of 768 threads)
-#pragma unroll
-        for (int qt = 0; qt < 4; ++qt) {
-            uint32_t v[16];
-            B2P_LD16(tm1 + tlane + 16 * qt, v);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            unsigned char *row = A2 + (gt >> 3) * SBO2 + (gt & 7) * 16 + (2 * qt) * 128;
-#pragma unroll
-            for (int c = 0; c < 2; ++c) {
-                uint32_t pk[4];
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const float v0 = __uint_as_float(v[8 * c + 2 * i]), v1 = __uint_as_float(v[8 * c + 2 * i + 1]);
-                    pk[i] = TANH >= 1 ? tanh_bf16x2(pack_bf16x2(v0, v1)) : pack_bf16x2(tanh_f32(v0), tanh_f32(v1));
-                }
-                *reinterpret_cast<uint4 *>(row + c * 128) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-            }
-        }
-        fence_async();
-        tc_fence_before();
-        group_bar(g);
-        if (gt == 0) {
+        // ---- the rest of a tower whose first-layer MMA has been issued: -> w3 . tanh(D2) + b3 of this thread's row
+        auto finish_tower = [&](uint64_t b2desc, const float *w3p, float bias) -> float {
+            mbar_wait(&mma_bar[g], mph);
+            mph ^= 1u;
             tc_fence_after();
+            // ---- A2 = tanh(D1) as bf16, 16 accumulator columns at a time (register budget of 768 threads)
 #pragma unroll
-            for (int kk = 0; kk < K2 / 16; ++kk)              // 16 K elements = two core matrices = 256 bytes per MMA
-                mma_bf16(tm2, a2d + (uint64_t)(kk * 16), b2d + (uint64_t)(kk * 16), idesc, kk ? 1u : 0u);
-            mma_commit(&mma_bar[g]);
-        }
-        mbar_wait(&mma_bar[g], mph);
-        mph ^= 1u;
-        tc_fence_after();
-        // ---- head: mean = tanh(D2) . w3 + b3
-        float acc0 = b3, acc1 = 0.f;
+            for (int qt = 0; qt < 4; ++qt) {
+                uint32_t v[16];
+                B2P_LD16(tm1 + tlane + 16 * qt, v);
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                unsigned char *row = A2 + (gt >> 3) * SBO2 + (gt & 7) * 16 + (2 * qt) * 128;
 #pragma unroll
-        for (int qt = 0; qt < 4; ++qt) {
-            uint32_t v[16];
-            B2P_LD16(tm2 + tlane + 16 * qt, v);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                for (int c = 0; c < 2; ++c) {
+                    uint32_t pk[4];
 #pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                const float4 w = *reinterpret_cast<const float4 *>(w3s + 16 * qt + 4 * c);
-                float t0, t1, t2, t3;
-                if (TANH == 2) {
-                    const uint32_t p0 = tanh_bf16x2(pack_bf16x2(__uint_as_float(v[4 * c]), __uint_as_float(v[4 * c + 1])));
-                    const uint32_t p1 = tanh_bf16x2(pack_bf16x2(__uint_as_float(v[4 * c + 2]), __uint_as_float(v[4 * c + 3])));
-                    t0 = __uint_as_float(p0 << 16); t1 = __uint_as_float(p0 & 0xFFFF0000u);
-                    t2 = __uint_as_float(p1 << 16); t3 = __uint_as_float(p1 & 0xFFFF0000u);
-                } else {
-                    t0 = tanh_f32(__uint_as_float(v[4 * c])); t1 = tanh_f32(__uint_as_float(v[4 * c + 1]));
-                    t2 = tanh_f32(__uint_as_float(v[4 * c + 2])); t3 = tanh_f32(__uint_as_float(v[4 * c + 3]));
+                    for (int i = 0; i < 4; ++i) {
+                        const float v0 = __uint_as_float(v[8 * c + 2 * i]), v1 = __uint_as_float(v[8 * c + 2 * i + 1]);
+                        pk[i] = TANH >= 1 ? tanh_bf16x2(pack_bf16x2(v0, v1)) : pack_bf16x2(tanh_f32(v0), tanh_f32(v1));
+                    }
+                    *reinterpret_cast<uint4 *>(row + c * 128) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
                 }
-                acc0 = fmaf(t0, w.x, acc0); acc1 = fmaf(t1, w.y, acc1);
-                acc0 = fmaf(t2, w.z, acc0); acc1 = fmaf(t3, w.w, acc1);
+            }
+            fence_async();
+            tc_fence_before();
+            group_bar(g);
+            if (gt == 0) {
+                tc_fence_after();
+#pragma unroll
+                for (int kk = 0; kk < K2 / 16; ++kk)              // 16 K elements = two core matrices = 256 bytes per MMA
+                    mma_bf16(tm2, a2d + (uint64_t)(kk * 16), b2desc + (uint64_t)(kk * 16), idesc, kk ? 1u : 0u);
+                mma_commit(&mma_bar[g]);
+            }
+            mbar_wait(&mma_bar[g], mph);
+            mph ^= 1u;
+            tc_fence_after();
+            // ---- head: tanh(D2) . w3 + b3
+            float acc0 = bias, acc1 = 0.f;
+#pragma unroll
+            for (int qt = 0; qt < 4; ++qt) {
+                uint32_t v[16];
+                B2P_LD16(tm2 + tlane + 16 * qt, v);
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+                for (int c = 0; c < 4; ++c) {
+                    const float4 w = *reinterpret_cast<const float4 *>(w3p + 16 * qt + 4 * c);
+                    float t0, t1, t2, t3;
+                    if (TANH == 2) {
+                        const uint32_t p0 = tanh_bf16x2(pack_bf16x2(__uint_as_float(v[4 * c]), __uint_as_float(v[4 * c + 1])));
+                        const uint32_t p1 = tanh_bf16x2(pack_bf16x2(__uint_as_float(v[4 * c + 2]), __uint_as_float(v[4 * c + 3])));
+                        t0 = __uint_as_float(p0 << 16); t1 = __uint_as_float(p0 & 0xFFFF0000u);
+                        t2 = __uint_as_float(p1 << 16); t3 = __uint_as_float(p1 & 0xFFFF0000u);
+                    } else {
+                        t0 = tanh_f32(__uint_as_float(v[4 * c])); t1 = tanh_f32(__uint_as_float(v[4 * c + 1]));
+                        t2 = tanh_f32(__uint_as_float(v[4 * c + 2])); t3 = tanh_f32(__uint_as_float(v[4 * c + 3]));
+                    }
+                    acc0 = fmaf(t0, w.x, acc0); acc1 = fmaf(t1, w.y, acc1);
+                    acc0 = fmaf(t2, w.z, acc0); acc1 = fmaf(t3, w.w, acc1);
+                }
+            }
+            tc_fence_before();
+            return acc0 + acc1;
+        };
+        if constexpr (!STEP) {
+            float mean = finish_tower(b2d, w3s, b3);
+            bool live;
+            const long long orow = out_row(live);
+            if (a.noise_std != 0.f) mean = fmaf(a.noise_std, row_noise(seed, orow), mean);
+            if (live) a.out[orow] = fminf(fmaxf(mean, a.low), a.high);
+        } else {
+            // the action outputs are stored before the value tower runs, so that nothing of them stays live across it
+            if (want_pi()) {
+                const float mean = finish_tower(b2d, w3s, w3s[HID]);
+                bool live;
+                const long long orow = out_row(live);
+                float z = 0.f, raw = mean;
+                if (a.noise_std != 0.f) { z = row_noise(seed, orow); raw = fmaf(a.noise_std, z, mean); }
+                if (live) {
+                    if (a.out) a.out[orow] = fminf(fmaxf(raw, a.low), a.high);
+                    if (s.raw) s.raw[orow] = raw;
+                    if (s.neglogp) s.neglogp[orow] = fmaf(0.5f * z, z, s.nlp_const);
+                }
+            }
+            if (want_v()) {
+                if (want_pi()) {          // the value tower reuses D1/D2 (read out above) and A2 (the last MMA has completed)
+                    group_bar(g);
+                    if (gt == 0) {
+                        tc_fence_after();
+                        mma_bf16(tm1, a1d, b1d + VDESC_SHIFT, idesc, 0u);
+                        mma_commit(&mma_bar[g]);
+                    }
+                }
+                const float *vw3s = reinterpret_cast<const float *>(sm + OFF_VW3);
+                const float value = finish_tower(b2d + VDESC_SHIFT, vw3s, vw3s[HID]);
+                bool live;
+                const long long orow = out_row(live);
+                if (live) s.values[orow] = value;
             }
         }
-        tc_fence_before();
-        float mean = acc0 + acc1;
-        // ---- action of the row (the next b2e_step gathers it through the same row table)
-        long long orow;
-        bool live;
-        if (RING) {
-            const int p = cur_tp * TILE + gt;
-            live = p < d.P;
-            orow = (long long)cur_e * d.P + (live ? (d.row_lex ? d.row_of_param[p] : p) : 0);
-        } else {
-            orow = tile * TILE + gt;
-            live = orow < a.rows;
-        }
-        if (a.noise_std != 0.f) mean = fmaf(a.noise_std, row_noise(seed, orow), mean);
-        if (live) a.out[orow] = fminf(fmaxf(mean, a.low), a.high);
         have = have_next; tile = next_tile; cur_e = next_e; cur_tp = next_tp;
     }
     tc_fence_before();
     __syncthreads();
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS));
+}
+
+// GAE of stable-baselines 2's PPO2 Runner (ppo2.py) over a time-major rollout, one thread per agent row, T sequential:
+//   nn = 1 - dones[t+1];  delta = r[t] + gamma * values[t+1] * nn - values[t];  adv[t] = last = delta + gamma * lam * nn * last
+//   ret[t] = adv[t] + values[t]
+// in the Runner's dtypes: gamma * values[t+1] is a float32 product (a Python float times a float32 array), the rest of
+// delta and the recursion are float64 (1.0 - a bool array is float64), adv is stored as float32 and ret = adv + value is
+// a float32 sum.  Explicit _rn intrinsics: no FMA contraction the numpy code does not have.  The values of U steps are
+// loaded ahead of their recursion; rewards and dones are per env (env = row / P) and shared by its rows through the cache.
+constexpr int GAE_THREADS = 256, GAE_U = 8;
+__global__ void __launch_bounds__(GAE_THREADS) gae_kernel(const float *__restrict__ values, const float *__restrict__ rewards,
+                                                          const uint8_t *__restrict__ dones, int T, long long rows, long long P,
+                                                          double gamma, double lam, float *__restrict__ adv, float *__restrict__ ret) {
+    const long long row = (long long)blockIdx.x * GAE_THREADS + threadIdx.x;
+    if (row >= rows) return;
+    const long long E = rows / P, e = row / P;
+    const double gl = __dmul_rn(gamma, lam);
+    const float g32 = (float)gamma;
+    double last = 0.0;
+    float nv = __ldcs(values + (size_t)T * rows + row);
+    for (int t0 = T - 1; t0 >= 0; t0 -= GAE_U) {
+        float v[GAE_U], r[GAE_U];
+        uint8_t dn[GAE_U];
+#pragma unroll
+        for (int i = 0; i < GAE_U; ++i) {
+            const int t = t0 - i;
+            if (t >= 0) {
+                v[i] = __ldcs(values + (size_t)t * rows + row);
+                r[i] = __ldg(rewards + (size_t)t * E + e);
+                dn[i] = __ldg(dones + (size_t)(t + 1) * E + e);
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < GAE_U; ++i) {
+            const int t = t0 - i;
+            if (t >= 0) {
+                const double nn = dn[i] ? 0.0 : 1.0;
+                const double delta = __dadd_rn(__dadd_rn((double)r[i], __dmul_rn((double)__fmul_rn(g32, nv), nn)), -(double)v[i]);
+                last = __dadd_rn(delta, __dmul_rn(__dmul_rn(gl, nn), last));
+                const float a32 = (float)last;
+                __stcs(adv + (size_t)t * rows + row, a32);
+                __stcs(ret + (size_t)t * rows + row, __fadd_rn(a32, v[i]));
+                nv = v[i];
+            }
+        }
+    }
 }
 
 }  // namespace pol
@@ -431,9 +562,9 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
 // ---------------------------------------------------------------- host side (C ABI)
 struct b2p_policy {
     int device, obs_dim, tanh_mode, num_sms;
-    float *weights;                  // w1 [64, obs_dim] | b1 | w2 [64, 64] | b2 | w3 | b3
+    float *weights;                  // w1 [64, obs_dim] | b1 | w2 [64, 64] | b2 | w3 | b3, then the value tower in the same layout
     const unsigned long long *seed_counter;
-    bool have_weights;
+    bool have_weights, have_value_weights;
     std::string error;
 };
 
@@ -455,21 +586,24 @@ struct PolicyDeviceGuard {
     ~PolicyDeviceGuard() { if (switched) cudaSetDevice(prev); }
 };
 
-template <int FRONT>
-cudaError_t launch_policy(int tanh_mode, int grid, cudaStream_t cs, const pol::Args &a, const Dev &d) {
+template <int FRONT, bool STEP = false>
+cudaError_t launch_policy(int tanh_mode, int grid, cudaStream_t cs, const pol::Args &a, const Dev &d,
+                          const pol::StepArgs &s = pol::StepArgs()) {
+    constexpr int smem = STEP ? pol::SMEM_STEP_BYTES : pol::SMEM_BYTES;
     switch (tanh_mode) {
-        case 2: pol::policy_kernel<FRONT, 2><<<grid, pol::THREADS, pol::SMEM_BYTES, cs>>>(a, d); break;
-        case 1: pol::policy_kernel<FRONT, 1><<<grid, pol::THREADS, pol::SMEM_BYTES, cs>>>(a, d); break;
-        default: pol::policy_kernel<FRONT, 0><<<grid, pol::THREADS, pol::SMEM_BYTES, cs>>>(a, d); break;
+        case 2: pol::policy_kernel<FRONT, 2, STEP><<<grid, pol::THREADS, smem, cs>>>(a, d, s); break;
+        case 1: pol::policy_kernel<FRONT, 1, STEP><<<grid, pol::THREADS, smem, cs>>>(a, d, s); break;
+        default: pol::policy_kernel<FRONT, 0, STEP><<<grid, pol::THREADS, smem, cs>>>(a, d, s); break;
     }
     return cudaGetLastError();
 }
 
-template <int FRONT>
+template <int FRONT, bool STEP>
 bool set_policy_smem() {
-    return cudaFuncSetAttribute(pol::policy_kernel<FRONT, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::SMEM_BYTES) == cudaSuccess &&
-           cudaFuncSetAttribute(pol::policy_kernel<FRONT, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::SMEM_BYTES) == cudaSuccess &&
-           cudaFuncSetAttribute(pol::policy_kernel<FRONT, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::SMEM_BYTES) == cudaSuccess;
+    constexpr int smem = STEP ? pol::SMEM_STEP_BYTES : pol::SMEM_BYTES;
+    return cudaFuncSetAttribute(pol::policy_kernel<FRONT, 0, STEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess &&
+           cudaFuncSetAttribute(pol::policy_kernel<FRONT, 1, STEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess &&
+           cudaFuncSetAttribute(pol::policy_kernel<FRONT, 2, STEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess;
 }
 
 void fill_weights(const b2p_policy *h, pol::Args &a) {
@@ -478,6 +612,71 @@ void fill_weights(const b2p_policy *h, pol::Args &a) {
     a.w1 = w; a.b1 = a.w1 + hid * od; a.w2 = a.b1 + hid; a.b2 = a.w2 + hid * hid; a.w3 = a.b2 + hid; a.b3 = a.w3 + hid;
     a.obs_dim = od;
 }
+
+size_t tower_floats(int obs_dim) {
+    return (size_t)pol::HID * obs_dim + pol::HID + pol::HID * pol::HID + pol::HID + pol::HID + 1;
+}
+
+int copy_tower(b2p_handle h, float *w, const float *const (&src)[6], cudaStream_t cs, const char *who) {
+    const int od = h->obs_dim, hid = pol::HID;
+    const size_t cnt[6] = {(size_t)hid * od, (size_t)hid, (size_t)hid * hid, (size_t)hid, (size_t)hid, 1};
+    for (int i = 0; i < 6; ++i) {
+        if (!src[i]) return pfail(h, std::string(who) + ": null pointer");
+        if (cudaMemcpyAsync(w, src[i], cnt[i] * sizeof(float), cudaMemcpyDeviceToDevice, cs) != cudaSuccess)
+            return pfail(h, std::string(who) + ": " + cudaGetErrorString(cudaGetLastError()));
+        w += cnt[i];
+    }
+    return 0;
+}
+
+// the ring front end's split of the env's tiles over the CTAs (b2p_act_env, b2p_step_env); NULL + error on a bad env
+const Dev *ring_setup(b2p_handle h, b2e_handle env, pol::Args &a, int &grid, const char *who) {
+    int ring_ok = 0, device = -1;
+    const Dev *dv = static_cast<const Dev *>(b2e_dev_view(env, &ring_ok, &device));
+    const std::string w(who);
+    if (!dv || !ring_ok) { pfail(h, w + ": the env has no MultiOptLRs adjusted-history rings (large-problem pipeline only)"); return nullptr; }
+    if (device != h->device) { pfail(h, w + ": policy and env live on different devices"); return nullptr; }
+    if (3 * dv->H != h->obs_dim) { pfail(h, w + ": obs_dim of the policy is not 3 x max_history of the env"); return nullptr; }
+    a.rows = (long long)dv->E * dv->P;
+    const int tiles_per_env = (dv->P + pol::TILE - 1) / pol::TILE;
+    a.tiles = (long long)dv->E * tiles_per_env;
+    // few envs: split every env's tiles into segments so that all SMs have work (>= 4 rounds of tiles per group and segment)
+    int segs = (3 * h->num_sms + dv->E - 1) / dv->E;
+    const int max_segs = tiles_per_env / (4 * pol::GROUPS);
+    segs = segs > max_segs ? max_segs : segs;
+    a.segs = segs < 1 ? 1 : segs;
+    a.units = dv->E * a.segs;
+    grid = a.units < h->num_sms ? a.units : h->num_sms;
+    return dv;
+}
+
+// Args / StepArgs of a b2p_step* launch; non-zero (error set) on a request the handle cannot serve
+int step_setup(b2p_handle h, const b2p_step_out *out, float noise_std, float log_std, uint64_t seed, float low, float high,
+               pol::Args &a, pol::StepArgs &s, const char *who) {
+    const std::string w(who);
+    if (!out) return pfail(h, w + ": null output set");
+    if (!out->actions && !out->actions_raw && !out->values && !out->neglogp && !out->obs_bf16)
+        return pfail(h, w + ": every output is NULL");
+    const bool want_pi = out->actions || out->actions_raw || out->neglogp;
+    if (want_pi && !h->have_weights) return pfail(h, w + ": b2p_set_weights has not been called");
+    if (out->values && !h->have_value_weights) return pfail(h, w + ": values requested but b2p_set_value_weights has not been called");
+    if (reinterpret_cast<uintptr_t>(out->obs_bf16) & 15u) return pfail(h, w + ": obs_bf16 must be 16-byte aligned");
+    memset(&a, 0, sizeof(a));
+    memset(&s, 0, sizeof(s));
+    fill_weights(h, a);
+    const float *v = h->weights + tower_floats(h->obs_dim);
+    const int od = h->obs_dim, hid = pol::HID;
+    s.w1 = v; s.b1 = s.w1 + hid * od; s.w2 = s.b1 + hid; s.b2 = s.w2 + hid * hid; s.w3 = s.b2 + hid; s.b3 = s.w3 + hid;
+    a.out = out->actions;
+    s.raw = out->actions_raw; s.values = out->values; s.neglogp = out->neglogp;
+    s.obs16 = static_cast<uint4 *>(out->obs_bf16);
+    s.nlp_const = (float)(0.91893853320467274178 + (double)log_std);      // 0.5 log(2 pi) + log_std
+    s.want_pi = want_pi ? 1 : 0;
+    a.seed_counter = h->seed_counter;
+    a.seed = seed; a.noise_std = noise_std; a.low = low; a.high = high;
+    return 0;
+}
+
 
 }  // namespace
 
@@ -494,15 +693,15 @@ int b2p_create(int device, int obs_dim, int tanh_mode, b2p_handle *out) {
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return pfail(nullptr, "b2p_create: no such CUDA device");
     if (prop.major != 10) return pfail(nullptr, "b2p_create: the policy kernel needs an sm_100 GPU (tcgen05); there is no fallback");
-    if (!(set_policy_smem<0>() && set_policy_smem<1>() && set_policy_smem<2>()))
+    if (!(set_policy_smem<0, false>() && set_policy_smem<1, false>() && set_policy_smem<2, false>() &&
+          set_policy_smem<0, true>() && set_policy_smem<1, true>() && set_policy_smem<2, true>()))
         return pfail(nullptr, "b2p_create: the policy kernel does not fit shared memory");
     b2p_policy *h = new (std::nothrow) b2p_policy();
     if (!h) return pfail(nullptr, "b2p_create: out of host memory");
     h->device = device; h->obs_dim = obs_dim; h->tanh_mode = tanh_mode; h->num_sms = prop.multiProcessorCount;
-    h->have_weights = false;
+    h->have_weights = h->have_value_weights = false;
     h->seed_counter = nullptr;
-    const size_t count = (size_t)pol::HID * obs_dim + pol::HID + pol::HID * pol::HID + pol::HID + pol::HID + 1;
-    if (cudaMalloc((void **)&h->weights, count * sizeof(float)) != cudaSuccess) {
+    if (cudaMalloc((void **)&h->weights, 2 * tower_floats(obs_dim) * sizeof(float)) != cudaSuccess) {
         delete h;
         return pfail(nullptr, "b2p_create: cudaMalloc failed");
     }
@@ -528,17 +727,19 @@ int b2p_set_weights(b2p_handle h, const float *w1, const float *b1, const float 
     if (!h) return 1;
     if (!w1 || !b1 || !w2 || !b2 || !w3 || !b3) return pfail(h, "b2p_set_weights: null pointer");
     PolicyDeviceGuard guard(h->device);
-    const cudaStream_t cs = (cudaStream_t)stream;
-    const int od = h->obs_dim, hid = pol::HID;
-    float *w = h->weights;
-    const float *src[6] = {w1, b1, w2, b2, w3, b3};
-    const size_t cnt[6] = {(size_t)hid * od, (size_t)hid, (size_t)hid * hid, (size_t)hid, (size_t)hid, 1};
-    for (int i = 0; i < 6; ++i) {
-        if (cudaMemcpyAsync(w, src[i], cnt[i] * sizeof(float), cudaMemcpyDeviceToDevice, cs) != cudaSuccess)
-            return pfail(h, std::string("b2p_set_weights: ") + cudaGetErrorString(cudaGetLastError()));
-        w += cnt[i];
-    }
+    const float *const src[6] = {w1, b1, w2, b2, w3, b3};
+    if (copy_tower(h, h->weights, src, (cudaStream_t)stream, "b2p_set_weights")) return 1;
     h->have_weights = true;
+    return 0;
+}
+
+int b2p_set_value_weights(b2p_handle h, const float *w1, const float *b1, const float *w2, const float *b2,
+                          const float *w3, const float *b3, void *stream) {
+    if (!h) return 1;
+    PolicyDeviceGuard guard(h->device);
+    const float *const src[6] = {w1, b1, w2, b2, w3, b3};
+    if (copy_tower(h, h->weights + tower_floats(h->obs_dim), src, (cudaStream_t)stream, "b2p_set_value_weights")) return 1;
+    h->have_value_weights = true;
     return 0;
 }
 
@@ -570,31 +771,74 @@ int b2p_act_env(b2p_handle h, b2e_handle env, float *actions_out, float noise_st
     if (!h) return 1;
     if (!env || !actions_out) return pfail(h, "b2p_act_env: null pointer");
     if (!h->have_weights) return pfail(h, "b2p_act_env: b2p_set_weights has not been called");
-    int ring_ok = 0, device = -1;
-    const Dev *dv = static_cast<const Dev *>(b2e_dev_view(env, &ring_ok, &device));
-    if (!dv || !ring_ok) return pfail(h, "b2p_act_env: the env has no MultiOptLRs adjusted-history rings (large-problem pipeline only)");
-    if (device != h->device) return pfail(h, "b2p_act_env: policy and env live on different devices");
-    if (3 * dv->H != h->obs_dim) return pfail(h, "b2p_act_env: obs_dim of the policy is not 3 x max_history of the env");
-    PolicyDeviceGuard guard(h->device);
     pol::Args a;
     memset(&a, 0, sizeof(a));
+    int grid = 0;
+    const Dev *dv = ring_setup(h, env, a, grid, "b2p_act_env");
+    if (!dv) return 1;
+    PolicyDeviceGuard guard(h->device);
     fill_weights(h, a);
     a.out = actions_out;
-    a.rows = (long long)dv->E * dv->P;
-    const int tiles_per_env = (dv->P + pol::TILE - 1) / pol::TILE;
-    a.tiles = (long long)dv->E * tiles_per_env;
-    // few envs: split every env's tiles into segments so that all SMs have work (>= 4 rounds of tiles per group and segment)
-    int segs = (3 * h->num_sms + dv->E - 1) / dv->E;
-    const int max_segs = tiles_per_env / (4 * pol::GROUPS);
-    segs = segs > max_segs ? max_segs : segs;
-    a.segs = segs < 1 ? 1 : segs;
-    a.units = dv->E * a.segs;
     a.seed_counter = h->seed_counter;
     a.seed = seed; a.noise_std = noise_std; a.low = low; a.high = high;
-    const int grid = a.units < h->num_sms ? a.units : h->num_sms;
     const cudaError_t err = dv->H == 5 ? launch_policy<1>(h->tanh_mode, grid, (cudaStream_t)stream, a, *dv)
                                       : launch_policy<2>(h->tanh_mode, grid, (cudaStream_t)stream, a, *dv);
     if (err != cudaSuccess) return pfail(h, std::string("b2p_act_env: ") + cudaGetErrorString(err));
+    return 0;
+}
+
+int b2p_step(b2p_handle h, const float *obs, int64_t rows, const b2p_step_out *out, float noise_std, float log_std,
+             uint64_t seed, float low, float high, void *stream) {
+    if (!h) return 1;
+    if (!obs || rows < 0) return pfail(h, "b2p_step: bad argument");
+    pol::Args a;
+    pol::StepArgs s;
+    if (step_setup(h, out, noise_std, log_std, seed, low, high, a, s, "b2p_step")) return 1;
+    if (rows == 0) return 0;
+    PolicyDeviceGuard guard(h->device);
+    a.obs = obs; a.rows = rows; a.tiles = (rows + pol::TILE - 1) / pol::TILE;
+    a.bulk_ok = (reinterpret_cast<uintptr_t>(obs) & 15u) == 0 ? 1 : 0;
+    Dev d;
+    memset(&d, 0, sizeof(d));
+    const long long want = (a.tiles + pol::GROUPS - 1) / pol::GROUPS;
+    const int grid = (int)(want < h->num_sms ? want : h->num_sms);
+    const cudaError_t err = launch_policy<0, true>(h->tanh_mode, grid, (cudaStream_t)stream, a, d, s);
+    if (err != cudaSuccess) return pfail(h, std::string("b2p_step: ") + cudaGetErrorString(err));
+    return 0;
+}
+
+int b2p_step_env(b2p_handle h, b2e_handle env, const b2p_step_out *out, float noise_std, float log_std, uint64_t seed,
+                 float low, float high, void *stream) {
+    if (!h) return 1;
+    if (!env) return pfail(h, "b2p_step_env: null pointer");
+    pol::Args a;
+    pol::StepArgs s;
+    if (step_setup(h, out, noise_std, log_std, seed, low, high, a, s, "b2p_step_env")) return 1;
+    int grid = 0;
+    const Dev *dv = ring_setup(h, env, a, grid, "b2p_step_env");
+    if (!dv) return 1;
+    PolicyDeviceGuard guard(h->device);
+    const cudaError_t err = dv->H == 5 ? launch_policy<1, true>(h->tanh_mode, grid, (cudaStream_t)stream, a, *dv, s)
+                                      : launch_policy<2, true>(h->tanh_mode, grid, (cudaStream_t)stream, a, *dv, s);
+    if (err != cudaSuccess) return pfail(h, std::string("b2p_step_env: ") + cudaGetErrorString(err));
+    return 0;
+}
+
+int b2p_gae(const float *values, const float *rewards, const uint8_t *dones, int T, int64_t rows, int64_t P, double gamma,
+            double lam, float *adv_out, float *ret_out, void *stream) {
+    if (!values || !rewards || !dones || !adv_out || !ret_out || T < 0 || rows < 0 || P < 1)
+        return pfail(nullptr, "b2p_gae: bad argument");
+    if (rows % P) return pfail(nullptr, "b2p_gae: rows is not a multiple of P (rows per env)");
+    if (T == 0 || rows == 0) return 0;
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, values) != cudaSuccess || attr.type != cudaMemoryTypeDevice)
+        return pfail(nullptr, "b2p_gae: values is not device memory");
+    PolicyDeviceGuard guard(attr.device);
+    const long long blocks = (rows + pol::GAE_THREADS - 1) / pol::GAE_THREADS;
+    pol::gae_kernel<<<(unsigned)blocks, pol::GAE_THREADS, 0, (cudaStream_t)stream>>>(values, rewards, dones, T, rows, P, gamma, lam,
+                                                                                   adv_out, ret_out);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return pfail(nullptr, std::string("b2p_gae: ") + cudaGetErrorString(err));
     return 0;
 }
 

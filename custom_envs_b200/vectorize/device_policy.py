@@ -7,8 +7,13 @@ action head of such a network -- taken from a ``SharedMlpPolicy`` / any ``torch.
 that shape -- with bf16 tcgen05 MMAs, either on a dense observation matrix (``act``) or straight on
 the env's adjusted-history rings (``act_env``), in which case the env can step ring-only and the
 [sum(P), 3H] matrix never exists.  There is no fallback: without the library / an sm_100 GPU the
-constructor raises (``SharedMlpPolicy.act`` is the torch path, and it is the caller's choice)."""
+constructor raises (``SharedMlpPolicy.act`` is the torch path, and it is the caller's choice).
+
+For PPO, ``step`` / ``value`` are the rest of stable-baselines' ``model.step`` / ``model.value`` (value
+tower, unclipped action, neglogp, bf16 observation store), ``DeviceRolloutBuffer`` and
+``device_ppo_rollout`` collect a whole rollout with its GAE advantages on the device."""
 import ctypes
+import math
 
 import torch
 
@@ -31,9 +36,10 @@ class DevicePolicy:
         self.device = torch.device(device)
         self.obs_dim = int(obs_dim)
         self.low, self.high = float(low), float(high)
-        self.noise_std = 0.0 if log_std is None else float(torch.as_tensor(log_std).exp())
+        self.set_log_std(log_std)
         self.calls = 0
         self.seed_counter = None
+        self.has_value = False
         handle = ctypes.c_void_p()
         if self.lib.b2p_create(self.device.index or 0, self.obs_dim, int(tanh_mode), ctypes.byref(handle)):
             raise _lib.B200EnvError(self.lib.b2p_last_error(None).decode())
@@ -42,18 +48,20 @@ class DevicePolicy:
     @classmethod
     def from_torch(cls, tower, obs_dim=None, **kwargs):
         """``tower``: Linear(obs_dim, 64), Tanh, Linear(64, 64), Tanh, Linear(64, 1) -- e.g.
-        ``SharedMlpPolicy.pi`` -- or a module with such a ``.pi`` (its ``log_std`` is taken along)."""
+        ``SharedMlpPolicy.pi`` -- or a module with such a ``.pi`` (its ``log_std`` is taken along, and
+        its ``.vf`` tower of the same shape, if any, becomes the value tower of ``step`` / ``value``)."""
+        vf = None
         if hasattr(tower, 'pi'):
             if 'log_std' not in kwargs and hasattr(tower, 'log_std'):
                 kwargs['log_std'] = tower.log_std.detach()
+            vf = getattr(tower, 'vf', None)
             tower = tower.pi
-        linears = [m for m in tower.modules() if isinstance(m, torch.nn.Linear)]
-        if len(linears) != 3 or linears[0].out_features != 64 or linears[1].out_features != 64 \
-                or linears[2].out_features != 1:
-            raise ValueError('DevicePolicy needs an obs_dim -> 64 -> 64 -> 1 tanh tower')
+        linears = _tower_linears(tower)
         device = linears[0].weight.device
         policy = cls(obs_dim or linears[0].in_features, device=device, **kwargs)
         policy.set_weights(*[t for lin in linears for t in (lin.weight, lin.bias)])
+        if vf is not None:
+            policy.set_value_weights(*[t for lin in _tower_linears(vf) for t in (lin.weight, lin.bias)])
         return policy
 
     def _stream(self):
@@ -69,6 +77,21 @@ class DevicePolicy:
         assert tensors[0].shape == (64, self.obs_dim) and tensors[2].shape == (64, 64) and tensors[4].numel() == 64
         self._check(self.lib.b2p_set_weights(self.handle, *[_ptr(t) for t in tensors], self._stream()))
         torch.cuda.current_stream(self.device).synchronize()      # the sources may be temporaries
+
+    def set_value_weights(self, w1, b1, w2, b2, w3, b3):
+        """The value tower (``SharedMlpPolicy.vf``), in the layouts of ``set_weights``."""
+        tensors = [t.detach().to(self.device, torch.float32).contiguous() for t in (w1, b1, w2, b2, w3, b3)]
+        assert tensors[0].shape == (64, self.obs_dim) and tensors[2].shape == (64, 64) and tensors[4].numel() == 64
+        self._check(self.lib.b2p_set_value_weights(self.handle, *[_ptr(t) for t in tensors], self._stream()))
+        torch.cuda.current_stream(self.device).synchronize()
+        self.has_value = True
+
+    def set_log_std(self, log_std):
+        """Log of the Gaussian's standard deviation (None = deterministic): the noise of later launches and the
+        neglogp of ``step``.  PPO trains it (``SharedMlpPolicy.log_std``): hand it over with the tower weights after
+        every update."""
+        self.log_std = None if log_std is None else float(torch.as_tensor(log_std))
+        self.noise_std = 0.0 if log_std is None else math.exp(self.log_std)
 
     def use_seed_counter(self, enabled=True):
         """Draw the noise seed from a device counter (``self.seed_counter``, int64 [1]) added to the seed argument:
@@ -104,6 +127,58 @@ class DevicePolicy:
                                          self.low, self.high, self._stream()))
         return out
 
+    def _launch(self, source, seed, actions=None, actions_raw=None, values=None, neglogp=None, obs_bf16=None):
+        """One b2p_step (``source`` = dense obs [rows, obs_dim] float32) or b2p_step_env (``source`` = a
+        ``BatchedOptEnv``, read from its rings) launch; None outputs are not computed."""
+        dense = torch.is_tensor(source)
+        if dense:
+            assert source.dtype == torch.float32 and source.is_contiguous() and source.shape[-1] == self.obs_dim
+            rows = source.numel() // self.obs_dim
+        else:
+            rows = source.num_rows
+        for t in (actions, actions_raw, values, neglogp):
+            assert t is None or (t.dtype == torch.float32 and t.is_contiguous() and t.numel() == rows
+                                 and t.device == self.device)
+        if obs_bf16 is not None:
+            assert obs_bf16.dtype == torch.bfloat16 and obs_bf16.is_contiguous() and obs_bf16.numel() == rows * 16
+        if neglogp is not None and self.log_std is None:
+            raise ValueError('neglogp needs a stochastic policy (log_std)')
+        out = _lib.StepOut(*[t.data_ptr() if t is not None else None
+                             for t in (actions, actions_raw, values, neglogp, obs_bf16)])
+        log_std = 0.0 if self.log_std is None else self.log_std
+        if dense:
+            code = self.lib.b2p_step(self.handle, _ptr(source), rows, ctypes.byref(out), self.noise_std, log_std, seed,
+                                     self.low, self.high, self._stream())
+        else:
+            code = self.lib.b2p_step_env(self.handle, source.handle, ctypes.byref(out), self.noise_std, log_std, seed,
+                                         self.low, self.high, self._stream())
+        self._check(code)
+
+    def _rows(self, source):
+        return source.numel() // self.obs_dim if torch.is_tensor(source) else source.num_rows
+
+    def step(self, source, seed=None, obs_bf16=None):
+        """stable-baselines' ``model.step`` on every row of ``source`` (dense obs [rows, obs_dim] float32, or a
+        ``BatchedOptEnv`` whose rings are read, VecEnv row order) -> (actions, actions_raw, values, neglogp,
+        obs_bf16), each [rows] float32: the clipped action the env steps with (bit for bit ``act`` /
+        ``act_env`` with the same seed), the unclipped one PPO stores, the value tower's output (None
+        without one) and -log p(actions_raw).  ``obs_bf16``: a bf16 [rows, 16] tensor to receive the
+        observation rows as the network read them (columns obs_dim..15 zero), or None."""
+        if self.log_std is None:
+            raise ValueError('step samples from the Gaussian policy: construct it with a log_std')
+        new = lambda: torch.empty(self._rows(source), dtype=torch.float32, device=self.device)   # noqa: E731
+        actions, actions_raw, neglogp = new(), new(), new()
+        values = new() if self.has_value else None
+        self._launch(source, self._seed(seed), actions, actions_raw, values, neglogp, obs_bf16)
+        return actions, actions_raw, values, neglogp, obs_bf16
+
+    def value(self, source, out=None):
+        """``model.value``: the value tower alone on every row of ``source`` (as in ``step``) -> [rows] float32."""
+        if out is None:
+            out = torch.empty(self._rows(source), dtype=torch.float32, device=self.device)
+        self._launch(source, ctypes.c_uint64(0), values=out)
+        return out
+
     def close(self):
         if getattr(self, 'handle', None):
             torch.cuda.synchronize(self.device)
@@ -115,6 +190,19 @@ class DevicePolicy:
             self.close()
         except Exception:      # noqa: BLE001 (interpreter shutdown)
             pass
+
+
+def _tower_linears(tower):
+    linears = [m for m in tower.modules() if isinstance(m, torch.nn.Linear)]
+    if len(linears) != 3 or linears[0].out_features != 64 or linears[1].out_features != 64 \
+            or linears[2].out_features != 1:
+        raise ValueError('DevicePolicy needs an obs_dim -> 64 -> 64 -> 1 tanh tower')
+    return linears
+
+
+def reference_values(tower, obs, bf16=True):
+    """The value tower (``SharedMlpPolicy.vf``) as the kernel evaluates it: ``reference_actions`` without the clip."""
+    return reference_actions(tower, obs, low=-math.inf, high=math.inf, bf16=bf16)
 
 
 def reference_actions(tower, obs, low=-4.0, high=6.0, bf16=True):
@@ -180,3 +268,99 @@ def device_policy_rollout(env, policy, steps, ring_only=True, on_step=None, use_
         if on_step is not None:
             on_step(t, obs, reward, done, info)
     return returns, int(finished.item())
+
+
+def gae(values, rewards, dones, rows_per_env, gamma=0.99, lam=0.95, advantages=None, returns=None):
+    """The PPO2 Runner's GAE on the device (b2p_gae): values [T+1, rows], rewards [T, E] float32, dones [T+1, E]
+    uint8 (dones[t+1] = done of step t) -> (advantages, returns) [T, rows] float32; float64 recursion."""
+    lib = _lib.load()
+    T, rows = values.shape[0] - 1, values.shape[1]
+    assert values.dtype == torch.float32 and rewards.dtype == torch.float32 and dones.dtype == torch.uint8
+    assert all(t.is_contiguous() for t in (values, rewards, dones))
+    assert rewards.shape == (T, rows // rows_per_env) and dones.shape == (T + 1, rows // rows_per_env)
+    if advantages is None:
+        advantages = torch.empty((T, rows), dtype=torch.float32, device=values.device)
+    if returns is None:
+        returns = torch.empty((T, rows), dtype=torch.float32, device=values.device)
+    stream = ctypes.c_void_p(torch.cuda.current_stream(values.device).cuda_stream)
+    if lib.b2p_gae(_ptr(values), _ptr(rewards), _ptr(dones), T, rows, int(rows_per_env), float(gamma), float(lam),
+                   _ptr(advantages), _ptr(returns), stream):
+        raise _lib.B200EnvError(lib.b2p_last_error(None).decode())
+    return advantages, returns
+
+
+class DeviceRolloutBuffer:
+    """PPO rollout storage of ``n_steps`` steps of every agent row of ``env``, on its device, allocated once.
+
+    Time-major: ``obs_bf16`` [T, rows, 16] bf16 (the observation rows as the policy read them, columns
+    obs_dim..15 zero), ``actions_raw`` / ``neglogp`` / ``advantages`` / ``returns`` [T, rows] float32,
+    ``values`` [T+1, rows] float32 (``values[T]`` = value of the observation after the last step),
+    ``rewards`` [T, E] float32 and ``dones`` [T+1, E] uint8 (per env; env = row // P; ``dones[0]`` = the
+    flags at the rollout's first observation, ``dones[t+1]`` = done of step t).  stable-baselines'
+    ``swap_and_flatten`` order is ``.transpose(0, 1)`` of these arrays; PPO samples random minibatches of
+    flat indices, so no copy is needed.
+
+    ``actions`` [rows] float32 holds the clipped actions of the current step (what the env steps with).
+
+    Memory: 52 bytes per agent row and step (32 observation + 5 x 4), plus 8 bytes per agent row (the last
+    value slot and ``actions``), e.g. 10.8 GB per step for the 2.08e8 rows of 4096 envs of MLP 784-64-10
+    (88 GB for n_steps = 8); the constructor checks it against the device's free memory."""
+
+    BYTES_PER_ROW_STEP = 32 + 5 * 4
+
+    def __init__(self, env, n_steps):
+        self.n_steps = T = int(n_steps)
+        if T < 1:
+            raise ValueError('n_steps must be >= 1')
+        rows, E, dev = env.num_rows, env.num_envs, env.device
+        self.rows_per_env = env.num_params
+        need = rows * (self.BYTES_PER_ROW_STEP * T + 8) + E * (5 * T + 1)
+        free, _ = torch.cuda.mem_get_info(dev)
+        if need > free:
+            raise MemoryError('DeviceRolloutBuffer: n_steps = %d needs %.2f GB (%d rows x %d B per step) but %s has '
+                              '%.2f GB free; use fewer steps per rollout' % (T, need / 1e9, rows, self.BYTES_PER_ROW_STEP,
+                                                                            dev, free / 1e9))
+        f32 = dict(dtype=torch.float32, device=dev)
+        self.obs_bf16 = torch.empty((T, rows, 16), dtype=torch.bfloat16, device=dev)
+        self.actions_raw = torch.empty((T, rows), **f32)
+        self.values = torch.empty((T + 1, rows), **f32)
+        self.neglogp = torch.empty((T, rows), **f32)
+        self.advantages = torch.empty((T, rows), **f32)
+        self.returns = torch.empty((T, rows), **f32)
+        self.rewards = torch.zeros((T, E), **f32)
+        self.dones = torch.zeros((T + 1, E), dtype=torch.uint8, device=dev)
+        self.actions = torch.empty(rows, **f32)
+
+    def reset(self):
+        """Forget the carried done flags (call after ``env.reset()``): the next rollout starts with dones[0] = 0."""
+        self.dones.zero_()
+
+
+@torch.no_grad()
+def device_ppo_rollout(env, policy, buffer, gamma=0.99, lam=0.95, ring_only=True, on_step=None):
+    """One PPO2 ``Runner.run`` on the device: ``buffer.n_steps`` times ``model.step`` (``policy.step`` into the
+    buffer) then the env step with the clipped actions, then ``model.value`` of the last observation and GAE.
+    ``ring_only``: the policy reads the env's rings and the env writes no observation rows (MultiOptLRs, large
+    problems); otherwise the policy reads ``env.obs``, which must hold the current observation (the only path
+    of the small problems).  ``on_step(t, obs, reward, done, info)`` as in ``device_rollout``.  The done flags
+    of the last step become ``dones[0]`` of the next rollout; after ``env.reset()`` call ``buffer.reset()`` so that
+    they are zero, as the Runner starts.  Returns (buffer, finished episodes)."""
+    T = buffer.n_steps
+    assert buffer.actions.numel() == env.num_rows and buffer.rewards.shape[1] == env.num_envs
+    if not policy.has_value:
+        raise ValueError('device_ppo_rollout needs a policy with a value tower (set_value_weights)')
+    finished = torch.zeros((), dtype=torch.int64, device=env.device)
+    buffer.dones[0].copy_(buffer.dones[T])
+    for t in range(T):
+        source = env if ring_only else env.obs
+        policy._launch(source, policy._seed(None), buffer.actions, buffer.actions_raw[t], buffer.values[t],
+                       buffer.neglogp[t], buffer.obs_bf16[t])
+        obs, reward, done, info = env.step(buffer.actions, ring_only=ring_only)
+        buffer.rewards[t].copy_(reward)
+        buffer.dones[t + 1].copy_(done)
+        finished.add_(done.sum())
+        if on_step is not None:
+            on_step(t, obs, reward, done, info)
+    policy.value(env if ring_only else env.obs, out=buffer.values[T])
+    gae(buffer.values, buffer.rewards, buffer.dones, buffer.rows_per_env, gamma, lam, buffer.advantages, buffer.returns)
+    return buffer, int(finished.item())

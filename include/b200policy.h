@@ -70,6 +70,52 @@ int b2p_act(b2p_handle h, const float *obs, int64_t rows, float *actions_out, fl
 int b2p_act_env(b2p_handle h, b2e_handle env, float *actions_out, float noise_std, uint64_t seed,
                 float low, float high, void *stream);
 
+/* ---- PPO rollouts: the rest of stable-baselines' model.step / model.value, and GAE.
+ *
+ * MlpPolicy has a second tower of the same shape for the value (net_arch pi = vf = [64, 64]); it is
+ * set in the torch.nn.Linear layouts of b2p_set_weights.  The handle keeps its own copy. */
+int b2p_set_value_weights(b2p_handle h, const float *w1, const float *b1, const float *w2,
+                          const float *b2, const float *w3, const float *b3, void *stream);
+
+/* Outputs of one step launch, each [rows] float32 in the row order of the front end (VecEnv order on
+ * the rings), any of them NULL = not computed:
+ *   actions      clip(raw, low, high): bit for bit what b2p_act / b2p_act_env write with the same
+ *                seed, noise and bounds (the env steps with these)
+ *   actions_raw  raw = mean + noise_std * z, z = the row's N(0, 1) draw (PPO stores and scores this)
+ *   values       the value tower's output (model.value)
+ *   neglogp      0.5 z^2 + 0.5 log(2 pi) + log_std: -log density of raw under the diagonal Gaussian
+ *   obs_bf16     [rows][16] bf16, 16-byte aligned: the observation row the first layer read, already
+ *                rounded to bf16, columns obs_dim..15 zero (32 bytes per row)
+ * The action tower runs only for actions / actions_raw / neglogp, the value tower only for values
+ * (values alone = model.value).  values needs b2p_set_value_weights; an all-NULL set is an error. */
+typedef struct b2p_step_out {
+    float *actions;
+    float *actions_raw;
+    float *values;
+    float *neglogp;
+    void *obs_bf16;
+} b2p_step_out;
+
+/* Dense front end: obs float32 [rows, obs_dim], as b2p_act.  `out` is read when the call is made. */
+int b2p_step(b2p_handle h, const float *obs, int64_t rows, const b2p_step_out *out, float noise_std,
+             float log_std, uint64_t seed, float low, float high, void *stream);
+
+/* Ring front end: every agent row of `env`, as b2p_act_env. */
+int b2p_step_env(b2p_handle h, b2e_handle env, const b2p_step_out *out, float noise_std, float log_std,
+                 uint64_t seed, float low, float high, void *stream);
+
+/* Generalised advantage estimation of the PPO2 Runner over a time-major rollout of T steps:
+ *   values float32 [T+1, rows] (values[T] = the value of the observation after the last step),
+ *   rewards float32 [T, E], dones uint8 [T+1, E] (dones[t+1] = done returned by step t; dones[0] is
+ *   not read), E = rows / P with P rows per env (env = row / P in both VecEnv row orders)
+ *   -> adv_out, ret_out float32 [T, rows]:
+ *   nn = 1 - dones[t+1], delta = r[t] + gamma values[t+1] nn - values[t],
+ *   adv[t] = last = delta + gamma lam nn last, ret[t] = adv[t] + values[t]
+ * with the Runner's precision (float64 recursion, float32 stores).  Runs on the device of `values`;
+ * errors are read with b2p_last_error(NULL). */
+int b2p_gae(const float *values, const float *rewards, const uint8_t *dones, int T, int64_t rows,
+            int64_t P, double gamma, double lam, float *adv_out, float *ret_out, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
