@@ -29,7 +29,8 @@ EXPORTS = (
     'b2d_normalize', 'b2d_rank_workspace', 'b2d_label_ranks', 'b2d_onehot', 'b2d_shuffle_permutations',
     # shared per-agent policy (include/b200policy.h)
     'b2p_create', 'b2p_destroy', 'b2p_last_error', 'b2p_set_weights', 'b2p_act', 'b2p_act_env', 'b2p_set_seed_counter',
-    'b2p_set_value_weights', 'b2p_step', 'b2p_step_env', 'b2p_gae')
+    'b2p_set_value_weights', 'b2p_step', 'b2p_step_env', 'b2p_gae',
+    'b2p_tanh_table', 'b2p_ppo_indices', 'b2p_ppo_adv_stats_workspace_size', 'b2p_ppo_adv_stats', 'b2p_ppo_workspace_size', 'b2p_ppo_grad')
 DTYPE_U8, DTYPE_I32, DTYPE_F32, DTYPE_F64 = range(4)
 
 
@@ -45,6 +46,18 @@ class Config(ctypes.Structure):
 class StepOut(ctypes.Structure):
     """b2p_step_out: device pointers of the outputs of one b2p_step / b2p_step_env launch (NULL = not computed)."""
     _fields_ = [(name, ctypes.c_void_p) for name in ('actions', 'actions_raw', 'values', 'neglogp', 'obs_bf16')]
+
+
+class PpoBatch(ctypes.Structure):
+    """b2p_ppo_batch: device pointers of a time-major rollout buffer."""
+    _fields_ = [(name, ctypes.c_void_p) for name in ('obs_bf16', 'actions_raw', 'neglogp', 'values', 'returns')] + [
+        ('T', ctypes.c_int), ('rows', ctypes.c_int64)]
+
+
+class PpoParams(ctypes.Structure):
+    """b2p_ppo_params: loss coefficients and the minibatch of one b2p_ppo_grad call."""
+    _fields_ = [(name, ctypes.c_float) for name in ('cliprange', 'cliprange_vf', 'ent_coef', 'vf_coef', 'log_std')] + [
+        ('key', ctypes.c_uint64), ('begin', ctypes.c_int64), ('count', ctypes.c_int64), ('adv_stats', ctypes.c_void_p)]
 
 
 class B200EnvError(RuntimeError):
@@ -114,6 +127,14 @@ def load():
     lib.b2p_step.argtypes = [vp, vp, i64, ctypes.POINTER(StepOut), f32, f32, u64, f32, f32, vp]
     lib.b2p_step_env.argtypes = [vp, vp, ctypes.POINTER(StepOut), f32, f32, u64, f32, f32, vp]
     lib.b2p_gae.argtypes = [vp, vp, vp, i32, i64, i64, ctypes.c_double, ctypes.c_double, vp, vp, vp]
+    lib.b2p_tanh_table.argtypes = [vp, vp]
+    lib.b2p_ppo_indices.argtypes = [u64, i64, i64, i64, vp, vp]
+    lib.b2p_ppo_adv_stats_workspace_size.argtypes = [i64, i64]
+    lib.b2p_ppo_adv_stats_workspace_size.restype = usize
+    lib.b2p_ppo_adv_stats.argtypes = [ctypes.POINTER(PpoBatch), u64, i64, vp, vp, vp]
+    lib.b2p_ppo_workspace_size.argtypes = [vp]
+    lib.b2p_ppo_workspace_size.restype = usize
+    lib.b2p_ppo_grad.argtypes = [vp, ctypes.POINTER(PpoBatch), ctypes.POINTER(PpoParams), vp, vp, vp, vp]
     if lib.b2e_abi_version() != 2:
         raise B200EnvError('libb200env.so ABI version mismatch')
     _lib = lib

@@ -27,6 +27,7 @@
 #include <stdint.h>
 #include <string.h>
 
+#include <algorithm>
 #include <new>
 #include <string>
 
@@ -556,6 +557,496 @@ __global__ void __launch_bounds__(GAE_THREADS) gae_kernel(const float *__restric
     }
 }
 
+// ---------------------------------------------------------------- PPO update (b2p_ppo_*)
+// Minibatch order: a keyed Feistel network on 2 x `bits` bits (4^bits >= n), cycle-walked into [0, n): a
+// permutation of [0, n) that needs no stored index array.  Position p of the order is perm(p).
+constexpr int FEISTEL_ROUNDS = 6;
+struct Feistel {
+    unsigned long long key[FEISTEL_ROUNDS], mask, n;
+    int bits;
+};
+__host__ __device__ __forceinline__ unsigned long long mix64(unsigned long long z) {
+    z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
+    z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
+    return z ^ (z >> 31);
+}
+__device__ __forceinline__ long long feistel_at(const Feistel &f, long long p) {
+    unsigned long long v = (unsigned long long)p;
+    do {
+        unsigned long long L = v >> f.bits, R = v & f.mask;
+#pragma unroll
+        for (int r = 0; r < FEISTEL_ROUNDS; ++r) {
+            const unsigned long long nr = L ^ (mix64(R ^ f.key[r]) & f.mask);
+            L = R;
+            R = nr;
+        }
+        v = (L << f.bits) | R;
+    } while (v >= f.n);
+    return (long long)v;
+}
+
+// tanh.approx.bf16x2 of every bf16 input, as the policy kernels evaluate it in the bf16 tanh modes (b2p_tanh_table)
+__global__ void tanh_bf16_table_kernel(float *__restrict__ out) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < 65536) out[i] = __uint_as_float(tanh_bf16x2((uint32_t)i) << 16);
+}
+
+__global__ void ppo_indices_kernel(const Feistel f, long long begin, long long count, long long *__restrict__ out) {
+    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (long long)gridDim.x * blockDim.x)
+        out[i] = feistel_at(f, begin + i);
+}
+
+// a DeviceRolloutBuffer seen through flat time-major indices j = t * rows + row (values: its first T rows)
+struct PpoBatch {
+    const uint4 *obs;                                  // 2 x uint4 per row
+    const float *act, *nlp, *val, *ret;
+};
+
+// Advantage statistics of every minibatch of an epoch: block (m, c) sums A - K over its slice of minibatch m's
+// positions in fp64, thread-strided then a fixed tree (K = A at the minibatch's first position: a shift that keeps
+// the sum of squares well conditioned); ppo_adv_final sums a minibatch's slices in order.
+constexpr int ADV_THREADS = 256;
+constexpr long long ADV_SLICE = 65536;
+__device__ __forceinline__ float adv_of(const PpoBatch &b, long long j) { return __fsub_rn(b.ret[j], b.val[j]); }
+__global__ void __launch_bounds__(ADV_THREADS) ppo_adv_partial(const PpoBatch b, const Feistel f, long long mb, int slices,
+                                                               double *__restrict__ part) {
+    __shared__ double s1[ADV_THREADS], s2[ADV_THREADS];
+    const long long m = blockIdx.x / slices;
+    const int c = (int)(blockIdx.x - m * slices);
+    const long long len = (mb + slices - 1) / slices, lo = m * mb + c * len, hi = min(m * mb + mb, lo + len);
+    const double K = (double)adv_of(b, feistel_at(f, m * mb));
+    double a1 = 0.0, a2 = 0.0;
+    for (long long p = lo + threadIdx.x; p < hi; p += ADV_THREADS) {
+        const double d = (double)adv_of(b, feistel_at(f, p)) - K;
+        a1 += d;
+        a2 = fma(d, d, a2);
+    }
+    s1[threadIdx.x] = a1; s2[threadIdx.x] = a2;
+    __syncthreads();
+    for (int w = ADV_THREADS / 2; w > 0; w >>= 1) {
+        if ((int)threadIdx.x < w) { s1[threadIdx.x] += s1[threadIdx.x + w]; s2[threadIdx.x] += s2[threadIdx.x + w]; }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) { part[2 * blockIdx.x] = s1[0]; part[2 * blockIdx.x + 1] = s2[0]; }
+}
+__global__ void ppo_adv_final(const PpoBatch b, const Feistel f, long long mb, long long nmb, int slices,
+                              const double *__restrict__ part, double *__restrict__ stats) {
+    const long long m = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (m >= nmb) return;
+    double a1 = 0.0, a2 = 0.0;
+    for (int c = 0; c < slices; ++c) { a1 += part[2 * (m * slices + c)]; a2 += part[2 * (m * slices + c) + 1]; }
+    const double mean = a1 / (double)mb, var = a2 / (double)mb - mean * mean;
+    stats[2 * m] = (double)adv_of(b, feistel_at(f, m * mb)) + mean;
+    stats[2 * m + 1] = sqrt(var > 0.0 ? var : 0.0);                 // population std
+}
+
+// The clipped-surrogate gradient of both towers over one minibatch (b2p_ppo_grad).  Per 128-row tile a group
+// gathers its rows by index, runs the forward of each tower exactly as policy_kernel's step variant does (same
+// operands, MMAs, tanh and head FMA order, so the values at the rollout's weights are the rollout's bits), forms the
+// per-row loss derivative g, and runs the tower's backward on the tensor cores:
+//   dPre2 = g w3 (1 - h2^2)             bf16 tile [128 rows x 64], K-major (the thread's row)
+//   dH1   = dPre2 . W2                   M 128, N 64, K 64: A = dPre2 (K-major), B = [W2 | b2] operand read MN-major
+//   dPre1 = dH1 (1 - h1^2)               h1 = the bf16 operand of the second forward MMA
+//   [dW2 | db2] += dPre2^T . [h1 | 1]    M 64, N 80, K 128 rows: both operands read MN-major
+//   [dW1 | db1] += dPre1^T . A1          M 64, N 16, K 128 rows
+//   dw3 += g h2, db3 += g                FFMA: g h2 staged in shared memory as fp32, column sums in fixed order
+// MN-major no-swizzle descriptors for bf16: LBO = stride between 8-row K groups, SBO = stride between 8-element MN
+// groups (128 B).  An M = 64 accumulator holds row j in TMEM lane (j % 16) + 32 (j / 16).
+// TMEM: 256 columns per group = 64 working (D1, D2 / h2, dH1) + 2 x (80 + 16) private accumulators, so two groups.
+// The accumulators are read out and added into the group's fp32 slot of the workspace every FLUSH tiles (the tensor
+// core's adder truncates over long sums); ppo_reduce sums the slots in fp64 in a fixed order.
+namespace ppo {
+constexpr int GROUPS = 2, THREADS = GROUPS * 128, FLUSH = 16;
+constexpr int SBO_P = (HID / 8) * 128, P_BYTES = (TILE / 8) * SBO_P;      // dPre tiles [128 x 64] bf16
+constexpr int S_STRIDE = HID + 1, S_BYTES = (TILE * S_STRIDE * 4 + 127) / 128 * 128;   // g h2 stage, fp32
+constexpr int G_BYTES = A1_BYTES + A2_BYTES + 2 * P_BYTES + S_BYTES;
+constexpr int TOWER_OPS = B1_BYTES + B2_BYTES;                            // [W1 | b1] and [W2 | b2] of one tower
+constexpr int OFF_W = GROUPS * G_BYTES, OFF_W3 = OFF_W + 2 * TOWER_OPS;
+constexpr int SMEM_BYTES = OFF_W3 + 2 * (HID + 4) * 4 + 128;
+constexpr int TMEM_COLS = 512;
+constexpr int NSTATS = 5;                     // per-slot sums: pg, max(vf losses), (nlp - nlp_old)^2, clipped, dL/dlog_std
+static_assert(G_BYTES % 128 == 0 && OFF_W % 128 == 0 && TOWER_OPS % 128 == 0, "operand blocks are 128-byte aligned");
+static_assert(SMEM_BYTES <= 227 * 1024, "shared memory");
+static_assert(GROUPS * 256 <= TMEM_COLS, "tensor memory");
+}  // namespace ppo
+
+struct GradArgs {
+    const float *w;                   // the handle's weights: action tower, value tower
+    PpoBatch b;
+    Feistel f;
+    long long begin, count, tiles;
+    const double *adv_stats;          // mean, std of this minibatch's advantages
+    float clip, clip_vf, vf_coef, inv_n, inv_sigma, nlp_const;
+    float *ws_grad;                   // [slots][stride]
+    double *ws_stats;                 // [slots][NSTATS]
+    int od, tf, stride;
+};
+
+#define B2P_ST16(taddr, v) \
+    asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16};" \
+                 ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), \
+                   "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]) : "memory")
+
+template <int TANH>
+__global__ void __launch_bounds__(ppo::THREADS, 1) ppo_grad_kernel(const __grid_constant__ GradArgs a) {
+    constexpr int GROUPS = ppo::GROUPS, THREADS = ppo::THREADS, FLUSH = ppo::FLUSH, SBO_P = ppo::SBO_P, P_BYTES = ppo::P_BYTES;
+    constexpr int S_STRIDE = ppo::S_STRIDE, G_BYTES = ppo::G_BYTES, TOWER_OPS = ppo::TOWER_OPS, OFF_W = ppo::OFF_W;
+    constexpr int OFF_W3 = ppo::OFF_W3, TMEM_COLS = ppo::TMEM_COLS, NSTATS = ppo::NSTATS;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    __shared__ __align__(8) uint64_t mma_bar[GROUPS];
+    __shared__ uint32_t tmem_slot;
+    const int tid = threadIdx.x, warp = tid >> 5;
+    const int g = warp >> 2, wq = warp & 3, gt = tid & 127;
+    const uint32_t sbase = (smem_u32(smem_raw) + 127u) & ~127u;
+    unsigned char *const sm = smem_raw + (sbase - smem_u32(smem_raw));
+    unsigned char *const A1 = sm + g * G_BYTES, *const H = A1 + A1_BYTES, *const P2 = H + A2_BYTES, *const P1 = P2 + P_BYTES;
+    float *const S = reinterpret_cast<float *>(P1 + P_BYTES);
+    const uint32_t a1s = sbase + g * G_BYTES, hs = a1s + A1_BYTES, p2s = hs + A2_BYTES, p1s = p2s + P_BYTES;
+    const int od = a.od;
+    const int slot = blockIdx.x * GROUPS + g;
+    float *const wsg = a.ws_grad + (size_t)slot * a.stride;
+
+    if (tid == 0) {
+        for (int i = 0; i < GROUPS; ++i) mbar_init(&mma_bar[i], 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (warp == 0) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(TMEM_COLS));
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
+    }
+    for (int tw = 0; tw < 2; ++tw) {      // both towers' operands, in policy_kernel's layouts
+        const float *w1 = a.w + tw * a.tf, *b1 = w1 + HID * od, *w2 = b1 + HID, *b2 = w2 + HID * HID, *w3 = b2 + HID;
+        unsigned char *ob1 = sm + OFF_W + tw * TOWER_OPS, *ob2 = ob1 + B1_BYTES;
+        for (int i = tid; i < HID * K1; i += THREADS) {
+            const int n = i / K1, k = i - n * K1;
+            const float v = k < od ? w1[n * od + k] : (k == K1 - 1 ? b1[n] : 0.f);
+            *reinterpret_cast<unsigned short *>(ob1 + (n >> 3) * SBO1 + (k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2) = bf16_bits(v);
+        }
+        for (int i = tid; i < HID * K2; i += THREADS) {
+            const int n = i / K2, k = i - n * K2;
+            const float v = k < HID ? w2[n * HID + k] : (k == HID ? b2[n] : 0.f);
+            *reinterpret_cast<unsigned short *>(ob2 + (n >> 3) * SBO2 + (k >> 3) * 128 + (n & 7) * 16 + (k & 7) * 2) = bf16_bits(v);
+        }
+        float *w3s = reinterpret_cast<float *>(sm + OFF_W3) + tw * (HID + 4);
+        if (tid <= HID) w3s[tid] = w3[tid];                 // w3 then b3
+    }
+    {
+        unsigned char *row = H + (gt >> 3) * SBO2 + (gt & 7) * 16;
+        *reinterpret_cast<uint4 *>(row + 8 * 128) = make_uint4(0x00003F80u, 0u, 0u, 0u);
+        *reinterpret_cast<uint4 *>(row + 9 * 128) = make_uint4(0u, 0u, 0u, 0u);
+    }
+    for (int i = gt; i < a.stride; i += 128) wsg[i] = 0.f;
+    fence_async();
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const uint32_t tmem = tmem_slot;
+    const uint32_t twk = tmem + 256 * g;                  // working columns; accumulators of tower tw at + 64 + 96 tw
+    const uint32_t tlane = (uint32_t)(wq * 32) << 16;
+    constexpr uint32_t F32_BF16 = (1u << 4) | (1u << 7) | (1u << 10), A_MN = 1u << 15, B_MN = 1u << 16;
+    const uint32_t idesc = F32_BF16 | ((uint32_t)(HID >> 3) << 17) | ((uint32_t)(TILE >> 4) << 24);
+    const uint32_t idesc_dh = idesc | B_MN;
+    const uint32_t idesc_w2 = F32_BF16 | A_MN | B_MN | ((uint32_t)(K2 >> 3) << 17) | ((uint32_t)(64 >> 4) << 24);
+    const uint32_t idesc_w1 = F32_BF16 | A_MN | B_MN | ((uint32_t)(K1 >> 3) << 17) | ((uint32_t)(64 >> 4) << 24);
+    const uint64_t a1d = make_desc(a1s, 128, SBO1), hd = make_desc(hs, 128, SBO2);
+    const uint64_t b1d = make_desc(sbase + OFF_W, 128, SBO1), b2d = make_desc(sbase + OFF_W + B1_BYTES, 128, SBO2);
+    const uint64_t b2mn = make_desc(sbase + OFF_W + B1_BYTES, SBO2, 128);        // [W2 | b2] read as B[N = in][K = out]
+    const uint64_t p2k = make_desc(p2s, 128, SBO_P), p2mn = make_desc(p2s, SBO_P, 128), p1mn = make_desc(p1s, SBO_P, 128);
+    const uint64_t hmn = make_desc(hs, SBO2, 128), a1mn = make_desc(a1s, SBO1, 128);
+    const float *const w3all = reinterpret_cast<const float *>(sm + OFF_W3);
+    const double adv_mean = a.adv_stats[0], adv_inv = 1.0 / (a.adv_stats[1] + 1e-8);
+
+    uint32_t mph = 0;
+    auto mma_wait = [&]() { mbar_wait(&mma_bar[g], mph); mph ^= 1u; tc_fence_after(); };
+    auto issue_begin = [&]() -> bool {                     // every thread's operand writes are visible to the MMA issuer
+        fence_async();
+        tc_fence_before();
+        group_bar(g);
+        if (gt == 0) tc_fence_after();
+        return gt == 0;
+    };
+    // forward of tower tw on the A1 tile: policy_kernel's finish_tower, plus h2 written back over D2 for the backward
+    auto forward = [&](int tw) -> float {
+        const uint64_t shift = (uint64_t)(tw * (TOWER_OPS >> 4));
+        if (issue_begin()) { mma_bf16(twk, a1d, b1d + shift, idesc, 0u); mma_commit(&mma_bar[g]); }
+        mma_wait();
+#pragma unroll
+        for (int qt = 0; qt < 4; ++qt) {
+            uint32_t v[16];
+            B2P_LD16(twk + tlane + 16 * qt, v);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            unsigned char *row = H + (gt >> 3) * SBO2 + (gt & 7) * 16 + (2 * qt) * 128;
+#pragma unroll
+            for (int c = 0; c < 2; ++c) {
+                uint32_t pk[4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const float v0 = __uint_as_float(v[8 * c + 2 * i]), v1 = __uint_as_float(v[8 * c + 2 * i + 1]);
+                    pk[i] = TANH >= 1 ? tanh_bf16x2(pack_bf16x2(v0, v1)) : pack_bf16x2(tanh_f32(v0), tanh_f32(v1));
+                }
+                *reinterpret_cast<uint4 *>(row + c * 128) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+            }
+        }
+        if (issue_begin()) {
+#pragma unroll
+            for (int kk = 0; kk < K2 / 16; ++kk)
+                mma_bf16(twk, hd + (uint64_t)(kk * 16), b2d + shift + (uint64_t)(kk * 16), idesc, kk ? 1u : 0u);
+            mma_commit(&mma_bar[g]);
+        }
+        mma_wait();
+        const float *w3p = w3all + tw * (HID + 4);
+        float acc0 = w3p[HID], acc1 = 0.f;
+#pragma unroll
+        for (int qt = 0; qt < 4; ++qt) {
+            uint32_t v[16];
+            B2P_LD16(twk + tlane + 16 * qt, v);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+            for (int c = 0; c < 4; ++c) {
+                const float4 w = *reinterpret_cast<const float4 *>(w3p + 16 * qt + 4 * c);
+                float t0, t1, t2, t3;
+                if (TANH == 2) {
+                    const uint32_t q0 = tanh_bf16x2(pack_bf16x2(__uint_as_float(v[4 * c]), __uint_as_float(v[4 * c + 1])));
+                    const uint32_t q1 = tanh_bf16x2(pack_bf16x2(__uint_as_float(v[4 * c + 2]), __uint_as_float(v[4 * c + 3])));
+                    t0 = __uint_as_float(q0 << 16); t1 = __uint_as_float(q0 & 0xFFFF0000u);
+                    t2 = __uint_as_float(q1 << 16); t3 = __uint_as_float(q1 & 0xFFFF0000u);
+                } else {
+                    t0 = tanh_f32(__uint_as_float(v[4 * c])); t1 = tanh_f32(__uint_as_float(v[4 * c + 1]));
+                    t2 = tanh_f32(__uint_as_float(v[4 * c + 2])); t3 = tanh_f32(__uint_as_float(v[4 * c + 3]));
+                }
+                acc0 = fmaf(t0, w.x, acc0); acc1 = fmaf(t1, w.y, acc1);
+                acc0 = fmaf(t2, w.z, acc0); acc1 = fmaf(t3, w.w, acc1);
+                v[4 * c] = __float_as_uint(t0); v[4 * c + 1] = __float_as_uint(t1);
+                v[4 * c + 2] = __float_as_uint(t2); v[4 * c + 3] = __float_as_uint(t3);
+            }
+            B2P_ST16(twk + tlane + 16 * qt, v);
+        }
+        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+        return acc0 + acc1;
+    };
+    float dw3acc[2] = {0.f, 0.f}, db3acc[2] = {0.f, 0.f};
+    bool fresh = true;                                     // the accumulators start from zero at the next tile
+    // backward of tower tw for this row's dL/d(output) = gr (0 for rows past the minibatch)
+    auto backward = [&](int tw, float gr) {
+        const float *w3p = w3all + tw * (HID + 4);
+        unsigned char *prow = P2 + (gt >> 3) * SBO_P + (gt & 7) * 16;
+        float *srow = S + gt * S_STRIDE;
+#pragma unroll
+        for (int qt = 0; qt < 4; ++qt) {
+            uint32_t v[16];
+            B2P_LD16(twk + tlane + 16 * qt, v);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+            for (int c = 0; c < 2; ++c) {
+                uint32_t pk[4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const int j0 = 16 * qt + 8 * c + 2 * i;
+                    const float h0 = __uint_as_float(v[8 * c + 2 * i]), h1 = __uint_as_float(v[8 * c + 2 * i + 1]);
+                    pk[i] = pack_bf16x2(gr * w3p[j0] * fmaf(-h0, h0, 1.f), gr * w3p[j0 + 1] * fmaf(-h1, h1, 1.f));
+                    srow[j0] = gr * h0;
+                    srow[j0 + 1] = gr * h1;
+                }
+                *reinterpret_cast<uint4 *>(prow + (2 * qt + c) * 128) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+            }
+        }
+        const uint32_t acc_w2 = twk + 64 + 96 * tw, acc_w1 = acc_w2 + 80;
+        if (issue_begin()) {
+            const uint64_t shift = (uint64_t)(tw * (TOWER_OPS >> 4));
+#pragma unroll
+            for (int kk = 0; kk < HID / 16; ++kk)
+                mma_bf16(twk, p2k + (uint64_t)(kk * 16), b2mn + shift + (uint64_t)(kk * (2 * SBO2 >> 4)), idesc_dh, kk ? 1u : 0u);
+#pragma unroll
+            for (int kk = 0; kk < TILE / 16; ++kk)
+                mma_bf16(acc_w2, p2mn + (uint64_t)(kk * (2 * SBO_P >> 4)), hmn + (uint64_t)(kk * (2 * SBO2 >> 4)), idesc_w2,
+                         (kk || !fresh) ? 1u : 0u);
+            mma_commit(&mma_bar[g]);
+        }
+        {   // dw3 under the MMAs: column j = gt % 64 over rows 64 (gt / 64) .. + 63
+            const float *col = S + (gt >> 6) * 64 * S_STRIDE + (gt & 63);
+            float s = 0.f;
+#pragma unroll 8
+            for (int r = 0; r < 64; ++r) s += col[r * S_STRIDE];
+            dw3acc[tw] += s;
+            db3acc[tw] += gr;
+        }
+        mma_wait();
+        const unsigned char *hrow = H + (gt >> 3) * SBO2 + (gt & 7) * 16;
+        unsigned char *p1row = P1 + (gt >> 3) * SBO_P + (gt & 7) * 16;
+#pragma unroll
+        for (int qt = 0; qt < 4; ++qt) {
+            uint32_t v[16];
+            B2P_LD16(twk + tlane + 16 * qt, v);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+            for (int c = 0; c < 2; ++c) {
+                const uint4 hv = *reinterpret_cast<const uint4 *>(hrow + (2 * qt + c) * 128);
+                const uint32_t hw[4] = {hv.x, hv.y, hv.z, hv.w};
+                uint32_t pk[4];
+#pragma unroll
+                for (int i = 0; i < 4; ++i) {
+                    const float h0 = __uint_as_float(hw[i] << 16), h1 = __uint_as_float(hw[i] & 0xFFFF0000u);
+                    pk[i] = pack_bf16x2(__uint_as_float(v[8 * c + 2 * i]) * fmaf(-h0, h0, 1.f),
+                                        __uint_as_float(v[8 * c + 2 * i + 1]) * fmaf(-h1, h1, 1.f));
+                }
+                *reinterpret_cast<uint4 *>(p1row + (2 * qt + c) * 128) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
+            }
+        }
+        if (issue_begin()) {
+#pragma unroll
+            for (int kk = 0; kk < TILE / 16; ++kk)
+                mma_bf16(acc_w1, p1mn + (uint64_t)(kk * (2 * SBO_P >> 4)), a1mn + (uint64_t)(kk * (2 * SBO1 >> 4)), idesc_w1,
+                         (kk || !fresh) ? 1u : 0u);
+            mma_commit(&mma_bar[g]);
+        }
+        mma_wait();
+    };
+    // accumulators -> the group's workspace slot (fp32 adds, one owner per element)
+    auto flush = [&]() {
+        const int lane = gt & 31, j = wq * 16 + (lane & 15);
+        for (int tw = 0; tw < 2; ++tw) {
+            float *base = wsg + tw * a.tf;
+            float *dw1 = base, *db1 = dw1 + HID * od, *dw2 = db1 + HID, *db2 = dw2 + HID * HID;
+            const uint32_t acc_w2 = twk + 64 + 96 * tw, acc_w1 = acc_w2 + 80;
+            for (int q = 0; q < K2 / 16; ++q) {
+                uint32_t v[16];
+                B2P_LD16(acc_w2 + tlane + 16 * q, v);
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                if (lane < 16) {
+#pragma unroll
+                    for (int i = 0; i < 16; ++i) {
+                        const int col = 16 * q + i;
+                        if (col < HID) dw2[j * HID + col] += __uint_as_float(v[i]);
+                        else if (col == HID) db2[j] += __uint_as_float(v[i]);
+                    }
+                }
+            }
+            uint32_t v[16];
+            B2P_LD16(acc_w1 + tlane, v);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            if (lane < 16) {
+#pragma unroll
+                for (int k = 0; k < K1 - 1; ++k)
+                    if (k < od) dw1[j * od + k] += __uint_as_float(v[k]);
+                db1[j] += __uint_as_float(v[K1 - 1]);
+            }
+            S[gt] = dw3acc[tw];
+            S[128 + gt] = db3acc[tw];
+            group_bar(g);
+            float *dw3 = db2 + HID;
+            if (gt < HID) dw3[gt] += S[gt] + S[gt + 64];
+            if (gt == 0) {
+                float s = 0.f;
+                for (int r = 0; r < 128; ++r) s += S[128 + r];
+                dw3[HID] += s;
+            }
+            group_bar(g);
+            dw3acc[tw] = db3acc[tw] = 0.f;
+        }
+        tc_fence_before();
+    };
+
+    double st[NSTATS] = {0.0, 0.0, 0.0, 0.0, 0.0};
+    struct Row { uint4 o0, o1; float act, nlp, val, ret; bool live; };
+    auto fetch = [&](long long tile, Row &r) {
+        const long long q = tile * TILE + gt;
+        r.live = q < a.count;
+        if (r.live) {
+            const long long j = feistel_at(a.f, a.begin + q);
+            r.o0 = __ldg(a.b.obs + 2 * j); r.o1 = __ldg(a.b.obs + 2 * j + 1);
+            r.act = __ldg(a.b.act + j); r.nlp = __ldg(a.b.nlp + j); r.val = __ldg(a.b.val + j); r.ret = __ldg(a.b.ret + j);
+        } else {
+            r.o0 = r.o1 = make_uint4(0u, 0u, 0u, 0u);
+            r.act = r.nlp = r.val = r.ret = 0.f;
+        }
+    };
+    const long long step = (long long)gridDim.x * GROUPS;
+    long long tile = (long long)blockIdx.x * GROUPS + g;
+    Row nx;
+    if (tile < a.tiles) fetch(tile, nx);
+    for (int since = 0; tile < a.tiles; tile += step) {
+        const Row cur = nx;
+        {   // A1 = the stored bf16 row with the bias column 15 set to 1
+            unsigned char *row = A1 + (gt >> 3) * SBO1 + (gt & 7) * 16;
+            uint4 o1 = cur.o1;
+            if (cur.live) o1.w = (o1.w & 0xFFFFu) | 0x3F800000u;
+            *reinterpret_cast<uint4 *>(row) = cur.o0;
+            *reinterpret_cast<uint4 *>(row + 128) = o1;
+        }
+        if (tile + step < a.tiles) fetch(tile + step, nx);      // in flight under this tile's work
+        // ---- action tower: dL/dmu of the clipped surrogate (TF gradient rules: max -> first operand on ties,
+        // clip passes inside the closed interval)
+        const float mu = forward(0);
+        float gpi = 0.f;
+        if (cur.live) {
+            const float adv = (float)(((double)__fsub_rn(cur.ret, cur.val) - adv_mean) * adv_inv);
+            const float z = (cur.act - mu) * a.inv_sigma;
+            const float nlp = fmaf(0.5f * z, z, a.nlp_const);
+            const float ratio = expf(cur.nlp - nlp);
+            const float lo = 1.f - a.clip, hi = 1.f + a.clip;
+            const float l1 = -adv * ratio, l2 = -adv * fminf(fmaxf(ratio, lo), hi);
+            const float dratio = (l1 >= l2 || (ratio >= lo && ratio <= hi)) ? -adv : 0.f;
+            const float dnlp = -dratio * ratio * a.inv_n;            // d pg / d nlp of this row
+            gpi = -dnlp * z * a.inv_sigma;                           // d nlp / d mu = -(a - mu) / sigma^2
+            st[0] += (double)fmaxf(l1, l2);
+            st[2] += (double)(nlp - cur.nlp) * (double)(nlp - cur.nlp);
+            st[3] += fabsf(ratio - 1.f) > a.clip ? 1.0 : 0.0;
+            st[4] += (double)(dnlp * fmaf(-z, z, 1.f));              // d nlp / d log_std = 1 - z^2
+        }
+        backward(0, gpi);
+        // ---- value tower
+        const float V = forward(1);
+        float gv = 0.f;
+        if (cur.live) {
+            const float d1 = V - cur.ret, dv = V - cur.val;
+            const bool clipv = a.clip_vf >= 0.f;
+            const float vc = clipv ? cur.val + fminf(fmaxf(dv, -a.clip_vf), a.clip_vf) : V;
+            const float d2 = vc - cur.ret;
+            const float l1 = d1 * d1, l2 = d2 * d2;
+            const float dl = l1 >= l2 ? 2.f * d1 : ((clipv && fabsf(dv) <= a.clip_vf) ? 2.f * d2 : 0.f);
+            gv = 0.5f * a.vf_coef * a.inv_n * dl;
+            st[1] += (double)fmaxf(l1, l2);
+        }
+        backward(1, gv);
+        fresh = false;
+        if (++since == FLUSH || tile + step >= a.tiles) { flush(); since = 0; fresh = true; }
+    }
+    {   // the group's statistics, fixed order
+        double *sd = reinterpret_cast<double *>(S);
+        group_bar(g);
+        for (int s = 0; s < NSTATS; ++s) sd[s * 128 + gt] = st[s];
+        group_bar(g);
+        if (gt < NSTATS) {
+            double s = 0.0;
+            for (int r = 0; r < 128; ++r) s += sd[gt * 128 + r];
+            a.ws_stats[(size_t)slot * NSTATS + gt] = s;
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS));
+}
+
+// slots -> grad_out (fp64 sums in slot order; the last entry is d loss / d log_std) and the six statistics
+__global__ void ppo_reduce_kernel(const float *__restrict__ ws_grad, const double *__restrict__ ws_stats, int slots, int stride,
+                                  double inv_n, double log_std, double ent_coef, double vf_coef, float *__restrict__ grad,
+                                  double *__restrict__ stats) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < stride - 1) {
+        double s = 0.0;
+        for (int k = 0; k < slots; ++k) s += (double)ws_grad[(size_t)k * stride + i];
+        grad[i] = (float)s;
+    } else if (i == stride - 1) {
+        double s[ppo::NSTATS] = {0.0, 0.0, 0.0, 0.0, 0.0};
+        for (int k = 0; k < slots; ++k)
+            for (int q = 0; q < ppo::NSTATS; ++q) s[q] += ws_stats[(size_t)k * ppo::NSTATS + q];
+        grad[i] = (float)(s[4] - ent_coef);                       // the entropy term: d ent / d log_std = 1
+        const double pg = s[0] * inv_n, vf = 0.5 * s[1] * inv_n, ent = log_std + 1.4189385332046727418;   // 0.5 log(2 pi e)
+        stats[0] = pg; stats[1] = vf; stats[2] = ent; stats[3] = 0.5 * s[2] * inv_n; stats[4] = s[3] * inv_n;
+        stats[5] = pg - ent_coef * ent + vf_coef * vf;
+    }
+}
+
 }  // namespace pol
 }  // namespace
 
@@ -677,6 +1168,33 @@ int step_setup(b2p_handle h, const b2p_step_out *out, float noise_std, float log
     return 0;
 }
 
+pol::Feistel feistel_setup(uint64_t key, int64_t n) {
+    pol::Feistel f;
+    f.n = (unsigned long long)n;
+    f.bits = 1;
+    while ((1ull << (2 * f.bits)) < f.n) ++f.bits;
+    f.mask = (1ull << f.bits) - 1ull;
+    for (int r = 0; r < pol::FEISTEL_ROUNDS; ++r) f.key[r] = pol::mix64(key + 0x9E3779B97F4A7C15ull * (unsigned long long)(r + 1));
+    return f;
+}
+
+int adv_slices(int64_t mb_size) { return (int)((mb_size + pol::ADV_SLICE - 1) / pol::ADV_SLICE); }
+
+size_t grad_stride(int obs_dim) { return 2 * tower_floats(obs_dim) + 1; }
+
+// a b2p_ppo_batch -> PpoBatch; n = T * rows; non-zero (error set on h, or the global error for h = NULL) if malformed
+int check_batch(b2p_handle h, const b2p_ppo_batch *b, pol::PpoBatch &pb, int64_t &n, const char *who) {
+    const std::string w(who);
+    if (!b || !b->obs_bf16 || !b->actions_raw || !b->neglogp || !b->values || !b->returns)
+        return pfail(h, w + ": null batch pointer");
+    if (reinterpret_cast<uintptr_t>(b->obs_bf16) & 15u) return pfail(h, w + ": obs_bf16 must be 16-byte aligned");
+    if (b->T < 1 || b->rows < 1 || b->rows > B2P_PPO_MAX_SAMPLES / b->T) return pfail(h, w + ": bad T or rows");
+    n = (int64_t)b->T * b->rows;
+    pb.obs = static_cast<const uint4 *>(b->obs_bf16);
+    pb.act = b->actions_raw; pb.nlp = b->neglogp; pb.val = b->values; pb.ret = b->returns;
+    return 0;
+}
+
 
 }  // namespace
 
@@ -696,6 +1214,10 @@ int b2p_create(int device, int obs_dim, int tanh_mode, b2p_handle *out) {
     if (!(set_policy_smem<0, false>() && set_policy_smem<1, false>() && set_policy_smem<2, false>() &&
           set_policy_smem<0, true>() && set_policy_smem<1, true>() && set_policy_smem<2, true>()))
         return pfail(nullptr, "b2p_create: the policy kernel does not fit shared memory");
+    if (cudaFuncSetAttribute(pol::ppo_grad_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::ppo::SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(pol::ppo_grad_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::ppo::SMEM_BYTES) != cudaSuccess ||
+        cudaFuncSetAttribute(pol::ppo_grad_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::ppo::SMEM_BYTES) != cudaSuccess)
+        return pfail(nullptr, "b2p_create: the PPO gradient kernel does not fit shared memory");
     b2p_policy *h = new (std::nothrow) b2p_policy();
     if (!h) return pfail(nullptr, "b2p_create: out of host memory");
     h->device = device; h->obs_dim = obs_dim; h->tanh_mode = tanh_mode; h->num_sms = prop.multiProcessorCount;
@@ -839,6 +1361,115 @@ int b2p_gae(const float *values, const float *rewards, const uint8_t *dones, int
                                                                                    adv_out, ret_out);
     const cudaError_t err = cudaGetLastError();
     if (err != cudaSuccess) return pfail(nullptr, std::string("b2p_gae: ") + cudaGetErrorString(err));
+    return 0;
+}
+
+int b2p_tanh_table(float *out, void *stream) {
+    if (!out) return pfail(nullptr, "b2p_tanh_table: null output");
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, out) != cudaSuccess || attr.type != cudaMemoryTypeDevice)
+        return pfail(nullptr, "b2p_tanh_table: out is not device memory");
+    PolicyDeviceGuard guard(attr.device);
+    pol::tanh_bf16_table_kernel<<<256, 256, 0, (cudaStream_t)stream>>>(out);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return pfail(nullptr, std::string("b2p_tanh_table: ") + cudaGetErrorString(err));
+    return 0;
+}
+
+int b2p_ppo_indices(uint64_t key, int64_t n, int64_t begin, int64_t count, int64_t *out, void *stream) {
+    if (n < 1 || n > B2P_PPO_MAX_SAMPLES) return pfail(nullptr, "b2p_ppo_indices: n must be 1..2^62");
+    if (count < 1) return pfail(nullptr, "b2p_ppo_indices: count must be >= 1");
+    if (begin < 0 || begin > n - count) return pfail(nullptr, "b2p_ppo_indices: range outside [0, n)");
+    if (!out) return pfail(nullptr, "b2p_ppo_indices: null output");
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, out) != cudaSuccess || attr.type != cudaMemoryTypeDevice)
+        return pfail(nullptr, "b2p_ppo_indices: out is not device memory");
+    PolicyDeviceGuard guard(attr.device);
+    const pol::Feistel f = feistel_setup(key, n);
+    const long long blocks = std::min<long long>((count + 255) / 256, 1 << 16);
+    pol::ppo_indices_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)stream>>>(f, begin, count, reinterpret_cast<long long *>(out));
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return pfail(nullptr, std::string("b2p_ppo_indices: ") + cudaGetErrorString(err));
+    return 0;
+}
+
+size_t b2p_ppo_adv_stats_workspace_size(int64_t n, int64_t mb_size) {
+    if (n < 1 || mb_size < 1 || n % mb_size) return 0;
+    return (size_t)(n / mb_size) * (size_t)adv_slices(mb_size) * 2 * sizeof(double);
+}
+
+int b2p_ppo_adv_stats(const b2p_ppo_batch *b, uint64_t key, int64_t mb_size, double *stats_out, void *workspace,
+                      void *stream) {
+    pol::PpoBatch pb;
+    int64_t n = 0;
+    if (check_batch(nullptr, b, pb, n, "b2p_ppo_adv_stats")) return 1;
+    if (!stats_out || !workspace) return pfail(nullptr, "b2p_ppo_adv_stats: null output or workspace");
+    if (mb_size < 1 || n % mb_size) return pfail(nullptr, "b2p_ppo_adv_stats: T * rows is not a multiple of the minibatch size");
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, b->returns) != cudaSuccess || attr.type != cudaMemoryTypeDevice)
+        return pfail(nullptr, "b2p_ppo_adv_stats: returns is not device memory");
+    PolicyDeviceGuard guard(attr.device);
+    const pol::Feistel f = feistel_setup(key, n);
+    const long long nmb = n / mb_size;
+    const int slices = adv_slices(mb_size);
+    if (nmb > 0x7FFFFFFFLL / slices)
+        return pfail(nullptr, "b2p_ppo_adv_stats: too many minibatches for one launch (more than 2^31 - 1 blocks)");
+    double *part = static_cast<double *>(workspace);
+    pol::ppo_adv_partial<<<(unsigned)(nmb * slices), pol::ADV_THREADS, 0, (cudaStream_t)stream>>>(pb, f, mb_size, slices, part);
+    pol::ppo_adv_final<<<(unsigned)((nmb + 255) / 256), 256, 0, (cudaStream_t)stream>>>(pb, f, mb_size, nmb, slices, part, stats_out);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return pfail(nullptr, std::string("b2p_ppo_adv_stats: ") + cudaGetErrorString(err));
+    return 0;
+}
+
+size_t b2p_ppo_workspace_size(b2p_handle h) {
+    if (!h) return 0;
+    const size_t slots = (size_t)h->num_sms * pol::ppo::GROUPS;
+    return slots * (grad_stride(h->obs_dim) * sizeof(float) + pol::ppo::NSTATS * sizeof(double)) + 256;
+}
+
+int b2p_ppo_grad(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, float *grad_out, double *stats_out,
+                 void *workspace, void *stream) {
+    if (!h) return 1;
+    if (!h->have_weights || !h->have_value_weights)
+        return pfail(h, "b2p_ppo_grad: weights not set (b2p_set_weights and b2p_set_value_weights)");
+    pol::PpoBatch pb;
+    int64_t n = 0;
+    if (check_batch(h, b, pb, n, "b2p_ppo_grad")) return 1;
+    if (!p || !grad_out || !stats_out || !workspace || !p->adv_stats)
+        return pfail(h, "b2p_ppo_grad: null params, adv_stats, output or workspace");
+    if (p->count < 1) return pfail(h, "b2p_ppo_grad: count must be >= 1");
+    if (p->begin < 0 || p->begin > n - p->count) return pfail(h, "b2p_ppo_grad: range outside [0, T * rows)");
+    if (!(p->cliprange > 0.f)) return pfail(h, "b2p_ppo_grad: cliprange must be > 0");
+    PolicyDeviceGuard guard(h->device);
+    pol::GradArgs a;
+    memset(&a, 0, sizeof(a));
+    a.w = h->weights;
+    a.b = pb;
+    a.f = feistel_setup(p->key, n);
+    a.begin = p->begin; a.count = p->count; a.tiles = (p->count + pol::TILE - 1) / pol::TILE;
+    a.adv_stats = p->adv_stats;
+    a.clip = p->cliprange; a.clip_vf = p->cliprange_vf; a.vf_coef = p->vf_coef;
+    a.inv_n = (float)(1.0 / (double)p->count);
+    a.inv_sigma = (float)exp(-(double)p->log_std);
+    a.nlp_const = (float)(0.91893853320467274178 + (double)p->log_std);      // as b2p_step: 0.5 log(2 pi) + log_std
+    a.od = h->obs_dim; a.tf = (int)tower_floats(h->obs_dim); a.stride = (int)grad_stride(h->obs_dim);
+    const long long want = (a.tiles + pol::ppo::GROUPS - 1) / pol::ppo::GROUPS;
+    const int grid = (int)(want < h->num_sms ? want : h->num_sms), slots = grid * pol::ppo::GROUPS;
+    const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
+    a.ws_grad = reinterpret_cast<float *>(base);
+    a.ws_stats = reinterpret_cast<double *>(base + (((size_t)slots * a.stride * sizeof(float) + 7) & ~(size_t)7));
+    cudaStream_t cs = (cudaStream_t)stream;
+    switch (h->tanh_mode) {
+        case 2: pol::ppo_grad_kernel<2><<<grid, pol::ppo::THREADS, pol::ppo::SMEM_BYTES, cs>>>(a); break;
+        case 1: pol::ppo_grad_kernel<1><<<grid, pol::ppo::THREADS, pol::ppo::SMEM_BYTES, cs>>>(a); break;
+        default: pol::ppo_grad_kernel<0><<<grid, pol::ppo::THREADS, pol::ppo::SMEM_BYTES, cs>>>(a); break;
+    }
+    pol::ppo_reduce_kernel<<<(a.stride + 255) / 256, 256, 0, cs>>>(a.ws_grad, a.ws_stats, slots, a.stride, 1.0 / (double)p->count,
+                                                                   (double)p->log_std, (double)p->ent_coef, (double)p->vf_coef,
+                                                                   grad_out, stats_out);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return pfail(h, std::string("b2p_ppo_grad: ") + cudaGetErrorString(err));
     return 0;
 }
 

@@ -11,7 +11,8 @@ constructor raises (``SharedMlpPolicy.act`` is the torch path, and it is the cal
 
 For PPO, ``step`` / ``value`` are the rest of stable-baselines' ``model.step`` / ``model.value`` (value
 tower, unclipped action, neglogp, bf16 observation store), ``DeviceRolloutBuffer`` and
-``device_ppo_rollout`` collect a whole rollout with its GAE advantages on the device."""
+``device_ppo_rollout`` collect a whole rollout with its GAE advantages on the device, and ``ppo_grad`` /
+``device_ppo_update`` run PPO2's minibatch updates over it with a fused clipped-surrogate gradient kernel."""
 import ctypes
 import math
 
@@ -178,6 +179,33 @@ class DevicePolicy:
             out = torch.empty(self._rows(source), dtype=torch.float32, device=self.device)
         self._launch(source, ctypes.c_uint64(0), values=out)
         return out
+
+    def ppo_grad(self, buffer, key, begin, count, adv_stats, cliprange=0.2, cliprange_vf=None, ent_coef=0.01,
+                 vf_coef=0.5, grad=None, stats=None):
+        """Gradient of PPO2's loss over the minibatch at positions [begin, begin + count) of the permutation ``key`` of
+        ``buffer``'s T * rows samples, at this policy's weights and ``log_std`` (b2p_ppo_grad).  ``adv_stats``: device
+        float64 [2] (mean, std of the minibatch's returns - values, e.g. a row of ``ppo_adv_stats``);
+        ``cliprange_vf`` None = ``cliprange`` (stable-baselines' default), negative = no value clipping.  Returns
+        (grad float32 [2 * tower + 1]: action tower, value tower in ``set_weights`` layouts, then log_std; stats float64
+        [6]: pg_loss, vf_loss, entropy, approxkl, clipfrac, loss), both on the device, not synchronised."""
+        if self.log_std is None:
+            raise ValueError('ppo_grad needs a stochastic policy (log_std)')
+        tower = 64 * self.obs_dim + 64 + 64 * 64 + 64 + 64 + 1
+        if grad is None:
+            grad = torch.empty(2 * tower + 1, dtype=torch.float32, device=self.device)
+        if stats is None:
+            stats = torch.empty(6, dtype=torch.float64, device=self.device)
+        assert grad.dtype == torch.float32 and grad.numel() == 2 * tower + 1 and grad.is_contiguous()
+        assert stats.dtype == torch.float64 and stats.numel() == 6 and adv_stats.dtype == torch.float64
+        if getattr(self, '_ppo_ws', None) is None:
+            self._ppo_ws = torch.empty(self.lib.b2p_ppo_workspace_size(self.handle), dtype=torch.uint8, device=self.device)
+        params = _lib.PpoParams(float(cliprange), float(cliprange if cliprange_vf is None else cliprange_vf),
+                                float(ent_coef), float(vf_coef), float(self.log_std), int(key) & (2 ** 64 - 1),
+                                int(begin), int(count), adv_stats.data_ptr())
+        batch = _ppo_batch(buffer)
+        self._check(self.lib.b2p_ppo_grad(self.handle, ctypes.byref(batch), ctypes.byref(params), _ptr(grad), _ptr(stats),
+                                          _ptr(self._ppo_ws), self._stream()))
+        return grad, stats
 
     def close(self):
         if getattr(self, 'handle', None):
@@ -364,3 +392,123 @@ def device_ppo_rollout(env, policy, buffer, gamma=0.99, lam=0.95, ring_only=True
     policy.value(env if ring_only else env.obs, out=buffer.values[T])
     gae(buffer.values, buffer.rewards, buffer.dones, buffer.rows_per_env, gamma, lam, buffer.advantages, buffer.returns)
     return buffer, int(finished.item())
+
+
+# ------------------------------------------------------------------ PPO updates
+def _ppo_batch(buffer):
+    T, rows = buffer.actions_raw.shape
+    return _lib.PpoBatch(buffer.obs_bf16.data_ptr(), buffer.actions_raw.data_ptr(), buffer.neglogp.data_ptr(),
+                         buffer.values.data_ptr(), buffer.returns.data_ptr(), T, rows)
+
+
+def _check_global(code):
+    if code:
+        raise _lib.B200EnvError(_lib.load().b2p_last_error(None).decode())
+
+
+def tanh_bf16_table(device='cuda'):
+    """float32 [65536]: the bf16 tanh the kernels evaluate in the bf16 tanh modes, indexed by the input's bf16 bit
+    pattern (b2p_tanh_table) -- for references that reproduce those modes exactly."""
+    lib = _lib.load()
+    out = torch.empty(65536, dtype=torch.float32, device=device)
+    _check_global(lib.b2p_tanh_table(_ptr(out), ctypes.c_void_p(torch.cuda.current_stream(out.device).cuda_stream)))
+    return out
+
+
+def ppo_minibatch_indices(n, key, begin, count, out=None, device='cuda'):
+    """The flat sample indices (t * rows + row) at positions [begin, begin + count) of the keyed permutation of
+    [0, n) that ``ppo_grad`` reads (b2p_ppo_indices) -> int64 [count] on the device."""
+    lib = _lib.load()
+    if out is None:
+        out = torch.empty(int(count), dtype=torch.int64, device=device)
+    assert out.dtype == torch.int64 and out.is_contiguous() and out.numel() == count
+    stream = ctypes.c_void_p(torch.cuda.current_stream(out.device).cuda_stream)
+    _check_global(lib.b2p_ppo_indices(int(key) & (2 ** 64 - 1), int(n), int(begin), int(count), _ptr(out), stream))
+    return out
+
+
+def ppo_adv_stats(buffer, key, mb_size):
+    """Mean and population std (float64 sums) of returns - values over every minibatch of one epoch's permutation
+    ``key`` -> float64 [T * rows / mb_size, 2] on the device (b2p_ppo_adv_stats)."""
+    lib = _lib.load()
+    T, rows = buffer.actions_raw.shape
+    n = T * rows
+    if mb_size < 1 or n % mb_size:
+        raise ValueError('the %d samples of the buffer do not split into minibatches of %d' % (n, mb_size))
+    dev = buffer.returns.device
+    stats = torch.empty((n // mb_size, 2), dtype=torch.float64, device=dev)
+    ws = torch.empty(max(1, lib.b2p_ppo_adv_stats_workspace_size(n, mb_size)), dtype=torch.uint8, device=dev)
+    batch = _ppo_batch(buffer)
+    stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    _check_global(lib.b2p_ppo_adv_stats(ctypes.byref(batch), int(key) & (2 ** 64 - 1), int(mb_size), _ptr(stats),
+                                        _ptr(ws), stream))
+    return stats
+
+
+def epoch_key(seed, epoch):
+    """The permutation key of epoch ``epoch`` of an update seeded ``seed`` (splitmix64 of both)."""
+    z = (int(seed) * 0x9E3779B97F4A7C15 + int(epoch) + 1) & (2 ** 64 - 1)
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & (2 ** 64 - 1)
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & (2 ** 64 - 1)
+    return z ^ (z >> 31)
+
+
+def _model_params(model):
+    """The parameters in the order of ``ppo_grad``'s flat gradient: pi (w1, b1, w2, b2, w3, b3), vf (...), log_std."""
+    params = []
+    for tower in (model.pi, model.vf):
+        for lin in _tower_linears(tower):
+            params += [lin.weight, lin.bias]
+    return params + [model.log_std]
+
+
+def load_model(policy, model):
+    """Hand ``model``'s (a ``SharedMlpPolicy``) towers and ``log_std`` to ``policy``."""
+    policy.set_weights(*[t for lin in _tower_linears(model.pi) for t in (lin.weight, lin.bias)])
+    policy.set_value_weights(*[t for lin in _tower_linears(model.vf) for t in (lin.weight, lin.bias)])
+    policy.set_log_std(model.log_std.detach())
+
+
+def device_ppo_update(model, policy, buffer, optimizer, n_epochs=4, n_minibatches=4, cliprange=0.2, cliprange_vf=None,
+                      ent_coef=0.01, vf_coef=0.5, max_grad_norm=0.5, seed=None):
+    """stable-baselines 2 ``PPO2.learn``'s inner loop over a filled ``DeviceRolloutBuffer``: ``n_epochs`` passes, each
+    over a fresh permutation of the T * rows samples cut into ``n_minibatches`` minibatches.  Per minibatch: ``model``'s
+    towers and ``log_std`` go to ``policy``, ``policy.ppo_grad`` computes the gradient of PPO2's loss, it is copied into
+    the parameters' ``.grad``, then ``clip_grad_norm_(max_grad_norm)`` (skipped for None, as in PPO2) and
+    ``optimizer.step()``.  ``model`` (a ``SharedMlpPolicy``) stays the fp32 master copy; the optimizer is the
+    caller's -- PPO2's is Adam with eps = 1e-5, i.e. ``torch.optim.Adam(model.parameters(), lr, eps=1e-5)`` (torch places eps outside the square root like TF's
+    Adam but without TF's bias-corrected epsilon, so parity with TF is not pinned).  ``seed`` picks the permutations
+    (None: drawn from torch's generator).  On return ``policy`` holds the trained weights and ``log_std``.  Returns
+    the statistics averaged over minibatches (pg_loss, vf_loss, entropy, approxkl, clipfrac, loss) as float64 numpy
+    [6], with one host synchronisation."""
+    T, rows = buffer.actions_raw.shape
+    n = T * rows
+    if n % n_minibatches:
+        raise ValueError('T * rows = %d is not a multiple of n_minibatches = %d' % (n, n_minibatches))
+    mb = n // n_minibatches
+    if seed is None:
+        seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+    params = _model_params(model)
+    total = torch.zeros(6, dtype=torch.float64, device=policy.device)
+    grad = stats = None
+    for epoch in range(n_epochs):
+        key = epoch_key(seed, epoch)
+        adv = ppo_adv_stats(buffer, key, mb)
+        for m in range(n_minibatches):
+            load_model(policy, model)
+            grad, stats = policy.ppo_grad(buffer, key, m * mb, mb, adv[m], cliprange, cliprange_vf, ent_coef, vf_coef,
+                                          grad, stats)
+            offset = 0
+            for p in params:
+                g = grad[offset:offset + p.numel()].view_as(p)
+                if p.grad is None:
+                    p.grad = g.clone()
+                else:
+                    p.grad.copy_(g)
+                offset += p.numel()
+            if max_grad_norm is not None:
+                torch.nn.utils.clip_grad_norm_(params, max_grad_norm)
+            optimizer.step()
+            total += stats
+    load_model(policy, model)
+    return (total / (n_epochs * n_minibatches)).cpu().numpy()

@@ -70,6 +70,11 @@ int b2p_act(b2p_handle h, const float *obs, int64_t rows, float *actions_out, fl
 int b2p_act_env(b2p_handle h, b2e_handle env, float *actions_out, float noise_std, uint64_t seed,
                 float low, float high, void *stream);
 
+/* out float32 [65536]: out[x] = the bf16 tanh of the bf16 with bit pattern x, as the kernels evaluate it in
+ * B2P_TANH_BF16X2 and the mode that also uses it for the second layer (tanh.approx.bf16x2).  For references that
+ * reproduce those modes exactly.  Errors: b2p_last_error(NULL). */
+int b2p_tanh_table(float *out, void *stream);
+
 /* ---- PPO rollouts: the rest of stable-baselines' model.step / model.value, and GAE.
  *
  * MlpPolicy has a second tower of the same shape for the value (net_arch pi = vf = [64, 64]); it is
@@ -115,6 +120,55 @@ int b2p_step_env(b2p_handle h, b2e_handle env, const b2p_step_out *out, float no
  * errors are read with b2p_last_error(NULL). */
 int b2p_gae(const float *values, const float *rewards, const uint8_t *dones, int T, int64_t rows,
             int64_t P, double gamma, double lam, float *adv_out, float *ret_out, void *stream);
+
+/* ---- PPO updates: the gradient of stable-baselines 2's PPO2 loss over one minibatch of a rollout.
+ *
+ * A minibatch is a range of positions of a keyed permutation of the T * rows flat sample indices
+ * j = t * rows + row (a Feistel bijection, cycle-walked into [0, T * rows); no index array is stored):
+ * epoch e of PPO2 uses one key and minibatch m the positions [m * n, (m + 1) * n). */
+#define B2P_PPO_MAX_SAMPLES (1LL << 62)
+
+typedef struct b2p_ppo_batch {          /* a DeviceRolloutBuffer, time-major */
+    const void *obs_bf16;               /* [T][rows][16] bf16, 16-byte aligned (column 15 is not read: the bias 1) */
+    const float *actions_raw, *neglogp, *values, *returns;   /* [T][rows] (values: first T rows of [T+1][rows]) */
+    int T;
+    int64_t rows;
+} b2p_ppo_batch;
+
+typedef struct b2p_ppo_params {
+    float cliprange, cliprange_vf;      /* cliprange_vf < 0: no value clipping (the None default is resolved by the caller) */
+    float ent_coef, vf_coef, log_std;
+    uint64_t key;                       /* permutation key of the epoch */
+    int64_t begin, count;               /* the minibatch = positions [begin, begin + count) of the permutation */
+    const double *adv_stats;            /* device [2]: mean and population std of this minibatch's returns - values */
+} b2p_ppo_params;
+
+/* out int64 [count] = the flat sample indices at positions [begin, begin + count) of the permutation of [0, n)
+ * with `key`.  Errors: b2p_last_error(NULL). */
+int b2p_ppo_indices(uint64_t key, int64_t n, int64_t begin, int64_t count, int64_t *out, void *stream);
+
+/* Advantage statistics of every minibatch of an epoch: stats_out double [T * rows / mb_size][2] = mean and population
+ * std of A = returns - values (float32 difference, fp64 sums in a fixed order) over each minibatch's samples.
+ * T * rows must be a multiple of mb_size.  workspace: b2p_ppo_adv_stats_workspace_size(T * rows, mb_size) bytes.
+ * Errors: b2p_last_error(NULL). */
+size_t b2p_ppo_adv_stats_workspace_size(int64_t n, int64_t mb_size);
+int b2p_ppo_adv_stats(const b2p_ppo_batch *b, uint64_t key, int64_t mb_size, double *stats_out, void *workspace,
+                      void *stream);
+
+/* The gradient of PPO2's loss over one minibatch, with the weights of the last b2p_set_weights /
+ * b2p_set_value_weights and the handle's tanh_mode:
+ *   A_n = (A - mean) / (std + 1e-8);  ratio = exp(neglogp_old - neglogp(actions_raw | mu, log_std))
+ *   pg = mean(max(-A_n ratio, -A_n clip(ratio, 1 - c, 1 + c)))
+ *   vf = 0.5 mean(max((V - R)^2, (V_old + clip(V - V_old, -c_vf, c_vf) - R)^2))   (c_vf < 0: vf = 0.5 mean((V - R)^2))
+ *   ent = log_std + 0.5 log(2 pi e);  loss = pg - ent_coef ent + vf_coef vf
+ * grad_out float [2 * tower + 1]: d loss / d (action tower, value tower, log_std), the towers in b2p_set_weights layouts
+ * (w1, b1, w2, b2, w3, b3); stats_out double [6]: pg, vf, ent, approxkl = 0.5 mean((nlp - nlp_old)^2),
+ * clipfrac = mean(|ratio - 1| > c), loss.  Gradients follow TensorFlow's rules (max: the first operand on ties; clip:
+ * passes inside the closed interval).  workspace: b2p_ppo_workspace_size(h) bytes.  The result is bit-identical from
+ * call to call for the same inputs on the same device.  Nothing is allocated. */
+size_t b2p_ppo_workspace_size(b2p_handle h);
+int b2p_ppo_grad(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, float *grad_out, double *stats_out,
+                 void *workspace, void *stream);
 
 #ifdef __cplusplus
 }
