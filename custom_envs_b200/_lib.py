@@ -30,7 +30,7 @@ EXPORTS = (
     # shared per-agent policy (include/b200policy.h)
     'b2p_create', 'b2p_destroy', 'b2p_last_error', 'b2p_set_weights', 'b2p_act', 'b2p_act_env', 'b2p_set_seed_counter',
     'b2p_set_value_weights', 'b2p_step', 'b2p_step_env', 'b2p_gae',
-    'b2p_tanh_table', 'b2p_ppo_indices', 'b2p_ppo_adv_stats_workspace_size', 'b2p_ppo_adv_stats', 'b2p_ppo_workspace_size', 'b2p_ppo_grad')
+    'b2p_obs_width', 'b2p_tanh_table', 'b2p_ppo_indices', 'b2p_ppo_adv_stats_workspace_size', 'b2p_ppo_adv_stats', 'b2p_ppo_workspace_size', 'b2p_ppo_grad')
 DTYPE_U8, DTYPE_I32, DTYPE_F32, DTYPE_F64 = range(4)
 
 
@@ -115,6 +115,8 @@ def load():
     lib.b2d_shuffle_permutations.argtypes = [vp, i32, i64, i32, vp, vp]
     f32, u64 = ctypes.c_float, ctypes.c_uint64
     lib.b2p_create.argtypes = [i32, i32, i32, ctypes.POINTER(vp)]
+    lib.b2p_obs_width.argtypes = [i32]
+    lib.b2p_obs_width.restype = i32
     lib.b2p_destroy.argtypes = [vp]
     lib.b2p_destroy.restype = None
     lib.b2p_last_error.argtypes = [vp]

@@ -30,6 +30,7 @@
 #include <algorithm>
 #include <new>
 #include <string>
+#include <type_traits>
 
 #include "b200env_shared.cuh"
 #include "b200env_internal.h"
@@ -41,25 +42,50 @@ namespace pol {
 #ifndef B2P_GROUPS
 #define B2P_GROUPS 6
 #endif
-constexpr int TILE = 128, HID = B2P_HIDDEN, K1 = 16, K2 = 80, GROUPS = B2P_GROUPS, THREADS = GROUPS * 128;
-constexpr int NSTG = GROUPS <= 4 ? 2 : 1;        // staging buffers of the dense front end per group (shared memory budget)
-constexpr int XMAX = B2P_MAX_OBS_DIM;
-constexpr int SBO1 = (K1 / 8) * 128, SBO2 = (K2 / 8) * 128;
-constexpr int A1_BYTES = (TILE / 8) * SBO1, A2_BYTES = (TILE / 8) * SBO2;
-constexpr int STAGE_BYTES = TILE * XMAX * 4;
-constexpr int G_BYTES = NSTG * STAGE_BYTES + A1_BYTES + A2_BYTES;
-constexpr int OFF_B1 = GROUPS * G_BYTES, B1_BYTES = (HID / 8) * SBO1;
-constexpr int OFF_B2 = OFF_B1 + B1_BYTES, B2_BYTES = (HID / 8) * SBO2;
-constexpr int OFF_W3 = OFF_B2 + B2_BYTES;
-constexpr int SMEM_BYTES = OFF_W3 + (HID + 4) * 4 + 128;   // + slack to align the base to 128 bytes
-constexpr int TMEM_COLS = GROUPS <= 4 ? 256 : 512;    // 64 columns per group: D2 overwrites D1, which is fully read before the second layer's MMAs are issued
-// the step kernel (b2p_step*) adds the value tower's operands behind the action tower's; it runs the two towers
-// one after the other in the same TMEM columns and A2 buffer
-constexpr int OFF_VB1 = (OFF_W3 + (HID + 4) * 4 + 127) / 128 * 128, OFF_VB2 = OFF_VB1 + B1_BYTES, OFF_VW3 = OFF_VB2 + B2_BYTES;
-constexpr int SMEM_STEP_BYTES = OFF_VW3 + (HID + 4) * 4 + 128;
-static_assert(G_BYTES % 128 == 0 && OFF_B1 % 128 == 0 && OFF_B2 % 128 == 0 && OFF_VB1 % 128 == 0 && OFF_VB2 % 128 == 0,
-              "operand blocks are 128-byte aligned");
-static_assert(SMEM_BYTES <= 227 * 1024 && SMEM_STEP_BYTES <= 227 * 1024, "shared memory");
+constexpr int TILE = 128, HID = B2P_HIDDEN, K2 = 80;
+constexpr int XMAX = 15;                          // the narrow row (K1 = 16): obs_dim <= 15, held in registers
+constexpr int SBO2 = (K2 / 8) * 128, A2_BYTES = (TILE / 8) * SBO2, B2_BYTES = (HID / 8) * SBO2;
+constexpr int W3_BYTES = (HID + 4) * 4;
+constexpr int SMEM_LIMIT = 227 * 1024;
+
+// First-layer K of an observation row (b2p_obs_width): the row and the bias column, rounded up to the MMA's K of 16.
+// K1 = 16 is the narrow kernel (obs_dim <= 15); K1 = 32 .. 80 the wide variants.
+__host__ __device__ constexpr int obs_width(int obs_dim) { return 16 * ((obs_dim + 16) / 16); }
+
+// policy_kernel's shared memory: per group [dense staging (narrow only) | A1 | A2], then [W1 | b1], [W2 | b2], w3 of the
+// action tower; the step kernel (b2p_step*) adds the value tower's operands behind them and runs the two towers one
+// after the other in the same TMEM columns and A2 buffer
+constexpr int policy_smem(int groups, int g_bytes, int b1_bytes, bool step) {
+    const int off_w3 = groups * g_bytes + b1_bytes + B2_BYTES;
+    const int off_vw3 = (off_w3 + W3_BYTES + 127) / 128 * 128 + b1_bytes + B2_BYTES;
+    return (step ? off_vw3 : off_w3) + W3_BYTES + 128;   // + slack to align the base to 128 bytes
+}
+// the wide variants: as many groups as the shared memory holds (at most the narrow kernel's six); no staging buffers,
+// the front end writes A1 directly
+constexpr int wide_groups(int g_bytes, int b1_bytes, bool step) {
+    int g = 6;
+    while (g > 1 && policy_smem(g, g_bytes, b1_bytes, step) > SMEM_LIMIT - 256) --g;     // 256: the static barriers
+    return g;
+}
+template <int K1, bool STEP>
+struct Geo {
+    static constexpr bool WIDE = K1 > 16;
+    static constexpr int SBO1 = (K1 / 8) * 128, A1_BYTES = (TILE / 8) * SBO1, B1_BYTES = (HID / 8) * SBO1;
+    static constexpr int GROUPS = WIDE ? wide_groups(A1_BYTES + A2_BYTES, B1_BYTES, STEP) : B2P_GROUPS;
+    static constexpr int THREADS = GROUPS * 128;
+    static constexpr int NSTG = WIDE ? 0 : GROUPS <= 4 ? 2 : 1;     // staging buffers of the dense front end per group
+    static constexpr int STAGE_BYTES = TILE * XMAX * 4;
+    static constexpr int G_BYTES = NSTG * STAGE_BYTES + A1_BYTES + A2_BYTES;
+    static constexpr int OFF_B1 = GROUPS * G_BYTES, OFF_B2 = OFF_B1 + B1_BYTES, OFF_W3 = OFF_B2 + B2_BYTES;
+    static constexpr int OFF_VB1 = (OFF_W3 + W3_BYTES + 127) / 128 * 128, OFF_VB2 = OFF_VB1 + B1_BYTES, OFF_VW3 = OFF_VB2 + B2_BYTES;
+    static constexpr int SMEM_BYTES = policy_smem(GROUPS, G_BYTES, B1_BYTES, STEP);
+    static constexpr int TMEM_COLS = GROUPS <= 4 ? 256 : 512;   // 64 columns per group: D2 overwrites D1, which is fully read before the second layer's MMAs are issued
+    static_assert(K1 % 16 == 0 && K1 >= 16 && K1 <= K2, "first-layer K");
+    static_assert(G_BYTES % 128 == 0 && OFF_B1 % 128 == 0 && OFF_B2 % 128 == 0 && OFF_VB1 % 128 == 0 && OFF_VB2 % 128 == 0,
+                  "operand blocks are 128-byte aligned");
+    static_assert(SMEM_BYTES <= SMEM_LIMIT, "shared memory");
+};
+static_assert(Geo<16, true>::GROUPS == 6 && Geo<32, true>::GROUPS == 6 && Geo<80, true>::GROUPS == 4, "group counts");
 
 struct Args {
     const float *w1, *b1, *w2, *b2, *w3, *b3;
@@ -77,7 +103,7 @@ struct Args {
 struct StepArgs {
     const float *w1, *b1, *w2, *b2, *w3, *b3;      // value tower (vf), NULL without values
     float *raw, *values, *neglogp;                  // [rows]; Args::out holds the clipped actions
-    uint4 *obs16;                                   // [rows][16] bf16 = 2 x uint4 per row
+    uint4 *obs16;                                   // [rows][K1] bf16 = K1 / 8 x uint4 per row
     float nlp_const;                                // 0.5 log(2 pi) + log_std
     int want_pi;                                    // any action output requested
 };
@@ -160,9 +186,14 @@ __device__ __forceinline__ float row_noise(unsigned long long seed, long long ro
 // 2 = rings with any max_history <= 5
 // STEP: the b2p_step* variant (value tower, raw actions, neglogp, observation store; StepArgs); the b2p_act* instantiations
 // ignore `s`
-template <int FRONT, int TANH, bool STEP = false>
-__global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constant__ Args a, const __grid_constant__ Dev d,
-                                                            const __grid_constant__ StepArgs s) {
+template <int FRONT, int TANH, bool STEP = false, int K1 = 16>
+__global__ void __launch_bounds__(Geo<K1, STEP>::THREADS, 1) policy_kernel(const __grid_constant__ Args a, const __grid_constant__ Dev d,
+                                                                          const __grid_constant__ StepArgs s) {
+    using G = Geo<K1, STEP>;
+    constexpr bool WIDE = G::WIDE;
+    constexpr int GROUPS = G::GROUPS, THREADS = G::THREADS, NSTG = G::NSTG, STAGE_BYTES = G::STAGE_BYTES, G_BYTES = G::G_BYTES;
+    constexpr int SBO1 = G::SBO1, A1_BYTES = G::A1_BYTES, OFF_B1 = G::OFF_B1, OFF_B2 = G::OFF_B2;
+    constexpr int OFF_W3 = G::OFF_W3, OFF_VB1 = G::OFF_VB1, OFF_VB2 = G::OFF_VB2, OFF_VW3 = G::OFF_VW3, TMEM_COLS = G::TMEM_COLS;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t obs_full[GROUPS][2];
     __shared__ __align__(8) uint64_t mma_bar[GROUPS];
@@ -236,6 +267,12 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
     auto want_pi = [&]() -> bool { return !STEP || s.want_pi; };     // read from the parameter space, never held in a register
     auto want_v = [&]() -> bool { return STEP && s.values; };
     const uint32_t tm1 = tmem + 64 * g, tm2 = tm1;
+    // D1 = A1 . [W1 | b1]^T: K1 / 16 MMAs into the same accumulator, in K order (ppo_grad_kernel repeats it)
+    auto layer1 = [&](uint64_t b1desc) {
+#pragma unroll
+        for (int kk = 0; kk < K1 / 16; ++kk)
+            mma_bf16(tm1, a1d + (uint64_t)(kk * 16), b1desc + (uint64_t)(kk * 16), idesc, kk ? 1u : 0u);
+    };
     const uint32_t tlane = (uint32_t)(wq * 32) << 16;
     const float b3 = w3s[HID];
     const unsigned long long seed = a.seed + (a.seed_counter ? *a.seed_counter : 0ull);
@@ -279,12 +316,14 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
             if (lo + g >= hi) continue;
             const EnvScalars *sc = d.sc + e;
             c.e = e; c.tp = lo + g; c.hi = hi; c.head = sc->head; c.nvalid = sc->nvalid; c.valid = true;
+            if constexpr (!WIDE) {
 #pragma unroll
-            for (int h = 0; h < XMAX / 3; ++h) {
-                const int H = FRONT == 1 ? 5 : d.H;
-                int slot = c.head - h;
-                slot += slot < 0 ? H : 0;
-                c.lv[h] = (h < H && h < c.nvalid) ? sc->adj_loss[slot] : 0.f;
+                for (int h = 0; h < XMAX / 3; ++h) {
+                    const int H = FRONT == 1 ? 5 : d.H;
+                    int slot = c.head - h;
+                    slot += slot < 0 ? H : 0;
+                    c.lv[h] = (h < H && h < c.nvalid) ? sc->adj_loss[slot] : 0.f;
+                }
             }
             return;
         }
@@ -312,6 +351,26 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
                 if (ok && h < c.nvalid) { wv = d.ringw[off]; gv = d.ringg[off]; }
             }
             x[3 * h] = wv; x[3 * h + 1] = c.lv[h]; x[3 * h + 2] = gv;
+        }
+    };
+    // Wide rows (K1 > 16): too many values to hold in registers, so the group's loads of the next tile are L2
+    // prefetches issued under this tile's work, and the row is read when the tile's turn comes (wide_row below)
+    auto prefetch_next = [&](const Cursor &c) {
+        auto prefetch_l2 = [](const void *ptr) { asm volatile("prefetch.global.L2 [%0];" ::"l"(ptr)); };
+        if (RING) {                                         // 2H slot rows of 128 floats = 8H lines of 128 bytes
+            const int H = d.H;
+            for (int i = gt; i < 8 * H; i += 128) {
+                const int h = i >> 3, p = c.tp * TILE + (i & 3) * 32;
+                if (h < c.nvalid && p < d.P) {
+                    int slot = c.head - h;
+                    slot += slot < 0 ? H : 0;
+                    prefetch_l2(((i >> 2) & 1 ? d.ringg : d.ringw) + ((size_t)c.e * H + slot) * d.Pp + p);
+                }
+            }
+        } else {                                            // the tile's rows are contiguous
+            const long long row0 = c.tile * TILE, n = min((long long)TILE, a.rows - row0) * od;
+            const float *src = a.obs + row0 * od;
+            for (long long i = gt * 32; i < n; i += 128 * 32) prefetch_l2(src + i);
         }
     };
     auto ring_row = [&](const float (&raw)[XMAX], float (&x)[XMAX]) {   // [adj_w (H) | adj_L (H) | adj_g (H)], clip, -1
@@ -347,11 +406,61 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
     int cur_e = 0, cur_tp = 0;
     bool have = c.valid;
     if (have) {
-        if (RING) { load_ring(c, nxt); cur_e = c.e; cur_tp = c.tp; }
-        else { fetch_dense(c.tile, 0); tile = c.tile; }
+        if (RING) { if constexpr (!WIDE) load_ring(c, nxt); cur_e = c.e; cur_tp = c.tp; }
+        else { if constexpr (!WIDE) fetch_dense(c.tile, 0); tile = c.tile; }
         advance(c);
     }
     for (int n = 0; have; ++n) {
+        // ---- row of the output vectors (the next b2e_step gathers the action through the same row table)
+        auto out_row = [&](bool &live) -> long long {
+            if (RING) {
+                const int p = cur_tp * TILE + gt;
+                live = p < d.P;
+                return (long long)cur_e * d.P + (live ? (d.row_lex ? d.row_of_param[p] : p) : 0);
+            }
+            live = tile * TILE + gt < a.rows;
+            return tile * TILE + gt;
+        };
+        if constexpr (WIDE) {
+            // ---- A1 = [row | 0 | 1] as bf16, 16 columns at a time; the observation store gets the same chunks with
+            // the bias column 0.  Ring rows are assembled column by column, [adj_w (H) | adj_L (H) | adj_g (H)] newest
+            // first, with the narrow front end's values and rounding, so that they equal the dense rows bit for bit.
+            unsigned char *row = A1 + (gt >> 3) * SBO1 + (gt & 7) * 16;
+            bool live;
+            const long long orow = out_row(live);
+            uint4 *const store = (STEP && s.obs16 && live) ? s.obs16 + orow * (K1 / 8) : nullptr;
+            const int H = RING ? d.H : 0, p = cur_tp * TILE + gt;
+            const EnvScalars *sc = d.sc + cur_e;
+            const int head = RING ? sc->head : 0, nvalid = RING ? sc->nvalid : 0;
+            const float *src = a.obs + (tile * TILE + gt) * od;
+            auto col = [&](int k) -> float {
+                if (RING) {
+                    if (k >= 3 * H) return 0.f;
+                    const int sg = k >= 2 * H ? 2 : (k >= H ? 1 : 0), h = k - sg * H;
+                    float v = 0.f;
+                    if (h < nvalid) {
+                        int slot = head - h;
+                        slot += slot < 0 ? H : 0;
+                        if (sg == 1) v = sc->adj_loss[slot];
+                        else if (p < d.P) v = (sg == 0 ? d.ringw : d.ringg)[((size_t)cur_e * H + slot) * d.Pp + p];
+                    }
+                    return clip_m1(v);
+                }
+                return (live && k < od) ? src[k] : 0.f;
+            };
+#pragma unroll 1
+            for (int k0 = 0; k0 < K1; k0 += 16) {
+                float v[16];
+#pragma unroll
+                for (int i = 0; i < 16; ++i) v[i] = col(k0 + i);
+                const uint4 c0 = make_uint4(pack_bf16x2(v[0], v[1]), pack_bf16x2(v[2], v[3]), pack_bf16x2(v[4], v[5]), pack_bf16x2(v[6], v[7]));
+                uint4 c1 = make_uint4(pack_bf16x2(v[8], v[9]), pack_bf16x2(v[10], v[11]), pack_bf16x2(v[12], v[13]), pack_bf16x2(v[14], v[15]));
+                if (store) { store[k0 / 8] = c0; store[k0 / 8 + 1] = c1; }
+                if (k0 + 16 == K1) c1.w = (c1.w & 0xFFFFu) | 0x3F800000u;      // column K1 - 1 >= obs_dim: the bias 1
+                *reinterpret_cast<uint4 *>(row + (k0 / 8) * 128) = c0;
+                *reinterpret_cast<uint4 *>(row + (k0 / 8 + 1) * 128) = c1;
+            }
+        } else {
         float x[XMAX];
         if (RING) {
             ring_row(nxt, x);
@@ -364,16 +473,6 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
 #pragma unroll
             for (int k = 0; k < XMAX; ++k) x[k] = (live && k < od) ? st[k] : 0.f;
         }
-        // ---- row of the output vectors (the next b2e_step gathers the action through the same row table)
-        auto out_row = [&](bool &live) -> long long {
-            if (RING) {
-                const int p = cur_tp * TILE + gt;
-                live = p < d.P;
-                return (long long)cur_e * d.P + (live ? (d.row_lex ? d.row_of_param[p] : p) : 0);
-            }
-            live = tile * TILE + gt < a.rows;
-            return tile * TILE + gt;
-        };
         // ---- A1 = [x | 0 | 1] as bf16, this thread's row
         {
             unsigned char *row = A1 + (gt >> 3) * SBO1 + (gt & 7) * 16;
@@ -391,19 +490,26 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
                 }
             }
         }
+        }
         fence_async();
         tc_fence_before();
         group_bar(g);
         if (gt == 0 && (want_pi() || want_v())) {
             tc_fence_after();
-            mma_bf16(tm1, a1d, want_pi() ? b1d : b1d + VDESC_SHIFT, idesc, 0u);
+            layer1(want_pi() ? b1d : b1d + VDESC_SHIFT);
             mma_commit(&mma_bar[g]);
         }
-        if (!RING && NSTG == 1 && c.valid) fetch_dense(c.tile, 0);      // the single staging buffer is free again (barrier above)
+        if constexpr (!WIDE) {
+            if (!RING && NSTG == 1 && c.valid) fetch_dense(c.tile, 0);      // the single staging buffer is free again (barrier above)
+        }
         const bool have_next = c.valid;
         const long long next_tile = c.tile;
         const int next_e = c.e, next_tp = c.tp;
-        if (RING && have_next) load_ring(c, nxt);             // in flight under this tile's work
+        if constexpr (WIDE) {
+            if (have_next) prefetch_next(c);
+        } else {
+            if (RING && have_next) load_ring(c, nxt);             // in flight under this tile's work
+        }
         if (have_next) advance(c);
         // ---- the rest of a tower whose first-layer MMA has been issued: -> w3 . tanh(D2) + b3 of this thread's row
         auto finish_tower = [&](uint64_t b2desc, const float *w3p, float bias) -> float {
@@ -493,7 +599,7 @@ __global__ void __launch_bounds__(THREADS, 1) policy_kernel(const __grid_constan
                     group_bar(g);
                     if (gt == 0) {
                         tc_fence_after();
-                        mma_bf16(tm1, a1d, b1d + VDESC_SHIFT, idesc, 0u);
+                        layer1(b1d + VDESC_SHIFT);
                         mma_commit(&mma_bar[g]);
                     }
                 }
@@ -598,7 +704,7 @@ __global__ void ppo_indices_kernel(const Feistel f, long long begin, long long c
 
 // a DeviceRolloutBuffer seen through flat time-major indices j = t * rows + row (values: its first T rows)
 struct PpoBatch {
-    const uint4 *obs;                                  // 2 x uint4 per row
+    const uint4 *obs;                                  // K1 / 8 x uint4 per row (b2p_obs_width bf16)
     const float *act, *nlp, *val, *ret;
 };
 
@@ -648,26 +754,37 @@ __global__ void ppo_adv_final(const PpoBatch b, const Feistel f, long long mb, l
 //   dH1   = dPre2 . W2                   M 128, N 64, K 64: A = dPre2 (K-major), B = [W2 | b2] operand read MN-major
 //   dPre1 = dH1 (1 - h1^2)               h1 = the bf16 operand of the second forward MMA
 //   [dW2 | db2] += dPre2^T . [h1 | 1]    M 64, N 80, K 128 rows: both operands read MN-major
-//   [dW1 | db1] += dPre1^T . A1          M 64, N 16, K 128 rows
+//   [dW1 | db1] += dPre1^T . A1          M 64, N K1, K 128 rows
 //   dw3 += g h2, db3 += g                FFMA: g h2 staged in shared memory as fp32, column sums in fixed order
 // MN-major no-swizzle descriptors for bf16: LBO = stride between 8-row K groups, SBO = stride between 8-element MN
 // groups (128 B).  An M = 64 accumulator holds row j in TMEM lane (j % 16) + 32 (j / 16).
-// TMEM: 256 columns per group = 64 working (D1, D2 / h2, dH1) + 2 x (80 + 16) private accumulators, so two groups.
+// TMEM per group: 64 working columns (D1, D2 / h2, dH1) + 2 x (80 + K1) private accumulators.  That is 256 at K1 = 16,
+// so two groups share the 512 columns; the wide variants (K1 = 32 .. 80) need 288 .. 384 and run one group per CTA.
 // The accumulators are read out and added into the group's fp32 slot of the workspace every FLUSH tiles (the tensor
 // core's adder truncates over long sums); ppo_reduce sums the slots in fp64 in a fixed order.
 namespace ppo {
-constexpr int GROUPS = 2, THREADS = GROUPS * 128, FLUSH = 16;
+constexpr int FLUSH = 16;
 constexpr int SBO_P = (HID / 8) * 128, P_BYTES = (TILE / 8) * SBO_P;      // dPre tiles [128 x 64] bf16
 constexpr int S_STRIDE = HID + 1, S_BYTES = (TILE * S_STRIDE * 4 + 127) / 128 * 128;   // g h2 stage, fp32
-constexpr int G_BYTES = A1_BYTES + A2_BYTES + 2 * P_BYTES + S_BYTES;
-constexpr int TOWER_OPS = B1_BYTES + B2_BYTES;                            // [W1 | b1] and [W2 | b2] of one tower
-constexpr int OFF_W = GROUPS * G_BYTES, OFF_W3 = OFF_W + 2 * TOWER_OPS;
-constexpr int SMEM_BYTES = OFF_W3 + 2 * (HID + 4) * 4 + 128;
 constexpr int TMEM_COLS = 512;
 constexpr int NSTATS = 5;                     // per-slot sums: pg, max(vf losses), (nlp - nlp_old)^2, clipped, dL/dlog_std
-static_assert(G_BYTES % 128 == 0 && OFF_W % 128 == 0 && TOWER_OPS % 128 == 0, "operand blocks are 128-byte aligned");
-static_assert(SMEM_BYTES <= 227 * 1024, "shared memory");
-static_assert(GROUPS * 256 <= TMEM_COLS, "tensor memory");
+constexpr int tmem_per_group(int k1) { return 64 + 2 * (K2 + k1); }
+constexpr int groups(int k1) { return tmem_per_group(k1) <= 256 ? 2 : 1; }
+template <int K1>
+struct Geo {
+    static constexpr int GROUPS = groups(K1), THREADS = GROUPS * 128;
+    static constexpr int SBO1 = pol::Geo<K1, true>::SBO1, A1_BYTES = pol::Geo<K1, true>::A1_BYTES, B1_BYTES = pol::Geo<K1, true>::B1_BYTES;
+    static constexpr int ACC_STRIDE = K2 + K1;                                // accumulator columns of one tower: [dW2 | db2 | 0], [dW1 | db1]
+    static constexpr int TMEM_STRIDE = TMEM_COLS / GROUPS;                    // TMEM columns of one group
+    static constexpr int G_BYTES = A1_BYTES + A2_BYTES + 2 * P_BYTES + S_BYTES;
+    static constexpr int TOWER_OPS = B1_BYTES + B2_BYTES;                     // [W1 | b1] and [W2 | b2] of one tower
+    static constexpr int OFF_W = GROUPS * G_BYTES, OFF_W3 = OFF_W + 2 * TOWER_OPS;
+    static constexpr int SMEM_BYTES = OFF_W3 + 2 * W3_BYTES + 128;
+    static_assert(G_BYTES % 128 == 0 && OFF_W % 128 == 0 && TOWER_OPS % 128 == 0, "operand blocks are 128-byte aligned");
+    static_assert(SMEM_BYTES <= SMEM_LIMIT, "shared memory");
+    static_assert(tmem_per_group(K1) <= TMEM_STRIDE, "tensor memory");
+};
+static_assert(Geo<16>::GROUPS == 2 && Geo<16>::TMEM_STRIDE == 256 && Geo<80>::GROUPS == 1, "group counts");
 }  // namespace ppo
 
 struct GradArgs {
@@ -687,11 +804,14 @@ struct GradArgs {
                  ::"r"(taddr), "r"(v[0]), "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7]), \
                    "r"(v[8]), "r"(v[9]), "r"(v[10]), "r"(v[11]), "r"(v[12]), "r"(v[13]), "r"(v[14]), "r"(v[15]) : "memory")
 
-template <int TANH>
-__global__ void __launch_bounds__(ppo::THREADS, 1) ppo_grad_kernel(const __grid_constant__ GradArgs a) {
-    constexpr int GROUPS = ppo::GROUPS, THREADS = ppo::THREADS, FLUSH = ppo::FLUSH, SBO_P = ppo::SBO_P, P_BYTES = ppo::P_BYTES;
-    constexpr int S_STRIDE = ppo::S_STRIDE, G_BYTES = ppo::G_BYTES, TOWER_OPS = ppo::TOWER_OPS, OFF_W = ppo::OFF_W;
-    constexpr int OFF_W3 = ppo::OFF_W3, TMEM_COLS = ppo::TMEM_COLS, NSTATS = ppo::NSTATS;
+template <int TANH, int K1 = 16>
+__global__ void __launch_bounds__(ppo::Geo<K1>::THREADS, 1) ppo_grad_kernel(const __grid_constant__ GradArgs a) {
+    using PG = ppo::Geo<K1>;
+    constexpr bool WIDE = K1 > 16;
+    constexpr int GROUPS = PG::GROUPS, THREADS = PG::THREADS, FLUSH = ppo::FLUSH, SBO_P = ppo::SBO_P, P_BYTES = ppo::P_BYTES;
+    constexpr int S_STRIDE = ppo::S_STRIDE, G_BYTES = PG::G_BYTES, TOWER_OPS = PG::TOWER_OPS, OFF_W = PG::OFF_W;
+    constexpr int OFF_W3 = PG::OFF_W3, TMEM_COLS = ppo::TMEM_COLS, NSTATS = ppo::NSTATS;
+    constexpr int SBO1 = PG::SBO1, A1_BYTES = PG::A1_BYTES, B1_BYTES = PG::B1_BYTES, ACC = PG::ACC_STRIDE;
     extern __shared__ __align__(128) unsigned char smem_raw[];
     __shared__ __align__(8) uint64_t mma_bar[GROUPS];
     __shared__ uint32_t tmem_slot;
@@ -741,7 +861,7 @@ __global__ void __launch_bounds__(ppo::THREADS, 1) ppo_grad_kernel(const __grid_
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem = tmem_slot;
-    const uint32_t twk = tmem + 256 * g;                  // working columns; accumulators of tower tw at + 64 + 96 tw
+    const uint32_t twk = tmem + PG::TMEM_STRIDE * g;      // working columns; accumulators of tower tw at + 64 + (80 + K1) tw
     const uint32_t tlane = (uint32_t)(wq * 32) << 16;
     constexpr uint32_t F32_BF16 = (1u << 4) | (1u << 7) | (1u << 10), A_MN = 1u << 15, B_MN = 1u << 16;
     const uint32_t idesc = F32_BF16 | ((uint32_t)(HID >> 3) << 17) | ((uint32_t)(TILE >> 4) << 24);
@@ -768,7 +888,12 @@ __global__ void __launch_bounds__(ppo::THREADS, 1) ppo_grad_kernel(const __grid_
     // forward of tower tw on the A1 tile: policy_kernel's finish_tower, plus h2 written back over D2 for the backward
     auto forward = [&](int tw) -> float {
         const uint64_t shift = (uint64_t)(tw * (TOWER_OPS >> 4));
-        if (issue_begin()) { mma_bf16(twk, a1d, b1d + shift, idesc, 0u); mma_commit(&mma_bar[g]); }
+        if (issue_begin()) {                                // policy_kernel's layer1: the same MMAs in the same K order
+#pragma unroll
+            for (int kk = 0; kk < K1 / 16; ++kk)
+                mma_bf16(twk, a1d + (uint64_t)(kk * 16), b1d + shift + (uint64_t)(kk * 16), idesc, kk ? 1u : 0u);
+            mma_commit(&mma_bar[g]);
+        }
         mma_wait();
 #pragma unroll
         for (int qt = 0; qt < 4; ++qt) {
@@ -850,7 +975,7 @@ __global__ void __launch_bounds__(ppo::THREADS, 1) ppo_grad_kernel(const __grid_
                 *reinterpret_cast<uint4 *>(prow + (2 * qt + c) * 128) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
             }
         }
-        const uint32_t acc_w2 = twk + 64 + 96 * tw, acc_w1 = acc_w2 + 80;
+        const uint32_t acc_w2 = twk + 64 + ACC * tw, acc_w1 = acc_w2 + K2;
         if (issue_begin()) {
             const uint64_t shift = (uint64_t)(tw * (TOWER_OPS >> 4));
 #pragma unroll
@@ -907,7 +1032,7 @@ __global__ void __launch_bounds__(ppo::THREADS, 1) ppo_grad_kernel(const __grid_
         for (int tw = 0; tw < 2; ++tw) {
             float *base = wsg + tw * a.tf;
             float *dw1 = base, *db1 = dw1 + HID * od, *dw2 = db1 + HID, *db2 = dw2 + HID * HID;
-            const uint32_t acc_w2 = twk + 64 + 96 * tw, acc_w1 = acc_w2 + 80;
+            const uint32_t acc_w2 = twk + 64 + ACC * tw, acc_w1 = acc_w2 + K2;
             for (int q = 0; q < K2 / 16; ++q) {
                 uint32_t v[16];
                 B2P_LD16(acc_w2 + tlane + 16 * q, v);
@@ -921,14 +1046,30 @@ __global__ void __launch_bounds__(ppo::THREADS, 1) ppo_grad_kernel(const __grid_
                     }
                 }
             }
-            uint32_t v[16];
-            B2P_LD16(acc_w1 + tlane, v);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            if (lane < 16) {
+            if constexpr (!WIDE) {
+                uint32_t v[16];
+                B2P_LD16(acc_w1 + tlane, v);
+                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                if (lane < 16) {
 #pragma unroll
-                for (int k = 0; k < K1 - 1; ++k)
-                    if (k < od) dw1[j * od + k] += __uint_as_float(v[k]);
-                db1[j] += __uint_as_float(v[K1 - 1]);
+                    for (int k = 0; k < K1 - 1; ++k)
+                        if (k < od) dw1[j * od + k] += __uint_as_float(v[k]);
+                    db1[j] += __uint_as_float(v[K1 - 1]);
+                }
+            } else {
+                for (int q = 0; q < K1 / 16; ++q) {
+                    uint32_t v[16];
+                    B2P_LD16(acc_w1 + tlane + 16 * q, v);
+                    asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                    if (lane < 16) {
+#pragma unroll
+                        for (int i = 0; i < 16; ++i) {
+                            const int k = 16 * q + i;
+                            if (k < od) dw1[j * od + k] += __uint_as_float(v[i]);
+                            else if (k == K1 - 1) db1[j] += __uint_as_float(v[i]);
+                        }
+                    }
+                }
             }
             S[gt] = dw3acc[tw];
             S[128 + gt] = db3acc[tw];
@@ -960,20 +1101,57 @@ __global__ void __launch_bounds__(ppo::THREADS, 1) ppo_grad_kernel(const __grid_
             r.act = r.nlp = r.val = r.ret = 0.f;
         }
     };
+    // wide rows (K1 > 16) are not held in registers a tile ahead: the next tile's sample index is, and its row and
+    // scalars are prefetched to L2 under this tile's work
+    auto locate = [&](long long tile) -> long long {       // -1 past the minibatch
+        const long long q = tile * TILE + gt;
+        if (q >= a.count) return -1;
+        const long long j = feistel_at(a.f, a.begin + q);
+        auto prefetch_l2 = [](const void *ptr) { asm volatile("prefetch.global.L2 [%0];" ::"l"(ptr)); };
+        const unsigned char *o = reinterpret_cast<const unsigned char *>(a.b.obs + j * (K1 / 8));
+        prefetch_l2(o);
+        prefetch_l2(o + 2 * K1 - 1);
+        prefetch_l2(a.b.act + j); prefetch_l2(a.b.nlp + j); prefetch_l2(a.b.val + j); prefetch_l2(a.b.ret + j);
+        return j;
+    };
     const long long step = (long long)gridDim.x * GROUPS;
     long long tile = (long long)blockIdx.x * GROUPS + g;
     Row nx;
-    if (tile < a.tiles) fetch(tile, nx);
+    long long nj = -1;
+    if (tile < a.tiles) {
+        if constexpr (WIDE) nj = locate(tile);
+        else fetch(tile, nx);
+    }
     for (int since = 0; tile < a.tiles; tile += step) {
-        const Row cur = nx;
-        {   // A1 = the stored bf16 row with the bias column 15 set to 1
+        const Row cur = [&]() -> Row {
+            if constexpr (WIDE) {                   // A1 = the stored bf16 row with the bias column K1 - 1 set to 1
+                Row r;
+                r.live = nj >= 0;
+                r.act = r.live ? __ldg(a.b.act + nj) : 0.f; r.nlp = r.live ? __ldg(a.b.nlp + nj) : 0.f;
+                r.val = r.live ? __ldg(a.b.val + nj) : 0.f; r.ret = r.live ? __ldg(a.b.ret + nj) : 0.f;
+                unsigned char *row = A1 + (gt >> 3) * SBO1 + (gt & 7) * 16;
+#pragma unroll
+                for (int c = 0; c < K1 / 8; ++c) {
+                    uint4 o = r.live ? __ldg(a.b.obs + nj * (K1 / 8) + c) : make_uint4(0u, 0u, 0u, 0u);
+                    if (c == K1 / 8 - 1 && r.live) o.w = (o.w & 0xFFFFu) | 0x3F800000u;
+                    *reinterpret_cast<uint4 *>(row + c * 128) = o;
+                }
+                return r;
+            } else {
+                return nx;
+            }
+        }();
+        if constexpr (!WIDE) {   // A1 = the stored bf16 row with the bias column 15 set to 1
             unsigned char *row = A1 + (gt >> 3) * SBO1 + (gt & 7) * 16;
             uint4 o1 = cur.o1;
             if (cur.live) o1.w = (o1.w & 0xFFFFu) | 0x3F800000u;
             *reinterpret_cast<uint4 *>(row) = cur.o0;
             *reinterpret_cast<uint4 *>(row + 128) = o1;
         }
-        if (tile + step < a.tiles) fetch(tile + step, nx);      // in flight under this tile's work
+        if (tile + step < a.tiles) {                        // in flight under this tile's work
+            if constexpr (WIDE) nj = locate(tile + step);
+            else fetch(tile + step, nx);
+        }
         // ---- action tower: dL/dmu of the clipped surrogate (TF gradient rules: max -> first operand on ties,
         // clip passes inside the closed interval)
         const float mu = forward(0);
@@ -1077,24 +1255,69 @@ struct PolicyDeviceGuard {
     ~PolicyDeviceGuard() { if (switched) cudaSetDevice(prev); }
 };
 
-template <int FRONT, bool STEP = false>
+// f(std::integral_constant<int, K1>()) with the first-layer K of a validated obs_dim (1 .. B2P_MAX_OBS_DIM): the kernels
+// are instantiated per K1, and the handle's obs_dim picks them
+template <class F>
+auto with_k1(int obs_dim, F &&f) {
+    switch (pol::obs_width(obs_dim)) {
+        case 32: return f(std::integral_constant<int, 32>());
+        case 48: return f(std::integral_constant<int, 48>());
+        case 64: return f(std::integral_constant<int, 64>());
+        case 80: return f(std::integral_constant<int, 80>());
+        default: return f(std::integral_constant<int, 16>());
+    }
+}
+
+template <int FRONT, bool STEP = false, int K1 = 16>
 cudaError_t launch_policy(int tanh_mode, int grid, cudaStream_t cs, const pol::Args &a, const Dev &d,
                           const pol::StepArgs &s = pol::StepArgs()) {
-    constexpr int smem = STEP ? pol::SMEM_STEP_BYTES : pol::SMEM_BYTES;
+    constexpr int smem = pol::Geo<K1, STEP>::SMEM_BYTES, threads = pol::Geo<K1, STEP>::THREADS;
     switch (tanh_mode) {
-        case 2: pol::policy_kernel<FRONT, 2, STEP><<<grid, pol::THREADS, smem, cs>>>(a, d, s); break;
-        case 1: pol::policy_kernel<FRONT, 1, STEP><<<grid, pol::THREADS, smem, cs>>>(a, d, s); break;
-        default: pol::policy_kernel<FRONT, 0, STEP><<<grid, pol::THREADS, smem, cs>>>(a, d, s); break;
+        case 2: pol::policy_kernel<FRONT, 2, STEP, K1><<<grid, threads, smem, cs>>>(a, d, s); break;
+        case 1: pol::policy_kernel<FRONT, 1, STEP, K1><<<grid, threads, smem, cs>>>(a, d, s); break;
+        default: pol::policy_kernel<FRONT, 0, STEP, K1><<<grid, threads, smem, cs>>>(a, d, s); break;
     }
     return cudaGetLastError();
 }
 
-template <int FRONT, bool STEP>
+// the ring front end: FRONT 1 (max_history 5, constant indices) exists only for the narrow row
+template <bool STEP, int K1>
+cudaError_t launch_ring(int H, int tanh_mode, int grid, cudaStream_t cs, const pol::Args &a, const Dev &d,
+                        const pol::StepArgs &s = pol::StepArgs()) {
+    if constexpr (K1 == 16) {
+        if (H == 5) return launch_policy<1, STEP>(tanh_mode, grid, cs, a, d, s);
+    }
+    return launch_policy<2, STEP, K1>(tanh_mode, grid, cs, a, d, s);
+}
+
+template <int FRONT, bool STEP, int K1 = 16>
 bool set_policy_smem() {
-    constexpr int smem = STEP ? pol::SMEM_STEP_BYTES : pol::SMEM_BYTES;
-    return cudaFuncSetAttribute(pol::policy_kernel<FRONT, 0, STEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess &&
-           cudaFuncSetAttribute(pol::policy_kernel<FRONT, 1, STEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess &&
-           cudaFuncSetAttribute(pol::policy_kernel<FRONT, 2, STEP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess;
+    constexpr int smem = pol::Geo<K1, STEP>::SMEM_BYTES;
+    return cudaFuncSetAttribute(pol::policy_kernel<FRONT, 0, STEP, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess &&
+           cudaFuncSetAttribute(pol::policy_kernel<FRONT, 1, STEP, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess &&
+           cudaFuncSetAttribute(pol::policy_kernel<FRONT, 2, STEP, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess;
+}
+
+template <int K1>
+bool set_smem_all() {
+    bool ok = set_policy_smem<0, false, K1>() && set_policy_smem<2, false, K1>() && set_policy_smem<0, true, K1>() &&
+              set_policy_smem<2, true, K1>();
+    if constexpr (K1 == 16) ok = ok && set_policy_smem<1, false>() && set_policy_smem<1, true>();
+    return ok;
+}
+
+template <int K1>
+bool set_ppo_smem() {
+    constexpr int smem = pol::ppo::Geo<K1>::SMEM_BYTES;
+    return cudaFuncSetAttribute(pol::ppo_grad_kernel<0, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess &&
+           cudaFuncSetAttribute(pol::ppo_grad_kernel<1, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess &&
+           cudaFuncSetAttribute(pol::ppo_grad_kernel<2, K1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem) == cudaSuccess;
+}
+
+// grid of a dense front-end launch: one CTA per GROUPS tiles, at most one per SM
+int dense_grid(const b2p_policy *h, long long tiles, int groups) {
+    const long long want = (tiles + groups - 1) / groups;
+    return (int)(want < h->num_sms ? want : h->num_sms);
 }
 
 void fill_weights(const b2p_policy *h, pol::Args &a) {
@@ -1121,7 +1344,7 @@ int copy_tower(b2p_handle h, float *w, const float *const (&src)[6], cudaStream_
 }
 
 // the ring front end's split of the env's tiles over the CTAs (b2p_act_env, b2p_step_env); NULL + error on a bad env
-const Dev *ring_setup(b2p_handle h, b2e_handle env, pol::Args &a, int &grid, const char *who) {
+const Dev *ring_setup(b2p_handle h, b2e_handle env, pol::Args &a, int &grid, int groups, const char *who) {
     int ring_ok = 0, device = -1;
     const Dev *dv = static_cast<const Dev *>(b2e_dev_view(env, &ring_ok, &device));
     const std::string w(who);
@@ -1133,7 +1356,7 @@ const Dev *ring_setup(b2p_handle h, b2e_handle env, pol::Args &a, int &grid, con
     a.tiles = (long long)dv->E * tiles_per_env;
     // few envs: split every env's tiles into segments so that all SMs have work (>= 4 rounds of tiles per group and segment)
     int segs = (3 * h->num_sms + dv->E - 1) / dv->E;
-    const int max_segs = tiles_per_env / (4 * pol::GROUPS);
+    const int max_segs = tiles_per_env / (4 * groups);
     segs = segs > max_segs ? max_segs : segs;
     a.segs = segs < 1 ? 1 : segs;
     a.units = dv->E * a.segs;
@@ -1202,21 +1425,21 @@ extern "C" {
 
 const char *b2p_last_error(b2p_handle h) { return h ? h->error.c_str() : g_policy_create_error.c_str(); }
 
+int b2p_obs_width(int obs_dim) { return obs_dim >= 1 && obs_dim <= B2P_MAX_OBS_DIM ? pol::obs_width(obs_dim) : 0; }
+
 int b2p_create(int device, int obs_dim, int tanh_mode, b2p_handle *out) {
     if (!out) return pfail(nullptr, "b2p_create: null output pointer");
     *out = nullptr;
-    if (obs_dim < 1 || obs_dim > B2P_MAX_OBS_DIM) return pfail(nullptr, "b2p_create: obs_dim must be 1..15");
+    if (obs_dim < 1 || obs_dim > B2P_MAX_OBS_DIM)
+        return pfail(nullptr, "b2p_create: obs_dim must be 1..79 (3 x max_history up to max_history 26)");
     if (tanh_mode < 0 || tanh_mode > 2) return pfail(nullptr, "b2p_create: unknown tanh_mode");
     PolicyDeviceGuard guard(device);
     cudaDeviceProp prop;
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) return pfail(nullptr, "b2p_create: no such CUDA device");
     if (prop.major != 10) return pfail(nullptr, "b2p_create: the policy kernel needs an sm_100 GPU (tcgen05); there is no fallback");
-    if (!(set_policy_smem<0, false>() && set_policy_smem<1, false>() && set_policy_smem<2, false>() &&
-          set_policy_smem<0, true>() && set_policy_smem<1, true>() && set_policy_smem<2, true>()))
+    if (!with_k1(obs_dim, [](auto k) { return set_smem_all<decltype(k)::value>(); }))
         return pfail(nullptr, "b2p_create: the policy kernel does not fit shared memory");
-    if (cudaFuncSetAttribute(pol::ppo_grad_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::ppo::SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(pol::ppo_grad_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::ppo::SMEM_BYTES) != cudaSuccess ||
-        cudaFuncSetAttribute(pol::ppo_grad_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, pol::ppo::SMEM_BYTES) != cudaSuccess)
+    if (!with_k1(obs_dim, [](auto k) { return set_ppo_smem<decltype(k)::value>(); }))
         return pfail(nullptr, "b2p_create: the PPO gradient kernel does not fit shared memory");
     b2p_policy *h = new (std::nothrow) b2p_policy();
     if (!h) return pfail(nullptr, "b2p_create: out of host memory");
@@ -1281,9 +1504,11 @@ int b2p_act(b2p_handle h, const float *obs, int64_t rows, float *actions_out, fl
     a.bulk_ok = (reinterpret_cast<uintptr_t>(obs) & 15u) == 0 ? 1 : 0;
     Dev d;
     memset(&d, 0, sizeof(d));
-    const long long want = (a.tiles + pol::GROUPS - 1) / pol::GROUPS;
-    const int grid = (int)(want < h->num_sms ? want : h->num_sms);
-    const cudaError_t err = launch_policy<0>(h->tanh_mode, grid, (cudaStream_t)stream, a, d);
+    const cudaError_t err = with_k1(h->obs_dim, [&](auto k) {
+        constexpr int K1 = decltype(k)::value;
+        const int grid = dense_grid(h, a.tiles, pol::Geo<K1, false>::GROUPS);
+        return launch_policy<0, false, K1>(h->tanh_mode, grid, (cudaStream_t)stream, a, d);
+    });
     if (err != cudaSuccess) return pfail(h, std::string("b2p_act: ") + cudaGetErrorString(err));
     return 0;
 }
@@ -1296,15 +1521,17 @@ int b2p_act_env(b2p_handle h, b2e_handle env, float *actions_out, float noise_st
     pol::Args a;
     memset(&a, 0, sizeof(a));
     int grid = 0;
-    const Dev *dv = ring_setup(h, env, a, grid, "b2p_act_env");
+    const int groups = with_k1(h->obs_dim, [](auto k) { return pol::Geo<decltype(k)::value, false>::GROUPS; });
+    const Dev *dv = ring_setup(h, env, a, grid, groups, "b2p_act_env");
     if (!dv) return 1;
     PolicyDeviceGuard guard(h->device);
     fill_weights(h, a);
     a.out = actions_out;
     a.seed_counter = h->seed_counter;
     a.seed = seed; a.noise_std = noise_std; a.low = low; a.high = high;
-    const cudaError_t err = dv->H == 5 ? launch_policy<1>(h->tanh_mode, grid, (cudaStream_t)stream, a, *dv)
-                                      : launch_policy<2>(h->tanh_mode, grid, (cudaStream_t)stream, a, *dv);
+    const cudaError_t err = with_k1(h->obs_dim, [&](auto k) {
+        return launch_ring<false, decltype(k)::value>(dv->H, h->tanh_mode, grid, (cudaStream_t)stream, a, *dv);
+    });
     if (err != cudaSuccess) return pfail(h, std::string("b2p_act_env: ") + cudaGetErrorString(err));
     return 0;
 }
@@ -1322,9 +1549,11 @@ int b2p_step(b2p_handle h, const float *obs, int64_t rows, const b2p_step_out *o
     a.bulk_ok = (reinterpret_cast<uintptr_t>(obs) & 15u) == 0 ? 1 : 0;
     Dev d;
     memset(&d, 0, sizeof(d));
-    const long long want = (a.tiles + pol::GROUPS - 1) / pol::GROUPS;
-    const int grid = (int)(want < h->num_sms ? want : h->num_sms);
-    const cudaError_t err = launch_policy<0, true>(h->tanh_mode, grid, (cudaStream_t)stream, a, d, s);
+    const cudaError_t err = with_k1(h->obs_dim, [&](auto k) {
+        constexpr int K1 = decltype(k)::value;
+        const int grid = dense_grid(h, a.tiles, pol::Geo<K1, true>::GROUPS);
+        return launch_policy<0, true, K1>(h->tanh_mode, grid, (cudaStream_t)stream, a, d, s);
+    });
     if (err != cudaSuccess) return pfail(h, std::string("b2p_step: ") + cudaGetErrorString(err));
     return 0;
 }
@@ -1337,11 +1566,13 @@ int b2p_step_env(b2p_handle h, b2e_handle env, const b2p_step_out *out, float no
     pol::StepArgs s;
     if (step_setup(h, out, noise_std, log_std, seed, low, high, a, s, "b2p_step_env")) return 1;
     int grid = 0;
-    const Dev *dv = ring_setup(h, env, a, grid, "b2p_step_env");
+    const int groups = with_k1(h->obs_dim, [](auto k) { return pol::Geo<decltype(k)::value, true>::GROUPS; });
+    const Dev *dv = ring_setup(h, env, a, grid, groups, "b2p_step_env");
     if (!dv) return 1;
     PolicyDeviceGuard guard(h->device);
-    const cudaError_t err = dv->H == 5 ? launch_policy<1, true>(h->tanh_mode, grid, (cudaStream_t)stream, a, *dv, s)
-                                      : launch_policy<2, true>(h->tanh_mode, grid, (cudaStream_t)stream, a, *dv, s);
+    const cudaError_t err = with_k1(h->obs_dim, [&](auto k) {
+        return launch_ring<true, decltype(k)::value>(dv->H, h->tanh_mode, grid, (cudaStream_t)stream, a, *dv, s);
+    });
     if (err != cudaSuccess) return pfail(h, std::string("b2p_step_env: ") + cudaGetErrorString(err));
     return 0;
 }
@@ -1424,7 +1655,7 @@ int b2p_ppo_adv_stats(const b2p_ppo_batch *b, uint64_t key, int64_t mb_size, dou
 
 size_t b2p_ppo_workspace_size(b2p_handle h) {
     if (!h) return 0;
-    const size_t slots = (size_t)h->num_sms * pol::ppo::GROUPS;
+    const size_t slots = (size_t)h->num_sms * pol::ppo::groups(pol::obs_width(h->obs_dim));
     return slots * (grad_stride(h->obs_dim) * sizeof(float) + pol::ppo::NSTATS * sizeof(double)) + 256;
 }
 
@@ -1454,17 +1685,21 @@ int b2p_ppo_grad(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, 
     a.inv_sigma = (float)exp(-(double)p->log_std);
     a.nlp_const = (float)(0.91893853320467274178 + (double)p->log_std);      // as b2p_step: 0.5 log(2 pi) + log_std
     a.od = h->obs_dim; a.tf = (int)tower_floats(h->obs_dim); a.stride = (int)grad_stride(h->obs_dim);
-    const long long want = (a.tiles + pol::ppo::GROUPS - 1) / pol::ppo::GROUPS;
-    const int grid = (int)(want < h->num_sms ? want : h->num_sms), slots = grid * pol::ppo::GROUPS;
+    const int groups = pol::ppo::groups(pol::obs_width(h->obs_dim));
+    const int grid = dense_grid(h, a.tiles, groups), slots = grid * groups;
     const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
     a.ws_grad = reinterpret_cast<float *>(base);
     a.ws_stats = reinterpret_cast<double *>(base + (((size_t)slots * a.stride * sizeof(float) + 7) & ~(size_t)7));
     cudaStream_t cs = (cudaStream_t)stream;
-    switch (h->tanh_mode) {
-        case 2: pol::ppo_grad_kernel<2><<<grid, pol::ppo::THREADS, pol::ppo::SMEM_BYTES, cs>>>(a); break;
-        case 1: pol::ppo_grad_kernel<1><<<grid, pol::ppo::THREADS, pol::ppo::SMEM_BYTES, cs>>>(a); break;
-        default: pol::ppo_grad_kernel<0><<<grid, pol::ppo::THREADS, pol::ppo::SMEM_BYTES, cs>>>(a); break;
-    }
+    with_k1(h->obs_dim, [&](auto k) {
+        using PG = pol::ppo::Geo<decltype(k)::value>;
+        switch (h->tanh_mode) {
+            case 2: pol::ppo_grad_kernel<2, decltype(k)::value><<<grid, PG::THREADS, PG::SMEM_BYTES, cs>>>(a); break;
+            case 1: pol::ppo_grad_kernel<1, decltype(k)::value><<<grid, PG::THREADS, PG::SMEM_BYTES, cs>>>(a); break;
+            default: pol::ppo_grad_kernel<0, decltype(k)::value><<<grid, PG::THREADS, PG::SMEM_BYTES, cs>>>(a); break;
+        }
+        return 0;
+    });
     pol::ppo_reduce_kernel<<<(a.stride + 255) / 256, 256, 0, cs>>>(a.ws_grad, a.ws_stats, slots, a.stride, 1.0 / (double)p->count,
                                                                    (double)p->log_std, (double)p->ent_coef, (double)p->vf_coef,
                                                                    grad_out, stats_out);

@@ -45,6 +45,7 @@ class DevicePolicy:
         if self.lib.b2p_create(self.device.index or 0, self.obs_dim, int(tanh_mode), ctypes.byref(handle)):
             raise _lib.B200EnvError(self.lib.b2p_last_error(None).decode())
         self.handle = handle
+        self.obs_width = obs_width(self.obs_dim)
 
     @classmethod
     def from_torch(cls, tower, obs_dim=None, **kwargs):
@@ -141,7 +142,7 @@ class DevicePolicy:
             assert t is None or (t.dtype == torch.float32 and t.is_contiguous() and t.numel() == rows
                                  and t.device == self.device)
         if obs_bf16 is not None:
-            assert obs_bf16.dtype == torch.bfloat16 and obs_bf16.is_contiguous() and obs_bf16.numel() == rows * 16
+            assert obs_bf16.dtype == torch.bfloat16 and obs_bf16.is_contiguous() and obs_bf16.numel() == rows * self.obs_width
         if neglogp is not None and self.log_std is None:
             raise ValueError('neglogp needs a stochastic policy (log_std)')
         out = _lib.StepOut(*[t.data_ptr() if t is not None else None
@@ -163,8 +164,8 @@ class DevicePolicy:
         ``BatchedOptEnv`` whose rings are read, VecEnv row order) -> (actions, actions_raw, values, neglogp,
         obs_bf16), each [rows] float32: the clipped action the env steps with (bit for bit ``act`` /
         ``act_env`` with the same seed), the unclipped one PPO stores, the value tower's output (None
-        without one) and -log p(actions_raw).  ``obs_bf16``: a bf16 [rows, 16] tensor to receive the
-        observation rows as the network read them (columns obs_dim..15 zero), or None."""
+        without one) and -log p(actions_raw).  ``obs_bf16``: a bf16 [rows, obs_width] tensor to receive the
+        observation rows as the network read them (columns obs_dim..obs_width-1 zero), or None."""
         if self.log_std is None:
             raise ValueError('step samples from the Gaussian policy: construct it with a log_std')
         new = lambda: torch.empty(self._rows(source), dtype=torch.float32, device=self.device)   # noqa: E731
@@ -197,6 +198,7 @@ class DevicePolicy:
             stats = torch.empty(6, dtype=torch.float64, device=self.device)
         assert grad.dtype == torch.float32 and grad.numel() == 2 * tower + 1 and grad.is_contiguous()
         assert stats.dtype == torch.float64 and stats.numel() == 6 and adv_stats.dtype == torch.float64
+        assert buffer.obs_bf16.shape[-1] == self.obs_width, 'the buffer\'s rows are not this policy\'s obs_width wide'
         if getattr(self, '_ppo_ws', None) is None:
             self._ppo_ws = torch.empty(self.lib.b2p_ppo_workspace_size(self.handle), dtype=torch.uint8, device=self.device)
         params = _lib.PpoParams(float(cliprange), float(cliprange if cliprange_vf is None else cliprange_vf),
@@ -218,6 +220,16 @@ class DevicePolicy:
             self.close()
         except Exception:      # noqa: BLE001 (interpreter shutdown)
             pass
+
+
+def obs_width(obs_dim):
+    """W, the bf16 columns of a stored observation row for ``obs_dim`` (b2p_obs_width): 16 up to obs_dim 15, then 32,
+    48, 64 and 80 (obs_dim 64..79).  Columns obs_dim..W-1 are zero; the last is the bias slot.  Raises outside the
+    supported 1..79."""
+    width = _lib.load().b2p_obs_width(int(obs_dim))
+    if not width:
+        raise _lib.B200EnvError('obs_dim %d is outside the policy kernels\' 1..79' % obs_dim)
+    return width
 
 
 def _tower_linears(tower):
@@ -320,8 +332,8 @@ def gae(values, rewards, dones, rows_per_env, gamma=0.99, lam=0.95, advantages=N
 class DeviceRolloutBuffer:
     """PPO rollout storage of ``n_steps`` steps of every agent row of ``env``, on its device, allocated once.
 
-    Time-major: ``obs_bf16`` [T, rows, 16] bf16 (the observation rows as the policy read them, columns
-    obs_dim..15 zero), ``actions_raw`` / ``neglogp`` / ``advantages`` / ``returns`` [T, rows] float32,
+    Time-major: ``obs_bf16`` [T, rows, W] bf16 (the observation rows as the policy read them, W = ``obs_width(obs_dim)``,
+    columns obs_dim..W-1 zero), ``actions_raw`` / ``neglogp`` / ``advantages`` / ``returns`` [T, rows] float32,
     ``values`` [T+1, rows] float32 (``values[T]`` = value of the observation after the last step),
     ``rewards`` [T, E] float32 and ``dones`` [T+1, E] uint8 (per env; env = row // P; ``dones[0]`` = the
     flags at the rollout's first observation, ``dones[t+1]`` = done of step t).  stable-baselines'
@@ -330,11 +342,11 @@ class DeviceRolloutBuffer:
 
     ``actions`` [rows] float32 holds the clipped actions of the current step (what the env steps with).
 
-    Memory: 52 bytes per agent row and step (32 observation + 5 x 4), plus 8 bytes per agent row (the last
-    value slot and ``actions``), e.g. 10.8 GB per step for the 2.08e8 rows of 4096 envs of MLP 784-64-10
-    (88 GB for n_steps = 8); the constructor checks it against the device's free memory."""
-
-    BYTES_PER_ROW_STEP = 32 + 5 * 4
+    Memory: 2W + 20 bytes per agent row and step (the observation row + 5 x 4), plus 8 bytes per agent row (the
+    last value slot and ``actions``).  That is 52 B at W = 16, e.g. 10.8 GB per step for the 2.08e8 rows of 4096
+    envs of MLP 784-64-10 (88 GB for n_steps = 8), and 180 B at max_history 25 (W = 80: 37.5 GB per step, so
+    n_steps = 2 fits a 180 GB card beside the env's rings and 8 does not); the constructor checks it against the
+    device's free memory."""
 
     def __init__(self, env, n_steps):
         self.n_steps = T = int(n_steps)
@@ -342,14 +354,16 @@ class DeviceRolloutBuffer:
             raise ValueError('n_steps must be >= 1')
         rows, E, dev = env.num_rows, env.num_envs, env.device
         self.rows_per_env = env.num_params
-        need = rows * (self.BYTES_PER_ROW_STEP * T + 8) + E * (5 * T + 1)
+        self.obs_width = W = obs_width(env.obs_dim)
+        self.bytes_per_row_step = 2 * W + 5 * 4
+        need = rows * (self.bytes_per_row_step * T + 8) + E * (5 * T + 1)
         free, _ = torch.cuda.mem_get_info(dev)
         if need > free:
             raise MemoryError('DeviceRolloutBuffer: n_steps = %d needs %.2f GB (%d rows x %d B per step) but %s has '
-                              '%.2f GB free; use fewer steps per rollout' % (T, need / 1e9, rows, self.BYTES_PER_ROW_STEP,
+                              '%.2f GB free; use fewer steps per rollout' % (T, need / 1e9, rows, self.bytes_per_row_step,
                                                                             dev, free / 1e9))
         f32 = dict(dtype=torch.float32, device=dev)
-        self.obs_bf16 = torch.empty((T, rows, 16), dtype=torch.bfloat16, device=dev)
+        self.obs_bf16 = torch.empty((T, rows, W), dtype=torch.bfloat16, device=dev)
         self.actions_raw = torch.empty((T, rows), **f32)
         self.values = torch.empty((T + 1, rows), **f32)
         self.neglogp = torch.empty((T, rows), **f32)

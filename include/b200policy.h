@@ -37,7 +37,7 @@ extern "C" {
 #endif
 
 #define B2P_HIDDEN 64            /* units of both hidden layers (stable-baselines MlpPolicy) */
-#define B2P_MAX_OBS_DIM 15       /* 3H with H <= 5 (envs/multioptlrs.py:39, utils/utils_env.py:32-36) */
+#define B2P_MAX_OBS_DIM 79       /* 3H with H <= 26 (MultiOptLRs; the reference's max_history search space is 5..25) */
 
 /* tanh_mode */
 #define B2P_TANH_F32    0        /* tanh.approx.f32 on the fp32 accumulators (default)                      */
@@ -45,7 +45,14 @@ extern "C" {
 
 typedef struct b2p_policy *b2p_handle;
 
+/* obs_dim 1..B2P_MAX_OBS_DIM; anything else is rejected. */
 int b2p_create(int device, int obs_dim, int tanh_mode, b2p_handle *out);
+
+/* W, the bf16 columns of a stored observation row (b2p_step_out.obs_bf16, b2p_ppo_batch.obs_bf16) for obs_dim:
+ * 16 * ceil((obs_dim + 1) / 16), i.e. 16 for obs_dim 1..15, 32 for 16..31, 48 for 32..47, 64 for 48..63 and 80 for
+ * 64..79.  Columns obs_dim..W-1 are stored as zero; column W-1 is the bias slot the kernels set to 1 when they read
+ * the row.  0 outside 1..B2P_MAX_OBS_DIM.  Needs no device. */
+int b2p_obs_width(int obs_dim);
 void b2p_destroy(b2p_handle h);
 const char *b2p_last_error(b2p_handle h);
 
@@ -89,8 +96,8 @@ int b2p_set_value_weights(b2p_handle h, const float *w1, const float *b1, const 
  *   actions_raw  raw = mean + noise_std * z, z = the row's N(0, 1) draw (PPO stores and scores this)
  *   values       the value tower's output (model.value)
  *   neglogp      0.5 z^2 + 0.5 log(2 pi) + log_std: -log density of raw under the diagonal Gaussian
- *   obs_bf16     [rows][16] bf16, 16-byte aligned: the observation row the first layer read, already
- *                rounded to bf16, columns obs_dim..15 zero (32 bytes per row)
+ *   obs_bf16     [rows][W] bf16, W = b2p_obs_width(obs_dim), 16-byte aligned: the observation row the first
+ *                layer read, already rounded to bf16, columns obs_dim..W-1 zero (2W bytes per row)
  * The action tower runs only for actions / actions_raw / neglogp, the value tower only for values
  * (values alone = model.value).  values needs b2p_set_value_weights; an all-NULL set is an error. */
 typedef struct b2p_step_out {
@@ -129,7 +136,8 @@ int b2p_gae(const float *values, const float *rewards, const uint8_t *dones, int
 #define B2P_PPO_MAX_SAMPLES (1LL << 62)
 
 typedef struct b2p_ppo_batch {          /* a DeviceRolloutBuffer, time-major */
-    const void *obs_bf16;               /* [T][rows][16] bf16, 16-byte aligned (column 15 is not read: the bias 1) */
+    const void *obs_bf16;               /* [T][rows][W] bf16, W = b2p_obs_width(obs_dim), 16-byte aligned (column W-1
+                                           is not read: the bias 1) */
     const float *actions_raw, *neglogp, *values, *returns;   /* [T][rows] (values: first T rows of [T+1][rows]) */
     int T;
     int64_t rows;
