@@ -30,7 +30,9 @@ EXPORTS = (
     # shared per-agent policy (include/b200policy.h)
     'b2p_create', 'b2p_destroy', 'b2p_last_error', 'b2p_set_weights', 'b2p_act', 'b2p_act_env', 'b2p_set_seed_counter',
     'b2p_set_value_weights', 'b2p_step', 'b2p_step_env', 'b2p_gae',
-    'b2p_obs_width', 'b2p_tanh_table', 'b2p_ppo_indices', 'b2p_ppo_adv_stats_workspace_size', 'b2p_ppo_adv_stats', 'b2p_ppo_workspace_size', 'b2p_ppo_grad')
+    'b2p_obs_width', 'b2p_tanh_table', 'b2p_ppo_indices', 'b2p_ppo_adv_stats_workspace_size', 'b2p_ppo_adv_stats', 'b2p_ppo_workspace_size', 'b2p_ppo_grad',
+    'b2p_set_row_base', 'b2p_ppo_partial_size', 'b2p_ppo_grad_partial', 'b2p_ppo_combine', 'b2p_ppo_adv_moments',
+    'b2p_ppo_adv_combine')
 DTYPE_U8, DTYPE_I32, DTYPE_F32, DTYPE_F64 = range(4)
 
 
@@ -39,7 +41,7 @@ class Config(ctypes.Structure):
         'struct_size', 'device', 'env_kind', 'problem_kind', 'num_features', 'num_hidden',
         'num_outputs', 'num_rows', 'batch_size', 'num_envs', 'max_batches', 'max_history',
         'history_version', 'observation_version', 'action_version', 'reward_version',
-        'row_order', 'index_mode', 'auto_reset', 'reserved')] + [
+        'row_order', 'index_mode', 'auto_reset', 'env_base')] + [
         ('hidden_more', ctypes.c_int32 * MAX_LAYERS), ('init_seed', ctypes.c_uint64)]
 
 
@@ -137,6 +139,13 @@ def load():
     lib.b2p_ppo_workspace_size.argtypes = [vp]
     lib.b2p_ppo_workspace_size.restype = usize
     lib.b2p_ppo_grad.argtypes = [vp, ctypes.POINTER(PpoBatch), ctypes.POINTER(PpoParams), vp, vp, vp, vp]
+    lib.b2p_set_row_base.argtypes = [vp, i64]
+    lib.b2p_ppo_partial_size.argtypes = [vp]
+    lib.b2p_ppo_partial_size.restype = usize
+    lib.b2p_ppo_grad_partial.argtypes = [vp, ctypes.POINTER(PpoBatch), ctypes.POINTER(PpoParams), i64, vp, vp, vp]
+    lib.b2p_ppo_combine.argtypes = [vp, vp, i32, i64, f32, f32, f32, vp, vp, vp]
+    lib.b2p_ppo_adv_moments.argtypes = [ctypes.POINTER(PpoBatch), u64, i64, vp, vp, vp]
+    lib.b2p_ppo_adv_combine.argtypes = [vp, i32, i64, vp, vp]
     if lib.b2e_abi_version() != 2:
         raise B200EnvError('libb200env.so ABI version mismatch')
     _lib = lib

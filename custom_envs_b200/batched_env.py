@@ -105,10 +105,16 @@ class BatchedOptEnv:
                  history_version=3, observation_version=3, action_version=0, reward_version=6,
                  row_order='lexicographic', index_mode='internal', auto_reset=True,
                  seeds=None, perms=None, init_orders=None, device='cuda:0', init_seed=0,
-                 materialize_obs=True):
+                 materialize_obs=True, env_base=0):
         """``materialize_obs=False``: no [E*P, obs_dim] observation matrix is allocated (12.5 GB at
         BASELINE config 4); every step is then ring-only and the consumer reads the adjusted-history
-        rings in place (``custom_envs_b200.vectorize.device_policy.DevicePolicy.act_env``)."""
+        rings in place (``custom_envs_b200.vectorize.device_policy.DevicePolicy.act_env``).
+
+        ``env_base``: the global index of this batch's env 0, when it is the shard
+        ``[env_base, env_base + num_envs)`` of a larger batch (``sharding.shard_bases``).  The on-device Glorot
+        initialiser and the default ``seeds`` then follow the global index, so the shard's envs start and
+        auto-reset exactly as they do inside the whole batch; pass that batch's ``init_seed`` and the shard's
+        slice of its ``seeds``."""
         self.lib = _lib.load()
         if not torch.cuda.is_available():
             raise _lib.B200EnvError('BatchedOptEnv needs a CUDA device (no CPU fallback)')
@@ -145,6 +151,7 @@ class BatchedOptEnv:
         cfg.index_mode = _lib.INDEX_INTERNAL if index_mode == 'internal' else _lib.INDEX_EXTERNAL
         cfg.auto_reset = int(bool(auto_reset))
         cfg.init_seed = int(init_seed)
+        self.env_base = cfg.env_base = int(env_base)
         self.max_batches, self.max_history = int(max_batches), int(max_history)
         handle = ctypes.c_void_p()
         with torch.cuda.device(self.device):
@@ -174,7 +181,7 @@ class BatchedOptEnv:
             self._check(self.lib.b2e_bind_dataset(handle, _ptr(features), _ptr(targets), self._stream()))
             if index_mode == 'internal':
                 if perms is None:                    # the epoch permutation of every env, generated on the device
-                    seeds = range(self.num_envs) if seeds is None else seeds
+                    seeds = range(self.env_base, self.env_base + self.num_envs) if seeds is None else seeds
                     perms = env_permutations_device(num_rows, list(seeds), dev)
                 if torch.is_tensor(perms):
                     perms = perms.to(dev, torch.int32).contiguous()

@@ -883,9 +883,9 @@ __device__ void reset_env(const Dev &d, const StepArgs &a, float *sm, int e) {
         if (p < d.P) {
             if (a.init_params) v = a.init_params[(size_t)e * d.P + p];
             else if (d.kind == B2E_PROBLEM_FUNC) v = p == 0 ? -1.9f : 2.0f;   // optimize_function.py:37
-            else if (p < d.P1) v = glorot(d.seed, e, episode, p, d.lim1);
+            else if (p < d.P1) v = glorot(d.seed, e + d.env_base, episode, p, d.lim1);
             else if (d.hidden && p >= d.P1 + d.N1 && p < d.P1 + d.N1 + d.N1 * d.C)
-                v = glorot(d.seed, e, episode, p, d.lim2);
+                v = glorot(d.seed, e + d.env_base, episode, p, d.lim2);
         }
         if (d.w2) d.w2[(size_t)e * d.Pp + p] = cx.wE[p];         // raw History keeps the older weights
         cx.wE[p] = v;
@@ -2803,8 +2803,8 @@ __global__ void __launch_bounds__(256) reset_prepare_kernel(const __grid_constan
             float v = 0.f;
             if (p < d.P) {
                 if (a.init_params) v = a.init_params[(size_t)e * d.P + p];
-                else if (p < d.P1) v = glorot(d.seed, e, episode, p, d.lim1);
-                else if (d.hidden && p >= d.P1 + d.N1 && p < d.P1 + d.N1 + d.N1 * d.C) v = glorot(d.seed, e, episode, p, d.lim2);
+                else if (p < d.P1) v = glorot(d.seed, e + d.env_base, episode, p, d.lim1);
+                else if (d.hidden && p >= d.P1 + d.N1 && p < d.P1 + d.N1 + d.N1 * d.C) v = glorot(d.seed, e + d.env_base, episode, p, d.lim2);
             }
             wE[p] = v;
         }
@@ -3121,7 +3121,7 @@ __global__ void __launch_bounds__(256, 2) gen_eval_kernel(const __grid_constant_
                 for (int p = lo + tid; p < hi; p += nt) {
                     float v = 0.f;
                     if (a.init_params) v = a.init_params[(size_t)e * d.P + p];
-                    else if (p < d.boff[l]) v = glorot(d.seed, e, episode, p, limit);
+                    else if (p < d.boff[l]) v = glorot(d.seed, e + d.env_base, episode, p, limit);
                     if (d.w2) d.w2[(size_t)e * d.Pp + p] = wE[p];
                     wE[p] = v;
                 }
@@ -3517,7 +3517,7 @@ int configure(b2e_handle h) {
     d.E = c.num_envs; d.H = c.max_history; d.max_batches = c.max_batches;
     d.act_ver = c.action_version; d.rew_ver = c.reward_version; d.obs_ver = c.observation_version;
     d.row_lex = c.row_order == B2E_ROWS_LEXICOGRAPHIC;
-    d.index_mode = c.index_mode; d.auto_reset = c.auto_reset; d.seed = c.init_seed;
+    d.index_mode = c.index_mode; d.auto_reset = c.auto_reset; d.seed = c.init_seed; d.env_base = c.env_base;
     if (d.kind == B2E_PROBLEM_FUNC) {
         d.D = 0; d.N1 = 8; d.C = 0; d.N = 0; d.B = 1; d.P1 = 0; d.tailP = 2; d.P = 2;
     } else {
@@ -3834,6 +3834,8 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
         return fail(nullptr, "b2e_create: bad problem shape");
     if (cfg->problem_kind == B2E_PROBLEM_LINREG && cfg->num_hidden != 0)
         return fail(nullptr, "b2e_create: linreg has no hidden layer");
+    if (cfg->env_base < 0 || cfg->env_base > 0x7FFFFFFF - cfg->num_envs)
+        return fail(nullptr, "b2e_create: env_base must be 0..2^31-1-num_envs");
     if (cfg->auto_reset && cfg->index_mode == B2E_INDEX_EXTERNAL && cfg->problem_kind != B2E_PROBLEM_FUNC)
         return fail(nullptr, "b2e_create: auto_reset needs the internal index stream");
     b2e_handle h = new (std::nothrow) b2e_env();

@@ -36,6 +36,7 @@ struct Dev {
     int nsc, ncc, nks, fitems;
     int N1g, KR, gcc;
     int row_lex, index_mode, auto_reset;
+    int env_base;                    // global index of env 0 of this handle (b2e_config.env_base): the Glorot initialiser's env
     unsigned long long seed;
     float lim1, lim2;
     const float *X;

@@ -171,7 +171,9 @@ __device__ __forceinline__ uint32_t pack_bf16x2(float lo, float hi) {
 }
 __device__ __forceinline__ unsigned short bf16_bits(float v) { return (unsigned short)(pack_bf16x2(v, 0.f) & 0xFFFFu); }
 
-// N(0, 1) of an agent row: counter-based (splitmix64 of seed and row), Box-Muller
+// N(0, 1) of an agent row: counter-based (splitmix64 of seed and row), Box-Muller.  The row enters as seed + GOLDEN (row + 1),
+// so row_noise(seed, base + row) == row_noise(seed + GOLDEN base, row): b2p_set_row_base's global row offset is folded into
+// the seed on the host (row_seed) and the kernels see only local rows.
 __device__ __forceinline__ float row_noise(unsigned long long seed, long long row) {
     unsigned long long z = seed + 0x9E3779B97F4A7C15ull * (unsigned long long)(row + 1);
     z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
@@ -735,14 +737,37 @@ __global__ void __launch_bounds__(ADV_THREADS) ppo_adv_partial(const PpoBatch b,
     }
     if (threadIdx.x == 0) { part[2 * blockIdx.x] = s1[0]; part[2 * blockIdx.x + 1] = s2[0]; }
 }
-__global__ void ppo_adv_final(const PpoBatch b, const Feistel f, long long mb, long long nmb, int slices,
-                              const double *__restrict__ part, double *__restrict__ stats) {
+// moments[m] = {count, K, sum(A - K), sum((A - K)^2)} of minibatch m: its slices summed in order (b2p_ppo_adv_moments)
+__global__ void ppo_adv_moments_kernel(const PpoBatch b, const Feistel f, long long mb, long long nmb, int slices,
+                                       const double *__restrict__ part, double *__restrict__ moments) {
     const long long m = (long long)blockIdx.x * blockDim.x + threadIdx.x;
     if (m >= nmb) return;
     double a1 = 0.0, a2 = 0.0;
     for (int c = 0; c < slices; ++c) { a1 += part[2 * (m * slices + c)]; a2 += part[2 * (m * slices + c) + 1]; }
-    const double mean = a1 / (double)mb, var = a2 / (double)mb - mean * mean;
-    stats[2 * m] = (double)adv_of(b, feistel_at(f, m * mb)) + mean;
+    moments[4 * m] = (double)mb;
+    moments[4 * m + 1] = (double)adv_of(b, feistel_at(f, m * mb));
+    moments[4 * m + 2] = a1;
+    moments[4 * m + 3] = a2;
+}
+// the moments of `ranks` shards ([ranks][nmb][4], rank order) -> mean and population std of every union minibatch
+// (b2p_ppo_adv_combine).  Rank r's sums are moved to rank 0's shift K_0 (d = K_r - K_0):
+//   sum(A - K_0) += S1_r + n_r d,   sum((A - K_0)^2) += S2_r + d (2 S1_r + n_r d)
+// One rank is rank 0's sums as they are, so b2p_ppo_adv_stats (moments, then this with one rank) keeps its bits.
+__global__ void ppo_adv_combine_kernel(const double *__restrict__ moments, int ranks, long long nmb, double *__restrict__ stats) {
+    const long long m = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (m >= nmb) return;
+    const double *q = moments + 4 * m;
+    double n = q[0], a1 = q[2], a2 = q[3];
+    const double K = q[1];
+    for (int r = 1; r < ranks; ++r) {
+        q = moments + 4 * ((long long)r * nmb + m);
+        const double d = q[1] - K;
+        a1 += q[2] + q[0] * d;
+        a2 += q[3] + d * (2.0 * q[2] + q[0] * d);
+        n += q[0];
+    }
+    const double mean = a1 / n, var = a2 / n - mean * mean;
+    stats[2 * m] = K + mean;
     stats[2 * m + 1] = sqrt(var > 0.0 ? var : 0.0);                 // population std
 }
 
@@ -1205,19 +1230,38 @@ __global__ void __launch_bounds__(ppo::Geo<K1>::THREADS, 1) ppo_grad_kernel(cons
     if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS));
 }
 
-// slots -> grad_out (fp64 sums in slot order; the last entry is d loss / d log_std) and the six statistics
-__global__ void ppo_reduce_kernel(const float *__restrict__ ws_grad, const double *__restrict__ ws_stats, int slots, int stride,
-                                  double inv_n, double log_std, double ent_coef, double vf_coef, float *__restrict__ grad,
-                                  double *__restrict__ stats) {
+// The slots of one b2p_ppo_grad* launch -> one fp64 partial vector (b2p_ppo_grad_partial): [0, stride - 1) the gradient
+// sums, then the NSTATS statistic sums, each summed in slot order
+__global__ void ppo_partial_kernel(const float *__restrict__ ws_grad, const double *__restrict__ ws_stats, int slots, int stride,
+                                   double *__restrict__ partial) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i < stride - 1) {
         double s = 0.0;
         for (int k = 0; k < slots; ++k) s += (double)ws_grad[(size_t)k * stride + i];
-        grad[i] = (float)s;
+        partial[i] = s;
     } else if (i == stride - 1) {
         double s[ppo::NSTATS] = {0.0, 0.0, 0.0, 0.0, 0.0};
         for (int k = 0; k < slots; ++k)
             for (int q = 0; q < ppo::NSTATS; ++q) s[q] += ws_stats[(size_t)k * ppo::NSTATS + q];
+        for (int q = 0; q < ppo::NSTATS; ++q) partial[stride - 1 + q] = s[q];
+    }
+}
+
+// `ranks` partial vectors (rank order) -> grad_out (the last entry is d loss / d log_std) and the six statistics, summed in
+// fp64 from rank 0's vector on (b2p_ppo_combine); one rank is its partial as it is, so b2p_ppo_grad keeps its bits
+__global__ void ppo_combine_kernel(const double *__restrict__ partials, int ranks, int stride, double inv_n, double log_std,
+                                   double ent_coef, double vf_coef, float *__restrict__ grad, double *__restrict__ stats) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    const size_t len = (size_t)stride - 1 + ppo::NSTATS;
+    if (i < stride - 1) {
+        double s = partials[i];
+        for (int r = 1; r < ranks; ++r) s += partials[r * len + i];
+        grad[i] = (float)s;
+    } else if (i == stride - 1) {
+        double s[ppo::NSTATS];
+        for (int q = 0; q < ppo::NSTATS; ++q) s[q] = partials[stride - 1 + q];
+        for (int r = 1; r < ranks; ++r)
+            for (int q = 0; q < ppo::NSTATS; ++q) s[q] += partials[r * len + stride - 1 + q];
         grad[i] = (float)(s[4] - ent_coef);                       // the entropy term: d ent / d log_std = 1
         const double pg = s[0] * inv_n, vf = 0.5 * s[1] * inv_n, ent = log_std + 1.4189385332046727418;   // 0.5 log(2 pi e)
         stats[0] = pg; stats[1] = vf; stats[2] = ent; stats[3] = 0.5 * s[2] * inv_n; stats[4] = s[3] * inv_n;
@@ -1233,6 +1277,7 @@ struct b2p_policy {
     int device, obs_dim, tanh_mode, num_sms;
     float *weights;                  // w1 [64, obs_dim] | b1 | w2 [64, 64] | b2 | w3 | b3, then the value tower in the same layout
     const unsigned long long *seed_counter;
+    unsigned long long row_base;     // global index of row 0 of every launch's rows (b2p_set_row_base)
     bool have_weights, have_value_weights;
     std::string error;
 };
@@ -1245,6 +1290,9 @@ int pfail(b2p_handle h, const std::string &msg) {
     if (h) h->error = msg; else g_policy_create_error = msg;
     return 1;
 }
+
+// the seed argument of a launch with the handle's global row base folded in (see row_noise)
+unsigned long long row_seed(const b2p_policy *h, uint64_t seed) { return (unsigned long long)seed + 0x9E3779B97F4A7C15ull * h->row_base; }
 
 struct PolicyDeviceGuard {
     int prev;
@@ -1387,7 +1435,7 @@ int step_setup(b2p_handle h, const b2p_step_out *out, float noise_std, float log
     s.nlp_const = (float)(0.91893853320467274178 + (double)log_std);      // 0.5 log(2 pi) + log_std
     s.want_pi = want_pi ? 1 : 0;
     a.seed_counter = h->seed_counter;
-    a.seed = seed; a.noise_std = noise_std; a.low = low; a.high = high;
+    a.seed = row_seed(h, seed); a.noise_std = noise_std; a.low = low; a.high = high;
     return 0;
 }
 
@@ -1446,6 +1494,7 @@ int b2p_create(int device, int obs_dim, int tanh_mode, b2p_handle *out) {
     h->device = device; h->obs_dim = obs_dim; h->tanh_mode = tanh_mode; h->num_sms = prop.multiProcessorCount;
     h->have_weights = h->have_value_weights = false;
     h->seed_counter = nullptr;
+    h->row_base = 0;
     if (cudaMalloc((void **)&h->weights, 2 * tower_floats(obs_dim) * sizeof(float)) != cudaSuccess) {
         delete h;
         return pfail(nullptr, "b2p_create: cudaMalloc failed");
@@ -1457,6 +1506,13 @@ int b2p_create(int device, int obs_dim, int tanh_mode, b2p_handle *out) {
 int b2p_set_seed_counter(b2p_handle h, const uint64_t *counter) {
     if (!h) return 1;
     h->seed_counter = reinterpret_cast<const unsigned long long *>(counter);
+    return 0;
+}
+
+int b2p_set_row_base(b2p_handle h, int64_t row_base) {
+    if (!h) return 1;
+    if (row_base < 0) return pfail(h, "b2p_set_row_base: row_base must be >= 0");
+    h->row_base = (unsigned long long)row_base;
     return 0;
 }
 
@@ -1500,7 +1556,7 @@ int b2p_act(b2p_handle h, const float *obs, int64_t rows, float *actions_out, fl
     fill_weights(h, a);
     a.obs = obs; a.out = actions_out; a.rows = rows; a.tiles = (rows + pol::TILE - 1) / pol::TILE;
     a.seed_counter = h->seed_counter;
-    a.seed = seed; a.noise_std = noise_std; a.low = low; a.high = high;
+    a.seed = row_seed(h, seed); a.noise_std = noise_std; a.low = low; a.high = high;
     a.bulk_ok = (reinterpret_cast<uintptr_t>(obs) & 15u) == 0 ? 1 : 0;
     Dev d;
     memset(&d, 0, sizeof(d));
@@ -1528,7 +1584,7 @@ int b2p_act_env(b2p_handle h, b2e_handle env, float *actions_out, float noise_st
     fill_weights(h, a);
     a.out = actions_out;
     a.seed_counter = h->seed_counter;
-    a.seed = seed; a.noise_std = noise_std; a.low = low; a.high = high;
+    a.seed = row_seed(h, seed); a.noise_std = noise_std; a.low = low; a.high = high;
     const cudaError_t err = with_k1(h->obs_dim, [&](auto k) {
         return launch_ring<false, decltype(k)::value>(dv->H, h->tanh_mode, grid, (cudaStream_t)stream, a, *dv);
     });
@@ -1626,52 +1682,90 @@ int b2p_ppo_indices(uint64_t key, int64_t n, int64_t begin, int64_t count, int64
 
 size_t b2p_ppo_adv_stats_workspace_size(int64_t n, int64_t mb_size) {
     if (n < 1 || mb_size < 1 || n % mb_size) return 0;
-    return (size_t)(n / mb_size) * (size_t)adv_slices(mb_size) * 2 * sizeof(double);
+    const size_t nmb = (size_t)(n / mb_size);
+    return nmb * (size_t)adv_slices(mb_size) * 2 * sizeof(double) + nmb * 4 * sizeof(double);
 }
 
-int b2p_ppo_adv_stats(const b2p_ppo_batch *b, uint64_t key, int64_t mb_size, double *stats_out, void *workspace,
-                      void *stream) {
+}  // extern "C"
+
+namespace {
+
+// the slice sums of every minibatch of an epoch -> moments [nmb][4] (b2p_ppo_adv_moments, b2p_ppo_adv_stats); `part` holds
+// the slice sums, nmb * slices * 2 doubles
+int adv_moments(const b2p_ppo_batch *b, uint64_t key, int64_t mb_size, double *moments, double *part, void *stream,
+                int &device, const char *who) {
     pol::PpoBatch pb;
     int64_t n = 0;
-    if (check_batch(nullptr, b, pb, n, "b2p_ppo_adv_stats")) return 1;
-    if (!stats_out || !workspace) return pfail(nullptr, "b2p_ppo_adv_stats: null output or workspace");
-    if (mb_size < 1 || n % mb_size) return pfail(nullptr, "b2p_ppo_adv_stats: T * rows is not a multiple of the minibatch size");
+    const std::string w(who);
+    if (check_batch(nullptr, b, pb, n, who)) return 1;
+    if (!moments || !part) return pfail(nullptr, w + ": null output or workspace");
+    if (mb_size < 1 || n % mb_size) return pfail(nullptr, w + ": T * rows is not a multiple of the minibatch size");
     cudaPointerAttributes attr;
     if (cudaPointerGetAttributes(&attr, b->returns) != cudaSuccess || attr.type != cudaMemoryTypeDevice)
-        return pfail(nullptr, "b2p_ppo_adv_stats: returns is not device memory");
+        return pfail(nullptr, w + ": returns is not device memory");
+    device = attr.device;
     PolicyDeviceGuard guard(attr.device);
     const pol::Feistel f = feistel_setup(key, n);
     const long long nmb = n / mb_size;
     const int slices = adv_slices(mb_size);
     if (nmb > 0x7FFFFFFFLL / slices)
-        return pfail(nullptr, "b2p_ppo_adv_stats: too many minibatches for one launch (more than 2^31 - 1 blocks)");
-    double *part = static_cast<double *>(workspace);
+        return pfail(nullptr, w + ": too many minibatches for one launch (more than 2^31 - 1 blocks)");
     pol::ppo_adv_partial<<<(unsigned)(nmb * slices), pol::ADV_THREADS, 0, (cudaStream_t)stream>>>(pb, f, mb_size, slices, part);
-    pol::ppo_adv_final<<<(unsigned)((nmb + 255) / 256), 256, 0, (cudaStream_t)stream>>>(pb, f, mb_size, nmb, slices, part, stats_out);
+    pol::ppo_adv_moments_kernel<<<(unsigned)((nmb + 255) / 256), 256, 0, (cudaStream_t)stream>>>(pb, f, mb_size, nmb, slices, part,
+                                                                                                 moments);
     const cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return pfail(nullptr, std::string("b2p_ppo_adv_stats: ") + cudaGetErrorString(err));
+    if (err != cudaSuccess) return pfail(nullptr, w + ": " + cudaGetErrorString(err));
     return 0;
 }
 
-size_t b2p_ppo_workspace_size(b2p_handle h) {
-    if (!h) return 0;
-    const size_t slots = (size_t)h->num_sms * pol::ppo::groups(pol::obs_width(h->obs_dim));
-    return slots * (grad_stride(h->obs_dim) * sizeof(float) + pol::ppo::NSTATS * sizeof(double)) + 256;
+int adv_combine(const double *moments, int ranks, int64_t nmb, double *stats_out, void *stream, const char *who) {
+    pol::ppo_adv_combine_kernel<<<(unsigned)((nmb + 255) / 256), 256, 0, (cudaStream_t)stream>>>(moments, ranks, nmb, stats_out);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return pfail(nullptr, std::string(who) + ": " + cudaGetErrorString(err));
+    return 0;
 }
 
-int b2p_ppo_grad(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, float *grad_out, double *stats_out,
-                 void *workspace, void *stream) {
-    if (!h) return 1;
+// doubles of one partial vector: the gradient sums before log_std's, then the NSTATS statistic sums
+size_t partial_doubles(int obs_dim) { return grad_stride(obs_dim) - 1 + pol::ppo::NSTATS; }
+
+// The gradient workspace (b2p_ppo_workspace_size bytes): from its first 256-byte boundary the fp32 gradient slots
+// [slots][stride], from the next 8-byte boundary the fp64 statistic slots [slots][NSTATS], then b2p_ppo_grad's own
+// partial vector.  `slots` is that of the largest grid (num_sms x groups), so the layout does not depend on the launch.
+struct PpoWorkspace {
+    float *grad;
+    double *stats, *partial;
+};
+size_t max_slots(const b2p_policy *h) { return (size_t)h->num_sms * pol::ppo::groups(pol::obs_width(h->obs_dim)); }
+size_t ppo_workspace_bytes(const b2p_policy *h) {
+    return max_slots(h) * (grad_stride(h->obs_dim) * sizeof(float) + pol::ppo::NSTATS * sizeof(double)) +
+           partial_doubles(h->obs_dim) * sizeof(double) + 255 + 7;      // + the two alignments
+}
+PpoWorkspace ppo_workspace(const b2p_policy *h, void *workspace) {
+    const size_t slots = max_slots(h);
+    const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
+    PpoWorkspace w;
+    w.grad = reinterpret_cast<float *>(base);
+    w.stats = reinterpret_cast<double *>(base + ((slots * grad_stride(h->obs_dim) * sizeof(float) + 7) & ~(size_t)7));
+    w.partial = w.stats + slots * pol::ppo::NSTATS;
+    return w;
+}
+
+// the gradient kernel over one shard's minibatch and its slot reduction into `partial` (b2p_ppo_grad, b2p_ppo_grad_partial):
+// the per-row scale is 1 / count_total, the size of the union minibatch
+int grad_partial(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, int64_t count_total, double *partial,
+                 void *workspace, cudaStream_t cs, const char *who) {
+    const std::string w(who);
     if (!h->have_weights || !h->have_value_weights)
-        return pfail(h, "b2p_ppo_grad: weights not set (b2p_set_weights and b2p_set_value_weights)");
+        return pfail(h, w + ": weights not set (b2p_set_weights and b2p_set_value_weights)");
     pol::PpoBatch pb;
     int64_t n = 0;
-    if (check_batch(h, b, pb, n, "b2p_ppo_grad")) return 1;
-    if (!p || !grad_out || !stats_out || !workspace || !p->adv_stats)
-        return pfail(h, "b2p_ppo_grad: null params, adv_stats, output or workspace");
-    if (p->count < 1) return pfail(h, "b2p_ppo_grad: count must be >= 1");
-    if (p->begin < 0 || p->begin > n - p->count) return pfail(h, "b2p_ppo_grad: range outside [0, T * rows)");
-    if (!(p->cliprange > 0.f)) return pfail(h, "b2p_ppo_grad: cliprange must be > 0");
+    if (check_batch(h, b, pb, n, who)) return 1;
+    if (!p || !partial || !workspace || !p->adv_stats) return pfail(h, w + ": null params, adv_stats, output or workspace");
+    if (p->count < 1) return pfail(h, w + ": count must be >= 1");
+    if (p->begin < 0 || p->begin > n - p->count) return pfail(h, w + ": range outside [0, T * rows)");
+    if (count_total < p->count || count_total > B2P_PPO_MAX_SAMPLES)
+        return pfail(h, w + ": count_total must be count..2^62 (the size of the union minibatch)");
+    if (!(p->cliprange > 0.f)) return pfail(h, w + ": cliprange must be > 0");
     PolicyDeviceGuard guard(h->device);
     pol::GradArgs a;
     memset(&a, 0, sizeof(a));
@@ -1681,16 +1775,15 @@ int b2p_ppo_grad(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, 
     a.begin = p->begin; a.count = p->count; a.tiles = (p->count + pol::TILE - 1) / pol::TILE;
     a.adv_stats = p->adv_stats;
     a.clip = p->cliprange; a.clip_vf = p->cliprange_vf; a.vf_coef = p->vf_coef;
-    a.inv_n = (float)(1.0 / (double)p->count);
+    a.inv_n = (float)(1.0 / (double)count_total);
     a.inv_sigma = (float)exp(-(double)p->log_std);
     a.nlp_const = (float)(0.91893853320467274178 + (double)p->log_std);      // as b2p_step: 0.5 log(2 pi) + log_std
     a.od = h->obs_dim; a.tf = (int)tower_floats(h->obs_dim); a.stride = (int)grad_stride(h->obs_dim);
     const int groups = pol::ppo::groups(pol::obs_width(h->obs_dim));
     const int grid = dense_grid(h, a.tiles, groups), slots = grid * groups;
-    const uintptr_t base = (reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255;
-    a.ws_grad = reinterpret_cast<float *>(base);
-    a.ws_stats = reinterpret_cast<double *>(base + (((size_t)slots * a.stride * sizeof(float) + 7) & ~(size_t)7));
-    cudaStream_t cs = (cudaStream_t)stream;
+    const PpoWorkspace ws = ppo_workspace(h, workspace);
+    a.ws_grad = ws.grad;
+    a.ws_stats = ws.stats;
     with_k1(h->obs_dim, [&](auto k) {
         using PG = pol::ppo::Geo<decltype(k)::value>;
         switch (h->tanh_mode) {
@@ -1700,12 +1793,91 @@ int b2p_ppo_grad(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, 
         }
         return 0;
     });
-    pol::ppo_reduce_kernel<<<(a.stride + 255) / 256, 256, 0, cs>>>(a.ws_grad, a.ws_stats, slots, a.stride, 1.0 / (double)p->count,
-                                                                   (double)p->log_std, (double)p->ent_coef, (double)p->vf_coef,
-                                                                   grad_out, stats_out);
+    pol::ppo_partial_kernel<<<(a.stride + 255) / 256, 256, 0, cs>>>(a.ws_grad, a.ws_stats, slots, a.stride, partial);
     const cudaError_t err = cudaGetLastError();
-    if (err != cudaSuccess) return pfail(h, std::string("b2p_ppo_grad: ") + cudaGetErrorString(err));
+    if (err != cudaSuccess) return pfail(h, w + ": " + cudaGetErrorString(err));
     return 0;
+}
+
+int combine(b2p_handle h, const double *partials, int ranks, int64_t count_total, float log_std, float ent_coef, float vf_coef,
+            float *grad_out, double *stats_out, cudaStream_t cs, const char *who) {
+    PolicyDeviceGuard guard(h->device);
+    const int stride = (int)grad_stride(h->obs_dim);
+    pol::ppo_combine_kernel<<<(stride + 255) / 256, 256, 0, cs>>>(partials, ranks, stride, 1.0 / (double)count_total,
+                                                                  (double)log_std, (double)ent_coef, (double)vf_coef, grad_out,
+                                                                  stats_out);
+    const cudaError_t err = cudaGetLastError();
+    if (err != cudaSuccess) return pfail(h, std::string(who) + ": " + cudaGetErrorString(err));
+    return 0;
+}
+
+}  // namespace
+
+extern "C" {
+
+int b2p_ppo_adv_moments(const b2p_ppo_batch *b, uint64_t key, int64_t mb_size, double *moments_out, void *workspace,
+                        void *stream) {
+    int device = -1;
+    return adv_moments(b, key, mb_size, moments_out, static_cast<double *>(workspace), stream, device, "b2p_ppo_adv_moments");
+}
+
+int b2p_ppo_adv_combine(const double *moments, int ranks, int64_t nmb, double *stats_out, void *stream) {
+    if (!moments || !stats_out) return pfail(nullptr, "b2p_ppo_adv_combine: null moments or output");
+    if (ranks < 1) return pfail(nullptr, "b2p_ppo_adv_combine: ranks must be >= 1");
+    if (nmb < 1 || nmb > 0x7FFFFFFFLL * 256) return pfail(nullptr, "b2p_ppo_adv_combine: nmb must be 1..(2^31 - 1) x 256");
+    cudaPointerAttributes attr;
+    if (cudaPointerGetAttributes(&attr, moments) != cudaSuccess || attr.type != cudaMemoryTypeDevice)
+        return pfail(nullptr, "b2p_ppo_adv_combine: moments is not device memory");
+    PolicyDeviceGuard guard(attr.device);
+    return adv_combine(moments, ranks, nmb, stats_out, stream, "b2p_ppo_adv_combine");
+}
+
+int b2p_ppo_adv_stats(const b2p_ppo_batch *b, uint64_t key, int64_t mb_size, double *stats_out, void *workspace,
+                      void *stream) {
+    pol::PpoBatch pb;
+    int64_t n = 0;
+    if (check_batch(nullptr, b, pb, n, "b2p_ppo_adv_stats")) return 1;
+    if (!stats_out || !workspace) return pfail(nullptr, "b2p_ppo_adv_stats: null output or workspace");
+    if (mb_size < 1 || n % mb_size) return pfail(nullptr, "b2p_ppo_adv_stats: T * rows is not a multiple of the minibatch size");
+    const int64_t nmb = n / mb_size;
+    double *part = static_cast<double *>(workspace), *moments = part + nmb * adv_slices(mb_size) * 2;   // the slice sums, then the moments
+    int device = -1;
+    if (adv_moments(b, key, mb_size, moments, part, stream, device, "b2p_ppo_adv_stats")) return 1;
+    PolicyDeviceGuard guard(device);
+    return adv_combine(moments, 1, nmb, stats_out, stream, "b2p_ppo_adv_stats");
+}
+
+size_t b2p_ppo_workspace_size(b2p_handle h) {
+    if (!h) return 0;
+    return ppo_workspace_bytes(h);
+}
+
+size_t b2p_ppo_partial_size(b2p_handle h) { return h ? partial_doubles(h->obs_dim) : 0; }
+
+int b2p_ppo_grad_partial(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, int64_t count_total,
+                         double *partial_out, void *workspace, void *stream) {
+    if (!h) return 1;
+    return grad_partial(h, b, p, count_total, partial_out, workspace, (cudaStream_t)stream, "b2p_ppo_grad_partial");
+}
+
+int b2p_ppo_combine(b2p_handle h, const double *partials, int ranks, int64_t count_total, float log_std, float ent_coef,
+                    float vf_coef, float *grad_out, double *stats_out, void *stream) {
+    if (!h) return 1;
+    if (!partials || !grad_out || !stats_out) return pfail(h, "b2p_ppo_combine: null partials or output");
+    if (ranks < 1) return pfail(h, "b2p_ppo_combine: ranks must be >= 1");
+    if (count_total < 1 || count_total > B2P_PPO_MAX_SAMPLES) return pfail(h, "b2p_ppo_combine: count_total must be 1..2^62");
+    return combine(h, partials, ranks, count_total, log_std, ent_coef, vf_coef, grad_out, stats_out, (cudaStream_t)stream,
+                   "b2p_ppo_combine");
+}
+
+int b2p_ppo_grad(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, float *grad_out, double *stats_out,
+                 void *workspace, void *stream) {
+    if (!h) return 1;
+    // its own partial vector lives in the workspace (a NULL output makes grad_partial report the nulls)
+    double *partial = workspace && grad_out && stats_out ? ppo_workspace(h, workspace).partial : nullptr;
+    const cudaStream_t cs = (cudaStream_t)stream;
+    if (grad_partial(h, b, p, p ? p->count : 0, partial, workspace, cs, "b2p_ppo_grad")) return 1;
+    return combine(h, partial, 1, p->count, p->log_std, p->ent_coef, p->vf_coef, grad_out, stats_out, cs, "b2p_ppo_grad");
 }
 
 }  // extern "C"

@@ -160,7 +160,7 @@ __device__ __noinline__ void reset_one(const Dev &d, const StepArgs &a, WarpSmem
         float v = 0.f;
         if (p < d.P) {
             if (a.init_params) v = a.init_params[(size_t)e * d.P + p];
-            else if (p < d.P1) v = glorot(d.seed, e, episode, p, d.lim1);      // keras Dense: Glorot kernel, zero bias
+            else if (p < d.P1) v = glorot(d.seed, e + d.env_base, episode, p, d.lim1);      // keras Dense: Glorot kernel, zero bias
         }
         if (p < d.Pp) wE[p] = v;
         S.w[p] = v;

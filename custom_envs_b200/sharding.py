@@ -18,6 +18,15 @@ def shard_range(num_envs, world_size, rank):
     return first, count
 
 
+def shard_bases(num_envs, world_size, rank, rows_per_env):
+    """(env_base, row_base) of rank's shard for data-parallel PPO: ``BatchedOptEnv(..., env_base=env_base)`` draws the
+    shard's initial and auto-reset parameters by global env index, and ``DevicePolicy.set_row_base(row_base)`` its
+    exploration noise by global agent row (the rows of env e are [e P, (e + 1) P) in both VecEnv row orders), so the
+    shard's rollout is exactly its envs' part of one unsharded rollout."""
+    first, _ = shard_range(num_envs, world_size, rank)
+    return first, first * int(rows_per_env)
+
+
 def shard_seeds(seeds, world_size, rank):
     """Seeds (one per global env index) of the envs this rank owns."""
     first, count = shard_range(len(seeds), world_size, rank)

@@ -12,7 +12,12 @@ constructor raises (``SharedMlpPolicy.act`` is the torch path, and it is the cal
 For PPO, ``step`` / ``value`` are the rest of stable-baselines' ``model.step`` / ``model.value`` (value
 tower, unclipped action, neglogp, bf16 observation store), ``DeviceRolloutBuffer`` and
 ``device_ppo_rollout`` collect a whole rollout with its GAE advantages on the device, and ``ppo_grad`` /
-``device_ppo_update`` run PPO2's minibatch updates over it with a fused clipped-surrogate gradient kernel."""
+``device_ppo_update`` run PPO2's minibatch updates over it with a fused clipped-surrogate gradient kernel.
+
+Data-parallel PPO over several GPUs: every rank steps its env shard (``BatchedOptEnv(env_base=...)`` and
+``DevicePolicy.set_row_base``, ``sharding.shard_bases``), so its rollout holds exactly the rows of those envs in one
+unsharded run, and ``device_ppo_update(..., group=...)`` combines the ranks' fp64 partial sums in rank order, so every
+rank takes the same optimizer step bit for bit."""
 import ctypes
 import math
 
@@ -39,6 +44,7 @@ class DevicePolicy:
         self.low, self.high = float(low), float(high)
         self.set_log_std(log_std)
         self.calls = 0
+        self.row_base = 0
         self.seed_counter = None
         self.has_value = False
         handle = ctypes.c_void_p()
@@ -104,6 +110,14 @@ class DevicePolicy:
         self._check(self.lib.b2p_set_seed_counter(self.handle, ptr))
         if not enabled:
             self.seed_counter = None
+
+    def set_row_base(self, row_base):
+        """Global index of row 0 of every later launch (default 0): local row r draws the exploration noise of global
+        row ``row_base + r`` (b2p_set_row_base).  For the shard of envs starting at ``first_env`` with P rows per env
+        it is ``first_env * P`` in both VecEnv row orders (``sharding.shard_bases``); the shard's actions, neglogp and
+        stored rows then equal those rows of one unsharded batch."""
+        self._check(self.lib.b2p_set_row_base(self.handle, int(row_base)))
+        self.row_base = int(row_base)
 
     def _seed(self, seed):
         self.calls += 1
@@ -197,16 +211,65 @@ class DevicePolicy:
         if stats is None:
             stats = torch.empty(6, dtype=torch.float64, device=self.device)
         assert grad.dtype == torch.float32 and grad.numel() == 2 * tower + 1 and grad.is_contiguous()
-        assert stats.dtype == torch.float64 and stats.numel() == 6 and adv_stats.dtype == torch.float64
+        assert stats.dtype == torch.float64 and stats.numel() == 6
+        args = self._ppo_args(buffer, key, begin, count, adv_stats, cliprange, cliprange_vf, ent_coef, vf_coef)
+        self._check(self.lib.b2p_ppo_grad(self.handle, *args[:2], _ptr(grad), _ptr(stats), *args[2:]))
+        return grad, stats
+
+    def _ppo_args(self, buffer, key, begin, count, adv_stats, cliprange, cliprange_vf, ent_coef, vf_coef):
+        """(batch, params, workspace, stream) of a b2p_ppo_grad / b2p_ppo_grad_partial call."""
+        assert adv_stats.dtype == torch.float64
         assert buffer.obs_bf16.shape[-1] == self.obs_width, 'the buffer\'s rows are not this policy\'s obs_width wide'
         if getattr(self, '_ppo_ws', None) is None:
             self._ppo_ws = torch.empty(self.lib.b2p_ppo_workspace_size(self.handle), dtype=torch.uint8, device=self.device)
         params = _lib.PpoParams(float(cliprange), float(cliprange if cliprange_vf is None else cliprange_vf),
                                 float(ent_coef), float(vf_coef), float(self.log_std), int(key) & (2 ** 64 - 1),
                                 int(begin), int(count), adv_stats.data_ptr())
-        batch = _ppo_batch(buffer)
-        self._check(self.lib.b2p_ppo_grad(self.handle, ctypes.byref(batch), ctypes.byref(params), _ptr(grad), _ptr(stats),
-                                          _ptr(self._ppo_ws), self._stream()))
+        self._ppo_keep = (_ppo_batch(buffer), params)
+        return (ctypes.byref(self._ppo_keep[0]), ctypes.byref(params), _ptr(self._ppo_ws), self._stream())
+
+    @property
+    def ppo_partial_size(self):
+        """Length of the float64 partial vector of ``ppo_grad_partial``: the 2 * tower + 1 - 1 gradient sums before
+        log_std's, then the five loss sums."""
+        return int(self.lib.b2p_ppo_partial_size(self.handle))
+
+    def ppo_grad_partial(self, buffer, key, begin, count, count_total, adv_stats, cliprange=0.2, cliprange_vf=None,
+                         ent_coef=0.01, vf_coef=0.5, partial=None):
+        """This shard's part of PPO2's gradient over a minibatch split across shards (b2p_ppo_grad_partial): the rows
+        at positions [begin, begin + count) of the permutation ``key`` of ``buffer``, each scaled by 1 / ``count_total``
+        (the size of the union minibatch) rather than 1 / count, normalised with the union's ``adv_stats``
+        (``ppo_adv_combine``).  Returns float64 [``ppo_partial_size``] on the device, not synchronised; ``ppo_combine``
+        sums the shards' vectors in rank order.  With count_total = count, ``ppo_combine`` of this one vector is
+        ``ppo_grad`` bit for bit."""
+        if self.log_std is None:
+            raise ValueError('ppo_grad_partial needs a stochastic policy (log_std)')
+        size = self.ppo_partial_size
+        if partial is None:
+            partial = torch.empty(size, dtype=torch.float64, device=self.device)
+        if partial.dtype != torch.float64 or not partial.is_contiguous() or partial.numel() < size:
+            raise ValueError('the partial buffer must be a contiguous float64 tensor of at least %d elements' % size)
+        args = self._ppo_args(buffer, key, begin, count, adv_stats, cliprange, cliprange_vf, ent_coef, vf_coef)
+        self._check(self.lib.b2p_ppo_grad_partial(self.handle, *args[:2], int(count_total), _ptr(partial), *args[2:]))
+        return partial
+
+    def ppo_combine(self, partials, count_total, ent_coef=0.01, vf_coef=0.5, grad=None, stats=None):
+        """``partials`` float64 [ranks, ``ppo_partial_size``], the shards' ``ppo_grad_partial`` vectors in rank order ->
+        (grad, stats) as ``ppo_grad`` returns them for the union minibatch of ``count_total`` rows, at this policy's
+        ``log_std`` (b2p_ppo_combine: fp64 sums from rank 0 on, so every rank that combines the same vectors gets the
+        same bits)."""
+        size = self.ppo_partial_size
+        if partials.dtype != torch.float64 or not partials.is_contiguous() or partials.ndim != 2 or partials.shape[1] != size:
+            raise ValueError('partials must be a contiguous float64 [ranks, %d] tensor' % size)
+        if grad is None:
+            grad = torch.empty(size - 4, dtype=torch.float32, device=self.device)
+        if stats is None:
+            stats = torch.empty(6, dtype=torch.float64, device=self.device)
+        assert grad.dtype == torch.float32 and grad.numel() == size - 4 and grad.is_contiguous()
+        assert stats.dtype == torch.float64 and stats.numel() == 6
+        self._check(self.lib.b2p_ppo_combine(self.handle, _ptr(partials), int(partials.shape[0]), int(count_total),
+                                             float(self.log_std), float(ent_coef), float(vf_coef), _ptr(grad), _ptr(stats),
+                                             self._stream()))
         return grad, stats
 
     def close(self):
@@ -459,6 +522,52 @@ def ppo_adv_stats(buffer, key, mb_size):
     return stats
 
 
+def ppo_adv_moments(buffer, key, mb_size):
+    """This shard's advantage moments of every minibatch of one epoch's permutation ``key`` (b2p_ppo_adv_moments) ->
+    float64 [T * rows / mb_size, 4] on the device: count, shift K (the advantage at the minibatch's first position),
+    sum(A - K) and sum((A - K)^2), fp64 sums in the order of ``ppo_adv_stats``."""
+    lib = _lib.load()
+    T, rows = buffer.actions_raw.shape
+    n = T * rows
+    if mb_size < 1 or n % mb_size:
+        raise ValueError('the %d samples of the buffer do not split into minibatches of %d' % (n, mb_size))
+    dev = buffer.returns.device
+    moments = torch.empty((n // mb_size, 4), dtype=torch.float64, device=dev)
+    ws = torch.empty(max(1, lib.b2p_ppo_adv_stats_workspace_size(n, mb_size)), dtype=torch.uint8, device=dev)
+    batch = _ppo_batch(buffer)
+    stream = ctypes.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+    _check_global(lib.b2p_ppo_adv_moments(ctypes.byref(batch), int(key) & (2 ** 64 - 1), int(mb_size), _ptr(moments),
+                                          _ptr(ws), stream))
+    return moments
+
+
+def ppo_adv_combine(moments):
+    """``moments`` float64 [ranks, nmb, 4], the shards' ``ppo_adv_moments`` in rank order -> float64 [nmb, 2]: mean and
+    population std of the advantages of every union minibatch (b2p_ppo_adv_combine; one rank = ``ppo_adv_stats``)."""
+    lib = _lib.load()
+    if moments.dtype != torch.float64 or not moments.is_contiguous() or moments.ndim != 3 or moments.shape[2] != 4:
+        raise ValueError('moments must be a contiguous float64 [ranks, nmb, 4] tensor')
+    stats = torch.empty((moments.shape[1], 2), dtype=torch.float64, device=moments.device)
+    stream = ctypes.c_void_p(torch.cuda.current_stream(moments.device).cuda_stream)
+    _check_global(lib.b2p_ppo_adv_combine(_ptr(moments), int(moments.shape[0]), int(moments.shape[1]), _ptr(stats), stream))
+    return stats
+
+
+def _mix64(z):
+    z &= 2 ** 64 - 1
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & (2 ** 64 - 1)
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & (2 ** 64 - 1)
+    return z ^ (z >> 31)
+
+
+def rank_epoch_key(seed, epoch, rank):
+    """The permutation key of rank ``rank``'s shard in epoch ``epoch`` of a data-parallel update seeded ``seed``:
+    ``epoch_key(seed, epoch)`` on rank 0, so that a one-rank update is the single-GPU one, and on rank r > 0 the
+    splitmix64 finaliser of that key + r * 0x9E3779B97F4A7C15."""
+    key = epoch_key(seed, epoch)
+    return key if int(rank) == 0 else _mix64(key + int(rank) * 0x9E3779B97F4A7C15)
+
+
 def epoch_key(seed, epoch):
     """The permutation key of epoch ``epoch`` of an update seeded ``seed`` (splitmix64 of both)."""
     z = (int(seed) * 0x9E3779B97F4A7C15 + int(epoch) + 1) & (2 ** 64 - 1)
@@ -484,7 +593,7 @@ def load_model(policy, model):
 
 
 def device_ppo_update(model, policy, buffer, optimizer, n_epochs=4, n_minibatches=4, cliprange=0.2, cliprange_vf=None,
-                      ent_coef=0.01, vf_coef=0.5, max_grad_norm=0.5, seed=None):
+                      ent_coef=0.01, vf_coef=0.5, max_grad_norm=0.5, seed=None, group=None):
     """stable-baselines 2 ``PPO2.learn``'s inner loop over a filled ``DeviceRolloutBuffer``: ``n_epochs`` passes, each
     over a fresh permutation of the T * rows samples cut into ``n_minibatches`` minibatches.  Per minibatch: ``model``'s
     towers and ``log_std`` go to ``policy``, ``policy.ppo_grad`` computes the gradient of PPO2's loss, it is copied into
@@ -494,7 +603,28 @@ def device_ppo_update(model, policy, buffer, optimizer, n_epochs=4, n_minibatche
     Adam but without TF's bias-corrected epsilon, so parity with TF is not pinned).  ``seed`` picks the permutations
     (None: drawn from torch's generator).  On return ``policy`` holds the trained weights and ``log_std``.  Returns
     the statistics averaged over minibatches (pg_loss, vf_loss, entropy, approxkl, clipfrac, loss) as float64 numpy
-    [6], with one host synchronisation."""
+    [6], with one host synchronisation.
+
+    ``group``: a ``torch.distributed`` process group whose every rank holds the rollout of its own env shard (one GPU
+    per rank, e.g. under ``torchrun``); None = this GPU alone.  The ranks then train one policy on the union of their
+    samples, as PPO2 on the whole env batch with minibatches stratified by rank:
+
+    - rank 0's ``seed`` is used on every rank; rank r permutes its own N_r = T * rows_r samples with
+      ``rank_epoch_key(seed, epoch, r)``, and minibatch m is positions [m N_r / n_minibatches, (m + 1) N_r / n_minibatches)
+      of every rank, so its size n_m is the sum of the ranks' shares (every N_r must be a multiple of n_minibatches);
+    - the advantages are normalised with the mean and std of the union minibatch (``ppo_adv_moments``, all-gather,
+      ``ppo_adv_combine``), and gradient and statistics are means over n_m (``ppo_grad_partial``, all-gather,
+      ``ppo_combine``);
+    - the combine sums the ranks' fp64 vectors in rank order, so every rank applies the same gradient, clip and
+      optimizer step bit for bit and the models stay identical without a weight broadcast.
+
+    One all-gather first checks that the ranks agree on T, the observation width, obs_dim, n_epochs and n_minibatches;
+    on a mismatch every rank raises the same ValueError.  Per minibatch the exchange is one float64 vector of
+    ``policy.ppo_partial_size`` per rank (84 KB at obs_dim 15).  Returns the statistics of the union minibatches,
+    the same on every rank."""
+    if group is not None:
+        return _device_ppo_update_dist(model, policy, buffer, optimizer, n_epochs, n_minibatches, cliprange, cliprange_vf,
+                                       ent_coef, vf_coef, max_grad_norm, seed, group)
     T, rows = buffer.actions_raw.shape
     n = T * rows
     if n % n_minibatches:
@@ -512,14 +642,80 @@ def device_ppo_update(model, policy, buffer, optimizer, n_epochs=4, n_minibatche
             load_model(policy, model)
             grad, stats = policy.ppo_grad(buffer, key, m * mb, mb, adv[m], cliprange, cliprange_vf, ent_coef, vf_coef,
                                           grad, stats)
-            offset = 0
-            for p in params:
-                g = grad[offset:offset + p.numel()].view_as(p)
-                if p.grad is None:
-                    p.grad = g.clone()
-                else:
-                    p.grad.copy_(g)
-                offset += p.numel()
+            _set_grads(params, grad)
+            if max_grad_norm is not None:
+                torch.nn.utils.clip_grad_norm_(params, max_grad_norm)
+            optimizer.step()
+            total += stats
+    load_model(policy, model)
+    return (total / (n_epochs * n_minibatches)).cpu().numpy()
+
+
+def _set_grads(params, grad):
+    offset = 0
+    for p in params:
+        g = grad[offset:offset + p.numel()].view_as(p)
+        if p.grad is None:
+            p.grad = g.clone()
+        else:
+            p.grad.copy_(g)
+        offset += p.numel()
+
+
+def _check_rank_table(table, n_minibatches):
+    """The all-gathered [T, buffer width, obs_width, obs_dim, T * rows, n_epochs, n_minibatches, seed] of every rank ->
+    (rank 0's seed, n_m = the size of a union minibatch).  Every rank runs it on the same table, so all raise the same
+    ValueError or none does."""
+    for col, what in ((0, 'T (n_steps)'), (2, 'the observation width'), (3, 'obs_dim'), (5, 'n_epochs'),
+                      (6, 'n_minibatches')):
+        values = [row[col] for row in table]
+        if len(set(values)) > 1:
+            raise ValueError('data-parallel PPO: the ranks disagree on %s: %s' % (what, values))
+    bad = [r for r, row in enumerate(table) if row[1] != row[2]]
+    if bad:
+        raise ValueError('data-parallel PPO: the rollout rows of rank(s) %s are not the policy\'s obs_width wide' % bad)
+    bad = [r for r, row in enumerate(table) if n_minibatches < 1 or row[4] % n_minibatches]
+    if bad:
+        raise ValueError('data-parallel PPO: T * rows = %s of rank(s) %s is not a multiple of n_minibatches = %d'
+                         % ([table[r][4] for r in bad], bad, n_minibatches))
+    return table[0][7] & (2 ** 64 - 1), sum(row[4] // n_minibatches for row in table)
+
+
+def _device_ppo_update_dist(model, policy, buffer, optimizer, n_epochs, n_minibatches, cliprange, cliprange_vf, ent_coef,
+                            vf_coef, max_grad_norm, seed, group):
+    """``device_ppo_update`` over the ranks of ``group`` (see there)."""
+    import torch.distributed as dist
+    world, rank = dist.get_world_size(group), dist.get_rank(group)
+    dev = policy.device
+    T, rows = buffer.actions_raw.shape
+    n = T * rows
+    if seed is None:
+        seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+    seed = int(seed) & (2 ** 64 - 1)
+    mine = torch.tensor([T, buffer.obs_bf16.shape[-1], policy.obs_width, policy.obs_dim, n, n_epochs, n_minibatches,
+                         seed - 2 ** 64 if seed >= 2 ** 63 else seed], dtype=torch.int64, device=dev)
+    table = torch.empty((world, mine.numel()), dtype=torch.int64, device=dev)
+    dist.all_gather_into_tensor(table, mine, group=group)
+    seed, count_total = _check_rank_table(table.cpu().tolist(), n_minibatches)
+    mb = n // n_minibatches
+    params = _model_params(model)
+    f64 = dict(dtype=torch.float64, device=dev)
+    partial = torch.empty(policy.ppo_partial_size, **f64)
+    partials = torch.empty((world, partial.numel()), **f64)
+    moments_all = torch.empty((world, n_minibatches, 4), **f64)
+    total = torch.zeros(6, **f64)
+    grad = stats = None
+    for epoch in range(n_epochs):
+        key = rank_epoch_key(seed, epoch, rank)
+        dist.all_gather_into_tensor(moments_all, ppo_adv_moments(buffer, key, mb), group=group)
+        adv = ppo_adv_combine(moments_all)
+        for m in range(n_minibatches):
+            load_model(policy, model)
+            policy.ppo_grad_partial(buffer, key, m * mb, mb, count_total, adv[m], cliprange, cliprange_vf, ent_coef,
+                                    vf_coef, partial)
+            dist.all_gather_into_tensor(partials, partial, group=group)
+            grad, stats = policy.ppo_combine(partials, count_total, ent_coef, vf_coef, grad, stats)
+            _set_grads(params, grad)
             if max_grad_norm is not None:
                 torch.nn.utils.clip_grad_norm_(params, max_grad_norm)
             optimizer.step()

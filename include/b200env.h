@@ -77,7 +77,10 @@ typedef struct b2e_config {
     int32_t  auto_reset;          /* 1: finished envs are reset inside b2e_step, the row block
                                      of such an env holds the RESET observation
                                      (vectorize/concurrentvecenv.py:32-38) */
-    int32_t  reserved;
+    int32_t  env_base;            /* global index of this handle's env 0 (0..2^31-1-num_envs): the on-device
+                                     Glorot initialiser draws env e's parameters as those of env env_base + e,
+                                     so a shard of envs [env_base, env_base + num_envs) of a larger batch
+                                     starts and auto-resets from the weights that batch gives them */
     int32_t  hidden_more[B2E_MAX_LAYERS]; /* widths of the 2nd, 3rd ... hidden layers, 0 terminated
                                      (the reference default is layers=(256, 256)) */
     uint64_t init_seed;           /* seed of the on-device Glorot-uniform initialiser */

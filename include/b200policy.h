@@ -178,6 +178,49 @@ size_t b2p_ppo_workspace_size(b2p_handle h);
 int b2p_ppo_grad(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, float *grad_out, double *stats_out,
                  void *workspace, void *stream);
 
+/* ---- Data-parallel PPO: one policy trained on the rollouts of R env shards (one per GPU).
+ *
+ * Shard r rolls out envs [first_env, first_env + E_r) of the whole batch: b2e_config.env_base = first_env, and
+ * b2p_set_row_base(first_env * P) on the policy, so that its trajectories are those envs' rows of one unsharded run bit
+ * for bit.  Minibatch m of an epoch is the union over shards of positions [m N_r / n_mb, (m + 1) N_r / n_mb) of each
+ * shard's own permutation of its N_r = T * rows_r samples (every N_r a multiple of n_mb); its size is
+ * n_m = sum_r N_r / n_mb.  The advantages are normalised with the union's mean and std and the loss is a mean over n_m:
+ *   b2p_ppo_adv_moments on every shard, the R moment sets gathered in rank order, b2p_ppo_adv_combine;
+ *   per minibatch b2p_ppo_grad_partial on every shard, the R partial vectors gathered in rank order, b2p_ppo_combine.
+ * The combines sum in fp64 from rank 0 on, so every rank that combines the same inputs gets the same bits.
+ * b2p_ppo_adv_stats and b2p_ppo_grad are these with R = 1.  Nothing here allocates; transport is the caller's. */
+
+/* Global index of row 0 of every later b2p_act* / b2p_step* launch (default 0; >= 0): local row r draws the noise of
+ * row row_base + r, and everything that depends on it (actions, actions_raw, neglogp) follows. */
+int b2p_set_row_base(b2p_handle h, int64_t row_base);
+
+/* Doubles of one partial vector: the 2 * tower gradient sums before log_std's, then the five loss sums
+ * (2 * tower + 5; 0 for NULL). */
+size_t b2p_ppo_partial_size(b2p_handle h);
+
+/* This shard's part of the gradient over its rows [p->begin, p->begin + p->count) of the minibatch (permutation p->key):
+ * b2p_ppo_grad's kernel with every row scaled by 1 / count_total (count_total = n_m >= p->count), p->adv_stats the
+ * union's (mean, std) from b2p_ppo_adv_combine.  partial_out: double [b2p_ppo_partial_size(h)]; workspace:
+ * b2p_ppo_workspace_size(h) bytes.  p->ent_coef is not read (b2p_ppo_combine applies it). */
+int b2p_ppo_grad_partial(b2p_handle h, const b2p_ppo_batch *b, const b2p_ppo_params *p, int64_t count_total,
+                         double *partial_out, void *workspace, void *stream);
+
+/* partials double [ranks][b2p_ppo_partial_size(h)] (rank order, ranks >= 1) -> grad_out and stats_out as b2p_ppo_grad
+ * writes them, for the union minibatch of count_total rows. */
+int b2p_ppo_combine(b2p_handle h, const double *partials, int ranks, int64_t count_total, float log_std, float ent_coef,
+                    float vf_coef, float *grad_out, double *stats_out, void *stream);
+
+/* moments_out double [T * rows / mb_size][4] = count, shift K (A at the minibatch's first position), sum(A - K),
+ * sum((A - K)^2) of every minibatch of the permutation `key` of this shard's samples, summed as b2p_ppo_adv_stats does.
+ * workspace: b2p_ppo_adv_stats_workspace_size(T * rows, mb_size) bytes.  Errors: b2p_last_error(NULL). */
+int b2p_ppo_adv_moments(const b2p_ppo_batch *b, uint64_t key, int64_t mb_size, double *moments_out, void *workspace,
+                        void *stream);
+
+/* moments double [ranks][nmb][4] (rank order, ranks >= 1) -> stats_out double [nmb][2]: mean and population std of every
+ * union minibatch's advantages.  Shard r's sums are moved to rank 0's shift before they are added.
+ * Errors: b2p_last_error(NULL). */
+int b2p_ppo_adv_combine(const double *moments, int ranks, int64_t nmb, double *stats_out, void *stream);
+
 #ifdef __cplusplus
 }
 #endif
