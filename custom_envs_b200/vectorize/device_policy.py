@@ -442,14 +442,16 @@ class DeviceRolloutBuffer:
 
 
 @torch.no_grad()
-def device_ppo_rollout(env, policy, buffer, gamma=0.99, lam=0.95, ring_only=True, on_step=None):
+def device_ppo_rollout(env, policy, buffer, gamma=0.99, lam=0.95, ring_only=True, on_step=None, seed=None):
     """One PPO2 ``Runner.run`` on the device: ``buffer.n_steps`` times ``model.step`` (``policy.step`` into the
     buffer) then the env step with the clipped actions, then ``model.value`` of the last observation and GAE.
     ``ring_only``: the policy reads the env's rings and the env writes no observation rows (MultiOptLRs, large
     problems); otherwise the policy reads ``env.obs``, which must hold the current observation (the only path
     of the small problems).  ``on_step(t, obs, reward, done, info)`` as in ``device_rollout``.  The done flags
     of the last step become ``dones[0]`` of the next rollout; after ``env.reset()`` call ``buffer.reset()`` so that
-    they are zero, as the Runner starts.  Returns (buffer, finished episodes)."""
+    they are zero, as the Runner starts.  ``seed``: None draws the exploration noise of launch t from the policy's
+    call counter; otherwise launch t draws noise seed ``splitmix64(seed, t)``, so a rollout's noise depends on the
+    seed alone.  Returns (buffer, finished episodes)."""
     T = buffer.n_steps
     assert buffer.actions.numel() == env.num_rows and buffer.rewards.shape[1] == env.num_envs
     if not policy.has_value:
@@ -458,7 +460,8 @@ def device_ppo_rollout(env, policy, buffer, gamma=0.99, lam=0.95, ring_only=True
     buffer.dones[0].copy_(buffer.dones[T])
     for t in range(T):
         source = env if ring_only else env.obs
-        policy._launch(source, policy._seed(None), buffer.actions, buffer.actions_raw[t], buffer.values[t],
+        noise_seed = None if seed is None else splitmix64(seed, t)
+        policy._launch(source, policy._seed(noise_seed), buffer.actions, buffer.actions_raw[t], buffer.values[t],
                        buffer.neglogp[t], buffer.obs_bf16[t])
         obs, reward, done, info = env.step(buffer.actions, ring_only=ring_only)
         buffer.rewards[t].copy_(reward)
@@ -568,12 +571,15 @@ def rank_epoch_key(seed, epoch, rank):
     return key if int(rank) == 0 else _mix64(key + int(rank) * 0x9E3779B97F4A7C15)
 
 
+def splitmix64(seed, index):
+    """The splitmix64 finaliser of seed * 0x9E3779B97F4A7C15 + index + 1 (mod 2^64): the ``index``-th value derived
+    from ``seed``."""
+    return _mix64(int(seed) * 0x9E3779B97F4A7C15 + int(index) + 1)
+
+
 def epoch_key(seed, epoch):
-    """The permutation key of epoch ``epoch`` of an update seeded ``seed`` (splitmix64 of both)."""
-    z = (int(seed) * 0x9E3779B97F4A7C15 + int(epoch) + 1) & (2 ** 64 - 1)
-    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & (2 ** 64 - 1)
-    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & (2 ** 64 - 1)
-    return z ^ (z >> 31)
+    """The permutation key of epoch ``epoch`` of an update seeded ``seed`` (``splitmix64(seed, epoch)``)."""
+    return splitmix64(seed, epoch)
 
 
 def _model_params(model):

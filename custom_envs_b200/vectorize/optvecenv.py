@@ -399,45 +399,50 @@ class OptVecEnv(VecEnv):
         else:
             impl = self._impl
             impl._wait_outputs()
-            agents = impl.env.num_params
             states = impl._states()
-            reward_env = impl._rew_host.numpy()
-            done_env = impl._done_host.numpy().astype(bool)
             info_array = impl._info_host.numpy().copy()
-            overrides = {}
-            if self._fast_monitor:
-                # sum(self.rewards) in Monitor.step adds the float rewards in step order: a
-                # running float64 sum per env is the same arithmetic
-                self._ep_sum += reward_env.astype(np.float64)
-                self._ep_len += 1
-                self._steps[:] = info_array[:, 15].astype(np.int64)
-                for e in np.nonzero(done_env)[0]:
-                    env, core = self._chains[e], self._cores[e]
-                    self._steps[e] = 0
-                    if env is not core:
-                        info = info_row_to_dict(info_array[e])
-                        env._finish_episode(float(self._ep_sum[e]), int(self._ep_len[e]),
-                                            float(reward_env[e]), info)
-                        overrides[e] = info
-                        env.rewards = []                       # what Monitor.reset does
-                        env.current_episode += 1
-                    self._ep_sum[e] = 0.0
-                    self._ep_len[e] = 0
-            for e, (env, core) in enumerate(() if self._fast_monitor else zip(self._chains, self._cores)):
-                core._host_step_done(info_array[e], bool(done_env[e]))
-                if env is core:
-                    continue
-                # replay this env's result through its wrappers (Monitor bookkeeping)
-                core._pending = (float(reward_env[e]), bool(done_env[e]), info_row_to_dict(info_array[e]))
-                _, _, done, info = env.step(None)
-                overrides[e] = info
-                if done:
-                    env.reset()
+            infos = self.replay_env_step(impl._rew_host.numpy(), impl._done_host.numpy().astype(bool), info_array)
             rewards, terminals = impl._row_outputs()
-            infos = LazyInfos(info_array, agents, overrides)
         for callback in self.callbacks:
             callback(states, rewards, terminals, infos)
         return states, rewards, terminals, infos
+
+    def replay_env_step(self, reward_env, done_env, info_array):
+        """Per-env bookkeeping of one step of the fused batch (device-backed path): every env's step counter, and its
+        result replayed through its wrappers, so that Monitors write their ``.mon.csv`` rows, ``get_episode_rewards``
+        grows and ``info['episode']`` is the Monitor's.  ``reward_env`` float32 [E], ``done_env`` bool [E] and
+        ``info_array`` float64 [E, 16] are host arrays of that step (``info_array`` is kept by the result).  Returns
+        the step's ``LazyInfos``.  ``step_wait`` and the device trainer (``custom_envs_b200.ppo2.PPO2``) both call it."""
+        overrides = {}
+        if self._fast_monitor:
+            # sum(self.rewards) in Monitor.step adds the float rewards in step order: a
+            # running float64 sum per env is the same arithmetic
+            self._ep_sum += reward_env.astype(np.float64)
+            self._ep_len += 1
+            self._steps[:] = info_array[:, 15].astype(np.int64)
+            for e in np.nonzero(done_env)[0]:
+                env, core = self._chains[e], self._cores[e]
+                self._steps[e] = 0
+                if env is not core:
+                    info = info_row_to_dict(info_array[e])
+                    env._finish_episode(float(self._ep_sum[e]), int(self._ep_len[e]),
+                                        float(reward_env[e]), info)
+                    overrides[e] = info
+                    env.rewards = []                       # what Monitor.reset does
+                    env.current_episode += 1
+                self._ep_sum[e] = 0.0
+                self._ep_len[e] = 0
+        for e, (env, core) in enumerate(() if self._fast_monitor else zip(self._chains, self._cores)):
+            core._host_step_done(info_array[e], bool(done_env[e]))
+            if env is core:
+                continue
+            # replay this env's result through its wrappers (Monitor bookkeeping)
+            core._pending = (float(reward_env[e]), bool(done_env[e]), info_row_to_dict(info_array[e]))
+            _, _, done, info = env.step(None)
+            overrides[e] = info
+            if done:
+                env.reset()
+        return LazyInfos(info_array, self._impl.env.num_params, overrides)
 
     def close(self):
         if self.closed:
