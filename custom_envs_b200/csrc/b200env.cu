@@ -1157,14 +1157,12 @@ constexpr int OBS_WARPS = 8;
 constexpr int OBS_ITERS = 8;
 constexpr int SEG_ROWS = OBS_WARPS * OBS_ITERS * 32;
 
-template <int HT>
 __global__ void __launch_bounds__(OBS_WARPS * 32) obs_kernel(const __grid_constant__ Dev d,
-                                                             const __grid_constant__ StepArgs a) {
+                                                  const __grid_constant__ StepArgs a) {
     extern __shared__ __align__(16) float sm[];
     __shared__ double red[OBS_WARPS * 4];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int H = HT > 0 ? HT : d.H, OD = d.OD;
-    constexpr int HB = HT > 0 ? HT : 1;
+    const int H = d.H, OD = d.OD;
     float *obsL_s = sm;                                       // [B2E_MAX_HISTORY]
     float *stage = sm + B2E_MAX_HISTORY + warp * (32 * OD + 8);
     const int nitems = a.e_count * d.nseg;
@@ -1192,19 +1190,6 @@ __global__ void __launch_bounds__(OBS_WARPS * 32) obs_kernel(const __grid_consta
         float *rg = d.ringg + (size_t)e * H * d.Pp;
         float *rg_new = rg + (size_t)head * d.Pp;
         float *obs_env = a.obs + (size_t)e * d.P * OD;
-        // per-history-slot base pointers and loss columns (uniform across the CTA)
-        const float *rwh[HB], *rgh[HB];
-        float ol[HB];
-        if (HT > 0) {
-#pragma unroll
-            for (int h = 0; h < HB; ++h) {
-                int slot = head - h;
-                slot += slot < 0 ? HB : 0;
-                rwh[h] = rw + (size_t)slot * d.Pp;
-                rgh[h] = rg + (size_t)slot * d.Pp;
-                ol[h] = obsL_s[h];
-            }
-        }
         float s_absadjg = 0.f, s_gdiff = 0.f, s_state = 0.f;
         for (int it = 0; it < OBS_ITERS; ++it) {
             const int rbase = seg * SEG_ROWS + (it * OBS_WARPS + warp) * 32;
@@ -1213,17 +1198,6 @@ __global__ void __launch_bounds__(OBS_WARPS * 32) obs_kernel(const __grid_consta
             const bool ok = r < d.P;
             const int p = ok ? (d.row_lex ? d.param_of_row[r] : r) : 0;
             const float g = gnew[p], gp = gold[p];
-            float wv[HB], gv[HB];
-            if (HT > 0) {
-#pragma unroll
-                for (int h = 0; h < HB; ++h) {
-                    wv[h] = 0.f; gv[h] = 0.f;
-                    if (h < nvalid) {
-                        wv[h] = rwh[h][p];
-                        if (h > 0) gv[h] = rgh[h][p];
-                    }
-                }
-            }
             // stage so that shared and global memory share their 16-byte phase
             const unsigned w_lo = (unsigned)rbase * OD;           // word offset inside this env's block
             const unsigned sh = (unsigned)((((size_t)e * d.P * OD) + w_lo) & 3);
@@ -1234,29 +1208,18 @@ __global__ void __launch_bounds__(OBS_WARPS * 32) obs_kernel(const __grid_consta
                 s_absadjg += fabsf(ag);
                 s_gdiff += fabsf(g - gp);
             }
-            if (HT > 0) {
-                gv[0] = ag;
-#pragma unroll
-                for (int h = 0; h < HB; ++h) {
-                    if (ok) s_state += fabsf(wv[h]) + fabsf(gv[h]);
-                    srow[h] = clip_only_m1(wv[h]);
-                    srow[HB + h] = ol[h];
-                    srow[2 * HB + h] = clip_only_m1(gv[h]);
+            for (int h = 0; h < H; ++h) {
+                float w1 = 0.f, g1 = 0.f;
+                if (h < nvalid) {
+                    int slot = head - h;
+                    slot += slot < 0 ? H : 0;
+                    w1 = rw[(size_t)slot * d.Pp + p];
+                    g1 = h > 0 ? rg[(size_t)slot * d.Pp + p] : ag;
                 }
-            } else {
-                for (int h = 0; h < H; ++h) {
-                    float w1 = 0.f, g1 = 0.f;
-                    if (h < nvalid) {
-                        int slot = head - h;
-                        slot += slot < 0 ? H : 0;
-                        w1 = rw[(size_t)slot * d.Pp + p];
-                        g1 = h > 0 ? rg[(size_t)slot * d.Pp + p] : ag;
-                    }
-                    if (ok) s_state += fabsf(w1) + fabsf(g1);
-                    srow[h] = clip_only_m1(w1);
-                    srow[H + h] = obsL_s[h];
-                    srow[2 * H + h] = clip_only_m1(g1);
-                }
+                if (ok) s_state += fabsf(w1) + fabsf(g1);
+                srow[h] = clip_only_m1(w1);
+                srow[H + h] = obsL_s[h];
+                srow[2 * H + h] = clip_only_m1(g1);
             }
             __syncwarp();
             // contiguous write of this warp's rows: words [0, nw) of `dst`, stage word i at stage[sh + i]
@@ -1287,159 +1250,30 @@ __global__ void __launch_bounds__(OBS_WARPS * 32) obs_kernel(const __grid_consta
     }
 }
 
-// ------------------------------------------- observation kernel, asynchronous gathers
-// Same work as obs_kernel, organised for memory-level parallelism: a WARP owns 32 units of
-// 32 consecutive agent rows of one env and runs a private S-stage pipeline over them.  The
-// 2H+1 four-byte gathers of a row (g_t, g_{t-1}, H adjusted-weight slots, H-1 adjusted-gradient
-// slots) are cp.async copies into the warp's shared-memory stage, so S units of loads are in
-// flight per warp without holding registers or scoreboard slots; no CTA-wide barrier exists.
-// The 32 finished rows (32 * 3H words, contiguous in HBM) leave either through 16-byte stores
-// or as one cp.async.bulk shared->global copy issued by lane 0.
+// ------------------------------------------- observation kernel, register-batched gathers
+// Same work as obs_kernel, organised for memory-level parallelism (max_history 5): a WARP owns
+// d.obs_units units of 32 consecutive agent rows of one env; no CTA-wide barrier exists.  Every
+// lane issues the 2H+1 four-byte gathers (g_t, g_{t-1}, H adjusted-weight slots, H-1
+// adjusted-gradient slots) of R rows (R units per warp iteration) back to back before the first
+// use, so a warp has R*(2H+1) loads in flight at the LSU cost of plain LDG.  The 32 finished rows
+// (32 * 3H words, contiguous in HBM) leave as one cp.async.bulk shared->global copy issued by
+// lane 0, from two alternating stages.
 constexpr int O2_WARPS = 4;
 constexpr int O2_UNITS = 32;
 
-__device__ __forceinline__ void cp_async4(void *smem_dst, const void *gmem_src) {
-    const unsigned dst = (unsigned)__cvta_generic_to_shared(smem_dst);
-    asm volatile("cp.async.ca.shared.global [%0], [%1], 4;\n" ::"r"(dst), "l"(gmem_src) : "memory");
-}
 __device__ __forceinline__ void bulk_store(void *gmem_dst, const void *smem_src, unsigned bytes) {
     const unsigned src = (unsigned)__cvta_generic_to_shared(smem_src);
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;\n"
                  ::"l"(gmem_dst), "r"(src), "r"(bytes) : "memory");
 }
 
-template <int H, int S, bool BULK>
-__global__ void __launch_bounds__(O2_WARPS * 32) obs_kernel2(const __grid_constant__ Dev d,
-                                                             const __grid_constant__ StepArgs a) {
-    extern __shared__ __align__(16) float sm[];
-    constexpr int OD = 3 * H, NPL = 2 * H + 1, NPL1 = NPL + 1;   // + the row's parameter index
-    constexpr int STG = 32 * OD + 8;
-    constexpr int PER_WARP = S * NPL1 * 32 + (BULK ? 2 : 1) * STG;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int item = blockIdx.x * O2_WARPS + warp;
-    if (item >= a.e_count * d.nseg) return;                  // nseg = 32-unit chunks per env
-    float *gat = sm + warp * PER_WARP;
-    float *stage0 = gat + S * NPL1 * 32;
-    const int eo = item / d.nseg, chunk = item - eo * d.nseg;
-    const int e = a.e_begin + eo;
-    const EnvScalars *sc = d.sc + e;
-    const int head = sc->head, nvalid = sc->nvalid;          // already advanced by the second eval
-    float ol[H];
-    const float *src[NPL];
-    src[0] = d.gnext + (size_t)e * d.Pp;
-    src[1] = d.gprev + (size_t)e * d.Pp;
-#pragma unroll
-    for (int h = 0; h < H; ++h) {
-        int slot = head - h;
-        slot += slot < 0 ? H : 0;
-        ol[h] = clip_m1(h < nvalid ? sc->adj_loss[slot] : 0.f);
-        src[2 + h] = d.ringw + ((size_t)e * H + slot) * d.Pp;
-        if (h > 0) src[2 + H + h - 1] = d.ringg + ((size_t)e * H + slot) * d.Pp;
-    }
-    float *rg_new = d.ringg + ((size_t)e * H + head) * d.Pp;
-    float *obs_env = a.obs + (size_t)e * d.P * OD;
-    const int nblk = (d.P + 31) >> 5;
-    const int u0 = chunk * d.obs_units;
-    const int nu = min(d.obs_units, nblk - u0);
-    auto row_param = [&](int it) -> int {
-        const int r = (u0 + it) * 32 + lane;
-        return r < d.P ? (d.row_lex ? d.param_of_row[r] : r) : 0;
-    };
-    auto issue = [&](int it, int p) {
-        float *dst = gat + (it % S) * (NPL1 * 32) + lane;
-#pragma unroll
-        for (int k = 0; k < NPL; ++k) {
-            const int h = k < 2 ? 0 : (k < 2 + H ? k - 2 : k - 1 - H);
-            if (h < nvalid) cp_async4(dst + k * 32, src[k] + p);
-        }
-        reinterpret_cast<int *>(dst)[NPL * 32] = p;
-    };
-#pragma unroll
-    for (int it = 0; it < S; ++it) {
-        if (it < nu) issue(it, row_param(it));
-        cp_async_commit();
-    }
-    int p_next = S < nu ? row_param(S) : 0;
-    float s_absadjg = 0.f, s_gdiff = 0.f, s_state = 0.f;
-    for (int it = 0; it < nu; ++it) {
-        cp_async_wait<S - 1>();
-        const float *gs = gat + (it % S) * (NPL1 * 32) + lane;
-        const float g = gs[0], gp = gs[32];
-        const int p = reinterpret_cast<const int *>(gs)[NPL * 32];
-        float wv[H], gv[H];
-#pragma unroll
-        for (int h = 0; h < H; ++h) {
-            wv[h] = h < nvalid ? gs[(2 + h) * 32] : 0.f;
-            gv[h] = (h > 0 && h < nvalid) ? gs[(2 + H + h - 1) * 32] : 0.f;
-        }
-        if (it + S < nu) issue(it + S, p_next);              // refill the stage just consumed
-        cp_async_commit();
-        if (it + S + 1 < nu) p_next = row_param(it + S + 1);
-        const int rbase = (u0 + it) * 32;
-        const bool ok = rbase + lane < d.P;
-        const float ag = ratio_nn(g, gp);                    // utils_env.py:156-157
-        if (ok) {
-            rg_new[p] = ag;
-            s_absadjg += fabsf(ag);
-            s_gdiff += fabsf(g - gp);
-        }
-        gv[0] = ag;
-        // stage so that shared and global memory share their 16-byte phase
-        const unsigned w_lo = (unsigned)rbase * OD;
-        const unsigned sh = (unsigned)((((size_t)e * d.P * OD) + w_lo) & 3);
-        float *stage = stage0 + (BULK ? (it & 1) * STG : 0);
-        if (BULK) {
-            if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;\n" ::: "memory");
-            __syncwarp();
-        }
-        float *srow = stage + sh + lane * OD;
-#pragma unroll
-        for (int h = 0; h < H; ++h) {
-            if (ok) s_state += fabsf(wv[h]) + fabsf(gv[h]);
-            srow[h] = clip_only_m1(wv[h]);
-            srow[H + h] = ol[h];
-            srow[2 * H + h] = clip_only_m1(gv[h]);
-        }
-        if (BULK) asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
-        __syncwarp();
-        const unsigned nw = (unsigned)min(32, d.P - rbase) * OD;
-        float *dst = obs_env + w_lo;
-        const float *srcw = stage + sh;
-        const unsigned head_w = min(nw, (4u - sh) & 3u);     // scalars up to the first aligned word
-        const unsigned body_e = head_w + ((nw - head_w) & ~3u);
-        if (lane < head_w) dst[lane] = srcw[lane];
-        if (BULK) {
-            if (lane == 0) {
-                if (body_e > head_w) bulk_store(dst + head_w, srcw + head_w, (body_e - head_w) * 4u);
-                asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
-            }
-        } else {
-            for (unsigned i = head_w + lane * 4; i < body_e; i += 128)
-                *reinterpret_cast<float4 *>(dst + i) = *reinterpret_cast<const float4 *>(srcw + i);
-        }
-        if (body_e + lane < nw) dst[body_e + lane] = srcw[body_e + lane];
-        if (!BULK) __syncwarp();
-    }
-    if (BULK && lane == 0) asm volatile("cp.async.bulk.wait_group 0;\n" ::: "memory");
-    const double v0 = warp_sum((double)s_absadjg), v1 = warp_sum((double)s_gdiff);
-    const double v2 = warp_sum((double)s_state);
-    if (lane == 0) {
-        double *out = d.part + ((size_t)e * d.nseg + chunk) * 4;
-        out[0] = v0; out[1] = v1; out[2] = v2;
-    }
-}
-
-// ------------------------------------------- observation kernel, register-batched gathers
-// As obs_kernel2, but the loads stay in registers: every lane issues the 2H+1 gathers of R
-// rows (R units of 32 rows per warp iteration) back to back before the first use, so a warp
-// has R*(2H+1) loads in flight at the LSU cost of plain LDG.
-template <int H, int R, bool BULK>
+template <int H>
 __global__ void __launch_bounds__(O2_WARPS * 32) obs_kernel3(const __grid_constant__ Dev d,
                                                              const __grid_constant__ StepArgs a) {
     extern __shared__ __align__(16) float sm[];
-    constexpr int OD = 3 * H;
+    constexpr int OD = 3 * H, R = 4;
     constexpr int STG = 32 * OD + 8;
-    constexpr int PER_WARP = (BULK ? 2 : 1) * STG;
+    constexpr int PER_WARP = 2 * STG;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int item = blockIdx.x * O2_WARPS + warp;
     if (item >= a.e_count * d.nseg) return;
@@ -1506,12 +1340,10 @@ __global__ void __launch_bounds__(O2_WARPS * 32) obs_kernel3(const __grid_consta
             gv[j][0] = ag;
             const unsigned w_lo = (unsigned)rbase * OD;
             const unsigned sh = (unsigned)((((size_t)e * d.P * OD) + w_lo) & 3);
-            float *stage = stage0 + (BULK ? (nstore & 1) * STG : 0);
+            float *stage = stage0 + (nstore & 1) * STG;
             ++nstore;
-            if (BULK) {
-                if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;\n" ::: "memory");
-                __syncwarp();
-            }
+            if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;\n" ::: "memory");
+            __syncwarp();
             float *srow = stage + sh + lane * OD;
 #pragma unroll
             for (int h = 0; h < H; ++h) {
@@ -1520,7 +1352,7 @@ __global__ void __launch_bounds__(O2_WARPS * 32) obs_kernel3(const __grid_consta
                 srow[H + h] = ol[h];
                 srow[2 * H + h] = clip_only_m1(gv[j][h]);
             }
-            if (BULK) asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
+            asm volatile("fence.proxy.async.shared::cta;\n" ::: "memory");
             __syncwarp();
             const unsigned nw = (unsigned)min(32, d.P - rbase) * OD;
             float *dst = obs_env + w_lo;
@@ -1528,20 +1360,14 @@ __global__ void __launch_bounds__(O2_WARPS * 32) obs_kernel3(const __grid_consta
             const unsigned head_w = min(nw, (4u - sh) & 3u);
             const unsigned body_e = head_w + ((nw - head_w) & ~3u);
             if (lane < head_w) dst[lane] = srcw[lane];
-            if (BULK) {
-                if (lane == 0) {
-                    if (body_e > head_w) bulk_store(dst + head_w, srcw + head_w, (body_e - head_w) * 4u);
-                    asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
-                }
-            } else {
-                for (unsigned i = head_w + lane * 4; i < body_e; i += 128)
-                    *reinterpret_cast<float4 *>(dst + i) = *reinterpret_cast<const float4 *>(srcw + i);
+            if (lane == 0) {
+                if (body_e > head_w) bulk_store(dst + head_w, srcw + head_w, (body_e - head_w) * 4u);
+                asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
             }
             if (body_e + lane < nw) dst[body_e + lane] = srcw[body_e + lane];
-            if (!BULK) __syncwarp();
         }
     }
-    if (BULK && lane == 0) asm volatile("cp.async.bulk.wait_group 0;\n" ::: "memory");
+    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;\n" ::: "memory");
     const double v0 = warp_sum((double)s_absadjg), v1 = warp_sum((double)s_gdiff);
     const double v2 = warp_sum((double)s_state);
     if (lane == 0) {
@@ -1703,332 +1529,6 @@ __global__ void __launch_bounds__(256, 2) eval_kernel(const __grid_constant__ De
     }
 }
 
-// ------------------------------------------------ tensor-core eval kernel (tcgen05, 3xTF32)
-// The two per-env GEMMs of the one-hidden-layer MLP (BASELINE config 4: D = 784, N1 = 64,
-// B = 32) on the 5th-generation tensor cores:
-//   forward : Hpre^T[j][s] = sum_f W1[f][j] X[s][f]     M = 64 hidden, N = 32 samples, K = D
-//   backward: G[f][j]      = sum_s X[s][f] dPre[s][j]   M = 128 features per tile, N = 64, K = 32
-// fp32 parity (1e-5) is kept with the 3xTF32 split a = hi + lo (hi = the 19 leading bits, which
-// is what the tensor core reads of an fp32 word anyway: profiles/r1_tc_probe.txt):
-// a.b ~ lo.hi + hi.lo + hi.hi, accumulated in fp32 in TMEM; measured error 1.3e-6 of
-// sum|terms| (profiles/r1_tc_fb_probe_v4.txt).  Operands are staged by the threads (global ->
-// registers, one tile ahead -> 4x4 transpose, split -> shared memory) in the K-major
-// no-swizzle canonical layout (core matrix = 8 rows x 16 bytes, K chunks 128 bytes apart,
-// 8-row groups SBO apart; MN-major no-swizzle descriptors do not work for tf32).  One thread
-// issues the MMAs; tcgen05.commit arrives on an mbarrier when the stage may be overwritten.
-// One operand stage per CTA, two CTAs per SM overlap each other.  The tail of the network
-// (bias, relu, second layer, softmax-CE) is the shared-memory code of the FFMA kernels.
-namespace tc {
-constexpr int N1 = 64, B = 32, KT = 56, MT = 128;
-constexpr int SBO_FA = (KT / 4) * 128 + 16;           // forward A = W1^T tile [64 j  x 56 f]
-constexpr int SBO_FB = (KT / 4) * 128;                // forward B = X tile    [32 s  x 56 f]
-constexpr int SBO_BA = (B / 4) * 128 + 16;            // backward A = X^T tile [128 f x 32 s]
-constexpr int SBO_BB = (B / 4) * 128 + 16;            // backward B = dPre^T   [64 j  x 32 s]
-constexpr int A_F = (N1 / 8) * SBO_FA, B_F = (B / 8) * SBO_FB, A_B = (MT / 8) * SBO_BA;
-constexpr int STAGE = 2 * A_F + 2 * B_F;              // 43264 bytes >= 2 * A_B
-constexpr int DP_B = (N1 / 8) * SBO_BB;
-constexpr int OPERAND_BYTES = 2 * STAGE + 2 * DP_B;   // two operand stages + the dPre operand; float region follows
-constexpr int TMEM_COLS = 256;                        // forward 32 columns, backward 2 x 64
-
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ uint64_t make_desc(uint32_t saddr, uint32_t lbo, uint32_t sbo) {
-    return (uint64_t)((saddr >> 4) & 0x3FFF) | ((uint64_t)((lbo >> 4) & 0x3FFF) << 16) |
-           ((uint64_t)((sbo >> 4) & 0x3FFF) << 32) | ((uint64_t)1 << 46);
-}
-__device__ __forceinline__ void mma_tf32(uint32_t tmem, uint64_t ad, uint64_t bd, uint32_t idesc, uint32_t acc) {
-    asm volatile("{\n.reg .pred p;\nsetp.ne.b32 p, %4, 0;\n"
-                 "tcgen05.mma.cta_group::1.kind::tf32 [%0], %1, %2, %3, p;\n}"
-                 ::"r"(tmem), "l"(ad), "l"(bd), "r"(idesc), "r"(acc) : "memory");
-}
-__device__ __forceinline__ void mma_commit(uint64_t *bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool elect_one() {        // one lane of a converged warp (issues the MMAs)
-    uint32_t pred;
-    asm volatile("{\n.reg .pred p;\nelect.sync _|p, 0xffffffff;\nselp.u32 %0, 1, 0, p;\n}" : "=r"(pred));
-    return pred != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    uint32_t done = 0;
-    while (!done)
-        asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
-                     : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-}
-__device__ __forceinline__ void split_store(unsigned char *hi, unsigned char *lo, int off, float4 v) {
-    float4 h, l;
-    // hi = fp32 rounded to nearest at tf32 precision (the tensor core truncates, so the rounding
-    // is done here); lo = exact remainder, |lo| <= 2^-12 |v|
-    h.x = __uint_as_float((__float_as_uint(v.x) + 0x1000u) & 0xFFFFE000u); l.x = v.x - h.x;
-    h.y = __uint_as_float((__float_as_uint(v.y) + 0x1000u) & 0xFFFFE000u); l.y = v.y - h.y;
-    h.z = __uint_as_float((__float_as_uint(v.z) + 0x1000u) & 0xFFFFE000u); l.z = v.z - h.z;
-    h.w = __uint_as_float((__float_as_uint(v.w) + 0x1000u) & 0xFFFFE000u); l.w = v.w - h.w;
-    *reinterpret_cast<float4 *>(hi + off) = h;
-    *reinterpret_cast<float4 *>(lo + off) = l;
-}
-// 4x4 transpose (rows of v = 4 consecutive K indices, columns = 4 consecutive operand rows)
-__device__ __forceinline__ void split_store_t(unsigned char *hi, unsigned char *lo, int off, const float4 (&v)[4]) {
-    split_store(hi, lo, off, make_float4(v[0].x, v[1].x, v[2].x, v[3].x));
-    split_store(hi, lo, off + 16, make_float4(v[0].y, v[1].y, v[2].y, v[3].y));
-    split_store(hi, lo, off + 32, make_float4(v[0].z, v[1].z, v[2].z, v[3].z));
-    split_store(hi, lo, off + 48, make_float4(v[0].w, v[1].w, v[2].w, v[3].w));
-}
-#define B2E_TMEM_LD32(taddr, v) \
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, " \
-                 "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];" \
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), \
-                   "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), \
-                   "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), \
-                   "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31]) \
-                 : "r"(taddr))
-struct Pre { float4 w[4]; float4 x[2]; };            // one tile of global loads held in registers
-}  // namespace tc
-
-template <bool SECOND>
-__global__ void __launch_bounds__(256, 2) tc_eval_kernel(const __grid_constant__ Dev d,
-                                                         const __grid_constant__ StepArgs a) {
-    using namespace tc;
-    extern __shared__ __align__(1024) unsigned char smem_raw[];
-    __shared__ uint32_t tmem_slot;
-    __shared__ __align__(8) uint64_t bar[2];
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    float *sm = reinterpret_cast<float *>(smem_raw);              // Dev offsets (floats) index from here
-    unsigned char *dPhi = smem_raw + 2 * STAGE, *dPlo = dPhi + DP_B;
-    // row-major Hpre / dPre scratch of the tail lives in stage 1 (idle between the two passes);
-    // in the backward pass the same region stages the gradient rows for coalesced stores
-    float *Hb = sm + d.off_H, *dPs = sm + d.off_dP, *misc = sm + d.off_misc;
-    int *idx_s = reinterpret_cast<int *>(sm + d.off_idx);
-    int *ys = reinterpret_cast<int *>(sm + d.off_y);
-    const int D = d.D, NT_F = D / KT, NT_B = (D + MT - 1) / MT;
-    if (tid == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&bar[0])));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&bar[1])));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    if (warp == 0) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(TMEM_COLS));
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-    __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    const uint32_t tmem = tmem_slot;
-    uint32_t uses0 = 0, uses1 = 0;                    // commits issued to each stage barrier (uniform)
-    // forward: ONE 128x64x8 MMA per K step, A = [W_hi ; W_lo] rows, B = [X_hi ; X_lo] rows;
-    // backward: x_hi.[dP_hi ; dP_lo] (128x128x8) and x_lo.dP_hi (128x64x8)
-    const uint32_t idesc_f = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(2 * B >> 3) << 17) | ((uint32_t)(2 * N1 >> 4) << 24);
-    const uint32_t idesc_b = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(N1 >> 3) << 17) | ((uint32_t)(MT >> 4) << 24);
-    const uint32_t idesc_b2 = (1u << 4) | (2u << 7) | (2u << 10) | ((uint32_t)(2 * N1 >> 3) << 17) | ((uint32_t)(MT >> 4) << 24);
-    const uint64_t stage_step = (uint64_t)(STAGE >> 4);
-    const uint64_t dFA = make_desc(smem_u32(smem_raw), 128, SBO_FA);
-    const uint64_t dFB = make_desc(smem_u32(smem_raw + 2 * A_F), 128, SBO_FB);
-    const uint64_t dBAhi = make_desc(smem_u32(smem_raw), 128, SBO_BA), dBAlo = make_desc(smem_u32(smem_raw + A_B), 128, SBO_BA);
-    const uint64_t dBB = make_desc(smem_u32(dPhi), 128, SBO_BB);
-    const int r8 = lane & 7, q4 = lane >> 3;
-    const float4 zero4 = make_float4(0.f, 0.f, 0.f, 0.f);
-    auto wait_stage = [&](int b) {
-        const uint32_t u = b ? uses1 : uses0;
-        if (u) mbar_wait(&bar[b], (u - 1) & 1);
-    };
-    const int e_end = a.e_begin + a.e_count;
-
-    for (int e = a.e_begin + blockIdx.x; e < e_end; e += gridDim.x) {
-        EnvScalars *sc = d.sc + e;
-        const float *We = d.w + (size_t)e * d.Pp;
-        float *gout = d.gnext + (size_t)e * d.Pp;
-        const int *idx; int cnt;
-        current_batch(d, a, e, sc, idx, cnt);
-        __syncthreads();
-        if (tid < B) {
-            const int row = (tid < cnt) ? idx[tid] : -1;          // ragged last batch: missing rows are zeros
-            idx_s[tid] = row;
-            ys[tid] = row >= 0 ? d.labels[row] : 0;
-        }
-        for (int i = tid; i < d.tailP; i += blockDim.x) sm[d.off_tw + i] = We[d.P1 + i];
-        __syncthreads();
-        Pre pre;
-        auto load_fwd = [&](int t) {
-            const int f0 = t * KT;
-            if (tid < (KT / 4) * (N1 / 4)) {
-                const int jq = tid & 15, f4 = tid >> 4;
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-                    pre.w[i] = *reinterpret_cast<const float4 *>(We + (size_t)(f0 + 4 * f4 + i) * N1 + 4 * jq);
-            }
-#pragma unroll
-            for (int u = 0; u < 2; ++u) {
-                const int c = warp + 8 * u, sg = c >> 2, f4 = (c & 3) * 4 + q4;
-                if (f4 < KT / 4) {
-                    const int row = idx_s[sg * 8 + r8];
-                    pre.x[u] = row >= 0 ? *reinterpret_cast<const float4 *>(d.X + (size_t)row * d.Dp + f0 + 4 * f4) : zero4;
-                }
-            }
-        };
-        auto store_fwd = [&](int b) {
-            unsigned char *FAhi = smem_raw + b * STAGE, *FAlo = FAhi + A_F, *FBhi = FAlo + A_F, *FBlo = FBhi + B_F;
-            if (tid < (KT / 4) * (N1 / 4)) {
-                const int jq = tid & 15, f4 = tid >> 4;
-                split_store_t(FAhi, FAlo, (jq >> 1) * SBO_FA + f4 * 128 + (jq & 1) * 64, pre.w);
-            }
-#pragma unroll
-            for (int u = 0; u < 2; ++u) {
-                const int c = warp + 8 * u, sg = c >> 2, f4 = (c & 3) * 4 + q4;
-                if (f4 < KT / 4) split_store(FBhi, FBlo, sg * SBO_FB + f4 * 128 + r8 * 16, pre.x[u]);
-            }
-        };
-        auto load_bwd = [&](int m) {
-            const int f0 = m * MT, f4 = tid & 31, sq = tid >> 5;
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const int row = idx_s[4 * sq + i];
-                pre.w[i] = (row >= 0 && f0 + 4 * f4 < D)
-                               ? *reinterpret_cast<const float4 *>(d.X + (size_t)row * d.Dp + f0 + 4 * f4) : zero4;
-            }
-        };
-        auto store_bwd = [&]() {
-            const int f4 = tid & 31, sq = tid >> 5;
-            split_store_t(smem_raw, smem_raw + A_B, (f4 >> 1) * SBO_BA + sq * 128 + (f4 & 1) * 64, pre.w);
-        };
-
-        // ================= forward: two operand stages; accumulators: even K steps at TMEM columns
-        // [0, 64), odd K steps at [64, 128); rows 0..63 = W_hi, 64..127 = W_lo; columns 0..31 = X_hi
-        load_fwd(0);
-        for (int t = 0; t < NT_F; ++t) {
-            const int b = t & 1;
-            wait_stage(b);                                        // MMAs of tile t-2 done: stage b is free
-            store_fwd(b);
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            __syncthreads();
-            if (warp == 0 && elect_one()) {
-                // the barrier made every thread's st.shared visible to this thread; one proxy fence
-                // orders them before the tensor core's (async proxy) reads
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-                const uint64_t so = b ? stage_step : 0;
-#pragma unroll
-                for (int ks = 0; ks < KT / 8; ++ks) {                        // 8 features = two 16-byte chunks
-                    const uint64_t ko = so + (uint64_t)(ks * 256 >> 4);
-                    mma_tf32(tmem + 64 * (ks & 1), dFA + ko, dFB + ko, idesc_f, (t == 0 && ks < 2) ? 0u : 1u);
-                }
-                mma_commit(&bar[b]);
-            }
-            if (b) uses1++; else uses0++;
-            if (t + 1 < NT_F) load_fwd(t + 1); else load_bwd(0);     // in flight while the tensor core works
-        }
-        wait_stage(0);
-        wait_stage(1);
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-        if (warp < 4) {   // M = 128: accumulator row r sits in TMEM lane r
-            float acc[32];
-#pragma unroll
-            for (int i = 0; i < 32; ++i) acc[i] = 0.f;
-#pragma unroll
-            for (int k = 0; k < 4; ++k) {                         // small products first: X_lo columns, then X_hi
-                const int col = (k < 2 ? 32 : 0) + ((k & 1) ? 0 : 64);
-                uint32_t v[32];
-                B2E_TMEM_LD32(tmem + ((uint32_t)(warp * 32) << 16) + col, v);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-                for (int i = 0; i < 32; ++i) acc[i] += __uint_as_float(v[i]);
-            }
-            const int j = (warp & 1) * 32 + lane;
-            if (warp >= 2) {                                       // W_lo rows: hand the partial sums over
-#pragma unroll
-                for (int s = 0; s < B; ++s) dPs[s * N1 + j] = acc[s];
-            }
-            asm volatile("bar.sync 1, 128;" ::: "memory");
-            if (warp < 2) {
-#pragma unroll
-                for (int s = 0; s < B; ++s) Hb[s * N1 + j] = acc[s] + dPs[s * N1 + j];
-            }
-        }
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        __syncthreads();
-        // ================= tail: bias, relu, second layer, softmax-CE -> dPre [B][N1], tail gradient
-        const float loss = d.C == 10 ? tail_eval<64, 10>(d, sm, cnt) : tail_eval(d, sm, cnt);
-        float gsum = 0.f;
-        for (int i = tid; i < d.tailP; i += blockDim.x) {
-            const float g = sm[d.off_tg + i];
-            gout[d.P1 + i] = g;
-            gsum += g;
-        }
-        // dPre -> B operand (N = hidden j, K = sample s): thread = 4 samples x 4 hidden units
-        if (tid < (B / 4) * (N1 / 4)) {
-            const int jq = tid & 15, sq = tid >> 4;
-            float4 v[4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) v[i] = *reinterpret_cast<const float4 *>(dPs + (4 * sq + i) * N1 + 4 * jq);
-            split_store_t(dPhi, dPlo, (jq >> 1) * SBO_BB + sq * 128 + (jq & 1) * 64, v);
-        }
-        __syncthreads();                                          // the scratch in stage 1 is dead from here
-        // ================= backward: one operand stage (stage 0); accumulators P = x_hi.[dP_hi ; dP_lo]
-        // at TMEM columns [0, 128), Q = x_lo.dP_hi at [128, 192); G = P[:, 0:64] + P[:, 64:128] + Q
-        float *scr = reinterpret_cast<float *>(smem_raw + STAGE) + warp * (32 * 33);
-        auto readout = [&](int m) {
-            wait_stage(0);
-            asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            const int q = warp & 3, half = warp >> 2;                 // lanes 32q.., columns 32*half.. of each block
-            float acc[32];
-#pragma unroll
-            for (int i = 0; i < 32; ++i) acc[i] = 0.f;
-#pragma unroll
-            for (int k = 0; k < 3; ++k) {
-                const int col = (k == 0 ? 128 : k == 1 ? 64 : 0) + 32 * half;
-                uint32_t v[32];
-                B2E_TMEM_LD32(tmem + ((uint32_t)(q * 32) << 16) + col, v);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-                for (int i = 0; i < 32; ++i) acc[i] += __uint_as_float(v[i]);
-            }
-            // lane = feature row; transpose through shared memory so that a warp store covers one row
-#pragma unroll
-            for (int i = 0; i < 32; ++i) scr[lane * 33 + i] = acc[i];
-            __syncwarp();
-            const int fbase = m * MT + q * 32;
-            for (int r = 0; r < 32; ++r) {
-                if (fbase + r < D) {
-                    const float g = scr[r * 33 + lane];
-                    gout[(size_t)(fbase + r) * N1 + 32 * half + lane] = g;
-                    gsum += g;
-                }
-            }
-            __syncwarp();
-        };
-        for (int m = 0; m < NT_B; ++m) {
-            wait_stage(0);                                        // tile m-1 multiplied: stage and accumulators free
-            store_bwd();
-            if (m >= 1) readout(m - 1);
-            asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-            __syncthreads();
-            if (warp == 0 && elect_one()) {
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-#pragma unroll
-                for (int ks = 0; ks < B / 8; ++ks) {                     // 8 samples = two 16-byte chunks
-                    const uint64_t ko = (uint64_t)(ks * 256 >> 4);
-                    mma_tf32(tmem, dBAhi + ko, dBB + ko, idesc_b2, ks ? 1u : 0u);
-                    mma_tf32(tmem + 128, dBAlo + ko, dBB + ko, idesc_b, ks ? 1u : 0u);
-                }
-                mma_commit(&bar[0]);
-            }
-            uses0++;
-            if (m + 1 < NT_B) load_bwd(m + 1);
-        }
-        readout(NT_B - 1);
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        if (!SECOND) continue;
-        // ---- scalars of the step (thread 0): history bookkeeping, reward, done, info
-        __syncthreads();                                          // the reduction scratch shares stage 1
-        const double gtot = block_sum((double)gsum, reinterpret_cast<double *>(sm + d.off_red2));
-        if (tid == 0) step_scalars(d, a, sc, e, loss, gtot, misc);
-        __syncthreads();
-        const bool wrap = misc[4] != 0.f;
-        __syncthreads();
-        if (wrap) shuffle_order(d, e, sc);
-    }
-    __syncthreads();
-    if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(TMEM_COLS));
-}
-
 // ------------------------------------------------ eval kernel, bulk-copy operand pipeline
 // eval_kernel<., 64, 112> with the operand tiles moved by the copy engine instead of the threads:
 // per tile ONE cp.async.bulk for the contiguous 28 KB W1 tile and one per minibatch row piece
@@ -2037,38 +1537,35 @@ __global__ void __launch_bounds__(256, 2) tc_eval_kernel(const __grid_constant__
 // removes the per-thread cp.async issue loops and the two CTA barriers per tile.
 namespace bk {
 constexpr int N1 = 64, KT = 112, B = 32, XS = 116;
+__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void mbar_init(uint64_t *bar, int count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(tc::smem_u32(bar)), "r"(count));
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
 }
 __device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(tc::smem_u32(bar)) : "memory");
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void mbar_expect(uint64_t *bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(tc::smem_u32(bar)), "r"(bytes) : "memory");
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
+    uint32_t done = 0;
+    while (!done)
+        asm volatile("{\n.reg .pred p;\nmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\nselp.u32 %0, 1, 0, p;\n}"
+                     : "=r"(done) : "r"(smem_u32(bar)), "r"(parity) : "memory");
 }
 __device__ __forceinline__ void bulk_load(void *smem_dst, const void *gmem_src, unsigned bytes, uint64_t *bar) {
     asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(tc::smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(tc::smem_u32(bar)) : "memory");
+                 ::"r"(smem_u32(smem_dst)), "l"(gmem_src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 }  // namespace bk
 
-// FUSED (first eval only): the update w_t = w_{t-1} - g0 * lr(action) (update_kernel's work) happens in
-// the backward epilogue while the gradient tile is still in registers: the W1 tile is bulk-copied
-// a second time into the W stage that idles during the backward pass (an L2 hit mostly: this CTA
-// read it a few microseconds ago), so g0 is never written, and w / g0 are not re-read from HBM by a
-// separate kernel.  Saves 3 of the step's 35 words per parameter and one launch -- but no time:
-// measured 1.54 ms against 0.84 + 0.70 ms for the two kernels (profiles/r1_notes.md): the epilogue's
-// dependent chain (row lookup -> action gather -> arithmetic -> stores) is appended to each CTA's
-// timeline with nothing running underneath it, while the separate update kernel streams at 90 % of
-// the HBM rate.  Opt-in (B2E_FUSE_UPDATE=1).
-template <bool SECOND, bool FUSED = false>
+template <bool SECOND>
 __global__ void __launch_bounds__(256, 2) eval_bulk_kernel(const __grid_constant__ Dev d,
                                                            const __grid_constant__ StepArgs a) {
     using namespace bk;
     constexpr int PRODUCER = 7;       // the warp that refills the stages: idle in the backward tiles (kl >= KT)
     extern __shared__ __align__(16) float sm[];
-    __shared__ __align__(8) uint64_t full[2], empty[2], wfull[2];
-    static_assert(!(SECOND && FUSED), "the update belongs to the first eval");
+    __shared__ __align__(8) uint64_t full[2], empty[2];
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     float *const X0 = sm + d.ev_X0, *const W0 = sm + d.ev_W0;
     const int xstep = d.ev_X1 - d.ev_X0, wstep = d.ev_W1 - d.ev_W0;   // stage s at X0 + s * xstep
@@ -2079,21 +1576,15 @@ __global__ void __launch_bounds__(256, 2) eval_bulk_kernel(const __grid_constant
     if (tid == 0) {
         mbar_init(&full[0], 1); mbar_init(&full[1], 1);
         mbar_init(&empty[0], 8); mbar_init(&empty[1], 8);
-        mbar_init(&wfull[0], 1); mbar_init(&wfull[1], 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     __syncthreads();
-    unsigned fph = 0, eph = 0, wph = 0;                       // bit s: phase parity of stage s (warp-uniform)
+    unsigned fph = 0, eph = 0;                                // bit s: phase parity of stage s (warp-uniform)
     const int e_end = a.e_begin + a.e_count;
     for (int e = a.e_begin + blockIdx.x; e < e_end; e += gridDim.x) {
         EnvScalars *sc = d.sc + e;
         const float *wE = d.w + (size_t)e * d.Pp;
         float *gout = d.gnext + (size_t)e * d.Pp;
-        float *wOut = d.w + (size_t)e * d.Pp;                                                  // FUSED: updated in place
-        float *rw = d.ringw + ((size_t)e * d.H + (sc->head + 1) % d.H) * d.Pp;                 // FUSED: adjusted weights
-        const float *act = a.actions + (size_t)e * d.P;
-        float s_absw = 0.f;
-        double s_lr = 0.0, s_lr2 = 0.0;
         const int *idx; int cnt;
         current_batch(d, a, e, sc, idx, cnt);
         __syncthreads();
@@ -2115,18 +1606,8 @@ __global__ void __launch_bounds__(256, 2) eval_bulk_kernel(const __grid_constant
             if (lane < cnt) bulk_load(X0 + s * xstep + lane * XS, d.X + (size_t)idx_s[lane] * d.Dp + k0, KT * 4, &full[s]);
             if (with_w && lane == 0) bulk_load(W0 + s * wstep, wE + (size_t)k0 * N1, KT * N1 * 4, &full[s]);
         };
-        // FUSED: old weights of backward tile q into the idle W stage (own barrier: the first two are
-        // requested only after the forward partials have left the W stages)
-        auto issue_w = [&](int q) {                            // producer warp only
-            const int s = q & 1, k0 = (q - NT) * KT;
-            if (lane == 0) {
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                mbar_expect(&wfull[s], KT * N1 * 4);
-                bulk_load(W0 + s * wstep, wE + (size_t)k0 * N1, KT * N1 * 4, &wfull[s]);
-            }
-        };
         auto wait_full = [&](int s) {
-            tc::mbar_wait(&full[s], (fph >> s) & 1u);
+            mbar_wait(&full[s], (fph >> s) & 1u);
             fph ^= 1u << s;
         };
         // This warp is done with the stage of tile q.  The producer warp then waits until every warp
@@ -2138,12 +1619,9 @@ __global__ void __launch_bounds__(256, 2) eval_bulk_kernel(const __grid_constant
             if (lane == 0) mbar_arrive(&empty[q & 1]);
             if (warp == PRODUCER) {
                 const int s = q & 1;
-                tc::mbar_wait(&empty[s], (eph >> s) & 1u);
+                mbar_wait(&empty[s], (eph >> s) & 1u);
                 eph ^= 1u << s;
-                if (q + 2 < 2 * NT) {
-                    issue(q + 2);
-                    if (FUSED && q >= NT) issue_w(q + 2);
-                }
+                if (q + 2 < 2 * NT) issue(q + 2);
             }
         };
         if (warp == PRODUCER) { issue(0); issue(1); }
@@ -2161,26 +1639,13 @@ __global__ void __launch_bounds__(256, 2) eval_bulk_kernel(const __grid_constant
         }
         __syncthreads();                                      // every warp is done with the W tiles
         f_store_fast<N1>(d, sm, acc);                         // partials reduced through the W tiles
-        if (FUSED && warp == PRODUCER) { issue_w(NT); if (NT > 1) issue_w(NT + 1); }
         const float loss = d.C == 10 ? tail_eval<N1, 10>(d, sm, cnt) : tail_eval<N1, 0>(d, sm, cnt);
 
         // ---- backward: tail gradient, then g = X^T . dPre tile by tile, straight to HBM
         float gsum = 0.f;
         for (int i = tid; i < d.tailP; i += blockDim.x) {
             const float g = sm[d.off_tg + i];
-            if (FUSED) {                                      // b1, W2, b2: same update, one parameter at a time
-                const int p = d.P1 + i;
-                const float wo = wE[p];
-                const float lr = action_to_lr(act[d.row_lex ? d.row_of_param[p] : p], d.act_ver);
-                const float wn = fmaf(-g, lr, wo);
-                wOut[p] = wn;
-                rw[p] = ratio_nn(wn, wo);
-                s_absw += fabsf(wn);
-                s_lr += (double)lr;
-                s_lr2 += (double)lr * (double)lr;
-            } else {
-                gout[d.P1 + i] = g;
-            }
+            gout[d.P1 + i] = g;
             gsum += g;
         }
         const int rgi = tid >> 3, cgi = tid & 7, kl = rgi * 4;
@@ -2211,82 +1676,20 @@ __global__ void __launch_bounds__(256, 2) eval_bulk_kernel(const __grid_constant
                         ffma2(g2[j][3], x2, d1.y);
                     }
                 }
-                if (!FUSED) release(q);                       // the tile is in registers now
+                release(q);                                   // the tile is in registers now
 #pragma unroll
                 for (int j = 0; j < 4; ++j)
 #pragma unroll
                     for (int c = 0; c < 4; ++c) unpack2(g2[j][c], g[j][2 * c], g[j][2 * c + 1]);
-                if (FUSED) {
-                    // rows of the agents first (the only dependent loads), all in flight at once
-                    const int pbase = (k0 + kl) * N1 + 4 * cgi;
-                    int4 r4[4][2];
 #pragma unroll
-                    for (int j = 0; j < 4; ++j)
-#pragma unroll
-                        for (int hh = 0; hh < 2; ++hh) {
-                            const int p = pbase + j * N1 + hh * half;
-                            r4[j][hh] = d.row_lex ? *reinterpret_cast<const int4 *>(d.row_of_param + p)
-                                                  : make_int4(p, p + 1, p + 2, p + 3);
-                        }
-                    float av[4][8];
-#pragma unroll
-                    for (int j = 0; j < 4; ++j)
-#pragma unroll
-                        for (int hh = 0; hh < 2; ++hh) {
-                            av[j][4 * hh + 0] = act[r4[j][hh].x]; av[j][4 * hh + 1] = act[r4[j][hh].y];
-                            av[j][4 * hh + 2] = act[r4[j][hh].z]; av[j][4 * hh + 3] = act[r4[j][hh].w];
-                        }
-                    tc::mbar_wait(&wfull[q & 1], (wph >> (q & 1)) & 1u);
-                    wph ^= 1u << (q & 1);
-                    const float *ws = W0 + (q & 1) * wstep + kl * N1 + 4 * cgi;
-#pragma unroll
-                    for (int j = 0; j < 4; ++j)
-#pragma unroll
-                        for (int hh = 0; hh < 2; ++hh) {
-                            const float4 wo4 = *reinterpret_cast<const float4 *>(ws + j * N1 + hh * half);
-                            const float wo[4] = {wo4.x, wo4.y, wo4.z, wo4.w};
-                            float wn[4], aw[4];
-#pragma unroll
-                            for (int c = 0; c < 4; ++c) {
-                                const float lr = action_to_lr(av[j][4 * hh + c], d.act_ver);
-                                wn[c] = fmaf(-g[j][4 * hh + c], lr, wo[c]);
-                                aw[c] = ratio_nn(wn[c], wo[c]);          // utils_env.py:158-159
-                                s_absw += fabsf(wn[c]);
-                                s_lr += (double)lr;
-                                s_lr2 += (double)lr * (double)lr;
-                            }
-                            const int p = pbase + j * N1 + hh * half;
-                            *reinterpret_cast<float4 *>(wOut + p) = make_float4(wn[0], wn[1], wn[2], wn[3]);
-                            *reinterpret_cast<float4 *>(rw + p) = make_float4(aw[0], aw[1], aw[2], aw[3]);
-                        }
-                    release(q);                               // the old weights have been read
-#pragma unroll
-                    for (int j = 0; j < 4; ++j)
-                        gsum += ((g[j][0] + g[j][1]) + (g[j][2] + g[j][3])) + ((g[j][4] + g[j][5]) + (g[j][6] + g[j][7]));
-                } else {
-#pragma unroll
-                    for (int j = 0; j < 4; ++j) {
-                        float *dst = gout + (size_t)(k0 + kl + j) * N1 + 4 * cgi;
-                        *reinterpret_cast<float4 *>(dst) = make_float4(g[j][0], g[j][1], g[j][2], g[j][3]);
-                        *reinterpret_cast<float4 *>(dst + half) = make_float4(g[j][4], g[j][5], g[j][6], g[j][7]);
-                        gsum += ((g[j][0] + g[j][1]) + (g[j][2] + g[j][3])) + ((g[j][4] + g[j][5]) + (g[j][6] + g[j][7]));
-                    }
+                for (int j = 0; j < 4; ++j) {
+                    float *dst = gout + (size_t)(k0 + kl + j) * N1 + 4 * cgi;
+                    *reinterpret_cast<float4 *>(dst) = make_float4(g[j][0], g[j][1], g[j][2], g[j][3]);
+                    *reinterpret_cast<float4 *>(dst + half) = make_float4(g[j][4], g[j][5], g[j][6], g[j][7]);
+                    gsum += ((g[j][0] + g[j][1]) + (g[j][2] + g[j][3])) + ((g[j][4] + g[j][5]) + (g[j][6] + g[j][7]));
                 }
             } else {                                          // the producer warp has no rows here
-                if (FUSED) {
-                    tc::mbar_wait(&wfull[q & 1], (wph >> (q & 1)) & 1u);
-                    wph ^= 1u << (q & 1);
-                }
                 release(q);
-            }
-        }
-        if (FUSED) {                                          // update_kernel's statistics, whole env in segment 0
-            double *red = reinterpret_cast<double *>(sm + d.off_red2);
-            const double t0 = block_sum((double)s_absw, red), t1 = block_sum(s_lr, red), t2 = block_sum(s_lr2, red);
-            if (tid == 0) {
-                double *out = d.part_u + (size_t)e * d.nsegU * 4;
-                out[0] = t0; out[1] = t1; out[2] = t2;
-                for (int seg = 1; seg < d.nsegU; ++seg) { out[seg * 4] = 0.0; out[seg * 4 + 1] = 0.0; out[seg * 4 + 2] = 0.0; }
             }
         }
         if (!SECOND) continue;
@@ -3388,26 +2791,18 @@ struct b2e_env {
     double *part;
     EnvScalars *sc;
     size_t smem_obs;
-    int chunk_envs, obs_grid;
     bool use_eval_kernel;            // first layer fits the streamed-operand eval kernel
     bool eval_c;                     // eval_kernel instantiated for N1 = 64, KT = 112 (config 4)
-    bool fuse_update;                // first eval applies the update itself (eval_bulk_kernel<false, true>; opt-in with B2E_FUSE_UPDATE=1)
-    bool eval_bulk;                  // ... and its bulk-copy / mbarrier pipelined form (B2E_EVAL_BULK=0 disables)
-    int nchunks, eval_ctas_per_sm;   // B2E_CHUNKS experiment
+    bool eval_bulk;                  // ... and its bulk-copy / mbarrier pipelined form (softmax)
     bool use_thin;                   // softmax regression: thin_eval_kernel
-    bool thin_fused;                 // ... whose cluster form runs eval / update / eval of a MultiOptLRs step as ONE launch (opt-in: B2E_THIN_FUSE=1)
     bool use_thin2;                  // ... its shared-memory-resident successor for 10 classes (b200thin.cu; B2E_THIN2=0 disables)
     size_t smem_thin;
     int thin_kc;
-    bool use_tc;                     // tcgen05 eval kernel replaces eval_kernel
-    Dev d_tc;                        // Dev with the tensor-core kernel's shared-memory layout
-    size_t smem_tc;
-    int tc_grid;
     bool use_tc2;                    // warp-specialised tcgen05 eval kernel (b200tc.cu)
     b2e_tc2_ctx *tc2;                // its context: tensor map, watchdog word, grid
     bool tc2_check;                  // B2E_TC_CHECK=1: synchronise and test the watchdog after every step
     float *w2, *g2, *ws;
-    int obs_stages, obs_regs, obs_bulk;        // obs_kernel2 variant (0 stages = obs_kernel)
+    bool use_obs3;                   // observation rows by obs_kernel3 (max_history 5 on the large-problem pipeline)
     size_t smem_obs2;
     Dev d_eval;                      // Dev with the eval kernel's shared-memory layout
     size_t smem_eval;
@@ -3418,10 +2813,6 @@ struct b2e_env {
     bool reset_pipeline;
     bool use_tiny;                   // warp-per-env kernel for tiny problems (b200tiny.cu; B2E_TINY=0 disables)
     double *part_r, *slot_abs;       // ring-only steps: ring_adjg_kernel's partial sums, per-slot sums of |adjusted x|
-    cudaStream_t side;               // the observation kernel runs here (lowest priority) ...
-    cudaStream_t hi;                 // ... next to the compute kernel (highest priority)
-    cudaEvent_t ev_fork, ev_join;
-    cudaEvent_t ev_chunk[64];
     bool dataset_bound, stream_bound;
     bool trace;                      // record per-kernel events in b2e_step
     cudaEvent_t tr[8];
@@ -3484,27 +2875,6 @@ std::string lex_rows(int num_params, int *row_of_param_host) {
     }
     delete[] stack;
     return next_row == num_params ? "" : "internal error in lexicographic row table";
-}
-
-const void *obs2_fn(int stages, int regs, int bulk) {
-    if (regs) {
-        switch (regs * 2 + (bulk ? 1 : 0)) {
-            case 2: return (const void *)obs_kernel3<5, 1, false>;
-            case 3: return (const void *)obs_kernel3<5, 1, true>;
-            case 4: return (const void *)obs_kernel3<5, 2, false>;
-            case 5: return (const void *)obs_kernel3<5, 2, true>;
-            case 8: return (const void *)obs_kernel3<5, 4, false>;
-            default: return (const void *)obs_kernel3<5, 4, true>;
-        }
-    }
-    switch (stages * 2 + (bulk ? 1 : 0)) {
-        case 6: return (const void *)obs_kernel2<5, 3, false>;
-        case 7: return (const void *)obs_kernel2<5, 3, true>;
-        case 8: return (const void *)obs_kernel2<5, 4, false>;
-        case 9: return (const void *)obs_kernel2<5, 4, true>;
-        case 12: return (const void *)obs_kernel2<5, 6, false>;
-        default: return (const void *)obs_kernel2<5, 6, true>;
-    }
 }
 
 int configure(b2e_handle h) {
@@ -3656,31 +3026,15 @@ int configure(b2e_handle h) {
         d.doff1 = o; o += round_up(d.B * maxw, 4);
         d.ws_stride = o;
     }
-    {   // observation kernel variant: B2E_OBS = "<stages><b|s>" (cp.async gathers, e.g. "4b"),
-        // "r<rows><b|s>" (register-batched gathers, e.g. "r4b"), "0" = obs_kernel;
-        // b = cp.async.bulk row-block stores, s = 16-byte stores
-        const char *v = getenv("B2E_OBS");
-        h->obs_stages = 0; h->obs_regs = 4; h->obs_bulk = 1;
-        if (v && *v) {
-            h->obs_bulk = strchr(v, 's') ? 0 : 1;
-            if (*v == 'r') { h->obs_regs = atoi(v + 1); h->obs_stages = 0; }
-            else { h->obs_stages = atoi(v); h->obs_regs = 0; }
-        }
-        if (h->obs_stages != 0 && h->obs_stages != 3 && h->obs_stages != 4 && h->obs_stages != 6)
-            return fail(h, "B2E_OBS: stages must be 0, 3, 4 or 6");
-        if (h->obs_regs != 0 && h->obs_regs != 1 && h->obs_regs != 2 && h->obs_regs != 4)
-            return fail(h, "B2E_OBS: rows per lane must be 1, 2 or 4");
-        if (d.H != 5 || !d.split || c.env_kind != B2E_ENV_MULTIOPTLRS) h->obs_stages = h->obs_regs = 0;
-        if (h->obs_stages || h->obs_regs) {
-            // warp items of 32 units; small batches (BASELINE config 3: 8192 such items = 3.5 waves of the 296 resident
-            // CTAs) get 8-unit items, so that the last wave is 1/14 instead of 1/4 of the kernel
-            const int nblk = (d.P + 31) / 32;
-            const long long items32 = (long long)d.E * ((nblk + O2_UNITS - 1) / O2_UNITS);
-            d.obs_units = items32 < 8LL * 2 * O2_WARPS * h->num_sms ? 8 : O2_UNITS;
-            d.nseg = (nblk + d.obs_units - 1) / d.obs_units;
-            const int npl1 = 2 * d.H + 2, stg = 32 * d.OD + 8;
-            h->smem_obs2 = (size_t)O2_WARPS * (h->obs_stages * npl1 * 32 + (h->obs_bulk ? 2 : 1) * stg) * sizeof(float);
-        }
+    h->use_obs3 = d.H == 5 && d.split && c.env_kind == B2E_ENV_MULTIOPTLRS;
+    if (h->use_obs3) {
+        // obs_kernel3: warp items of 32 units; small batches (BASELINE config 3: 8192 such items = 3.5 waves of the 296
+        // resident CTAs) get 8-unit items, so that the last wave is 1/14 instead of 1/4 of the kernel
+        const int nblk = (d.P + 31) / 32;
+        const long long items32 = (long long)d.E * ((nblk + O2_UNITS - 1) / O2_UNITS);
+        d.obs_units = items32 < 8LL * 2 * O2_WARPS * h->num_sms ? 8 : O2_UNITS;
+        d.nseg = (nblk + d.obs_units - 1) / d.obs_units;
+        h->smem_obs2 = (size_t)O2_WARPS * 2 * (32 * d.OD + 8) * sizeof(float);
     }
     h->smem_obs = (size_t)(B2E_MAX_HISTORY + OBS_WARPS * (32 * d.OD + 8)) * sizeof(float);
     d.nsegU = (d.Pp + UPD_SEG - 1) / UPD_SEG;
@@ -3708,30 +3062,6 @@ int configure(b2e_handle h) {
         v.off_misc = o; o += 8 + 2 * B2E_MAX_HISTORY;
         h->smem_eval = (size_t)o * sizeof(float);
         v.split = d.split;
-    }
-    {   // tensor-core eval kernel: operand stage first, then the float regions of the tail
-        // opt-in (B2E_TC=1): parity-green, but in the step pipeline it is still slower than the FFMA
-        // eval kernel (1.24 vs 1.12 ms at 4096 envs; profiles/r1_notes.md has the analysis)
-        const char *tcv = getenv("B2E_TC");
-        h->use_tc = h->use_eval_kernel && d.hidden && d.N1 == tc::N1 && d.N1p == tc::N1 && d.B == tc::B &&
-                    d.D % tc::KT == 0 && d.kind == B2E_PROBLEM_SOFTMAX && tcv && atoi(tcv) != 0;
-        h->d_tc = d;
-        Dev &v = h->d_tc;
-        // scratch that only lives between the two passes sits inside operand stage 1
-        int in1 = tc::STAGE / 4;
-        v.off_H = in1; in1 += round_up(d.B * d.N1p, 4);
-        v.off_dP = in1; in1 += round_up(d.B * d.N1p, 4);
-        v.off_Z = in1; in1 += d.hidden ? round_up(d.B * d.Cp, 4) : 0;
-        v.off_lb = in1; in1 += round_up(d.B, 4);
-        v.off_red2 = in1; in1 += 2 * NSTAT * 16;
-        if (in1 > 2 * tc::STAGE / 4) h->use_tc = false;
-        int o = tc::OPERAND_BYTES / 4;
-        v.off_tw = o; o += round_up(d.tailP, 4);
-        v.off_tg = o; o += round_up(d.tailP, 4);
-        v.off_idx = o; o += round_up(d.B, 4);
-        v.off_y = o; o += round_up(d.B, 4);
-        v.off_misc = o; o += 8 + 2 * B2E_MAX_HISTORY;
-        h->smem_tc = (size_t)o * sizeof(float);
     }
     return 0;
 }
@@ -3777,6 +3107,38 @@ int launch(b2e_handle h, StepArgs args, void *stream) {
     } else {
         if (h->d.H == 5) optenv_kernel<5, false><<<h->grid, h->nthreads, h->smem_bytes, cs>>>(h->d, args);
         else optenv_kernel<0, false><<<h->grid, h->nthreads, h->smem_bytes, cs>>>(h->d, args);
+    }
+    h->launches++;
+    CUDA_TRY(h, cudaGetLastError());
+    return 0;
+}
+
+// One evaluation pass of a large-problem step on the kernel chosen at creation: the loss and gradient
+// (-> gnext) at w_{t-1} (SECOND = false) or at w_t together with the step's scalars (SECOND = true).
+// dv is h->d_eval with the step's pointers.
+template <bool SECOND>
+int eval_pass(b2e_handle h, const StepArgs &a, cudaStream_t s) {
+    const Dev &d = h->d, &dv = h->d_eval;
+    const int grid_ev = d.E < h->eval_grid ? d.E : h->eval_grid;
+    if (h->use_tc2) {
+        if (b2e_tc2_launch(h->tc2, &d, &a, SECOND, s)) return fail(h, "tc2 launch failed");
+    } else if (h->use_eval_kernel) {
+        if (h->eval_bulk) eval_bulk_kernel<SECOND><<<grid_ev, 256, h->smem_eval, s>>>(dv, a);
+        else if (h->eval_c) eval_kernel<SECOND, 64, 112><<<grid_ev, 256, h->smem_eval, s>>>(dv, a);
+        else eval_kernel<SECOND><<<grid_ev, 256, h->smem_eval, s>>>(dv, a);
+    } else if (h->use_thin) {
+        if (h->use_thin2) {
+            if (b2e_thin2_launch(&d, &a, SECOND, h->num_sms, s)) return fail(h, "thin2 launch failed");
+        } else {
+            Dev dt = d;
+            dt.KT = h->thin_kc;
+            if (d.C == 10) thin_eval_kernel<SECOND, 10><<<grid_ev, 256, h->smem_thin, s>>>(dt, a);
+            else thin_eval_kernel<SECOND><<<grid_ev, 256, h->smem_thin, s>>>(dt, a);
+        }
+    } else {                                                 // generic dense stack
+        StepArgs b = a;
+        b.mode = SECOND ? MODE_EVAL_STEP : MODE_EVAL_FIRST;
+        return launch(h, b, s);
     }
     h->launches++;
     CUDA_TRY(h, cudaGetLastError());
@@ -3842,16 +3204,14 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
     if (!h) return fail(nullptr, "b2e_create: out of host memory");
     h->cfg = *cfg;
     h->launches = 0;
-    h->nchunks = 1; h->eval_ctas_per_sm = 2; h->eval_c = false; h->eval_bulk = false;
+    h->eval_c = false; h->eval_bulk = false;
     h->dataset_bound = h->stream_bound = false;
     h->trace = false; h->tr_count = 0;
     for (auto &ev : h->tr) ev = nullptr;
     h->X = h->targets_f = nullptr; h->labels = h->ord = h->perm = h->row_of_param = h->param_of_row = nullptr;
     h->w2 = h->g2 = h->ws = nullptr;
     h->use_tc2 = false; h->tc2 = nullptr; h->tc2_check = false;
-    h->w = h->gprev = h->gnext = h->ringw = h->ringg = nullptr; h->sc = nullptr; h->part = nullptr; h->part_u = nullptr; h->part_r = nullptr; h->slot_abs = nullptr; h->reset_list = h->reset_count = nullptr; h->reset_loss = nullptr; h->reset_pipeline = false; h->use_tiny = false; h->use_thin2 = false; h->thin_fused = false;
-    h->side = h->hi = nullptr; h->ev_fork = h->ev_join = nullptr;
-    for (auto &ev : h->ev_chunk) ev = nullptr;
+    h->w = h->gprev = h->gnext = h->ringw = h->ringg = nullptr; h->sc = nullptr; h->part = nullptr; h->part_u = nullptr; h->part_r = nullptr; h->slot_abs = nullptr; h->reset_list = h->reset_count = nullptr; h->reset_loss = nullptr; h->reset_pipeline = false; h->use_tiny = false; h->use_thin2 = false;
     auto bail = [&](const std::string &msg) { g_create_error = msg; b2e_destroy(h); return 1; };
     int dev_count = 0;
     if (cudaGetDeviceCount(&dev_count) != cudaSuccess || cfg->device < 0 || cfg->device >= dev_count)
@@ -3920,13 +3280,11 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
             return bail("b2e_create: observation kernel does not fit (max_history too large)");
     }
     if (d.split) {
-        if (cudaFuncSetAttribute(obs_kernel<5>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)h->smem_obs) != cudaSuccess ||
-            cudaFuncSetAttribute(obs_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        if (cudaFuncSetAttribute(obs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)h->smem_obs) != cudaSuccess)
             return bail("b2e_create: observation kernel does not fit (max_history too large)");
-        if ((h->obs_stages || h->obs_regs) &&
-            cudaFuncSetAttribute(obs2_fn(h->obs_stages, h->obs_regs, h->obs_bulk), cudaFuncAttributeMaxDynamicSharedMemorySize,
+        if (h->use_obs3 &&
+            cudaFuncSetAttribute(obs_kernel3<5>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)h->smem_obs2) != cudaSuccess)
             return bail("b2e_create: observation kernel (batched gathers) does not fit shared memory");
     }
@@ -3946,29 +3304,12 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
             return bail("b2e_create: thin eval kernel does not fit an SM");
         h->eval_grid = occ_ev * h->num_sms;
     }
-    if (h->use_tc) {
-        if (cudaFuncSetAttribute(tc_eval_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)h->smem_tc) != cudaSuccess ||
-            cudaFuncSetAttribute(tc_eval_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 (int)h->smem_tc) != cudaSuccess)
-            return bail("b2e_create: tensor-core eval kernel does not fit shared memory");
-        int occ_tc = 0;
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_tc, tc_eval_kernel<true>, 256, h->smem_tc) !=
-                cudaSuccess || occ_tc < 1)
-            return bail("b2e_create: tensor-core eval kernel does not fit an SM");
-        if (occ_tc > 512 / tc::TMEM_COLS) occ_tc = 512 / tc::TMEM_COLS;    // TMEM: 512 columns per SM
-        h->tc_grid = occ_tc * h->num_sms;
-    }
     {   // tcgen05 eval kernel, warp-specialised (b200tc.cu); its context is made once the state
         // buffers exist (the tensor map holds the address of w)
-        // default for the shapes it covers (B2E_TC=0: the FFMA eval kernels, B2E_TC=1: the first,
-        // single-role tcgen05 kernel kept for comparison)
+        // default for the shapes it covers (B2E_TC=0: the FFMA eval kernels)
         const char *tcv = getenv("B2E_TC");
-        h->use_tc2 = h->use_eval_kernel && (!tcv || atoi(tcv) == 2) && b2e_tc2_supported(&h->d);
-        if (h->use_tc2) {
-            h->tc2_check = getenv("B2E_TC_CHECK") && atoi(getenv("B2E_TC_CHECK")) != 0;
-            h->use_tc = false;
-        }
+        h->use_tc2 = h->use_eval_kernel && !(tcv && atoi(tcv) == 0) && b2e_tc2_supported(&h->d);
+        h->tc2_check = h->use_tc2 && getenv("B2E_TC_CHECK") && atoi(getenv("B2E_TC_CHECK")) != 0;
     }
     if (h->use_eval_kernel) {
         if (cudaFuncSetAttribute(eval_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -3980,31 +3321,14 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
             cudaFuncSetAttribute(eval_kernel<true, 64, 112>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)h->smem_eval) != cudaSuccess)
             return bail("b2e_create: eval kernel does not fit shared memory");
-        h->eval_c = d.N1 == 64 && d.N1p == 64 && d.KT == 112 && d.B == 32 && d.D % 112 == 0 && d.Dp == d.D &&
-                    !getenv("B2E_EVAL_GENERIC");
-        h->eval_bulk = h->eval_c && d.kind == B2E_PROBLEM_SOFTMAX &&
-                       !(getenv("B2E_EVAL_BULK") && atoi(getenv("B2E_EVAL_BULK")) == 0);
+        h->eval_c = d.N1 == 64 && d.N1p == 64 && d.KT == 112 && d.B == 32 && d.D % 112 == 0 && d.Dp == d.D;
+        h->eval_bulk = h->eval_c && d.kind == B2E_PROBLEM_SOFTMAX;
         if (h->eval_bulk &&
             (cudaFuncSetAttribute(eval_bulk_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)h->smem_eval) != cudaSuccess ||
              cudaFuncSetAttribute(eval_bulk_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)h->smem_eval) != cudaSuccess))
             return bail("b2e_create: bulk eval kernel does not fit shared memory");
-        h->fuse_update = h->eval_bulk && !h->use_tc2 && d.env_kind == B2E_ENV_MULTIOPTLRS &&
-                         getenv("B2E_FUSE_UPDATE") && atoi(getenv("B2E_FUSE_UPDATE")) != 0 &&
-                         cudaFuncSetAttribute(eval_bulk_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                              (int)h->smem_eval) == cudaSuccess;
-        h->nchunks = getenv("B2E_CHUNKS") ? atoi(getenv("B2E_CHUNKS")) : 1;
-        if (h->nchunks > 1) {
-            int prio_least = 0, prio_greatest = 0;
-            cudaDeviceGetStreamPriorityRange(&prio_least, &prio_greatest);
-            if (cudaStreamCreateWithPriority(&h->side, cudaStreamNonBlocking, prio_least) != cudaSuccess ||
-                cudaStreamCreateWithPriority(&h->hi, cudaStreamNonBlocking, prio_least) != cudaSuccess ||
-                cudaEventCreateWithFlags(&h->ev_fork, cudaEventDisableTiming) != cudaSuccess ||
-                cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming) != cudaSuccess ||
-                cudaEventCreateWithFlags(&h->ev_chunk[0], cudaEventDisableTiming) != cudaSuccess)
-                return bail("b2e_create: stream/event creation failed");
-        }
         int occ_ev = 0;
         if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_ev, eval_kernel<true>, 256, h->smem_eval) !=
                 cudaSuccess || occ_ev < 1)
@@ -4014,17 +3338,8 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
             if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_b, eval_bulk_kernel<true>, 256, h->smem_eval) !=
                     cudaSuccess || occ_b < occ_ev)
                 h->eval_bulk = false;
-            if (h->fuse_update &&
-                (!h->eval_bulk || cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_b, eval_bulk_kernel<false, true>, 256,
-                                                                                h->smem_eval) != cudaSuccess || occ_b < occ_ev))
-                h->fuse_update = false;
-        } else {
-            h->fuse_update = false;
         }
         h->eval_grid = occ_ev * h->num_sms;
-        h->eval_ctas_per_sm = getenv("B2E_EVAL_CTAS") ? atoi(getenv("B2E_EVAL_CTAS")) : occ_ev;
-        h->chunk_envs = 4 * h->num_sms;
-        h->obs_grid = 1 << 30;
     }
     cudaMemset(h->w, 0, EP * 4); cudaMemset(h->gprev, 0, EP * 4);
     cudaMemset(h->ringw, 0, EP * d.H * 4); cudaMemset(h->ringg, 0, EP * d.H * 4);
@@ -4079,7 +3394,6 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
     h->use_tiny = b2e_tiny_supported(&h->d) && !(getenv("B2E_TINY") && atoi(getenv("B2E_TINY")) == 0);
     h->use_thin2 = h->use_thin && b2e_thin2_supported(&h->d) && !(getenv("B2E_THIN2") && atoi(getenv("B2E_THIN2")) == 0) &&
                    b2e_thin2_prepare(&h->d) == 0;
-    h->thin_fused = h->use_thin2 && b2e_thin2_fused_step(&h->d);
     init_scalars_kernel<<<(d.E + 127) / 128, 128>>>(d);
     if (cudaDeviceSynchronize() != cudaSuccess) return bail("b2e_create: device initialisation failed");
     *out = h;
@@ -4094,11 +3408,6 @@ void b2e_destroy(b2e_handle h) {
     cudaFree(h->w2); cudaFree(h->g2); cudaFree(h->ws);
     b2e_tc2_destroy(h->tc2);
     cudaFree(h->ringg); cudaFree(h->sc); cudaFree(h->gnext); cudaFree(h->part); cudaFree(h->part_u); cudaFree(h->part_r); cudaFree(h->slot_abs); cudaFree(h->reset_list); cudaFree(h->reset_count); cudaFree(h->reset_loss);
-    if (h->side) cudaStreamDestroy(h->side);
-    if (h->hi) cudaStreamDestroy(h->hi);
-    if (h->ev_fork) cudaEventDestroy(h->ev_fork);
-    if (h->ev_join) cudaEventDestroy(h->ev_join);
-    for (auto &ev : h->ev_chunk) if (ev) cudaEventDestroy(ev);
     for (auto &ev : h->tr) if (ev) cudaEventDestroy(ev);
     delete h;
 }
@@ -4172,7 +3481,7 @@ int b2e_step(b2e_handle h, const float *actions, const int32_t *batch_idx,
     if (!actions || !reward_out || !done_out || !info_out)
         return fail(h, "b2e_step: null pointer");
     // obs_out = NULL: ring-only step, the observation rows are not materialised (b200policy.h reads the rings)
-    if (!obs_out && !(h->d.split && h->d.env_kind == B2E_ENV_MULTIOPTLRS && h->slot_abs && !h->fuse_update && h->nchunks <= 1))
+    if (!obs_out && !(h->d.split && h->d.env_kind == B2E_ENV_MULTIOPTLRS && h->slot_abs))
         return fail(h, "b2e_step: obs_out = NULL needs a MultiOptLRs env on the large-problem pipeline");
     if (check_ready(h, batch_idx, batch_cnt)) return 1;
     StepArgs a;
@@ -4182,39 +3491,18 @@ int b2e_step(b2e_handle h, const float *actions, const int32_t *batch_idx,
     if (!h->d.split) return launch(h, a, stream);
     cudaStream_t main_s = (cudaStream_t)stream;
     Dev &d = h->d;
+    Dev &dv = h->d_eval;                                     // same pointers, eval-kernel smem layout
+    dv.gprev = d.gprev; dv.gnext = d.gnext; dv.perm_stride = d.perm_stride;
+    dv.X = d.X; dv.labels = d.labels; dv.targets = d.targets; dv.w = d.w; dv.sc = d.sc;
+    dv.ord = d.ord; dv.perm = d.perm; dv.part = d.part; dv.part_u = d.part_u;
+    dv.ringw = d.ringw; dv.ringg = d.ringg; dv.row_of_param = d.row_of_param; dv.param_of_row = d.param_of_row;
+    a.e_begin = 0; a.e_count = d.E;
     if (d.env_kind == B2E_ENV_MULTIOPTIMIZE) {
         // ---- update -> eval(w') + scalars -> observations (envs/multioptimize.py:90-154)
-        a.e_begin = 0; a.e_count = d.E;
         mo_update_kernel<<<dim3(d.nsegU, d.E), 256, 0, main_s>>>(d, a);
         h->launches++;
         CUDA_TRY(h, cudaGetLastError());
-        if (h->use_eval_kernel) {
-            Dev &v = h->use_tc ? h->d_tc : h->d_eval;
-            v.gprev = d.gprev; v.gnext = d.gnext; v.perm_stride = d.perm_stride;
-            v.X = d.X; v.labels = d.labels; v.targets = d.targets; v.w = d.w; v.sc = d.sc;
-            v.ord = d.ord; v.perm = d.perm;
-            const int cap = h->use_tc ? h->tc_grid : h->eval_grid;
-            const int grid_ev = d.E < cap ? d.E : cap;
-            if (h->use_tc2) { if (b2e_tc2_launch(h->tc2, &d, &a, 1, main_s)) return fail(h, "tc2 launch failed"); }
-            else if (h->use_tc) tc_eval_kernel<true><<<grid_ev, 256, h->smem_tc, main_s>>>(v, a);
-            else if (h->eval_bulk) eval_bulk_kernel<true><<<grid_ev, 256, h->smem_eval, main_s>>>(v, a);
-            else if (h->eval_c) eval_kernel<true, 64, 112><<<grid_ev, 256, h->smem_eval, main_s>>>(v, a);
-            else eval_kernel<true><<<grid_ev, 256, h->smem_eval, main_s>>>(v, a);
-            h->launches++;
-            CUDA_TRY(h, cudaGetLastError());
-        } else if (h->use_thin) {
-            const int grid_ev = d.E < h->eval_grid ? d.E : h->eval_grid;
-            if (h->use_thin2) { if (b2e_thin2_launch(&d, &a, 1, h->num_sms, main_s)) return fail(h, "thin2 launch failed"); }
-            else { Dev dt = d; dt.KT = h->thin_kc;
-          if (d.C == 10) thin_eval_kernel<true, 10><<<grid_ev, 256, h->smem_thin, main_s>>>(dt, a);
-          else thin_eval_kernel<true><<<grid_ev, 256, h->smem_thin, main_s>>>(dt, a); }
-            h->launches++;
-            CUDA_TRY(h, cudaGetLastError());
-        } else {
-            StepArgs b = a;
-            b.mode = MODE_EVAL_STEP;
-            if (launch(h, b, main_s)) return 1;
-        }
+        if (eval_pass<true>(h, a, main_s)) return 1;
         mo_obs_kernel<<<d.nseg * d.E, OBS_WARPS * 32, h->smem_obs, main_s>>>(d, a);
         info_finalize_kernel<<<(d.E + 127) / 128, 128, 0, main_s>>>(d, a);
         h->launches += 2;
@@ -4228,117 +3516,22 @@ int b2e_step(b2e_handle h, const float *actions, const int32_t *batch_idx,
         return 0;
     }
     // ---- large problems: eval(w) -> update -> eval(w') -> observations, all on the caller's stream
-    Dev &dv = h->use_tc ? h->d_tc : h->d_eval;               // same pointers, eval-kernel smem layout
-    dv.gprev = d.gprev; dv.gnext = d.gnext; dv.perm_stride = d.perm_stride;
-    dv.X = d.X; dv.labels = d.labels; dv.targets = d.targets; dv.w = d.w; dv.sc = d.sc;
-    dv.ord = d.ord; dv.perm = d.perm; dv.part = d.part; dv.part_u = d.part_u;
-    dv.ringw = d.ringw; dv.ringg = d.ringg; dv.row_of_param = d.row_of_param; dv.param_of_row = d.param_of_row;
-    a.e_begin = 0; a.e_count = d.E;
-    const int cap_ev = h->use_tc ? h->tc_grid : h->eval_grid;
-    const int grid_ev = d.E < cap_ev ? d.E : cap_ev;
     auto mark = [&](int i) { if (h->trace) cudaEventRecord(h->tr[i], main_s); };
-    if (h->nchunks > 1 && h->eval_c && !h->use_tc && (h->obs_stages || h->obs_regs)) {
-        // experiment (B2E_CHUNKS=n): env chunks alternate between two internal streams so that the
-        // FFMA-bound eval kernels of one chunk can share the SMs with the HBM-bound update /
-        // observation kernels of the other
-        cudaStream_t st[2] = {h->side, h->hi};
-        CUDA_TRY(h, cudaEventRecord(h->ev_fork, main_s));
-        CUDA_TRY(h, cudaStreamWaitEvent(st[0], h->ev_fork, 0));
-        CUDA_TRY(h, cudaStreamWaitEvent(st[1], h->ev_fork, 0));
-        const int chunk = (d.E + h->nchunks - 1) / h->nchunks;
-        const void *fn = obs2_fn(h->obs_stages, h->obs_regs, h->obs_bulk);
-        for (int c = 0; c < h->nchunks; ++c) {
-            StepArgs b = a;
-            b.e_begin = c * chunk;
-            b.e_count = d.E - b.e_begin < chunk ? d.E - b.e_begin : chunk;
-            if (b.e_count <= 0) break;
-            cudaStream_t s2 = st[c & 1];
-            const int cap = h->eval_ctas_per_sm * h->num_sms;
-            const int g = b.e_count < cap ? b.e_count : cap;
-            eval_kernel<false, 64, 112><<<g, 256, h->smem_eval, s2>>>(dv, b);
-            update_kernel<<<dim3(d.nsegU, b.e_count), 256, 0, s2>>>(d, b);
-            eval_kernel<true, 64, 112><<<g, 256, h->smem_eval, s2>>>(dv, b);
-            const int grid2 = (d.nseg * b.e_count + O2_WARPS - 1) / O2_WARPS;
-            void *params[2] = {(void *)&d, (void *)&b};
-            CUDA_TRY(h, cudaLaunchKernel(fn, dim3(grid2), dim3(O2_WARPS * 32), params, h->smem_obs2, s2));
-            h->launches += 4;
-        }
-        CUDA_TRY(h, cudaEventRecord(h->ev_join, st[0]));
-        CUDA_TRY(h, cudaStreamWaitEvent(main_s, h->ev_join, 0));
-        CUDA_TRY(h, cudaEventRecord(h->ev_chunk[0], st[1]));
-        CUDA_TRY(h, cudaStreamWaitEvent(main_s, h->ev_chunk[0], 0));
-        h->tr_count = 0;
-        CUDA_TRY(h, cudaGetLastError());
-        goto after_pipeline;
-    }
     mark(0);
-    if (h->use_tc2) {
-        if (b2e_tc2_launch(h->tc2, &d, &a, 0, main_s)) return fail(h, "tc2 launch failed");
-    } else if (h->use_tc) {
-        tc_eval_kernel<false><<<grid_ev, 256, h->smem_tc, main_s>>>(dv, a);
-    } else if (h->use_eval_kernel) {
-        if (h->eval_bulk && h->fuse_update) eval_bulk_kernel<false, true><<<grid_ev, 256, h->smem_eval, main_s>>>(dv, a);
-        else if (h->eval_bulk) eval_bulk_kernel<false><<<grid_ev, 256, h->smem_eval, main_s>>>(dv, a);
-        else if (h->eval_c) eval_kernel<false, 64, 112><<<grid_ev, 256, h->smem_eval, main_s>>>(dv, a);
-        else eval_kernel<false><<<grid_ev, 256, h->smem_eval, main_s>>>(dv, a);
-    } else if (h->use_thin) {
-        if (h->use_thin2) { if (b2e_thin2_launch(&d, &a, h->thin_fused ? 2 : 0, h->num_sms, main_s)) return fail(h, "thin2 launch failed"); }
-        else { Dev dt = d; dt.KT = h->thin_kc;
-          if (d.C == 10) thin_eval_kernel<false, 10><<<grid_ev, 256, h->smem_thin, main_s>>>(dt, a);
-          else thin_eval_kernel<false><<<grid_ev, 256, h->smem_thin, main_s>>>(dt, a); }
-    } else {                                                 // generic dense stack
-        StepArgs b = a;
-        b.mode = MODE_EVAL_FIRST;
-        if (launch(h, b, main_s)) return 1;
-        h->launches--;
-    }
+    if (eval_pass<false>(h, a, main_s)) return 1;
     mark(1);
-    if (h->fuse_update && h->eval_bulk && h->use_eval_kernel && !h->use_tc) h->launches--;   // the first eval did it
-    else if (h->thin_fused) h->launches--;                   // thin3_eval_kernel<2> did update and second eval as well
-    else update_kernel<<<dim3(d.nsegU, d.E), 256, 0, main_s>>>(d, a);
+    update_kernel<<<dim3(d.nsegU, d.E), 256, 0, main_s>>>(d, a);
     mark(2);
-    if (h->thin_fused) {
-        h->launches--;
-    } else if (h->use_tc2) {
-        if (b2e_tc2_launch(h->tc2, &d, &a, 1, main_s)) return fail(h, "tc2 launch failed");
-    } else if (h->use_tc) {
-        tc_eval_kernel<true><<<grid_ev, 256, h->smem_tc, main_s>>>(dv, a);
-    } else if (h->use_eval_kernel) {
-        if (h->eval_bulk) eval_bulk_kernel<true><<<grid_ev, 256, h->smem_eval, main_s>>>(dv, a);
-        else if (h->eval_c) eval_kernel<true, 64, 112><<<grid_ev, 256, h->smem_eval, main_s>>>(dv, a);
-        else eval_kernel<true><<<grid_ev, 256, h->smem_eval, main_s>>>(dv, a);
-    } else if (h->use_thin) {
-        if (h->use_thin2) { if (b2e_thin2_launch(&d, &a, 1, h->num_sms, main_s)) return fail(h, "thin2 launch failed"); }
-        else { Dev dt = d; dt.KT = h->thin_kc;
-          if (d.C == 10) thin_eval_kernel<true, 10><<<grid_ev, 256, h->smem_thin, main_s>>>(dt, a);
-          else thin_eval_kernel<true><<<grid_ev, 256, h->smem_thin, main_s>>>(dt, a); }
-    } else {
-        StepArgs b = a;
-        b.mode = MODE_EVAL_STEP;
-        if (launch(h, b, main_s)) return 1;
-        h->launches--;
-    }
+    if (eval_pass<true>(h, a, main_s)) return 1;
     mark(3);
-    if (!obs_out) {
-        ring_adjg_kernel<<<dim3(d.nsegU, d.E), 256, 0, main_s>>>(d, a);
-    } else {
-        const int items = d.nseg * d.E;
-        if (h->obs_stages || h->obs_regs) {
-            const int grid2 = (items + O2_WARPS - 1) / O2_WARPS;
-            const void *fn = obs2_fn(h->obs_stages, h->obs_regs, h->obs_bulk);
-            void *params[2] = {(void *)&d, (void *)&a};
-            CUDA_TRY(h, cudaLaunchKernel(fn, dim3(grid2), dim3(O2_WARPS * 32), params, h->smem_obs2, main_s));
-        }
-        else if (d.H == 5) obs_kernel<5><<<items, OBS_WARPS * 32, h->smem_obs, main_s>>>(d, a);
-        else obs_kernel<0><<<items, OBS_WARPS * 32, h->smem_obs, main_s>>>(d, a);
-    }
+    const int items = d.nseg * d.E;
+    if (!obs_out) ring_adjg_kernel<<<dim3(d.nsegU, d.E), 256, 0, main_s>>>(d, a);
+    else if (h->use_obs3) obs_kernel3<5><<<(items + O2_WARPS - 1) / O2_WARPS, O2_WARPS * 32, h->smem_obs2, main_s>>>(d, a);
+    else obs_kernel<<<items, OBS_WARPS * 32, h->smem_obs, main_s>>>(d, a);
     mark(4);
     h->tr_count = h->trace ? 4 : 0;
-    h->launches += 4;
-    CUDA_TRY(h, cudaGetLastError());
-after_pipeline:
     info_finalize_kernel<<<(d.E + 127) / 128, 128, 0, main_s>>>(d, a);
-    h->launches++;
+    h->launches += 3;
     CUDA_TRY(h, cudaGetLastError());
     if (h->use_tc2 && h->tc2_check) {                        // debugging aid: did the kernel's watchdog fire?
         int dbg[4] = {0, 0, 0, 0};

@@ -282,22 +282,16 @@ __global__ void __launch_bounds__(THREADS, 2) thin2_eval_kernel(const __grid_con
 //   backward : thread = features t, t + 256 of the half
 namespace cgx = cooperative_groups;
 
-// MODE 0: loss + gradient at the parameters in HBM (first evaluation of a step, b2e-style: g -> Dev::gnext)
-// MODE 1: the same + the step's scalars (second evaluation of a pipelined step)
-// MODE 2: the WHOLE compute part of a MultiOptLRs step in one launch (multioptlrs.py:85-88): gradient at w_{t-1},
-//         w_t = w_{t-1} - g0 * lr(action) and the adjusted-weight ring slot (what update_kernel does, same
-//         arithmetic per parameter), loss / gradient at w_t, scalars.  Rows and W never leave shared memory between the
-//         two evaluations, g0 never reaches HBM, update_kernel is not launched; CTA `rank` writes segment `rank` of the
-//         update statistics (nsegU >= 2 for these sizes).
-template <int MODE>
+// Loss + gradient at the parameters in HBM (-> Dev::gnext); SECOND: also the step's scalars (second evaluation of a
+// pipelined step).
+template <bool SECOND>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(THREADS, 3)
 thin3_eval_kernel(const __grid_constant__ Dev d, const __grid_constant__ StepArgs a) {
-    constexpr bool SECOND = MODE != 0, FUSED = MODE == 2;
     extern __shared__ __align__(16) float sm[];
     __shared__ float misc[8];
     __shared__ double red[8];
     __shared__ double gpart;
-    __shared__ float bs[C + 2];                       // the bias in use (FUSED: updated in place between the passes)
+    __shared__ float bs[C + 2];                       // the bias
     __shared__ int idx_s[BMAX], ys[BMAX];
     cgx::cluster_group cluster = cgx::this_cluster();
     const int rank = (int)cluster.block_rank(), peer = rank ^ 1;
@@ -313,7 +307,7 @@ thin3_eval_kernel(const __grid_constant__ Dev d, const __grid_constant__ StepArg
     int it = 0;
     for (int e = a.e_begin + cid; e < e_end; e += nclusters) {
         EnvScalars *sc = d.sc + e;
-        float *wE = d.w + (size_t)e * d.Pp;
+        const float *wE = d.w + (size_t)e * d.Pp;
         float *gout = d.gnext + (size_t)e * d.Pp;
         const int *idx; int cnt;
         current_batch(d, a, e, sc, idx, cnt);
@@ -350,186 +344,129 @@ thin3_eval_kernel(const __grid_constant__ Dev d, const __grid_constant__ StepArg
             asm volatile("cp.async.wait_group 0;\n" ::: "memory");
         }
         __syncthreads();
-        float s_absw = 0.f, s_absaw = 0.f;              // FUSED: update_kernel's statistics of this CTA's parameters
-        double s_lr = 0.0, s_lr2 = 0.0;
-        float gsum = 0.f, loss = 0.f;
-#pragma unroll 1
-        for (int pass = 0; pass < (FUSED ? 2 : 1); ++pass, ++it) {
-            float *Zmine = Zp + (it & 1) * BMAX * CP;
-            {   // ---- forward: warp = 4 samples, all Dh features of the half
-                f32x2 acc2[4][C / 2];
+        float gsum = 0.f;
+        float *Zmine = Zp + (it++ & 1) * BMAX * CP;     // alternates between envs: the peer may still read the last one
+        {   // ---- forward: warp = 4 samples, all Dh features of the half
+            f32x2 acc2[4][C / 2];
 #pragma unroll
-                for (int i = 0; i < 4; ++i)
+            for (int i = 0; i < 4; ++i)
 #pragma unroll
-                    for (int c = 0; c < C / 2; ++c) acc2[i][c] = pack2(0.f, 0.f);
-                const float *xr = Xs + (4 * warp) * Dh;
-                for (int k = lane; k < Dh; k += 32) {
-                    const f32x2 *wrow = reinterpret_cast<const f32x2 *>(Ws + k * C);
-                    f32x2 w2[C / 2];
+                for (int c = 0; c < C / 2; ++c) acc2[i][c] = pack2(0.f, 0.f);
+            const float *xr = Xs + (4 * warp) * Dh;
+            for (int k = lane; k < Dh; k += 32) {
+                const f32x2 *wrow = reinterpret_cast<const f32x2 *>(Ws + k * C);
+                f32x2 w2[C / 2];
 #pragma unroll
-                    for (int c = 0; c < C / 2; ++c) w2[c] = wrow[c];
+                for (int c = 0; c < C / 2; ++c) w2[c] = wrow[c];
 #pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const float x = xr[i * Dh + k];
-                        const f32x2 xx = pack2(x, x);
+                for (int i = 0; i < 4; ++i) {
+                    const float x = xr[i * Dh + k];
+                    const f32x2 xx = pack2(x, x);
 #pragma unroll
-                        for (int c = 0; c < C / 2; ++c) ffma2(acc2[i][c], xx, w2[c]);
-                    }
-                }
-                float v[40];
-#pragma unroll
-                for (int i = 0; i < 4; ++i)
-#pragma unroll
-                    for (int c = 0; c < C / 2; ++c) unpack2(acc2[i][c], v[i * C + 2 * c], v[i * C + 2 * c + 1]);
-                halve<20>(v, (lane & 16) != 0, 16);
-                halve<10>(v, (lane & 8) != 0, 8);
-                halve<5>(v, (lane & 4) != 0, 4);
-#pragma unroll
-                for (int i = 0; i < 5; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], 2);
-#pragma unroll
-                for (int i = 0; i < 5; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], 1);
-                if ((lane & 3) == 0) {
-                    const int base = ((lane >> 4) & 1) * 20 + ((lane >> 3) & 1) * 10 + ((lane >> 2) & 1) * 5;
-#pragma unroll
-                    for (int i = 0; i < 5; ++i) {
-                        const int flat = base + i, s = flat / C, c = flat - s * C;
-                        Zmine[(4 * warp + s) * CP + c] = v[i];
-                    }
+                    for (int c = 0; c < C / 2; ++c) ffma2(acc2[i][c], xx, w2[c]);
                 }
             }
-            cluster.sync();                           // both halves of the logits are in place
-            // ---- softmax cross-entropy per sample (both CTAs, redundantly), dZ (problems/optimize_nn.py:47-50)
-            if (tid < BMAX) {
-                const int s = tid;
-                const float *Zpeer = cluster.map_shared_rank(Zmine, peer);
-                const float *Z0 = rank == 0 ? Zmine : Zpeer, *Z1 = rank == 0 ? Zpeer : Zmine;     // feature order: the same sum in both CTAs
-                float z[C];
-                float ls = 0.f;
+            float v[40];
 #pragma unroll
-                for (int c = 0; c < C; ++c) z[c] = (Z0[s * CP + c] + Z1[s * CP + c]) + bs[c];
-                if (s < cnt) {
-                    const int y = ys[s];
-                    float m = z[0];
+            for (int i = 0; i < 4; ++i)
 #pragma unroll
-                    for (int c = 1; c < C; ++c) m = fmaxf(m, z[c]);
-                    float sum = 0.f, zy = 0.f;
+                for (int c = 0; c < C / 2; ++c) unpack2(acc2[i][c], v[i * C + 2 * c], v[i * C + 2 * c + 1]);
+            halve<20>(v, (lane & 16) != 0, 16);
+            halve<10>(v, (lane & 8) != 0, 8);
+            halve<5>(v, (lane & 4) != 0, 4);
 #pragma unroll
-                    for (int c = 0; c < C; ++c) { sum += expf(z[c] - m); if (c == y) zy = z[c]; }
-                    ls = (m + logf(sum)) - zy;
-                    const float inv = 1.0f / sum;
+            for (int i = 0; i < 5; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], 2);
 #pragma unroll
-                    for (int c = 0; c < C; ++c) z[c] = expf(z[c] - m) * inv - (c == y ? 1.f : 0.f);
-                } else {
+            for (int i = 0; i < 5; ++i) v[i] += __shfl_xor_sync(0xffffffffu, v[i], 1);
+            if ((lane & 3) == 0) {
+                const int base = ((lane >> 4) & 1) * 20 + ((lane >> 3) & 1) * 10 + ((lane >> 2) & 1) * 5;
 #pragma unroll
-                    for (int c = 0; c < C; ++c) z[c] = 0.f;
-                }
-#pragma unroll
-                for (int c = 0; c < C; ++c) dZ[s * CP + c] = z[c];
-                dZ[s * CP + 10] = 0.f; dZ[s * CP + 11] = 0.f;
-                lb[s] = ls;
-            }
-            __syncthreads();
-            if (tid == 0) {                           // mean loss, the samples in index order
-                float l = 0.f;
-                for (int s = 0; s < cnt; ++s) l += lb[s];
-                misc[0] = l / (float)cnt;
-            }
-            // ---- backward: thread = features tid, tid + 256 of the half
-            const bool update_pass = FUSED && pass == 0;
-            constexpr int KH = 2;
-            f32x2 g2[KH][C / 2];
-#pragma unroll
-            for (int j = 0; j < KH; ++j)
-#pragma unroll
-                for (int c = 0; c < C / 2; ++c) g2[j][c] = pack2(0.f, 0.f);
-            const int nk = (Dh - tid + THREADS - 1) / THREADS;     // 0, 1 or 2 features (Dh <= 512)
-#pragma unroll 4
-            for (int s = 0; s < cnt; ++s) {
-                const float4 z0 = *reinterpret_cast<const float4 *>(dZ + s * CP);
-                const float4 z1 = *reinterpret_cast<const float4 *>(dZ + s * CP + 4);
-                const float2 z2 = *reinterpret_cast<const float2 *>(dZ + s * CP + 8);
-                const f32x2 zz[C / 2] = {pack2(z0.x, z0.y), pack2(z0.z, z0.w), pack2(z1.x, z1.y), pack2(z1.z, z1.w), pack2(z2.x, z2.y)};
-                const float *xs = Xs + s * Dh;
-#pragma unroll
-                for (int j = 0; j < KH; ++j) {
-                    if (j < nk) {
-                        const float x = xs[tid + THREADS * j];
-                        const f32x2 xx = pack2(x, x);
-#pragma unroll
-                        for (int c = 0; c < C / 2; ++c) ffma2(g2[j][c], xx, zz[c]);
-                    }
+                for (int i = 0; i < 5; ++i) {
+                    const int flat = base + i, s = flat / C, c = flat - s * C;
+                    Zmine[(4 * warp + s) * CP + c] = v[i];
                 }
             }
-            float gb = 0.f;                           // bias gradient of class tid: column sum of dZ
-            if (tid < C) for (int s = 0; s < cnt; ++s) gb += dZ[s * CP + tid];
-            if (!update_pass) {
+        }
+        cluster.sync();                           // both halves of the logits are in place
+        // ---- softmax cross-entropy per sample (both CTAs, redundantly), dZ (problems/optimize_nn.py:47-50)
+        if (tid < BMAX) {
+            const int s = tid;
+            const float *Zpeer = cluster.map_shared_rank(Zmine, peer);
+            const float *Z0 = rank == 0 ? Zmine : Zpeer, *Z1 = rank == 0 ? Zpeer : Zmine;     // feature order: the same sum in both CTAs
+            float z[C];
+            float ls = 0.f;
 #pragma unroll
-                for (int j = 0; j < KH; ++j) {
-                    if (j < nk) {
-                        f32x2 *dst = reinterpret_cast<f32x2 *>(gout + (size_t)(kbase + tid + THREADS * j) * C);
+            for (int c = 0; c < C; ++c) z[c] = (Z0[s * CP + c] + Z1[s * CP + c]) + bs[c];
+            if (s < cnt) {
+                const int y = ys[s];
+                float m = z[0];
 #pragma unroll
-                        for (int c = 0; c < C / 2; ++c) {
-                            dst[c] = g2[j][c];
-                            float lo, hi;
-                            unpack2(g2[j][c], lo, hi);
-                            gsum += lo + hi;
-                        }
-                    }
-                }
-                if (rank == 0 && tid < C) { gout[d.P1 + tid] = gb; gsum += gb; }
-                __syncthreads();
-                loss = misc[0];
+                for (int c = 1; c < C; ++c) m = fmaxf(m, z[c]);
+                float sum = 0.f, zy = 0.f;
+#pragma unroll
+                for (int c = 0; c < C; ++c) { sum += expf(z[c] - m); if (c == y) zy = z[c]; }
+                ls = (m + logf(sum)) - zy;
+                const float inv = 1.0f / sum;
+#pragma unroll
+                for (int c = 0; c < C; ++c) z[c] = expf(z[c] - m) * inv - (c == y ? 1.f : 0.f);
             } else {
-                // ---- w_t = w_{t-1} - g0 * lr(action), adjusted weights (multioptlrs.py:86-87, utils_env.py:158-159)
-                const int head_new = (sc->head + 1) % d.H;
-                float *rw = d.ringw + ((size_t)e * d.H + head_new) * d.Pp;
-                const float *act = a.actions + (size_t)e * d.P;
-                auto update_one = [&](int p, float w, float g, bool count, float &wn, float &aw) {
-                    const float lr = action_to_lr(act[d.row_lex ? d.row_of_param[p] : p], d.act_ver);
-                    wn = fmaf(-g, lr, w);
-                    aw = nan_to_num_f(wn / fabsf(w));
-                    if (count) {
-                        s_absw += fabsf(wn);
-                        s_absaw += fabsf(aw);
-                        s_lr += (double)lr;
-                        s_lr2 += (double)lr * (double)lr;
-                    }
-                };
 #pragma unroll
-                for (int j = 0; j < KH; ++j) {
-                    if (j < nk) {
-                        const int kl = tid + THREADS * j, p0 = (kbase + kl) * C;
-                        float g[C], wn[C], aw[C];
+                for (int c = 0; c < C; ++c) z[c] = 0.f;
+            }
 #pragma unroll
-                        for (int c = 0; c < C / 2; ++c) unpack2(g2[j][c], g[2 * c], g[2 * c + 1]);
+            for (int c = 0; c < C; ++c) dZ[s * CP + c] = z[c];
+            dZ[s * CP + 10] = 0.f; dZ[s * CP + 11] = 0.f;
+            lb[s] = ls;
+        }
+        __syncthreads();
+        if (tid == 0) {                           // mean loss, the samples in index order
+            float l = 0.f;
+            for (int s = 0; s < cnt; ++s) l += lb[s];
+            misc[0] = l / (float)cnt;
+        }
+        // ---- backward: thread = features tid, tid + 256 of the half
+        constexpr int KH = 2;
+        f32x2 g2[KH][C / 2];
 #pragma unroll
-                        for (int c = 0; c < C; ++c) update_one(p0 + c, Ws[kl * C + c], g[c], true, wn[c], aw[c]);
+        for (int j = 0; j < KH; ++j)
 #pragma unroll
-                        for (int c = 0; c < C; ++c) Ws[kl * C + c] = wn[c];
-                        f32x2 *wdst = reinterpret_cast<f32x2 *>(wE + p0), *rdst = reinterpret_cast<f32x2 *>(rw + p0);
+            for (int c = 0; c < C / 2; ++c) g2[j][c] = pack2(0.f, 0.f);
+        const int nk = (Dh - tid + THREADS - 1) / THREADS;     // 0, 1 or 2 features (Dh <= 512)
+#pragma unroll 4
+        for (int s = 0; s < cnt; ++s) {
+            const float4 z0 = *reinterpret_cast<const float4 *>(dZ + s * CP);
+            const float4 z1 = *reinterpret_cast<const float4 *>(dZ + s * CP + 4);
+            const float2 z2 = *reinterpret_cast<const float2 *>(dZ + s * CP + 8);
+            const f32x2 zz[C / 2] = {pack2(z0.x, z0.y), pack2(z0.z, z0.w), pack2(z1.x, z1.y), pack2(z1.z, z1.w), pack2(z2.x, z2.y)};
+            const float *xs = Xs + s * Dh;
 #pragma unroll
-                        for (int c = 0; c < C / 2; ++c) { wdst[c] = pack2(wn[2 * c], wn[2 * c + 1]); rdst[c] = pack2(aw[2 * c], aw[2 * c + 1]); }
-                    }
+            for (int j = 0; j < KH; ++j) {
+                if (j < nk) {
+                    const float x = xs[tid + THREADS * j];
+                    const f32x2 xx = pack2(x, x);
+#pragma unroll
+                    for (int c = 0; c < C / 2; ++c) ffma2(g2[j][c], xx, zz[c]);
                 }
-                if (tid < C) {                        // the bias: both CTAs keep their copy current, CTA 0 owns HBM and the statistics
-                    float wn, aw;
-                    update_one(d.P1 + tid, bs[tid], gb, rank == 0, wn, aw);
-                    bs[tid] = wn;
-                    if (rank == 0) { wE[d.P1 + tid] = wn; rw[d.P1 + tid] = aw; }
-                }
-                __syncthreads();                      // Ws / bs hold w_t for the second pass
             }
         }
-        if (FUSED) {                                  // update statistics: segment `rank` of this env (info_finalize_kernel sums the segments)
-            const double t0 = block_sum((double)s_absw, red), t1 = block_sum(s_lr, red), t2 = block_sum(s_lr2, red);
-            const double t3 = block_sum((double)s_absaw, red);
-            if (tid == 0) {
-                double *out = d.part_u + ((size_t)e * d.nsegU + rank) * 4;
-                out[0] = t0; out[1] = t1; out[2] = t2; out[3] = t3;
-                if (rank == 0)
-                    for (int seg = 2; seg < d.nsegU; ++seg) { double *o = d.part_u + ((size_t)e * d.nsegU + seg) * 4; o[0] = o[1] = o[2] = o[3] = 0.0; }
+        float gb = 0.f;                           // bias gradient of class tid: column sum of dZ
+        if (tid < C) for (int s = 0; s < cnt; ++s) gb += dZ[s * CP + tid];
+#pragma unroll
+        for (int j = 0; j < KH; ++j) {
+            if (j < nk) {
+                f32x2 *dst = reinterpret_cast<f32x2 *>(gout + (size_t)(kbase + tid + THREADS * j) * C);
+#pragma unroll
+                for (int c = 0; c < C / 2; ++c) {
+                    dst[c] = g2[j][c];
+                    float lo, hi;
+                    unpack2(g2[j][c], lo, hi);
+                    gsum += lo + hi;
+                }
             }
         }
+        if (rank == 0 && tid < C) { gout[d.P1 + tid] = gb; gsum += gb; }
+        __syncthreads();
+        const float loss = misc[0];
         if (!SECOND) {
             if (rank == 0 && a.loss_out != nullptr && tid == 0) a.loss_out[e] = loss;
             continue;
@@ -570,24 +507,13 @@ static bool use_cluster_kernel(const Dev &d) {
            3 * (thin2::smem_bytes3(d) + 1024) <= 227 * 1024;
 }
 
-// the whole compute part of a MultiOptLRs step in one launch (thin3_eval_kernel<2>): opt-in with B2E_THIN_FUSE=1.
-// Bit-identical to the three launches and 4 words per parameter less HBM traffic, but not faster (0.215 ms against
-// 0.083 + 0.035 + 0.092 ms at 1024 envs): the kernel is bound by its per-env chain of latencies, which the fusion
-// lengthens by the action gathers of the update instead of shortening it.
-bool b2e_thin2_fused_step(const void *dev) {
-    const Dev &d = *static_cast<const Dev *>(dev);
-    const char *v = getenv("B2E_THIN_FUSE");
-    return use_cluster_kernel(d) && d.env_kind == B2E_ENV_MULTIOPTLRS && d.nsegU >= 2 && v && atoi(v) != 0;
-}
-
 int b2e_thin2_prepare(const void *dev) {
     const Dev &d = *static_cast<const Dev *>(dev);
     const int bytes = (int)thin2::smem_bytes(d), bytes3 = (int)thin2::smem_bytes3(d);
     return (cudaFuncSetAttribute(thin2::thin2_eval_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) == cudaSuccess &&
             cudaFuncSetAttribute(thin2::thin2_eval_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes) == cudaSuccess &&
-            cudaFuncSetAttribute(thin2::thin3_eval_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes3) == cudaSuccess &&
-            cudaFuncSetAttribute(thin2::thin3_eval_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes3) == cudaSuccess &&
-            cudaFuncSetAttribute(thin2::thin3_eval_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes3) == cudaSuccess) ? 0 : 1;
+            cudaFuncSetAttribute(thin2::thin3_eval_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes3) == cudaSuccess &&
+            cudaFuncSetAttribute(thin2::thin3_eval_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes3) == cudaSuccess) ? 0 : 1;
 }
 
 int b2e_thin2_launch(const void *dev, const void *args, int second, int num_sms, void *stream) {
@@ -600,9 +526,8 @@ int b2e_thin2_launch(const void *dev, const void *args, int second, int num_sms,
         const int rounds = (a.e_count + max_clusters - 1) / max_clusters;
         const int clusters = (a.e_count + rounds - 1) / rounds;
         const size_t bytes = thin2::smem_bytes3(d);
-        if (second == 2) thin2::thin3_eval_kernel<2><<<2 * clusters, thin2::THREADS, bytes, cs>>>(d, a);
-        else if (second) thin2::thin3_eval_kernel<1><<<2 * clusters, thin2::THREADS, bytes, cs>>>(d, a);
-        else thin2::thin3_eval_kernel<0><<<2 * clusters, thin2::THREADS, bytes, cs>>>(d, a);
+        if (second) thin2::thin3_eval_kernel<true><<<2 * clusters, thin2::THREADS, bytes, cs>>>(d, a);
+        else thin2::thin3_eval_kernel<false><<<2 * clusters, thin2::THREADS, bytes, cs>>>(d, a);
         return cudaGetLastError() == cudaSuccess ? 0 : 1;
     }
     const int cap = 2 * num_sms;

@@ -6,7 +6,5 @@
 bool b2e_thin2_supported(const void *dev);
 // shared-memory opt-in; 0 on success
 int b2e_thin2_prepare(const void *dev);
-// true: second = 2 runs eval(w_{t-1}) -> update -> eval(w_t) -> scalars of a MultiOptLRs step in ONE launch
-bool b2e_thin2_fused_step(const void *dev);
 // loss + gradient (-> Dev::gnext) of args.e_begin .. e_begin + e_count; second = 1: also the step's scalars
 int b2e_thin2_launch(const void *dev, const void *args, int second, int num_sms, void *stream);

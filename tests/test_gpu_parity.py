@@ -285,7 +285,7 @@ def test_loss_and_gradient_match_oracle(name, monkeypatch):
     env.close()
 
 
-@pytest.mark.parametrize('row_order', ['lexicographic', 'natural', 'lexicographic-generic', 'natural-tc',
+@pytest.mark.parametrize('row_order', ['lexicographic', 'natural', 'lexicographic-generic',
                                        'natural-tc2', 'lexicographic-tc2', 'lexicographic-ffma'])
 @pytest.mark.parametrize('name', list(SPECS))
 def test_step_parity_from_identical_states(name, row_order, monkeypatch):
@@ -314,12 +314,6 @@ def _step_parity(name, row_order, monkeypatch, depth):
         monkeypatch.setenv('B2E_TC', '2' if row_order.endswith('-tc2') else '0')
         monkeypatch.setenv('B2E_TC_CHECK', '1')
         row_order = row_order.rsplit('-', 1)[0]
-    if row_order.endswith('-tc'):
-        # the opt-in tcgen05 (3xTF32) eval kernel, held to the same oracle and tolerances
-        if name != 'mlp_784x64x10':
-            pytest.skip('the tensor-core eval kernel covers the config-4 shape')
-        monkeypatch.setenv('B2E_TC', '1')
-        row_order = 'natural'
     if row_order.endswith('-generic'):
         if spec.kind != 'softmax' or name in ('mlp_784x64x10', 'softmax_784x10') or len(spec.hidden) > 1:
             pytest.skip('generic path: softmax stacks; large / already-generic specs run it elsewhere')
@@ -727,40 +721,6 @@ def test_full_size_properties_mlp():
         assert np.array_equal(a[0], b[0]) and np.array_equal(a[1], b[1])
 
 
-def test_fused_update_variant_equals_the_four_kernel_pipeline(monkeypatch):
-    """B2E_FUSE_UPDATE=1 (the first eval kernel applies the update in its backward epilogue) against
-    the default pipeline on the config-4 shape: same arithmetic per parameter, so weights and
-    observations agree bit for bit; the per-env statistics are summed in another order."""
-    import torch
-    from custom_envs_b200.batched_env import BatchedOptEnv, ProblemSpec
-    rng = np.random.RandomState(11)
-    feats = rng.uniform(size=(256, 784)).astype(np.float32)
-    labels = rng.randint(0, 10, 256).astype(np.int32)
-    runs = []
-    for fused in (False, True):
-        monkeypatch.setenv('B2E_TC', '0')                   # the fusion lives in the FFMA eval kernel
-        if fused:
-            monkeypatch.setenv('B2E_FUSE_UPDATE', '1')
-        else:
-            monkeypatch.delenv('B2E_FUSE_UPDATE', raising=False)
-        env = BatchedOptEnv(ProblemSpec('softmax', 784, (64,), 10), feats, labels, 5, batch_size=32,
-                            max_batches=6, seeds=list(range(5)), init_seed=9)
-        env.reset()
-        act_rng = np.random.RandomState(4)
-        launches, trail = env.launch_count, []
-        for _ in range(8):                                   # crosses an auto-reset (max_batches=6)
-            actions = torch.as_tensor(act_rng.uniform(0, 3, env.num_rows).astype(np.float32), device=env.device)
-            obs, reward, done, info = env.step(actions)
-            trail.append((obs.cpu().numpy().copy(), reward.cpu().numpy().copy(), done.cpu().numpy().copy(),
-                          info.cpu().numpy().copy()))
-        runs.append((trail, env.launch_count - launches))
-        env.close()
-    assert runs[1][1] < runs[0][1]                           # one launch fewer per step
-    for (obs_a, rew_a, done_a, info_a), (obs_b, rew_b, done_b, info_b) in zip(runs[0][0], runs[1][0]):
-        assert np.array_equal(obs_a, obs_b) and np.array_equal(rew_a, rew_b) and np.array_equal(done_a, done_b)
-        assert np.allclose(info_a, info_b, rtol=1e-6, atol=1e-9, equal_nan=True)
-
-
 @pytest.mark.parametrize('after_reset', [False, True])
 def test_bench_sampled_parity_check_agrees_with_the_step(after_reset):
     """bench.py's ``parity`` entry (oracle/step_check.py seeded with the device's own state) on a
@@ -995,45 +955,3 @@ def test_resident_minibatch_eval_kernel_against_the_chunked_one(monkeypatch):
         np.testing.assert_allclose(new[4][:, 0], old[4][:, 0], rtol=RTOL, err_msg=str(t))
         np.testing.assert_allclose(new[0], old[0], rtol=20 * RTOL, atol=20 * RTOL, err_msg=str(t))
     assert ragged >= 2 * num_envs
-
-
-def test_one_launch_step_of_config_3_equals_the_three_launch_pipeline(monkeypatch):
-    """BASELINE config 3: `thin3_eval_kernel<2>` runs eval(w_{t-1}) -> update -> eval(w_t) -> scalars of a
-    MultiOptLRs step in one launch (rows and W stay in the cluster's shared memory, g0 never reaches HBM, no
-    update_kernel; opt-in with B2E_THIN_FUSE=1: it is not faster); the default runs the same arithmetic as eval /
-    update_kernel / eval.  Parameters, gradients,
-    rings, observation rows, rewards and done flags agree bit for bit over two episodes with a ragged last minibatch;
-    the update statistics (weights_mean/sum, actions_mean/std) are summed in another grouping."""
-    BatchedOptEnv, _ = _mods()
-    spec = SPECS['softmax_784x10'][0]
-    num_rows, num_envs = 304, 9
-    feats, targs = make_data(spec, num_rows)
-    perms = np.stack([orc.env_permutation(num_rows, 90 + s) for s in range(num_envs)])
-    runs = []
-    for fused in (True, False):
-        if fused:
-            monkeypatch.setenv('B2E_THIN_FUSE', '1')
-        else:
-            monkeypatch.delenv('B2E_THIN_FUSE', raising=False)
-        env = BatchedOptEnv(product_spec(spec), feats, targs, num_envs, batch_size=32, max_batches=11, perms=perms, init_seed=3)
-        rec = [env.reset().cpu().numpy().copy()]
-        launches = env.launch_count
-        gen = torch.Generator(device='cuda').manual_seed(2)
-        for t in range(24):
-            obs, rew, done, info = env.step(torch.rand(env.num_rows, device='cuda', generator=gen) * 2.5)
-            rec.append((obs.cpu().numpy().copy(), rew.cpu().numpy().copy(), done.cpu().numpy().copy(), info.cpu().numpy().copy(),
-                        {n: env.get_state(n).cpu().numpy() for n in ('params', 'grad_prev', 'adj_weights', 'adj_grads', 'adj_losses',
-                                                                    'raw_losses', 'raw_gsums', 'step', 'cursor')}))
-        runs.append((rec, env.launch_count - launches))
-        env.close()
-    assert runs[1][1] - runs[0][1] >= 2 * 24                  # two launches fewer per step
-    (fused_rec, _), (plain_rec, _) = runs
-    assert np.array_equal(fused_rec[0], plain_rec[0])
-    for t, (new, old) in enumerate(zip(fused_rec[1:], plain_rec[1:])):
-        assert np.array_equal(new[0], old[0]) and np.array_equal(new[1], old[1]) and np.array_equal(new[2], old[2]), t
-        for key in new[4]:
-            assert np.array_equal(new[4][key], old[4][key]), (t, key)
-        stats = [2, 3, 4, 5]
-        rest = [c for c in range(16) if c not in stats]
-        assert np.array_equal(new[3][:, rest], old[3][:, rest], equal_nan=True), t
-        np.testing.assert_allclose(new[3][:, stats], old[3][:, stats], rtol=1e-6, atol=1e-9, err_msg=str(t))
