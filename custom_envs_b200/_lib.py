@@ -22,6 +22,7 @@ MAX_LAYERS = 8
 EXPORTS = (
     'b2e_abi_version', 'b2e_create', 'b2e_destroy', 'b2e_last_error', 'b2e_num_params',
     'b2e_obs_dim', 'b2e_history_depth', 'b2e_bind_dataset', 'b2e_set_index_stream', 'b2e_reset', 'b2e_step',
+    'b2e_step_adam',
     'b2e_eval', 'b2e_get_state', 'b2e_set_state', 'b2e_get_batch_indices', 'b2e_next_batch',
     'b2e_set_trace', 'b2e_get_trace', 'b2e_launch_count',
     # data front-end (include/b200data.h)
@@ -43,6 +44,11 @@ class Config(ctypes.Structure):
         'history_version', 'observation_version', 'action_version', 'reward_version',
         'row_order', 'index_mode', 'auto_reset', 'env_base')] + [
         ('hidden_more', ctypes.c_int32 * MAX_LAYERS), ('init_seed', ctypes.c_uint64)]
+
+
+class Adam(ctypes.Structure):
+    """b2e_adam: the constants of b2e_step_adam (Keras 2.2 Adam)."""
+    _fields_ = [(name, ctypes.c_float) for name in ('beta_1', 'beta_2', 'epsilon')]
 
 
 class StepOut(ctypes.Structure):
@@ -93,6 +99,7 @@ def load():
     lib.b2e_set_index_stream.argtypes = [vp, vp, i32, vp, vp]
     lib.b2e_reset.argtypes = [vp, vp, vp, vp, vp, vp, vp]
     lib.b2e_step.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp]
+    lib.b2e_step_adam.argtypes = [vp, ctypes.POINTER(Adam), vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]
     lib.b2e_eval.argtypes = [vp, vp, vp, vp, vp, vp]
     lib.b2e_get_state.argtypes = [vp, i32, vp, usize, vp]
     lib.b2e_set_state.argtypes = [vp, i32, vp, usize, vp]

@@ -9,7 +9,7 @@ SOURCES = [os.path.join(_HERE, 'csrc', 'b200env.cu'), os.path.join(_HERE, 'csrc'
            os.path.join(_HERE, 'csrc', 'b200tiny.cu'), os.path.join(_HERE, 'csrc', 'b200thin.cu')]
 HEADERS = [os.path.join(ROOT, 'include', 'b200env.h'), os.path.join(ROOT, 'include', 'b200data.h'),
            os.path.join(ROOT, 'include', 'b200policy.h'),
-           os.path.join(_HERE, 'csrc', 'b200env_shared.cuh'), os.path.join(_HERE, 'csrc', 'b200tc.h'),
+           os.path.join(_HERE, 'csrc', 'b200env_shared.cuh'), os.path.join(_HERE, 'csrc', 'b200adam.cuh'), os.path.join(_HERE, 'csrc', 'b200tc.h'),
            os.path.join(_HERE, 'csrc', 'b200env_internal.h'), os.path.join(_HERE, 'csrc', 'b200tiny.h'), os.path.join(_HERE, 'csrc', 'b200thin.h')]
 OBJ_DIR = os.path.join(_HERE, 'csrc', '_obj')
 OUTPUT = os.path.join(_HERE, 'libb200env.so')

@@ -27,6 +27,7 @@
 #include "b200env.h"
 
 #include "b200env_shared.cuh"
+#include "b200adam.cuh"
 #include "b200tc.h"
 #include "b200env_internal.h"
 #include "b200tiny.h"
@@ -826,6 +827,36 @@ __device__ void epilogue(const Dev &d, const StepArgs &a, float *sm, const EpiCt
 }
 
 
+// b2e_step_adam's update pass over parameters [p_begin, p_end) of the fused step at env-step t (PASS_U of epilogue
+// with Keras' Adam in place of the action's learning rate; no row table, as no action is read): gsrc holds g0 at the
+// entry and w_t at the exit, as there
+__device__ void epilogue_adam(const Dev &d, const AdamArgs &o, const EpiCtx &cx, int p_begin, int p_end,
+                              float *gsrc, bool tile_mode, int k0, int t, float cnt, Stats &st) {
+    float *mE = o.m + (size_t)cx.e * d.P, *vE = o.v + (size_t)cx.e * d.P;
+    const float alpha = adam_alpha(o, cx.e, t);
+    const bool first = t == 1;
+    for (int p = p_begin + threadIdx.x; p < p_end; p += blockDim.x) {
+        int gi = p - p_begin;
+        if (tile_mode) {
+            const int k = p / d.N1;
+            gi = (k - k0) * d.N1p + (p - k * d.N1);
+        }
+        const float wv = cx.wE[p];
+        float mv = first ? 0.f : mE[p], vv = first ? 0.f : vE[p];
+        const float rate = adam_moments(o, alpha, first, adam_mean_grad(gsrc[gi], cnt), mv, vv);
+        const float wn = fmaf(-rate, mv, wv);
+        st.f[ST_ABSW] += fabsf(wn);
+        st.lr += (double)rate;
+        st.lr2 += (double)rate * (double)rate;
+        gsrc[gi] = wn;
+        cx.wE[p] = wn;
+        cx.rwE[(size_t)cx.head_new * d.Pp + p] = ratio_nn(wn, wv);          // utils_env.py:158-159
+        mE[p] = mv;
+        vE[p] = vv;
+    }
+}
+
+
 __device__ void load_tail(const Dev &d, float *sm, const float *wE) {
     float *tw = sm + d.off_tw;
     for (int i = threadIdx.x; i < d.tailP; i += blockDim.x) tw[i] = wE[d.P1 + i];
@@ -924,8 +955,10 @@ __device__ void reset_env(const Dev &d, const StepArgs &a, float *sm, int e) {
     __syncthreads();
 }
 
-template <int HT, bool BIG>
-__device__ void step_env(const Dev &d, const StepArgs &a, float *sm, int e) {
+// Adam: none for b2e_step, one AdamArgs for b2e_step_adam, whose update pass is epilogue_adam (Keras' Adam in place
+// of the action's learning rate); the pack leaves the action step's instantiations as they are
+template <int HT, bool BIG, class... Adam>
+__device__ void step_env(const Dev &d, const StepArgs &a, float *sm, int e, const Adam &...adam) {
     EnvScalars *sc = d.sc + e;
     EpiCtx cx;
     make_ctx(d, e, cx);
@@ -946,7 +979,10 @@ __device__ void step_env(const Dev &d, const StepArgs &a, float *sm, int e) {
     load_tail(d, sm, cx.wE);
     if (d.ntiles) { if (BIG && d.fast) forward_from_global_fast(d, sm, cx.wE); else forward_from_global(d, sm, cx.wE); }
     tail_eval(d, sm, cnt);
-    epilogue<PASS_U, 0>(d, a, sm, cx, d.P1, d.P, sm + d.off_tg, false, 0, st);
+    if constexpr (sizeof...(Adam) > 0)                          // this step is t = step + 1
+        epilogue_adam(d, adam_of(adam...), cx, d.P1, d.P, sm + d.off_tg, false, 0, sc->step + 1, (float)cnt, st);
+    else
+        epilogue<PASS_U, 0>(d, a, sm, cx, d.P1, d.P, sm + d.off_tg, false, 0, st);
     __syncthreads();
     {   // tail: tg now holds w_t of the tail; make it the live tail parameters
         float *tw = sm + d.off_tw, *tg = sm + d.off_tg;
@@ -959,7 +995,10 @@ __device__ void step_env(const Dev &d, const StepArgs &a, float *sm, int e) {
         const int krows = min(d.KT, d.D - k0), krows4 = (krows + 3) & ~3;
         if (BIG && d.fast) g_compute_fast(d, sm, T, k0, cnt); else g_compute(d, sm, T, k0, cnt);
         __syncthreads();
-        epilogue<PASS_U, 0>(d, a, sm, cx, k0 * d.N1, (k0 + krows) * d.N1, T, true, k0, st);
+        if constexpr (sizeof...(Adam) > 0)
+            epilogue_adam(d, adam_of(adam...), cx, k0 * d.N1, (k0 + krows) * d.N1, T, true, k0, sc->step + 1, (float)cnt, st);
+        else
+            epilogue<PASS_U, 0>(d, a, sm, cx, k0 * d.N1, (k0 + krows) * d.N1, T, true, k0, st);
         for (int i = krows * d.N1p + threadIdx.x; i < krows4 * d.N1p; i += blockDim.x) T[i] = 0.f;
         if (d.N1p != d.N1)
             for (int i = threadIdx.x; i < krows * (d.N1p - d.N1); i += blockDim.x) {
@@ -1128,13 +1167,16 @@ __device__ void eval_env(const Dev &d, const StepArgs &a, float *sm, int e) {
     __syncthreads();
 }
 
-template <int HT, bool BIG>
+// Adam: none, or the AdamArgs of b2e_step_adam (MODE_STEP only; finished envs auto-reset as in b2e_step)
+template <int HT, bool BIG, class... Adam>
 __global__ void __launch_bounds__(256, BIG ? 1 : 2) optenv_kernel(const __grid_constant__ Dev d,
-                                                     const __grid_constant__ StepArgs a) {
+                                                     const __grid_constant__ StepArgs a, const Adam... adam) {
     extern __shared__ __align__(16) float sm[];
     const int e_end = a.e_begin + a.e_count;
     for (int e = a.e_begin + blockIdx.x; e < e_end; e += gridDim.x) {
-        if (a.mode == MODE_STEP) {
+        if constexpr (sizeof...(Adam) > 0) {
+            step_env<HT, BIG>(d, a, sm, e, adam...);
+        } else if (a.mode == MODE_STEP) {
             step_env<HT, BIG>(d, a, sm, e);
         } else if (a.mode == MODE_RESET) {
             if (a.mask == nullptr || a.mask[e]) reset_env<BIG>(d, a, sm, e);
@@ -1993,6 +2035,114 @@ __global__ void __launch_bounds__(256) update_kernel(const __grid_constant__ Dev
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const double v0 = warp_sum((double)s_absw), v1 = warp_sum(s_lr), v2 = warp_sum(s_lr2);
     const double v3 = warp_sum((double)s_absaw);             // sum |adjusted weights| of the new ring slot
+    if (lane == 0) { red[warp * 4] = v0; red[warp * 4 + 1] = v1; red[warp * 4 + 2] = v2; red[warp * 4 + 3] = v3; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double *out = d.part_u + ((size_t)e * d.nsegU + seg) * 4;
+        for (int i = 0; i < 4; ++i) {
+            double v = 0.0;
+            for (int w = 0; w < 8; ++w) v += red[w * 4 + i];
+            out[i] = v;
+        }
+    }
+}
+
+// Quad p..p+3 of a caller-owned [E, P] row (b2e_step_adam's m and v): the row start e * P is only 4-byte
+// aligned, so the widest access the address allows; the components from P on read as 0 and are not stored.
+__device__ __forceinline__ float4 load_row_quad(const float *row, int p, int P) {
+    const float *q = row + p;
+    if (p + 4 <= P) {
+        if (((uintptr_t)q & 15) == 0) return *reinterpret_cast<const float4 *>(q);
+        if (((uintptr_t)q & 7) == 0) {
+            const float2 lo = *reinterpret_cast<const float2 *>(q), hi = *reinterpret_cast<const float2 *>(q + 2);
+            return make_float4(lo.x, lo.y, hi.x, hi.y);
+        }
+    }
+    return make_float4(q[0], p + 1 < P ? q[1] : 0.f, p + 2 < P ? q[2] : 0.f, p + 3 < P ? q[3] : 0.f);
+}
+__device__ __forceinline__ void store_row_quad(float *row, int p, int P, float4 x) {
+    float *q = row + p;
+    if (p + 4 <= P && ((uintptr_t)q & 15) == 0) {
+        *reinterpret_cast<float4 *>(q) = x;
+    } else if (p + 4 <= P && ((uintptr_t)q & 7) == 0) {
+        *reinterpret_cast<float2 *>(q) = make_float2(x.x, x.y);
+        *reinterpret_cast<float2 *>(q + 2) = make_float2(x.z, x.w);
+    } else {
+        q[0] = x.x;
+        if (p + 1 < P) q[1] = x.y;
+        if (p + 2 < P) q[2] = x.z;
+        if (p + 3 < P) q[3] = x.w;
+    }
+}
+
+// b2e_step_adam: update_kernel with Keras' Adam on the gradient of the mean minibatch loss, g0 / cnt, in place
+// of the action's learning rate.  Reads w, g0, m, v and writes w, m, v and the ring slot (8 words per parameter;
+// the action update moves 5); the partial sums take Adam's per-parameter rate alpha_t / (sqrt(v) + eps) for lr.
+__global__ void __launch_bounds__(256) update_adam_kernel(const __grid_constant__ Dev d,
+                                                          const __grid_constant__ StepArgs a,
+                                                          const __grid_constant__ AdamArgs o) {
+    const int e = a.e_begin + blockIdx.y;
+    const int seg = blockIdx.x;
+    const EnvScalars *sc = d.sc + e;
+    const int head_new = (sc->head + 1) % d.H;
+    float *wE = d.w + (size_t)e * d.Pp;
+    const float *gE = d.gnext + (size_t)e * d.Pp;             // g0, left there by the first eval
+    float *rw = d.ringw + ((size_t)e * d.H + head_new) * d.Pp;
+    float *mE = o.m + (size_t)e * d.P, *vE = o.v + (size_t)e * d.P;
+    const int t = sc->step + 1;                                // the second eval counts the step
+    const bool first = t == 1;
+    const int *idx; int cnt;
+    current_batch(d, a, e, sc, idx, cnt);                      // the first eval's minibatch (0 rows: func)
+    const float cntf = (float)cnt;
+    __shared__ float alpha_s;
+    if (threadIdx.x == 0) alpha_s = adam_alpha(o, e, t);
+    float4 w4[UPD_QUADS], g4[UPD_QUADS], m4[UPD_QUADS], v4[UPD_QUADS];
+    int pq[UPD_QUADS];
+#pragma unroll
+    for (int i = 0; i < UPD_QUADS; ++i) {
+        pq[i] = seg * UPD_SEG + (i * 256 + threadIdx.x) * 4;
+        if (pq[i] < d.P) {
+            w4[i] = *reinterpret_cast<const float4 *>(wE + pq[i]);
+            g4[i] = *reinterpret_cast<const float4 *>(gE + pq[i]);
+            m4[i] = first ? make_float4(0.f, 0.f, 0.f, 0.f) : load_row_quad(mE, pq[i], d.P);
+            v4[i] = first ? make_float4(0.f, 0.f, 0.f, 0.f) : load_row_quad(vE, pq[i], d.P);
+        }
+    }
+    __syncthreads();
+    const float alpha = alpha_s;
+    float s_absw = 0.f, s_absaw = 0.f;
+    double s_lr = 0.0, s_lr2 = 0.0;
+#pragma unroll
+    for (int i = 0; i < UPD_QUADS; ++i) {
+        if (pq[i] >= d.P) continue;
+        const float wv[4] = {w4[i].x, w4[i].y, w4[i].z, w4[i].w};
+        const float gv[4] = {g4[i].x, g4[i].y, g4[i].z, g4[i].w};
+        float mv[4] = {m4[i].x, m4[i].y, m4[i].z, m4[i].w};
+        float vv[4] = {v4[i].x, v4[i].y, v4[i].z, v4[i].w};
+        float wn[4], aw[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const float rate = adam_moments(o, alpha, first, adam_mean_grad(gv[j], cntf), mv[j], vv[j]);
+            wn[j] = fmaf(-rate, mv[j], wv[j]);
+            aw[j] = ratio_nn(wn[j], wv[j]);                      // utils_env.py:158-159
+            if (pq[i] + j < d.P) {
+                s_absw += fabsf(wn[j]);
+                s_absaw += fabsf(aw[j]);
+                s_lr += (double)rate;
+                s_lr2 += (double)rate * (double)rate;
+            } else {
+                wn[j] = 0.f; aw[j] = 0.f;
+            }
+        }
+        *reinterpret_cast<float4 *>(wE + pq[i]) = make_float4(wn[0], wn[1], wn[2], wn[3]);
+        *reinterpret_cast<float4 *>(rw + pq[i]) = make_float4(aw[0], aw[1], aw[2], aw[3]);
+        store_row_quad(mE, pq[i], d.P, make_float4(mv[0], mv[1], mv[2], mv[3]));
+        store_row_quad(vE, pq[i], d.P, make_float4(vv[0], vv[1], vv[2], vv[3]));
+    }
+    __shared__ double red[8 * 4];
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const double v0 = warp_sum((double)s_absw), v1 = warp_sum(s_lr), v2 = warp_sum(s_lr2);
+    const double v3 = warp_sum((double)s_absaw);
     if (lane == 0) { red[warp * 4] = v0; red[warp * 4 + 1] = v1; red[warp * 4 + 2] = v2; red[warp * 4 + 3] = v3; }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -3084,12 +3234,13 @@ int reset_through_pipeline(b2e_handle h, StepArgs a, void *stream) {
     return 0;
 }
 
-int launch(b2e_handle h, StepArgs args, void *stream) {
+// adam: b2e_step_adam's arguments (MODE_STEP), null on every other launch
+int launch(b2e_handle h, StepArgs args, void *stream, const AdamArgs *adam = nullptr) {
     if (args.mode == MODE_RESET && h->reset_pipeline) return reset_through_pipeline(h, args, stream);
     if (h->use_tiny && (args.mode == MODE_STEP || args.mode == MODE_RESET)) {
         if (args.e_count == 0) { args.e_begin = 0; args.e_count = h->d.E; }
         h->launches++;
-        if (b2e_tiny_launch(&h->d, &args, stream)) return fail(h, "tiny kernel launch failed");
+        if (b2e_tiny_launch(&h->d, &args, adam, stream)) return fail(h, "tiny kernel launch failed");
         return 0;
     }
     if (args.e_count == 0) { args.e_begin = 0; args.e_count = h->d.E; }
@@ -3101,7 +3252,15 @@ int launch(b2e_handle h, StepArgs args, void *stream) {
         CUDA_TRY(h, cudaGetLastError());
         return 0;
     }
-    if (h->d.fast) {
+    if (adam) {
+        if (h->d.fast) {
+            if (h->d.H == 5) optenv_kernel<5, true, AdamArgs><<<h->grid, h->nthreads, h->smem_bytes, cs>>>(h->d, args, *adam);
+            else optenv_kernel<0, true, AdamArgs><<<h->grid, h->nthreads, h->smem_bytes, cs>>>(h->d, args, *adam);
+        } else {
+            if (h->d.H == 5) optenv_kernel<5, false, AdamArgs><<<h->grid, h->nthreads, h->smem_bytes, cs>>>(h->d, args, *adam);
+            else optenv_kernel<0, false, AdamArgs><<<h->grid, h->nthreads, h->smem_bytes, cs>>>(h->d, args, *adam);
+        }
+    } else if (h->d.fast) {
         if (h->d.H == 5) optenv_kernel<5, true><<<h->grid, h->nthreads, h->smem_bytes, cs>>>(h->d, args);
         else optenv_kernel<0, true><<<h->grid, h->nthreads, h->smem_bytes, cs>>>(h->d, args);
     } else {
@@ -3228,6 +3387,9 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
     const void *kernel_fn = h->d.fast
         ? (h5 ? (const void *)optenv_kernel<5, true> : (const void *)optenv_kernel<0, true>)
         : (h5 ? (const void *)optenv_kernel<5, false> : (const void *)optenv_kernel<0, false>);
+    const void *adam_fn = h->d.fast
+        ? (h5 ? (const void *)optenv_kernel<5, true, AdamArgs> : (const void *)optenv_kernel<0, true, AdamArgs>)
+        : (h5 ? (const void *)optenv_kernel<5, false, AdamArgs> : (const void *)optenv_kernel<0, false, AdamArgs>);
     Dev &d = h->d;
     if (d.generic) {
         // per-CTA workspace of the generic dense stack; at most 4 GB of it
@@ -3242,6 +3404,8 @@ int b2e_create(const b2e_config *cfg, b2e_handle *out) {
                         std::to_string(ws_bytes * (size_t)ctas) + " bytes)");
     } else {
         if (cudaFuncSetAttribute(kernel_fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                 (int)h->smem_bytes) != cudaSuccess ||
+            cudaFuncSetAttribute(adam_fn, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                  (int)h->smem_bytes) != cudaSuccess)
             return bail("b2e_create: cudaFuncSetAttribute(smem) failed");
         int occ = 0;
@@ -3473,22 +3637,14 @@ int b2e_reset(b2e_handle h, const uint8_t *env_mask, const float *init_params,
     return launch(h, a, stream);
 }
 
-int b2e_step(b2e_handle h, const float *actions, const int32_t *batch_idx,
-             const int32_t *batch_cnt, float *obs_out, float *reward_out, uint8_t *done_out,
-             double *info_out, void *stream) {
-    if (!h) return 1;
-    DeviceGuard guard(h->cfg.device);
-    if (!actions || !reward_out || !done_out || !info_out)
-        return fail(h, "b2e_step: null pointer");
-    // obs_out = NULL: ring-only step, the observation rows are not materialised (b200policy.h reads the rings)
-    if (!obs_out && !(h->d.split && h->d.env_kind == B2E_ENV_MULTIOPTLRS && h->slot_abs))
-        return fail(h, "b2e_step: obs_out = NULL needs a MultiOptLRs env on the large-problem pipeline");
-    if (check_ready(h, batch_idx, batch_cnt)) return 1;
-    StepArgs a;
-    memset(&a, 0, sizeof(a));
-    a.mode = MODE_STEP; a.actions = actions; a.ext_idx = batch_idx; a.ext_cnt = batch_cnt;
-    a.obs = obs_out; a.reward = reward_out; a.done = done_out; a.info = info_out;
-    if (!h->d.split) return launch(h, a, stream);
+}  // extern "C"
+
+// b2e_step / b2e_step_adam once the arguments are checked: `a` holds the step's pointers, `adam` Adam's
+// arguments (null: the action update)
+static int step_launch(b2e_handle h, StepArgs &a, const AdamArgs *adam, void *stream) {
+    float *obs_out = a.obs;
+    uint8_t *done_out = a.done;
+    if (!h->d.split) return launch(h, a, stream, adam);
     cudaStream_t main_s = (cudaStream_t)stream;
     Dev &d = h->d;
     Dev &dv = h->d_eval;                                     // same pointers, eval-kernel smem layout
@@ -3520,7 +3676,8 @@ int b2e_step(b2e_handle h, const float *actions, const int32_t *batch_idx,
     mark(0);
     if (eval_pass<false>(h, a, main_s)) return 1;
     mark(1);
-    update_kernel<<<dim3(d.nsegU, d.E), 256, 0, main_s>>>(d, a);
+    if (adam) update_adam_kernel<<<dim3(d.nsegU, d.E), 256, 0, main_s>>>(d, a, *adam);
+    else update_kernel<<<dim3(d.nsegU, d.E), 256, 0, main_s>>>(d, a);
     mark(2);
     if (eval_pass<true>(h, a, main_s)) return 1;
     mark(3);
@@ -3551,6 +3708,49 @@ int b2e_step(b2e_handle h, const float *actions, const int32_t *batch_idx,
         return launch(h, r, main_s);
     }
     return 0;
+}
+
+extern "C" {
+
+int b2e_step(b2e_handle h, const float *actions, const int32_t *batch_idx,
+             const int32_t *batch_cnt, float *obs_out, float *reward_out, uint8_t *done_out,
+             double *info_out, void *stream) {
+    if (!h) return 1;
+    DeviceGuard guard(h->cfg.device);
+    if (!actions || !reward_out || !done_out || !info_out)
+        return fail(h, "b2e_step: null pointer");
+    // obs_out = NULL: ring-only step, the observation rows are not materialised (b200policy.h reads the rings)
+    if (!obs_out && !(h->d.split && h->d.env_kind == B2E_ENV_MULTIOPTLRS && h->slot_abs))
+        return fail(h, "b2e_step: obs_out = NULL needs a MultiOptLRs env on the large-problem pipeline");
+    if (check_ready(h, batch_idx, batch_cnt)) return 1;
+    StepArgs a;
+    memset(&a, 0, sizeof(a));
+    a.mode = MODE_STEP; a.actions = actions; a.ext_idx = batch_idx; a.ext_cnt = batch_cnt;
+    a.obs = obs_out; a.reward = reward_out; a.done = done_out; a.info = info_out;
+    return step_launch(h, a, nullptr, stream);
+}
+
+int b2e_step_adam(b2e_handle h, const b2e_adam *opt, const float *lr, float *m, float *v,
+                  const int32_t *batch_idx, const int32_t *batch_cnt, float *obs_out, float *reward_out,
+                  uint8_t *done_out, double *info_out, void *stream) {
+    if (!h) return 1;
+    DeviceGuard guard(h->cfg.device);
+    if (!opt || !lr || !m || !v || !reward_out || !done_out || !info_out)
+        return fail(h, "b2e_step_adam: null pointer");
+    if (h->d.env_kind != B2E_ENV_MULTIOPTLRS)
+        return fail(h, "b2e_step_adam: MultiOptLRs envs only (a MultiOptimize action is a weight delta and its "
+                       "minibatch never advances)");
+    if (!(opt->beta_1 >= 0.f && opt->beta_1 < 1.f && opt->beta_2 >= 0.f && opt->beta_2 < 1.f && opt->epsilon > 0.f))
+        return fail(h, "b2e_step_adam: need 0 <= beta_1, beta_2 < 1 and epsilon > 0");
+    if (!obs_out && !(h->d.split && h->slot_abs))
+        return fail(h, "b2e_step_adam: obs_out = NULL needs a MultiOptLRs env on the large-problem pipeline");
+    if (check_ready(h, batch_idx, batch_cnt)) return 1;
+    StepArgs a;
+    memset(&a, 0, sizeof(a));
+    a.mode = MODE_STEP; a.ext_idx = batch_idx; a.ext_cnt = batch_cnt;
+    a.obs = obs_out; a.reward = reward_out; a.done = done_out; a.info = info_out;
+    const AdamArgs adam = {lr, m, v, opt->beta_1, opt->beta_2, opt->epsilon};
+    return step_launch(h, a, &adam, stream);
 }
 
 int b2e_eval(b2e_handle h, const int32_t *batch_idx, const int32_t *batch_cnt, float *grad_out,

@@ -17,6 +17,7 @@
 #include <stdint.h>
 
 #include "b200env_shared.cuh"
+#include "b200adam.cuh"
 #include "b200tiny.h"
 
 namespace {
@@ -195,8 +196,12 @@ __device__ __noinline__ void reset_one(const Dev &d, const StepArgs &a, WarpSmem
     __syncwarp();
 }
 
-template <int HT, int DD, int CC>
-__global__ void __launch_bounds__(WARPS * 32) tiny_env_kernel(const __grid_constant__ Dev d, const __grid_constant__ StepArgs a) {
+// Adam: empty for b2e_step, one AdamArgs for b2e_step_adam (MODE_STEP only), whose update is Keras' Adam on the
+// gradient of the mean minibatch loss in place of the action's learning rate; m and v are loaded and stored per
+// lane = parameter.  The pack keeps the action step's instantiations (names and code) as they are.
+template <int HT, int DD, int CC, class... Adam>
+__global__ void __launch_bounds__(WARPS * 32) tiny_env_kernel(const __grid_constant__ Dev d, const __grid_constant__ StepArgs a,
+                                                               const Adam... adam) {
     __shared__ WarpSmem smem[WARPS];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int e = a.e_begin + blockIdx.x * WARPS + warp;
@@ -240,8 +245,21 @@ __global__ void __launch_bounds__(WARPS * 32) tiny_env_kernel(const __grid_const
                 row[j] = 0; aw[j] = 0.f;
                 if (p < P) {
                     row[j] = d.row_lex ? d.row_of_param[p] : p;
-                    const float lr = action_to_lr(a.actions[(size_t)e * P + row[j]], d.act_ver);
-                    const float wn = fmaf(-gt[j], lr, wv[j]);
+                    float lr, wn;
+                    if constexpr (sizeof...(Adam) > 0) {       // b2e_step_adam: t = step + 1, m = v = 0 before t = 1
+                        const AdamArgs &o = adam_of(adam...);
+                        const bool first = sc->step == 0;
+                        float *mp = o.m + (size_t)e * P + p, *vp = o.v + (size_t)e * P + p;
+                        float mv = first ? 0.f : *mp, vv = first ? 0.f : *vp;
+                        lr = adam_moments(o, adam_alpha(o, e, sc->step + 1), first,
+                                          adam_mean_grad(gt[j], (float)b.cnt), mv, vv);
+                        wn = fmaf(-lr, mv, wv[j]);
+                        *mp = mv;
+                        *vp = vv;
+                    } else {
+                        lr = action_to_lr(a.actions[(size_t)e * P + row[j]], d.act_ver);
+                        wn = fmaf(-gt[j], lr, wv[j]);
+                    }
                     aw[j] = ratio_nn(wn, wv[j]);
                     s_absw += fabsf(wn);
                     s_lr += (double)lr;
@@ -388,12 +406,17 @@ bool b2e_tiny_supported(const void *dev) {
            d.P <= tiny::PMAX && d.P * 3 * d.H <= tiny::OBS_MAX && d.H <= B2E_MAX_HISTORY && d.OD == 3 * d.H;
 }
 
-int b2e_tiny_launch(const void *dev, const void *args, void *stream) {
+int b2e_tiny_launch(const void *dev, const void *args, const void *adam, void *stream) {
     const Dev &d = *static_cast<const Dev *>(dev);
     const StepArgs &a = *static_cast<const StepArgs *>(args);
     const int grid = (a.e_count + tiny::WARPS - 1) / tiny::WARPS;
     const cudaStream_t cs = (cudaStream_t)stream;
-    if (d.H == 5 && d.D == 4 && d.C == 3) tiny::tiny_env_kernel<5, 4, 3><<<grid, tiny::WARPS * 32, 0, cs>>>(d, a);   // iris
+    if (adam) {                                                // b2e_step_adam
+        const AdamArgs &o = *static_cast<const AdamArgs *>(adam);
+        if (d.H == 5 && d.D == 4 && d.C == 3) tiny::tiny_env_kernel<5, 4, 3, AdamArgs><<<grid, tiny::WARPS * 32, 0, cs>>>(d, a, o);
+        else if (d.H == 5) tiny::tiny_env_kernel<5, 0, 0, AdamArgs><<<grid, tiny::WARPS * 32, 0, cs>>>(d, a, o);
+        else tiny::tiny_env_kernel<0, 0, 0, AdamArgs><<<grid, tiny::WARPS * 32, 0, cs>>>(d, a, o);
+    } else if (d.H == 5 && d.D == 4 && d.C == 3) tiny::tiny_env_kernel<5, 4, 3><<<grid, tiny::WARPS * 32, 0, cs>>>(d, a);   // iris
     else if (d.H == 5) tiny::tiny_env_kernel<5, 0, 0><<<grid, tiny::WARPS * 32, 0, cs>>>(d, a);
     else tiny::tiny_env_kernel<0, 0, 0><<<grid, tiny::WARPS * 32, 0, cs>>>(d, a);
     return cudaGetLastError() == cudaSuccess ? 0 : 1;

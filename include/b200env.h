@@ -136,6 +136,25 @@ int b2e_step(b2e_handle h, const float *actions, const int32_t *batch_idx,
              const int32_t *batch_cnt, float *obs_out, float *reward_out,
              uint8_t *done_out, double *info_out, void *stream);
 
+/* The Adam baseline: b2e_step of MultiOptLRs envs with the agent's learning rates replaced by Keras 2.2
+ * Adam.get_updates (amsgrad = False; search_baseline_hyperparam.py trains with it).  For env e at its step
+ * t (BaseEnvironment.current_step after the increment: t = 1 on the first step after any reset):
+ *   g   = g0 / cnt           g0 the batch-SUM gradient at w_{t-1}, cnt the minibatch's valid rows (1 for func)
+ *   m   = beta_1 m + (1 - beta_1) g,   v = beta_2 v + (1 - beta_2) g^2   (m = v = 0 before step 1, whatever
+ *                                                                         the buffers hold)
+ *   a_t = lr[e] sqrt(1 - beta_2^t) / (1 - beta_1^t)   (fp64, rounded to fp32)
+ *   w_t = w_{t-1} - a_t m / (sqrt(v) + epsilon)
+ * The rest is the ordinary step with the same outputs and the same obs_out = NULL rule; info's actions_mean
+ * / actions_std are taken over the per-parameter rate a_t / (sqrt(v) + epsilon).
+ *   opt       host pointer; Keras' defaults are {0.9, 0.999, 1e-7}
+ *   lr        float32 [E]
+ *   m, v      float32 [E, P], natural (flatten_arrays) order, owned by the caller, updated in place
+ * MultiOptimize handles are rejected. */
+typedef struct b2e_adam { float beta_1, beta_2, epsilon; } b2e_adam;
+int b2e_step_adam(b2e_handle h, const b2e_adam *opt, const float *lr, float *m, float *v,
+                  const int32_t *batch_idx, const int32_t *batch_cnt, float *obs_out,
+                  float *reward_out, uint8_t *done_out, double *info_out, void *stream);
+
 /* BaseProblem.get (problems/optimize_nn.py:152-159): gradient [E,P] and loss [E] of every
  * env's current parameters on its current minibatch.  Does not change env state. */
 int b2e_eval(b2e_handle h, const int32_t *batch_idx, const int32_t *batch_cnt,
